@@ -2,7 +2,7 @@
 """bench.py -- env-steps/s of the batched PCGRL step on B200 (the BASELINE.json metric).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--workload NAME] [--envs E]
-                    [--no-configs]
+                    [--no-configs] [--dump-outputs DIR]
 
 One "step" = one pass of the hot path (pcgrl_step: representation update -> get_stats -> reward) over the
 rank's whole env shard, with random actions, plus the auto-reset launches that episodes ending inside the
@@ -65,7 +65,9 @@ UNIT = "env-steps/s"
 def parse():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=800)
+    ap.add_argument("--steps", type=int, default=800,
+                    help="timed steps of the headline workload (its e2e arm times at most 200 of them; the secondary "
+                         "configs keep their own counts)")
     ap.add_argument("--warmup", type=int, default=10)
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--workload", default="binary-narrow-16x16", choices=sorted(WORKLOADS))
@@ -77,7 +79,13 @@ def parse():
     ap.add_argument("--int32-io", action="store_true", help="e2e through the int32 ABI (three dense result arrays) "
                     "instead of compact host I/O (uint8 actions, one packed record array)")
     ap.add_argument("--seed", type=int, default=0)
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step of the headline workload returned (rank 0's shard) to "
+                         "DIR/<name>.npy, for comparing two builds output for output")
+    a = ap.parse_args()
+    if a.dump_outputs and a.impl != "b200":
+        ap.error("--dump-outputs writes the GPU path's outputs: it needs --impl b200")
+    return a
 
 
 def peaks():
@@ -201,7 +209,28 @@ def cpu_arm(workload, seconds, cores, seed=0):
 
 
 # ------------------------------------------------------------------------------------------- GPU arms
-def run_workload(a, workload, n_envs, steps, warmup, e2e_steps, rank, world, local, clock_sampler=None):
+DUMP_ARRAY_BYTES = 12 << 20     # per array; five arrays stay under 64 MB
+
+
+def dump_outputs(env, out_dir):
+    """What a caller of BatchedPcgrlEnv.step holds after the last timed step (reward and done as returned, then the
+    stats, positions and maps, auto-reset applied) as float32 .npy files.  An array larger than DUMP_ARRAY_BYTES
+    keeps a fixed sample of env rows: the first k of np.random.default_rng(0).permutation(n_envs), in env order."""
+    import torch
+    arrays = {"reward": env.reward, "done": env.done, "stats": env.stats, "pos": env.pos[:, :env.ndim],
+              "maps": env.maps}
+    order = np.random.default_rng(0).permutation(env.n_envs)
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in arrays.items():
+        row_bytes = 4 * max(1, t[0].numel())
+        k = min(env.n_envs, DUMP_ARRAY_BYTES // row_bytes)
+        if k < env.n_envs:
+            t = t[torch.from_numpy(np.sort(order[:k])).to(t.device)]
+        np.save(os.path.join(out_dir, name + ".npy"), t.cpu().numpy().astype(np.float32))
+
+
+def run_workload(a, workload, n_envs, steps, warmup, e2e_steps, rank, world, local, clock_sampler=None,
+                 dump_dir=None):
     """value / e2e / roofline of one workload on this rank's GPU (max over ranks).  -> dict (same on every rank)"""
     import torch
     import torch.distributed as dist
@@ -291,13 +320,14 @@ def run_workload(a, workload, n_envs, steps, warmup, e2e_steps, rank, world, loc
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
     region_ms, kern_ms = float(t[0]), float(t[1])
     value = world * n_envs * steps / (region_ms * 1e-3)
+    if dump_dir is not None and rank == 0:
+        dump_outputs(env, dump_dir)
 
     # ---- end-to-end arm (host buffers through the public API) -----------------------------------
     e2e = None
     if not a.no_e2e:
         rng = np.random.default_rng(a.seed + 100 + rank)
-        # at least 50 host steps for the headline workload (20 steps are 8 ms: too short to average the host side)
-        k_e2e = max(3, min(steps, e2e_steps)) if e2e_steps < 200 else max(50, min(steps, e2e_steps))
+        k_e2e = min(steps, e2e_steps)      # never more timed steps than the device-resident arm was given
         HP = min(k_e2e + 3, max(8, int(2e9 // bytes_a)))
         if rep == "cellular":
             host_acts = [act_pool[i % POOL].cpu().pin_memory() for i in range(HP)]
@@ -425,7 +455,7 @@ def main():
     bound = bind_to_gpu_cpus(local) if world > 1 else []
 
     head = run_workload(a, a.workload, n_envs, a.steps, a.warmup, 200, rank, world, local,
-                        clock_sampler=ClockSampler(local) if rank == 0 else None)
+                        clock_sampler=ClockSampler(local) if rank == 0 else None, dump_dir=a.dump_outputs)
     configs = {}
     for wl, envs2, steps2, warm2, e2e2 in secondary:
         try:

@@ -38,6 +38,42 @@ def ref_problem(problem, map_shape):
     return p
 
 
+# (problem, map_shape) pairs of tests/golden/problem_tables.json
+PROBLEM_TABLE_CASES = [("binary", (16, 16)), ("binary", (10, 14)), ("zelda", (7, 11)), ("zelda", (16, 16)),
+                       ("sokoban", (5, 5)), ("sokoban", (6, 7)), ("smb", (116, 16)), ("minecraft_3D_maze", (14, 14, 14))]
+
+
+def problem_table_key(problem, map_shape):
+    return problem + "-" + "x".join(str(int(s)) for s in map_shape)
+
+
+def problem_table(tiles, static_trgs, cond_bounds, reward_weights, border_tile):
+    """What control_pcgrl_b200/problems.py restates of a Problem, in JSON form: the tile list, static targets and
+    condition bounds as floats (a range target as a pair), the keys of the reward weights and the border tile."""
+    def num(v):
+        return [float(x) for x in v] if isinstance(v, (tuple, list)) else float(v)
+    return {"tiles": [str(t) for t in tiles], "static_trgs": {k: num(v) for k, v in static_trgs.items()},
+            "cond_bounds": {k: num(v) for k, v in cond_bounds.items()},
+            "reward_weight_keys": sorted(reward_weights), "border_tile": str(border_tile)}
+
+
+def problem_tables_fixture():
+    """tests/golden/problem_tables.json: problem_table() of the reference's Problem classes for PROBLEM_TABLE_CASES.
+    The committed file was written from control_pcgrl_b200/problems.py, because no reference tree was at hand when
+    it was added; those tables had been compared with the real classes before, and the binary 16x16, zelda 7x11
+    and minecraft 15^3 values agree with SURVEY.md section A (items 13-15).  Running this job with a reference tree
+    rewrites it from the real classes."""
+    import json
+    out = {}
+    for problem, shape in PROBLEM_TABLE_CASES:
+        p = ref_problem(problem, shape)
+        out[problem_table_key(problem, shape)] = problem_table(p.get_tile_types(), p.static_trgs, p.cond_bounds,
+                                                               p._reward_weights, p._border_tile)
+    with open(os.path.join(OUT, "problem_tables.json"), "w") as f:
+        json.dump(out, f, indent=1, sort_keys=True)
+        f.write("\n")
+
+
 def ref_stats(problem_obj, problem, grid):
     H = R.load_helpers()
     helper = H.h3 if grid.ndim == 3 else H.h2
@@ -814,6 +850,7 @@ def main(which=None):
     jobs["stats_minecraft_2D_maze"] = minecraft_2d_maze_fixture
     jobs["stats_maze3d_holey"] = maze3d_holey_fixture
     jobs["stats_maze3d_holey_dungeon"] = maze3d_holey_dungeon_fixture
+    jobs["problem_tables"] = problem_tables_fixture
     for k, fn in jobs.items():
         if which and k not in which:
             continue

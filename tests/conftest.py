@@ -10,11 +10,13 @@ if ROOT not in sys.path:
 
 def pytest_configure(config):
     config.addinivalue_line("markers", "gpu: needs a CUDA device (run on the B200 box)")
-    config.addinivalue_line("markers", "needs_reference: needs /root/reference (build container only)")
+    config.addinivalue_line("markers", "needs_reference: needs a tree of the upstream control-pcgrl source "
+                                       "(found as oracle/refshim.py finds it)")
 
 
 def pytest_collection_modifyitems(config, items):
-    have_ref = os.path.isdir("/root/reference/control_pcgrl/envs")
+    from oracle import refshim
+    have_ref = refshim.available()
     try:
         import torch
         have_gpu = torch.cuda.is_available()
@@ -22,6 +24,6 @@ def pytest_collection_modifyitems(config, items):
         have_gpu = False
     for item in items:
         if "needs_reference" in item.keywords and not have_ref:
-            item.add_marker(pytest.mark.skip(reason="/root/reference not present"))
+            item.add_marker(pytest.mark.skip(reason="no control-pcgrl reference tree"))
         if "gpu" in item.keywords and not have_gpu:
             item.add_marker(pytest.mark.skip(reason="no CUDA device"))
