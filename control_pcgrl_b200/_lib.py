@@ -65,6 +65,7 @@ SYMBOLS = {
     "pcgrl_scratch_bytes": (C.c_int64, [C.POINTER(Config), C.c_int64]),
     "pcgrl_step_bytes": (C.c_int64, [C.POINTER(Config)]),
     "pcgrl_step": (C.c_int32, [C.POINTER(Config), C.POINTER(State), C.c_void_p, C.c_void_p]),
+    "pcgrl_update": (C.c_int32, [C.POINTER(Config), C.POINTER(State), C.c_void_p, C.c_void_p]),
     "pcgrl_reset": (C.c_int32, [C.POINTER(Config), C.POINTER(State), C.c_void_p, C.c_void_p, C.c_void_p,
                                 C.c_uint64, C.c_uint64, C.c_void_p]),
     "pcgrl_stats": (C.c_int32, [C.POINTER(Config), C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p]),

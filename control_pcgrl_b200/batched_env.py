@@ -206,6 +206,8 @@ class BatchedPcgrlEnv:
         self._pinned = {}
         self._epoch = 0
         self._synced_steps = None     # steps since the last full reset while all envs are in lock-step
+        # set by update(): stats (and the search cache) no longer describe the maps until the next full reset
+        self._stats_stale = False
         self.metric_trgs = OrderedDict(self.static_trgs)
         self._write_targets(self.metric_trgs)
 
@@ -399,6 +401,8 @@ class BatchedPcgrlEnv:
         if self.n_agents > 1:
             self._spawn_agents(agent_sp, m)
         self._synced_steps = 0 if mask is None else None
+        if mask is None:
+            self._stats_stale = False
         return self.stats
 
     def _spawn_agents(self, given, mask):
@@ -439,6 +443,7 @@ class BatchedPcgrlEnv:
         Returns (reward[N] f32, done[N] u8) device tensors (overwritten by the next step).
         agent: with n_agents > 1, whose turtle acts (MultiAgentWrapper.step, wrappers.py:724-731, steps the env once
         per agent)."""
+        self._check_fresh("step")
         a = self._check_actions(actions)
         with self._on_device():
             _lib.check(self.lib.pcgrl_step(self._cc, self._agent_state(agent), a.data_ptr(), self._stream()),
@@ -452,11 +457,33 @@ class BatchedPcgrlEnv:
 
     _in_agent_round = False
 
+    def update(self, actions: torch.Tensor, agent: int = 0) -> torch.Tensor:
+        """Representation.update for all N envs (envs/reps/*.py), the call evolution's generator loop makes at every
+        iteration (evo/evolve.py:1082-1085, _get_stats_on_step = False): edits the maps and advances pos / n_step,
+        nothing else -- no stats, reward, iteration / changes counters or done.  `actions` as for step() (same layout
+        and dtype, including compact_host_io's narrow types); agent: whose turtle acts with n_agents > 1.
+        Returns changed[N] u8 (the reference's `change`; overwritten by the next call).
+
+        Afterwards `stats` no longer describe the maps: step(), step_agents(), step_host() and observe() with control
+        planes raise until a full reset().  End-of-episode stats: compute_stats(env.maps, holes=env.holes)."""
+        a = self._check_actions(actions)
+        with self._on_device():
+            _lib.check(self.lib.pcgrl_update(self._cc, self._agent_state(agent), a.data_ptr(), self._stream()),
+                       "pcgrl_update")
+        self._stats_stale = True
+        return self.changed
+
+    def _check_fresh(self, what):
+        if self._stats_stale:
+            raise RuntimeError(f"{what}: update() edited the maps without recomputing stats, so stats (and the step's "
+                               "search cache) are stale; call reset() (all envs) before stepping again")
+
     def step_agents(self, actions: torch.Tensor):
         """One multi-agent step: actions[N, n_agents], agent a acts a-th (MultiAgentWrapper.step,
         wrappers.py:724-731: a full env step per agent, so iteration advances by n_agents).  Returns
         (reward[n_agents, N] f32, done[n_agents, N] u8); with auto_reset, envs restart once every agent of the round
         saw done (the wrapper's done['__all__'])."""
+        self._check_fresh("step_agents")
         A = max(self.n_agents, 1)
         if actions.dim() != 2 or tuple(actions.shape) != (self.n_envs, A):
             raise ValueError(f"actions must be [n_envs, n_agents] = {(self.n_envs, A)}")
@@ -560,6 +587,7 @@ class BatchedPcgrlEnv:
         next call.  By default these are three dense arrays (stats int32); with compact_host_io they are strided
         views of ONE packed record array (stats uint8 / int16 as the problem's bounds allow, see record_dtype()),
         downloaded with a single copy per pipeline chunk (pcgrl_step_host_packed)."""
+        self._check_fresh("step_host")
         h = self._host_io()
         a_ptr = h.known.get(id(actions))
         if a_ptr is None:
@@ -663,6 +691,8 @@ class BatchedPcgrlEnv:
         Cropped's own output (wrappers.py:407-437: 0 = out of bounds, tile t -> t + 1), one channel, for policies
         that embed the tile themselves (SURVEY 8f rank 3).
         agent: with n_agents > 1, whose crop (every agent sees the shared map around its own position)."""
+        if self.ctrl_metrics:
+            self._check_fresh("observe with control planes")
         if not onehot:
             if self.ctrl_metrics or (out is not None and out.dtype != torch.uint8):
                 raise ValueError("onehot=False is a uint8 observation without control planes")
@@ -752,11 +782,12 @@ class BatchedPcgrlEnv:
         sd["_epoch"] = int(self._epoch)
         sd["seed"] = int(self.seed)
         sd["_synced_steps"] = self._synced_steps
+        sd["_stats_stale"] = bool(self._stats_stale)
         return sd
 
     def load_state_dict(self, sd):
         want = {k for k in self._STATE_TENSORS if getattr(self, k) is not None}
-        have = {k for k in sd if k not in ("_epoch", "seed", "_synced_steps")}
+        have = {k for k in sd if k not in ("_epoch", "seed", "_synced_steps", "_stats_stale")}
         if want != have:
             raise KeyError(f"state_dict keys differ: missing {sorted(want - have)}, unexpected {sorted(have - want)}")
         for k in want:
@@ -768,3 +799,4 @@ class BatchedPcgrlEnv:
         self._epoch = int(sd.get("_epoch", self._epoch))
         self.seed = int(sd.get("seed", self.seed))
         self._synced_steps = sd.get("_synced_steps")     # lock-step episode clock (None: envs are out of step)
+        self._stats_stale = bool(sd.get("_stats_stale", False))    # checkpoints from before update() have no flag

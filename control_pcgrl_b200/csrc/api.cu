@@ -28,6 +28,7 @@ int64_t sokoban_scratch_bytes();
 int64_t smb_scratch_bytes(int64_t n_envs);
 int64_t maze3d_scratch_bytes();
 cudaError_t launch_observe(const pcgrl_config& cfg, const pcgrl_state& st, const pcgrl_obs_args& o, cudaStream_t s);
+cudaError_t launch_update(const KParams& p, cudaStream_t s);
 
 // split step path: up to WL_CHUNKS host-pipeline chunks, one 16-int work-list header each at the front of
 // pcgrl_state.worklist
@@ -426,6 +427,25 @@ static int32_t step_launch(const pcgrl_config* cfg, const pcgrl_state* st, const
 
 int32_t pcgrl_step(const pcgrl_config* cfg, const pcgrl_state* st, const void* actions, void* stream) {
     return step_launch(cfg, st, actions, stream, st ? st->worklist : nullptr, 0, 0);
+}
+
+int32_t pcgrl_update(const pcgrl_config* cfg, const pcgrl_state* st, const void* actions, void* stream) {
+    int r = check(cfg);
+    if (r) return r;
+    // only what the update touches: a holey problem's holes, the counters and the stats are not read
+    if (!st) return fail(PCGRL_E_ARG, "state is NULL");
+    if (st->n_envs < 0) return fail(PCGRL_E_ARG, "n_envs < 0");
+    if (!st->grids || !st->pos || !st->n_step || !st->changed)
+        return fail(PCGRL_E_ARG, "pcgrl_update needs grids, pos, n_step and changed");
+    if (!actions) return fail(PCGRL_E_ARG, "actions is NULL");
+    KParams p;
+    fill(p, cfg, st);
+    p.mode = MODE_STEP;
+    p.actions = actions;
+    const cudaError_t e = launch_update(p, (cudaStream_t)stream);
+    if (e != cudaSuccess) return cuda_fail(e, "update launch");
+    if (st->n_envs > 0) g_launches.fetch_add(1, std::memory_order_relaxed);
+    return 0;
 }
 
 int32_t pcgrl_reset(const pcgrl_config* cfg, const pcgrl_state* st, const uint8_t* mask, const int8_t* src_grids,

@@ -426,6 +426,73 @@ __device__ __forceinline__ void finish_env(const KParams& p, int64_t gid, const 
 }
 
 // ------------------------------------------------------------------------------------------------
+// Cellular representation update (reps/ca_rep.py:31-44) of the tile_n envs starting at `base`, cooperative over
+// the CTA: the whole map is replaced by the action.  s_flag[e] = 1 when env base + e's grid changed; the caller
+// zeroes s_flag[0 .. tile_n) before.  Shared by the step kernels (phase_a) and k_update.  Ends with a __syncthreads().
+// ------------------------------------------------------------------------------------------------
+template <int THREADS>
+__device__ __forceinline__ void cellular_rewrite(const KParams& p, int64_t base, int tile_n, uint8_t* s_flag) {
+    const int tid = threadIdx.x;
+    if (p.action_kind == PCGRL_ACT_CA_TILES) {
+        const int chunks = p.row_stride / 16;
+        for (int i = tid; i < tile_n * chunks; i += THREADS) {
+            const int e = i / chunks, c = i - e * chunks;
+            const int64_t off = (base + e) * p.row_stride + c * 16;
+            const uint4 nw = *(const uint4*)((const int8_t*)p.actions + off);
+            uint4* dst = (uint4*)(p.grids + off);
+            const uint4 od = *dst;
+            if (nw.x != od.x || nw.y != od.y || nw.z != od.z || nw.w != od.w) {
+                *dst = nw;
+                s_flag[e] = 1;
+            }
+        }
+    } else if (p.cells % 4 == 0 && ((uintptr_t)p.actions & 15) == 0) {
+        // PCGRL_ACT_CA_LOGITS, four cells per item: one 16-byte load per channel and one 4-byte grid word, so that a
+        // thread keeps C x 16 bytes in flight instead of C x 4 (the rewrite streams the logits once: HBM-bound)
+        const int q = p.cells / 4;
+        for (int i = tid; i < tile_n * q; i += THREADS) {
+            const int e = i / q, c = i - e * q;
+            const float4* lg = (const float4*)p.actions + (base + e) * (int64_t)p.n_tiles * q + c;
+            float4 best = __ldg(lg);
+            int b0 = 0, b1 = 0, b2 = 0, b3 = 0;
+            for (int t = 1; t < p.n_tiles; ++t) {   // strict > : ties keep the lowest channel
+                const float4 v = __ldg(lg + (int64_t)t * q);
+                if (v.x > best.x) best.x = v.x, b0 = t;
+                if (v.y > best.y) best.y = v.y, b1 = t;
+                if (v.z > best.z) best.z = v.z, b2 = t;
+                if (v.w > best.w) best.w = v.w, b3 = t;
+            }
+            const uint32_t nw = (uint32_t)b0 | ((uint32_t)b1 << 8) | ((uint32_t)b2 << 16) | ((uint32_t)b3 << 24);
+            uint32_t* g = (uint32_t*)(p.grids + (base + e) * p.row_stride) + c;
+            if (*g != nw) {
+                *g = nw;
+                s_flag[e] = 1;
+            }
+        }
+    } else {  // PCGRL_ACT_CA_LOGITS: float32 [N, C, cells]; argmax over C, ties -> lowest index
+        for (int i = tid; i < tile_n * p.cells; i += THREADS) {
+            const int e = i / p.cells, c = i - e * p.cells;
+            const float* lg = (const float*)p.actions + (base + e) * (int64_t)p.n_tiles * p.cells + c;
+            float best = lg[0];
+            int bi = 0;
+            for (int t = 1; t < p.n_tiles; ++t) {
+                const float v = lg[(int64_t)t * p.cells];
+                if (v > best) {
+                    best = v;
+                    bi = t;
+                }
+            }
+            int8_t* g = p.grids + (base + e) * p.row_stride + c;
+            if (*g != bi) {
+                *g = (int8_t)bi;
+                s_flag[e] = 1;
+            }
+        }
+    }
+    __syncthreads();
+}
+
+// ------------------------------------------------------------------------------------------------
 // phase A (whole CTA): apply the actions of the TILE envs starting at `base` (or reset them, or just list
 // them in MODE_STATS), advance the counters, decide done, and build the compact list of envs whose map
 // changed -- only those need get_stats (pcgrl_env.py:314).
@@ -437,43 +504,7 @@ __device__ __forceinline__ void phase_a(const KParams& p, int64_t base, int tile
                                         uint8_t* s_flag, int* s_count_ptr) {
     const int tid = threadIdx.x;
     int& s_count = *s_count_ptr;
-    // ---------------- cellular: whole-map rewrite, cooperative over the CTA -----------------------
-    if (p.mode == MODE_STEP && p.rep == PCGRL_REP_CELLULAR) {
-        if (p.action_kind == PCGRL_ACT_CA_TILES) {
-            const int chunks = p.row_stride / 16;
-            for (int i = tid; i < tile_n * chunks; i += THREADS) {
-                const int e = i / chunks, c = i - e * chunks;
-                const int64_t off = (base + e) * p.row_stride + c * 16;
-                const uint4 nw = *(const uint4*)((const int8_t*)p.actions + off);
-                uint4* dst = (uint4*)(p.grids + off);
-                const uint4 od = *dst;
-                if (nw.x != od.x || nw.y != od.y || nw.z != od.z || nw.w != od.w) {
-                    *dst = nw;
-                    s_flag[e] = 1;
-                }
-            }
-        } else {  // PCGRL_ACT_CA_LOGITS: float32 [N, C, cells]; argmax over C, ties -> lowest index
-            for (int i = tid; i < tile_n * p.cells; i += THREADS) {
-                const int e = i / p.cells, c = i - e * p.cells;
-                const float* lg = (const float*)p.actions + (base + e) * (int64_t)p.n_tiles * p.cells + c;
-                float best = lg[0];
-                int bi = 0;
-                for (int t = 1; t < p.n_tiles; ++t) {
-                    const float v = lg[(int64_t)t * p.cells];
-                    if (v > best) {
-                        best = v;
-                        bi = t;
-                    }
-                }
-                int8_t* g = p.grids + (base + e) * p.row_stride + c;
-                if (*g != bi) {
-                    *g = (int8_t)bi;
-                    s_flag[e] = 1;
-                }
-            }
-        }
-        __syncthreads();
-    }
+    if (p.mode == MODE_STEP && p.rep == PCGRL_REP_CELLULAR) cellular_rewrite<THREADS>(p, base, tile_n, s_flag);
 
     // ---------------- phase A: per-env action / reset, counters, change flag -----------------------
     for (int e = tid; e < TILE; e += THREADS) {

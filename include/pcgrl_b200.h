@@ -205,6 +205,15 @@ int32_t     pcgrl_cache_stride(const pcgrl_config* cfg);
 /* One env-step for every env of the shard.  `actions` layout depends on cfg->action_kind. */
 int32_t pcgrl_step(const pcgrl_config* cfg, const pcgrl_state* st, const void* actions, void* stream);
 
+/* Representation.update for every env (envs/reps/*.py update; what evo/evolve.py:1082-1085 calls): map edit,
+ * pos / n_step advance, changed[N] = the reference's `change`. No stats, reward, counters or done.
+ * Takes the same `actions` as pcgrl_step and sets status bit 0 for an invalid action as it does.  Writes only
+ * grids, pos, n_step, changed and status (reads static_mask when set); needs grids, pos, n_step and changed, and
+ * no holes for a holey problem.  One launch.  Afterwards `stats` no longer describe the maps (evolution calls
+ * pcgrl_stats / pcgrl_stats_holey at the end of the episode), and the search cache of a shard that has one
+ * (pcgrl_state.cache) no longer describes its grids: such a shard needs pcgrl_reset before its next pcgrl_step. */
+int32_t pcgrl_update(const pcgrl_config* cfg, const pcgrl_state* st, const void* actions, void* stream);
+
 /* (Re)start episodes: PcgrlEnv.reset (envs/pcgrl_env.py:158-188) + Representation.reset
  * (envs/reps/representation.py:65-76) + ControlWrapper.reset (control_wrappers.py:174-187).
  *   mask      [N] uint8 or NULL (= all envs): which envs to reset
