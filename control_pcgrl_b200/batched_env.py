@@ -749,8 +749,6 @@ class BatchedPcgrlEnv:
         (8, RuntimeError, "sokoban: a level with more than 15 crates met the solver preconditions; a packed solver "
                           "state holds 15, so its dist-win / sol-length were not computed"),
         (16, OverflowError, "a stat did not fit the packed result record (record_stat_bytes too small)"),
-        (32, RuntimeError, "step_host: a chunk's results waited more than two seconds for the search kernel "
-                           "(progressive host pipeline); the outputs of that step are invalid"),
     )
 
     def check_status(self):
@@ -760,7 +758,7 @@ class BatchedPcgrlEnv:
         if not s:
             return
         self.status.zero_()
-        for bit, exc, msg in sorted(self.STATUS_BITS, key=lambda b: b[0] not in (4, 8, 32)):
+        for bit, exc, msg in sorted(self.STATUS_BITS, key=lambda b: b[0] not in (4, 8)):
             if s & bit:
                 raise exc(f"{msg} [status word {s}]")
         raise RuntimeError(f"unknown device status word {s}")

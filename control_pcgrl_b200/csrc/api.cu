@@ -18,8 +18,6 @@ cudaError_t launch_bitboard_split(const KParams& p, int problem, cudaStream_t s,
                                   int& n_launches);
 cudaError_t launch_bitboard_lanegroup(const KParams& p, int problem, cudaStream_t s, bool& supported);
 int bitboard_cache_stride(int problem, int ndim, int d0, int d1, int rep, int action_kind);
-int split_prog_search_warps(int64_t n);
-bool split_prog_supported(const KParams& p, int problem);
 cudaError_t launch_maze3d(const KParams& p, cudaStream_t s, bool& supported);
 cudaError_t launch_maze3d_holey(const KParams& p, int problem, cudaStream_t s, bool& supported);
 cudaError_t launch_sokoban(const KParams& p, cudaStream_t s, bool& supported);
@@ -264,7 +262,6 @@ static int run(const KParams& p, int cfg_problem, void* stream, int force_path =
                 return 0;
             }
         }
-        if (p.split_phase != 0) return fail(PCGRL_E_UNSUPPORTED, "progressive host pipeline: config has no incremental split path");
         e = launch_bitboard(p, problem, (cudaStream_t)stream, supported);
         // maps beyond 32x32 (binary_bigger / zelda_bigger are 64x64): warp-per-grid boards
         if (!supported) e = launch_bigboard(p, problem, (cudaStream_t)stream, supported);
@@ -322,11 +319,6 @@ struct HostPipe {
 };
 static thread_local HostPipe g_pipe[16];
 
-// smallest shard the progressive host pipeline takes (read per call: the tests lower it)
-static int64_t prog_min_envs() {
-    const char* e = getenv("PCGRL_HOST_PROG_MIN");
-    return e ? atoll(e) : (int64_t)1 << 18;
-}
 static int host_chunks(const pcgrl_config* cfg, int64_t n, bool packed) {
     (void)packed;
     if (!is_bitboard(cfg) || cfg->dims[0] > 32 || cfg->dims[1] > 32) return 1;
@@ -402,8 +394,7 @@ int32_t pcgrl_record_stride(const pcgrl_config* cfg) {
 // pcgrl_state.worklist (host pipeline: st is a sub-range starting wl_off envs into the shard and `wl_base` is the
 // parent's buffer); a plain pcgrl_step is chunk 0 at offset 0 of its own buffer.
 static int32_t step_launch(const pcgrl_config* cfg, const pcgrl_state* st, const void* actions, void* stream,
-                           int32_t* wl_base, int wl_chunk, int64_t wl_off, int force_path = -1, int phase = 0,
-                           int ml_lists = 0, int64_t ml_per = 0, int ml_target = 0) {
+                           int32_t* wl_base, int wl_chunk, int64_t wl_off, int force_path = -1) {
     int r = check(cfg);
     if (r) return r;
     if ((r = check_state(st))) return r;
@@ -418,10 +409,6 @@ static int32_t step_launch(const pcgrl_config* cfg, const pcgrl_state* st, const
     p.mode = MODE_STEP;
     p.actions = actions;
     p.host_chunk = force_path >= 0;
-    p.split_phase = phase;
-    p.ml_lists = ml_lists;
-    p.ml_per = ml_per;
-    p.ml_target = ml_target;
     return run(p, cfg->problem, stream, force_path);
 }
 
@@ -528,7 +515,7 @@ static int32_t step_host_impl(const pcgrl_config* cfg, const pcgrl_state* st, co
         return fail(PCGRL_E_ARG, "packed host step needs cfg.record_stat_bytes and pcgrl_state.records");
     const int64_t n = st->n_envs;
     const int K = cfg->n_stats;
-    int chunks = (n > 0 && (!actions_host || action_bytes % n == 0)) ? host_chunks(cfg, n, records_host != nullptr) : 1;
+    const int chunks = (n > 0 && (!actions_host || action_bytes % n == 0)) ? host_chunks(cfg, n, records_host != nullptr) : 1;
     if (chunks <= 1) {
         if (actions_host &&
             (e = cudaMemcpyAsync(actions_dev, actions_host, (size_t)action_bytes, cudaMemcpyHostToDevice, s)) != cudaSuccess)
@@ -563,20 +550,6 @@ static int32_t step_host_impl(const pcgrl_config* cfg, const pcgrl_state* st, co
         hp.ready = true;
     }
     const int chunk_path = host_chunk_path(st->worklist && st->cache && cache_stride(cfg) > 0);
-    // Progressive pipeline (binary maps <= 16x16 with the incremental search, from 256 Ki envs): every chunk's update
-    // kernel, then ONE search over all the chunks' lists in chunk order (k_split_stats_inc_multi), and per chunk a
-    // wait kernel + output kernel + download that go as soon as the search has finished that chunk's list -- the
-    // search keeps the SIMT fill of the whole-shard launch and the downloads hide behind it.  PCGRL_HOST_PROG=0: the
-    // chunk-per-stream pipeline below (three launches per chunk on rotating streams).
-    const char* prog_env = getenv("PCGRL_HOST_PROG");
-    const bool prog_on = prog_env && atoi(prog_env) != 0;
-    bool prog = false;
-    if (prog_on && chunk_path == 2 && n >= prog_min_envs() && cfg->n_stats == 2) {
-        KParams probe;
-        fill(probe, cfg, st);
-        prog = split_prog_supported(probe, kernel_problem(cfg->problem));
-    }
-    if (prog && !getenv("PCGRL_HOST_CHUNKS")) chunks = n >= (1 << 19) ? 8 : 4;
     const int64_t per = ((n + chunks - 1) / chunks + 255) / 256 * 256;   // whole CTA tiles per chunk
     const int64_t a_env = actions_host ? action_bytes / n : 0;
 
@@ -599,8 +572,7 @@ static int32_t step_host_impl(const pcgrl_config* cfg, const pcgrl_state* st, co
     // Queue every chunk: its upload on the upload stream, its kernels on compute stream c % PIPE_COMPUTE, its download
     // on the download stream, chained by events.  (With the copies on the compute stream itself, chunk c + 3 could not
     // start before chunk c's DOWNLOAD had finished -- the device trace, PCGRL_HOST_TRACE, showed the fourth chunk's
-    // kernels starting 60 us after the first chunk's had ended.  PCGRL_HOST_SPLIT_COPIES=0 restores that order.)
-    static const bool split_copies = !(getenv("PCGRL_HOST_SPLIT_COPIES") && atoi(getenv("PCGRL_HOST_SPLIT_COPIES")) == 0);
+    // kernels starting 60 us after the first chunk's had ended.)
     auto enqueue_chunks = [&]() -> int {
         struct Chunk {
             int64_t off, m;
@@ -643,69 +615,20 @@ static int32_t step_host_impl(const pcgrl_config* cfg, const pcgrl_state* st, co
         }
         const int PIPE_COMPUTE = pipe_compute();
         cudaStream_t up = hp.s[PIPE_COMPUTE_MAX], down = hp.s[PIPE_COMPUTE_MAX + 1];
-        if (prog) {
-            cudaStream_t cs = hp.s[0], os = hp.s[1];
-            const int target = split_prog_search_warps(n);
-            if (target <= 0) return fail(PCGRL_E_CUDA, "progressive host pipeline: no SM count");
-            for (int c = 0; c < n_ck && actions_host; ++c) {
-                if ((e = cudaMemcpyAsync(ck[c].a_dev, (const char*)actions_host + ck[c].off * a_env, (size_t)(ck[c].m * a_env),
-                                         cudaMemcpyHostToDevice, up)) != cudaSuccess)
-                    return cuda_fail(e, "H2D actions");
-                if ((e = cudaEventRecord(hp.up_ev[c], up)) != cudaSuccess) return cuda_fail(e, "event record");
-                if (trace) cudaEventRecord(trace[3 * c + 0], up);
-            }
-            for (int c = 0; c < n_ck; ++c) {     // update kernels, chunk by chunk as the uploads land
-                if (actions_host && (e = cudaStreamWaitEvent(cs, hp.up_ev[c], 0)) != cudaSuccess) return cuda_fail(e, "stream wait");
-                if (!actions_host && trace) cudaEventRecord(trace[3 * c + 0], cs);
-                int rr = step_launch(cfg, &ck[c].sub, ck[c].a_dev, cs, st->worklist, c, ck[c].off, chunk_path, 1);
-                if (rr) return rr;
-            }
-            // ONE search over every chunk's list; queued BEFORE the wait kernels so that none of them can sit in front
-            // of it in a hardware queue
-            int rr = step_launch(cfg, st, actions_dev, cs, st->worklist, 0, 0, chunk_path, 2, n_ck, per);
-            if (rr) return rr;
-            for (int c = 0; c < n_ck; ++c) {     // per chunk: wait for its list, output kernel, download
-                const int64_t off = ck[c].off, m = ck[c].m;
-                const pcgrl_state& sub = ck[c].sub;
-                if ((rr = step_launch(cfg, &sub, ck[c].a_dev, os, st->worklist, c, off, chunk_path, 3, 0, 0, target))) return rr;
-                if (trace) cudaEventRecord(trace[3 * c + 1], os);
-                if ((e = cudaEventRecord(hp.k_ev[c], os)) != cudaSuccess) return cuda_fail(e, "event record");
-                if ((e = cudaStreamWaitEvent(down, hp.k_ev[c], 0)) != cudaSuccess) return cuda_fail(e, "stream wait");
-                if (records_host && (e = cudaMemcpyAsync(records_host + off * rs, sub.records, (size_t)(m * rs), cudaMemcpyDeviceToHost, down)) != cudaSuccess)
-                    return cuda_fail(e, "D2H records");
-                if (reward_host && (e = cudaMemcpyAsync(reward_host + off, sub.reward, m * sizeof(float), cudaMemcpyDeviceToHost, down)) != cudaSuccess)
-                    return cuda_fail(e, "D2H reward");
-                if (done_host && (e = cudaMemcpyAsync(done_host + off, sub.done, m, cudaMemcpyDeviceToHost, down)) != cudaSuccess)
-                    return cuda_fail(e, "D2H done");
-                if (stats_host && (e = cudaMemcpyAsync(stats_host + off * K, sub.stats, m * K * sizeof(int32_t), cudaMemcpyDeviceToHost, down)) != cudaSuccess)
-                    return cuda_fail(e, "D2H stats");
-                if (trace) cudaEventRecord(trace[3 * c + 2], down);
-            }
-            return 0;
-        }
         // every upload first: 1 B per env, on its own stream, long before the chunk's turn comes
         for (int c = 0; c < n_ck && actions_host; ++c) {
-            cudaStream_t us = split_copies ? up : hp.s[c % PIPE_COMPUTE];
-            if (!split_copies) continue;       // (old order: uploaded below, on the compute stream)
             if ((e = cudaMemcpyAsync(ck[c].a_dev, (const char*)actions_host + ck[c].off * a_env, (size_t)(ck[c].m * a_env),
-                                     cudaMemcpyHostToDevice, us)) != cudaSuccess)
+                                     cudaMemcpyHostToDevice, up)) != cudaSuccess)
                 return cuda_fail(e, "H2D actions");
-            if ((e = cudaEventRecord(hp.up_ev[c], us)) != cudaSuccess) return cuda_fail(e, "event record");
-            if (trace) cudaEventRecord(trace[3 * c + 0], us);
+            if ((e = cudaEventRecord(hp.up_ev[c], up)) != cudaSuccess) return cuda_fail(e, "event record");
+            if (trace) cudaEventRecord(trace[3 * c + 0], up);
         }
         for (int c = 0; c < n_ck; ++c) {
             const int64_t off = ck[c].off, m = ck[c].m;
             const pcgrl_state& sub = ck[c].sub;
             cudaStream_t cs = hp.s[c % PIPE_COMPUTE];
             if (actions_host) {
-                if (split_copies) {
-                    if ((e = cudaStreamWaitEvent(cs, hp.up_ev[c], 0)) != cudaSuccess) return cuda_fail(e, "stream wait");
-                } else {
-                    if ((e = cudaMemcpyAsync(ck[c].a_dev, (const char*)actions_host + off * a_env, (size_t)(m * a_env),
-                                             cudaMemcpyHostToDevice, cs)) != cudaSuccess)
-                        return cuda_fail(e, "H2D actions");
-                    if (trace) cudaEventRecord(trace[3 * c + 0], cs);
-                }
+                if ((e = cudaStreamWaitEvent(cs, hp.up_ev[c], 0)) != cudaSuccess) return cuda_fail(e, "stream wait");
             } else if (trace) {
                 cudaEventRecord(trace[3 * c + 0], cs);
             }
@@ -713,21 +636,17 @@ static int32_t step_host_impl(const pcgrl_config* cfg, const pcgrl_state* st, co
             int rr = step_launch(cfg, &sub, ck[c].a_dev, cs, st->worklist, c, off, chunk_path);
             if (rr) return rr;
             if (trace) cudaEventRecord(trace[3 * c + 1], cs);
-            cudaStream_t ds = cs;
-            if (split_copies) {
-                if ((e = cudaEventRecord(hp.k_ev[c], cs)) != cudaSuccess) return cuda_fail(e, "event record");
-                if ((e = cudaStreamWaitEvent(down, hp.k_ev[c], 0)) != cudaSuccess) return cuda_fail(e, "stream wait");
-                ds = down;
-            }
-            if (records_host && (e = cudaMemcpyAsync(records_host + off * rs, sub.records, (size_t)(m * rs), cudaMemcpyDeviceToHost, ds)) != cudaSuccess)
+            if ((e = cudaEventRecord(hp.k_ev[c], cs)) != cudaSuccess) return cuda_fail(e, "event record");
+            if ((e = cudaStreamWaitEvent(down, hp.k_ev[c], 0)) != cudaSuccess) return cuda_fail(e, "stream wait");
+            if (records_host && (e = cudaMemcpyAsync(records_host + off * rs, sub.records, (size_t)(m * rs), cudaMemcpyDeviceToHost, down)) != cudaSuccess)
                 return cuda_fail(e, "D2H records");
-            if (reward_host && (e = cudaMemcpyAsync(reward_host + off, sub.reward, m * sizeof(float), cudaMemcpyDeviceToHost, ds)) != cudaSuccess)
+            if (reward_host && (e = cudaMemcpyAsync(reward_host + off, sub.reward, m * sizeof(float), cudaMemcpyDeviceToHost, down)) != cudaSuccess)
                 return cuda_fail(e, "D2H reward");
-            if (done_host && (e = cudaMemcpyAsync(done_host + off, sub.done, m, cudaMemcpyDeviceToHost, ds)) != cudaSuccess)
+            if (done_host && (e = cudaMemcpyAsync(done_host + off, sub.done, m, cudaMemcpyDeviceToHost, down)) != cudaSuccess)
                 return cuda_fail(e, "D2H done");
-            if (stats_host && (e = cudaMemcpyAsync(stats_host + off * K, sub.stats, m * K * sizeof(int32_t), cudaMemcpyDeviceToHost, ds)) != cudaSuccess)
+            if (stats_host && (e = cudaMemcpyAsync(stats_host + off * K, sub.stats, m * K * sizeof(int32_t), cudaMemcpyDeviceToHost, down)) != cudaSuccess)
                 return cuda_fail(e, "D2H stats");
-            if (trace) cudaEventRecord(trace[3 * c + 2], ds);
+            if (trace) cudaEventRecord(trace[3 * c + 2], down);
         }
         return 0;
     };
@@ -740,9 +659,7 @@ static int32_t step_host_impl(const pcgrl_config* cfg, const pcgrl_state* st, co
     // with one cudaGraphLaunch; only the source addresses of the uploads change from step to step
     // (cudaGraphExecMemcpyNodeSetParams1D).  PCGRL_HOST_GRAPH=0 queues the operations directly, as before.
     static const bool use_graph = !(getenv("PCGRL_HOST_GRAPH") && atoi(getenv("PCGRL_HOST_GRAPH")) == 0);
-    // (the progressive pipeline is queued directly: only its first few operations -- uploads, update kernels, the search --
-    // sit on the critical path, the rest is queued while the search runs)
-    if (use_graph && !hp.graph_broken && !trace && !prog) {
+    if (use_graph && !hp.graph_broken && !trace) {
         HostGraphKey key;
         std::memset(&key, 0, sizeof(key));
         key.cfg = *cfg;

@@ -104,7 +104,6 @@ struct BinaryMachine {
     // the frontier died: next component / next phase; returns true when out[] holds the K stats
     __device__ __forceinline__ bool transition(int* out) {
         if (phase == 0) {
-#if PCGRL_OPT_BORROW
             uint32_t t[NW];
             B::minus_one(front, t);           // far tile of the component just swept (nothing on entry)
 #pragma unroll
@@ -118,22 +117,6 @@ struct BinaryMachine {
                 ++ncomp;
                 return false;
             }
-#else
-            uint32_t lo[NW];
-            B::lowest(front, lo);             // far tile of the component just swept (nothing on entry)
-#pragma unroll
-            for (int i = 0; i < NW; ++i) fars[i] |= lo[i];
-            B::lowest(avail, lo);             // first tile of the next component
-            if (B::any(lo)) {
-#pragma unroll
-                for (int i = 0; i < NW; ++i) {
-                    front[i] = lo[i];
-                    avail[i] ^= lo[i];
-                }
-                ++ncomp;
-                return false;
-            }
-#endif
             phase = 1;  // joint second sweep from every far tile
             uint32_t any = 0;
 #pragma unroll

@@ -9,18 +9,6 @@ constexpr int MAZE_QCAP = 256;    // FIFO ring capacity (entries); measured maxi
 #ifndef PCGRL_UF_RUNS32
 #define PCGRL_UF_RUNS32 1   // A/B on B200 (14^3): u16 per-cell parents / u32 run parents -> 2.12 / 2.26e7 env-steps/s
 #endif
-#ifndef PCGRL_MAZE_BATCH
-#define PCGRL_MAZE_BATCH 0   // 1: the player search pops up to 32 queue entries per round (search_batch), 0: one per round.
-                             // A/B on B200 (14^3, 65 536 envs, bench workload): 1.45e7 against 2.25e7 env-steps/s -- the
-                             // queue rarely holds more than 1-3 entries (a player's frontier in a 14^3 level is narrow:
-                             // 1.4 entries per round on 50 % AIR maps), and a round costs about four one-pop iterations.
-                             // Parity is green either way (fixtures, traces, CPU-restatement rollouts, holey problems).
-#endif
-#if PCGRL_MAZE_BATCH
-#define PCGRL_MAZE_SEARCH search_batch
-#else
-#define PCGRL_MAZE_SEARCH search
-#endif
 #ifndef PCGRL_MAZE_WARPS
 #define PCGRL_MAZE_WARPS 6   // A/B on B200 (14^3, 65 536 envs): 4 / 6 / 8 / 16 warps per CTA -> 1.81 / 2.13 / 2.05 / 1.41e7 env-steps/s
 #endif
@@ -142,6 +130,8 @@ struct Maze3DProb {
     // Leaves order[0..n) = cells in first-recording order, best[c] & 0x7FFF = len(paths[c]), nj[c] = jumps[c].
     // PARENTS: also leave par[c] = the cell the recorded path reaches c from (par[start] = start).  The start tile
     // needs head-room like every recorded tile (helper_3D.py:443-445), else nothing is recorded.
+    // One pop per round: the queue rarely holds more than 1-3 entries, and popping up to 32 per round measured
+    // 1.45e7 against 2.25e7 env-steps/s on B200 (14^3, 65 536 envs).
     template <bool PARENTS = false>
     __device__ static int search(Ctx& c, int start, int lane, bool& overflow) {
         const int XY = c.X * c.Y;
@@ -205,129 +195,6 @@ struct Maze3DProb {
         return n < c.order_cap ? n : c.order_cap;
     }
 
-    // ---- the same search, up to 32 queue entries per round ------------------------------------------------------------
-    // The reference pushes EVERY move and decides at pop time (`0 < len(old) <= len(path)`: skip).  Here a round takes
-    // the next B <= 32 entries; entry i is effective iff it is shorter than what is recorded for its cell and than
-    // every earlier entry of the round for the same cell (__match_any on the cell, then a loop over the few lanes that
-    // share one) -- exactly the sequential pop test.  The first effective entry of an unrecorded cell appends it to the
-    // recording order, the LAST effective entry of a cell leaves length / jumps / parent.  Then every effective lane
-    // evaluates its four moves and appends the candidates lane by lane, direction by direction (the sequential push
-    // order), dropping only those that are certain to be skipped when popped: the target already holds a recording
-    // that is not longer (recordings only get shorter; this round's are all in place before any of its candidates
-    // is popped).  No "best pushed" filter as in search(): it depends on the order of the pushes inside a round.
-    // On a queue overflow the cells are cleared and the search falls back to search().
-    template <bool PARENTS = false>
-    __device__ static int search_batch(Ctx& c, int start, int lane, bool& overflow) {
-        const int XY = c.X * c.Y;
-        unsigned head = 0, tail = 1;
-        int n = 0;
-        {
-            const int sz = div_by(start, c.magic_xy), srem = start - sz * XY;
-            if (sz + 1 >= c.Z || !((c.col[srem] >> (sz + 1)) & 1u)) return 0;
-        }
-        if (lane == 0) {
-            c.q_cl[0] = (uint32_t)start | (1u << 12);
-            c.q_nj[0] = 0;
-            if (PARENTS) c.q_par[0] = (uint16_t)start;
-        }
-        __syncwarp();
-        const unsigned lt = (1u << lane) - 1u;
-        bool spilled = false;
-        for (;;) {
-            const unsigned avail = tail - head;
-            if (!avail) break;
-            const int B = (int)min(32u, avail);
-            const bool mine = lane < B;
-            uint32_t cl = 0;
-            int nj_e = 0, par_e = 0;
-            if (mine) {
-                const unsigned slot = (head + lane) & (MAZE_QCAP - 1);
-                cl = c.q_cl[slot];
-                nj_e = c.q_nj[slot];
-                if (PARENTS) par_e = c.q_par[slot];
-            }
-            head += B;
-            const int cell = cl & 0xFFF, ln = cl >> 12;
-            const uint16_t rb = mine ? c.best[cell] : (uint16_t)0;
-            const unsigned mm = __ballot_sync(0xffffffffu, mine);
-            unsigned grp = 0;
-            if (mine) grp = __match_any_sync(mm, cell);
-            int minlow = 0x7FFFFFFF;
-            const unsigned dups = __ballot_sync(0xffffffffu, mine && (grp & (grp - 1u)) != 0u);
-            for (unsigned m = dups; m; m &= m - 1u) {       // rare: several entries of one cell in the same round
-                const int j = __ffs(m) - 1;
-                const int lj = __shfl_sync(0xffffffffu, ln, j), cj = __shfl_sync(0xffffffffu, cell, j);
-                if (mine && j < lane && cj == cell) minlow = min(minlow, lj);
-            }
-            const int rec_len = (rb & 0x8000u) ? (int)(rb & 0x7FFF) : 0x7FFFFFFF;
-            const bool eff = mine && ln < min(rec_len, minlow);                       // helper_3D.py:437-440
-            const bool first = eff && !(rb & 0x8000u) && (grp & lt) == 0u;
-            const unsigned fm = __ballot_sync(0xffffffffu, first);
-            const unsigned em = __ballot_sync(0xffffffffu, eff);
-            if (first) {
-                const int at = n + __popc(fm & lt);
-                if (at < c.order_cap) c.order[at] = (uint16_t)cell;
-            }
-            n += __popc(fm);
-            if (eff && (grp & em & ~lt & ~(1u << lane)) == 0u) {     // the last effective entry of this cell in the round
-                c.best[cell] = (uint16_t)(0x8000u | ln);
-                c.nj[cell] = (uint16_t)nj_e;
-                if (PARENTS) c.par[cell] = (uint16_t)par_e;
-            }
-            __syncwarp();
-            // moves of the effective entries (helper_3D.py:455-484), direction order of :220
-            uint32_t cand[4];
-            uint16_t cnj[4];
-            unsigned ok = 0;
-            if (eff) {
-                const int z = div_by(cell, c.magic_xy), rem = cell - z * XY, y = div_by(rem, c.magic_x), x = rem - y * c.X;
-#pragma unroll
-                for (int d = 0; d < 4; ++d) {
-                    const int dx = d == 0 ? 1 : (d == 2 ? -1 : 0), dy = d == 1 ? 1 : (d == 3 ? -1 : 0);
-                    int ncell = 0, cost = 0, jump = 0;
-                    if (move(c, x, y, z, dx, dy, ncell, cost, jump)) {
-                        const uint16_t r = c.best[ncell];
-                        if (!(r & 0x8000u) || (int)(r & 0x7FFF) > ln + cost) {
-                            ok |= 1u << d;
-                            cand[d] = (uint32_t)ncell | ((uint32_t)(ln + cost) << 12);
-                            cnj[d] = (uint16_t)(nj_e + jump);
-                        }
-                    }
-                }
-            }
-            const int cnt = __popc(ok);
-            int incl = cnt;
-#pragma unroll
-            for (int o = 1; o < 32; o <<= 1) {
-                const int v = __shfl_up_sync(0xffffffffu, incl, o);
-                if (lane >= o) incl += v;
-            }
-            const int total = __shfl_sync(0xffffffffu, incl, 31);
-            if (tail + total - head > (unsigned)MAZE_QCAP || n > c.order_cap) {
-                spilled = true;
-                break;
-            }
-            unsigned at = tail + incl - cnt;
-#pragma unroll
-            for (int d = 0; d < 4; ++d)
-                if (ok & (1u << d)) {
-                    const unsigned slot = at & (MAZE_QCAP - 1);
-                    c.q_cl[slot] = cand[d];
-                    c.q_nj[slot] = cnj[d];
-                    if (PARENTS) c.q_par[slot] = (uint16_t)cell;
-                    ++at;
-                }
-            tail += total;
-            __syncwarp();
-        }
-        __syncwarp();
-        if (spilled) {       // more candidates in flight than the ring holds: start over with the filtered, one-pop loop
-            clear_search(c, n < c.order_cap ? n : c.order_cap, lane);
-            return search<PARENTS>(c, start, lane, overflow);
-        }
-        return n;
-    }
-
     // first maximum of len(paths[.]) in insertion order (np.argmax, helper_3D.py:538-541)
     __device__ static __forceinline__ void far_tile(const Ctx& c, int n, int lane, int& cell, int& dist) {
         uint32_t key = 0;
@@ -385,7 +252,7 @@ struct Maze3DProb {
             const int x = __ffs(__shfl_sync(0xffffffffu, cand, y)) - 1;
             const int start = (z * Y + y) * X + x;
 
-            int n = PCGRL_MAZE_SEARCH(c, start, lane, overflow);                         // :529
+            int n = search(c, start, lane, overflow);                                    // :529
             uint32_t mark = 0;
             for (int i = lane; i < n; i += 32) {                                          // :531
                 const int cell = c.order[i];
@@ -399,7 +266,7 @@ struct Maze3DProb {
             int far, dist;
             far_tile(c, n, lane, far, dist);                                             // :538-541
             clear_search(c, n, lane);
-            n = PCGRL_MAZE_SEARCH(c, far, lane, overflow);                               // :548
+            n = search(c, far, lane, overflow);                                          // :548
             far_tile(c, n, lane, far, dist);                                             // :549-552
             last_far = far;                                                              // :553 last component wins
             if (dist > final_value) final_value = dist;                                  // :558

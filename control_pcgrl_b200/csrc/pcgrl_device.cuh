@@ -4,41 +4,6 @@
 #include <stdint.h>
 #include "../../include/pcgrl_b200.h"
 
-// tuning knobs (A/B-tested on B200, see profiles/)
-#ifndef PCGRL_OPT_SHR_IMAD
-#define PCGRL_OPT_SHR_IMAD 0   // 1: issue x>>1 as IMAD.HI on the FMA pipe instead of SHF on the ALU pipe
-#endif
-#ifndef PCGRL_OPT_WORKERS
-#define PCGRL_OPT_WORKERS 0    // 1: only ceil(M/rounds) threads take part in the stats phase
-#endif
-#ifndef PCGRL_OPT_IMAD_SUB
-#define PCGRL_OPT_IMAD_SUB 1   // 1: remove a subset from a board with x - n (IMAD, FMA pipe) instead of x ^ n (LOP3, ALU pipe)
-#endif
-#ifndef PCGRL_OPT_BORROW
-#define PCGRL_OPT_BORROW 1     // 1: lowest-cell extraction through x - 1 (minus_one) fused into its consumers
-#endif
-#ifndef PCGRL_OPT_FUNNEL_IMAD
-#define PCGRL_OPT_FUNNEL_IMAD 0   // 1: the 16-bit funnel shift between board words as IMAD.HI + IMAD (FMA pipe) instead of SHF (ALU pipe)
-#endif
-#if PCGRL_OPT_FUNNEL_IMAD
-// (lo >> 16) | (hi << 16): the two halves occupy disjoint bits, so the OR is an add -- mul.hi + mad.  The multiplier
-// comes from constant memory: a literal 65536 is strength-reduced back into a shift
-static __constant__ unsigned int c_pcgrl_k16 = 65536u;
-#define PCGRL_FUNNEL16(lo, hi) ((hi) * c_pcgrl_k16 + __umulhi((lo), c_pcgrl_k16))
-#else
-#define PCGRL_FUNNEL16(lo, hi) __funnelshift_l((lo), (hi), 16)
-#endif
-#if PCGRL_OPT_SHR_IMAD == 2
-// x >> 1 as a multiply-high by 2^31 that the compiler cannot turn back into a shift (with the literal it does: the
-// SASS of the search kernels showed SHF.R.U32.HI, ALU pipe)
-static __constant__ unsigned int c_pcgrl_k31 = 0x80000000u;
-#define PCGRL_SHR1(x) __umulhi((x), c_pcgrl_k31)
-#elif PCGRL_OPT_SHR_IMAD
-#define PCGRL_SHR1(x) __umulhi((x), 0x80000000u)
-#else
-#define PCGRL_SHR1(x) ((x) >> 1)
-#endif
-
 namespace pcgrl {
 
 enum { MODE_STEP = 0, MODE_RESET = 1, MODE_STATS = 2 };
@@ -92,12 +57,6 @@ struct KParams {
     uint8_t* cache;               // [N, cache_stride]
     int32_t cache_stride;
     int32_t host_chunk;           // 1: this launch is one chunk of the host pipeline (other chunks run beside it)
-    // progressive host pipeline (api.cu, step_split.cu): the three kernels of the split path launched separately
-    int32_t split_phase;          // 0: update + search + output; 1: update only; 2: ONE search over ml_lists chunk lists; 3: wait for
-                                  // this chunk's list to be searched (header word 5 == ml_target), then output
-    int32_t ml_lists;             // phase 2: number of chunk lists (headers 16 ints apart from wl_hdr)
-    int32_t ml_target;            // phase 3: search warps that must have reported the list
-    int64_t ml_per;               // phase 2: envs per chunk (the last chunk may hold fewer)
 };
 
 // one scalar action (narrow / turtle / flat wide) in the width the caller chose (cfg.action_elem_bytes)
@@ -224,11 +183,9 @@ struct Board {
     //
     // TWO layout: the "row above" word of board word i and the "row below" word of board word i-1 are the
     // same 32-bit window straddling words i-1 and i (high row of i-1, low row of i), so one funnel shift
-    // per word boundary serves both directions.  x<<1 is an add (IMAD.IADD, FMA pipe).  x>>1 is written as a
-    // multiply-high by 2^31, which nvcc 12.9 turns back into SHF.R; forcing real IMAD.HI for it and for the 16-bit
-    // funnel shifts (multipliers from constant memory, PCGRL_OPT_SHR_IMAD=2 / PCGRL_OPT_FUNNEL_IMAD=1) takes every
-    // shift off the ALU pipe but is SLOWER on B200: 0.2997 ms per step against 0.3064 (shr), 0.3092 (funnel),
-    // 0.3225 (both) at 1 Mi envs -- IMAD.HI is not a full-rate instruction.
+    // per word boundary serves both directions.  x<<1 is an add (IMAD.IADD, FMA pipe).  x>>1 and the 16-bit funnel
+    // shifts stay SHF on the ALU pipe: issuing them as IMAD.HI was SLOWER on B200, 0.2997 ms per step against 0.3064
+    // (shr), 0.3092 (funnel), 0.3225 (both) at 1 Mi envs -- IMAD.HI is not a full-rate instruction.
     __device__ static __forceinline__ uint32_t expand_and(const uint32_t (&f)[NW], const uint32_t (&av)[NW],
                                                           uint32_t (&n)[NW]) {
         uint32_t any = 0;
@@ -236,14 +193,14 @@ struct Board {
             uint32_t s[NW + 1];  // s[i] = rows (2i-1, 2i): window between word i-1 and word i
             s[0] = f[0] << 16;
 #pragma unroll
-            for (int i = 1; i < NW; ++i) s[i] = PCGRL_FUNNEL16(f[i - 1], f[i]);
+            for (int i = 1; i < NW; ++i) s[i] = __funnelshift_l(f[i - 1], f[i], 16);
             s[NW] = f[NW - 1] >> 16;
 #pragma unroll
             for (int i = 0; i < NW; ++i) {
                 // the two 16-bit rows of a word must not leak into each other.  Rows narrower than 16 have
                 // never-passable padding bits, for which the masks are no-ops, so they are always applied.
                 const uint32_t l = (f[i] + f[i]) & 0xFFFEFFFEu;
-                const uint32_t r = PCGRL_SHR1(f[i]) & 0x7FFF7FFFu;
+                const uint32_t r = (f[i] >> 1) & 0x7FFF7FFFu;
                 n[i] = (l | r | s[i] | s[i + 1]) & av[i];
                 any |= n[i];
             }
@@ -252,47 +209,15 @@ struct Board {
             for (int i = 0; i < NW; ++i) {
                 const uint32_t up = i > 0 ? f[i - 1] : 0u;
                 const uint32_t dn = i < NW - 1 ? f[i + 1] : 0u;
-                n[i] = ((f[i] + f[i]) | PCGRL_SHR1(f[i]) | up | dn) & av[i];
+                n[i] = ((f[i] + f[i]) | (f[i] >> 1) | up | dn) & av[i];
                 any |= n[i];
             }
         }
         return any;
     }
-    // One-hot board holding only the lowest set cell of x (all zero if x is empty): the multi-word
-    // two's-complement identity  X & -X, with the borrow rippling through the words as a carry chain
-    // (sub.cc / subc.cc), i.e. 2 ALU ops per word and no compares, selects or indices.
-    __device__ static __forceinline__ void lowest(const uint32_t (&x)[NW], uint32_t (&out)[NW]) {
-        uint32_t neg[NW];
-        if constexpr (NW == 1) {
-            neg[0] = 0u - x[0];
-        } else if constexpr (NW == 2) {
-            asm("sub.cc.u32 %0, 0, %2;\n\tsubc.u32 %1, 0, %3;" : "=r"(neg[0]), "=r"(neg[1]) : "r"(x[0]), "r"(x[1]));
-        } else if constexpr (NW == 4) {
-            asm("sub.cc.u32 %0, 0, %4;\n\tsubc.cc.u32 %1, 0, %5;\n\tsubc.cc.u32 %2, 0, %6;\n\tsubc.u32 %3, 0, %7;"
-                : "=r"(neg[0]), "=r"(neg[1]), "=r"(neg[2]), "=r"(neg[3])
-                : "r"(x[0]), "r"(x[1]), "r"(x[2]), "r"(x[3]));
-        } else if constexpr (NW == 8) {
-            asm("sub.cc.u32 %0, 0, %8;\n\tsubc.cc.u32 %1, 0, %9;\n\tsubc.cc.u32 %2, 0, %10;\n\t"
-                "subc.cc.u32 %3, 0, %11;\n\tsubc.cc.u32 %4, 0, %12;\n\tsubc.cc.u32 %5, 0, %13;\n\t"
-                "subc.cc.u32 %6, 0, %14;\n\tsubc.u32 %7, 0, %15;"
-                : "=r"(neg[0]), "=r"(neg[1]), "=r"(neg[2]), "=r"(neg[3]), "=r"(neg[4]), "=r"(neg[5]), "=r"(neg[6]),
-                  "=r"(neg[7])
-                : "r"(x[0]), "r"(x[1]), "r"(x[2]), "r"(x[3]), "r"(x[4]), "r"(x[5]), "r"(x[6]), "r"(x[7]));
-        } else {
-            // wide boards (maps up to 32x32): ripple the borrow by hand
-            uint32_t borrow = 0;
-#pragma unroll
-            for (int i = 0; i < NW; ++i) {
-                neg[i] = 0u - x[i] - borrow;
-                borrow = (x[i] | borrow) ? 1u : 0u;
-            }
-        }
-#pragma unroll
-        for (int i = 0; i < NW; ++i) out[i] = x[i] & neg[i];
-    }
     // t = x - 1 as one multi-word integer (borrow rippling up through sub.cc / subc.cc); returns true iff x != 0.
     // With it the lowest set cell of x is x & ~t and x without that cell is x & t -- one LOP3 per word each, which
-    // ptxas fuses with the consumer (fars |= x & ~t), instead of the negate / and / xor sequence of lowest().
+    // ptxas fuses with the consumer (fars |= x & ~t), instead of a negate / and / xor sequence (X & -X).
     __device__ static __forceinline__ bool minus_one(const uint32_t (&x)[NW], uint32_t (&t)[NW]) {
         uint32_t b;
         if constexpr (NW == 1) {
@@ -328,13 +253,9 @@ struct Board {
     }
     // x \ n for n a subset of x, as x - n: an IMAD on the FMA pipe instead of a LOP3 on the (saturated) ALU pipe
     __device__ static __forceinline__ uint32_t minus_subset(uint32_t x, uint32_t n) {
-#if PCGRL_OPT_IMAD_SUB
         uint32_t r;
         asm("mad.lo.u32 %0, %1, 0xFFFFFFFF, %2;" : "=r"(r) : "r"(n), "r"(x));
         return r;
-#else
-        return x ^ n;
-#endif
     }
     __device__ static __forceinline__ uint32_t any(const uint32_t (&x)[NW]) {
         uint32_t r = 0;

@@ -28,31 +28,8 @@ namespace pcgrl {
 #ifndef PCGRL_MIN_CTAS
 #define PCGRL_MIN_CTAS 10  // boards of <= 8 words: 48 registers, 10 CTAs (40 warps) per SM; A/B 1 / 10 -> 2.88 / 2.95e9
 #endif
-#ifndef PCGRL_CARVEOUT
-#define PCGRL_CARVEOUT 0
-#endif
-#ifndef PCGRL_SKIP_CLAIM
-#define PCGRL_SKIP_CLAIM 0
-#endif
-#ifndef PCGRL_STATIC_ITEMS
-#define PCGRL_STATIC_ITEMS 0
-#endif
 #ifndef PCGRL_EXPAND_R
 #define PCGRL_EXPAND_R 3
-#endif
-#ifndef PCGRL_THETA_F
-#define PCGRL_THETA_F 0     // expand while >= THETA_F/32 of a warp's active lanes are alive (0: fixed windows of PCGRL_EXPAND_R);
-                            // A/B 8 / 12 / 16 / 20: 0.60 / 0.53 / 0.47 / 0.45 ms per step against 0.385 with fixed windows
-#endif
-#ifndef PCGRL_CONVERGE
-#define PCGRL_CONVERGE 0    // 1: every lane of a warp starts every search trip together (vote at the loop head); A/B in the
-                            // fused kernel 0.393 against 0.385 ms without (it does pay in the split kernel: 0.381 / 0.432)
-#endif
-#ifndef PCGRL_WARP_BATCH
-#define PCGRL_WARP_BATCH 0  // 1: warps claim batches of 32 changed envs; 0: per-thread claims
-#endif
-#ifndef PCGRL_BATCH_K
-#define PCGRL_BATCH_K 0     // lanes of a warp that must be waiting for a transition before the warp takes it
 #endif
 #ifndef PCGRL_TILE8
 #define PCGRL_TILE8 256   // envs per CTA when a board is <= 8 words (binary 16x16); A/B: 2 envs per thread is best
@@ -156,131 +133,14 @@ __global__ void __launch_bounds__(THREADS, NW <= 8 ? PCGRL_MIN_CTAS : 1) k_step_
     // Each thread pulls the next changed env from the shared-memory queue as soon as it finishes one, so
     // lanes with short searches do not idle behind long ones; the search itself is a flat loop (one board
     // expansion per trip) so lanes in different phases of different grids execute the same instructions.
-    // Only as many threads as finish in whole rounds take part (R = ceil(M/THREADS) items each), so a warp's
-    // lanes run out of work together instead of a few lanes dragging a mostly idle warp through a last round.
+    // Fixed windows of PCGRL_EXPAND_R expansions: adaptive rounds (expand while a share of the warp's lanes is
+    // alive) measured 0.45-0.60 ms per step against 0.385, and a warp-wide vote that starts every trip together
+    // 0.393 against 0.385 (it pays in the split kernel, step_split.cu).
     {
         Machine m;
-#if PCGRL_WARP_BATCH
-        // Warp-synchronous batches: a warp claims 32 consecutive changed envs at a time and its lanes start their
-        // searches together, so at most ONE warp of the CTA runs a partly filled batch (with per-thread claims
-        // the few envs beyond THREADS were picked up by lanes scattered over every warp, each of which then ran
-        // a whole extra search at 1/32..7/32 lane occupancy).
-        for (;;) {
-            int b0 = 0;
-            if ((tid & 31) == 0) b0 = atomicAdd(&s_next, 32);
-            b0 = __shfl_sync(0xffffffffu, b0, 0);
-            if (b0 >= M) break;
-            const int item = b0 + (tid & 31);
-            if (item < M) {
-                m.init(s_bb + item * BBW, p, base + s_list[item]);
-                int out[K];
-                for (;;) {
-                    if (m.expand()) continue;
-                    if (m.transition(out)) break;
-                }
-#pragma unroll
-                for (int k = 0; k < K; ++k) s_stats[item * K + k] = out[k];
-            }
-            __syncwarp();
-        }
-#else
-#if PCGRL_STATIC_ITEMS
-        // static round-robin claims: the changed envs beyond THREADS all land in the lowest warp(s), so only those
-        // run a second, partly filled round (dynamic claims scatter them over lanes of every warp, and each such
-        // warp then runs a whole extra search at 1/32 lane occupancy)
-#define PCGRL_NEXT_ITEM(cur) ((cur) + THREADS)
-        int item = tid;
-#else
-#define PCGRL_NEXT_ITEM(cur) ((PCGRL_SKIP_CLAIM && M <= THREADS) ? M : atomicAdd(&s_next, 1))
         int item = atomicAdd(&s_next, 1);
-#endif
         bool active = item < M;
         if (active) m.init(s_bb + item * BBW, p, base + s_list[item]);
-#if PCGRL_BATCH_K > 0
-        // Expansions and transitions are different instruction streams; with 32 independent grids per warp some
-        // lane needs a transition on almost every trip, so an unbatched loop pays for both streams every trip
-        // with the transition stream running at 1/8 lane occupancy.  Lanes whose frontier died therefore WAIT
-        // (masked off during the expansions) until PCGRL_BATCH_K lanes of the warp are waiting, or nobody can
-        // expand; then all of them take their transition together.
-        bool pend = active;   // a fresh machine has an empty frontier: its first act is a transition
-        while (__any_sync(0xffffffffu, active)) {
-            if (active && !pend) pend = !m.expand();
-            const unsigned pb = __ballot_sync(0xffffffffu, pend);
-            const unsigned cb = __ballot_sync(0xffffffffu, active && !pend);
-            if (__popc(pb) >= PCGRL_BATCH_K || cb == 0) {
-                if (pend) {
-                    int out[K];
-                    while (m.transition(out)) {
-#pragma unroll
-                        for (int k = 0; k < K; ++k) s_stats[item * K + k] = out[k];
-                        item = atomicAdd(&s_next, 1);
-                        active = item < M;
-                        if (!active) break;
-                        m.init(s_bb + item * BBW, p, base + s_list[item]);
-                    }
-                    pend = false;
-                }
-            }
-        }
-#else
-#if PCGRL_THETA_F > 0
-        // Rounds: the warp keeps expanding while at least PCGRL_THETA_F/32 of its active lanes still have a live
-        // frontier (the others wait), then every waiting lane takes its transition (and claims its next grid) in
-        // ONE pass of the transition stream, so both streams run with many lanes.
-        bool alive = false;   // a fresh machine has an empty frontier: its first act is a transition
-        for (;;) {
-            const unsigned act = __ballot_sync(0xffffffffu, active);
-            if (!act) break;
-            const int need = max(1, (__popc(act) * PCGRL_THETA_F) >> 5);
-            for (;;) {
-                if (__popc(__ballot_sync(0xffffffffu, active && alive)) < need) break;
-                if (active && alive) alive = m.expand();
-            }
-            if (active && !alive) {
-                int out[K];
-                if (m.transition(out)) {
-#pragma unroll
-                    for (int k = 0; k < K; ++k) s_stats[item * K + k] = out[k];
-                    if constexpr (Machine::HAS_CACHE)
-                        if (p.cache && p.mode != MODE_STATS)
-                            m.store_cache((uint32_t*)(p.cache + (base + s_list[item]) * p.cache_stride));
-                    item = PCGRL_NEXT_ITEM(item);
-                    active = item < M;
-                    if (active) m.init(s_bb + item * BBW, p, base + s_list[item]);
-                } else {
-                    alive = true;
-                }
-            }
-        }
-#elif PCGRL_CONVERGE
-        // One trip = PCGRL_EXPAND_R board expansions, then the transition stream for the lanes whose frontier died.
-        // The warp-wide vote at the top makes every lane start every trip together (finished lanes stay in the
-        // loop until the whole warp is done): without it the lanes that loop back early run ahead of the ones in a
-        // transition and the warp falls apart into groups that issue both streams separately.
-        for (;;) {
-            if (!__any_sync(0xffffffffu, active)) break;
-            bool dead = false;
-            if (active) {
-                bool alive = m.expand();
-#pragma unroll
-                for (int r = 1; r < PCGRL_EXPAND_R; ++r)
-                    if (alive) alive = m.expand();
-                dead = !alive;
-            }
-            __syncwarp();
-            int out[K];
-            if (dead && m.transition(out)) {
-#pragma unroll
-                for (int k = 0; k < K; ++k) s_stats[item * K + k] = out[k];
-                if constexpr (Machine::HAS_CACHE)
-                    if (p.cache && p.mode != MODE_STATS)
-                        m.store_cache((uint32_t*)(p.cache + (base + s_list[item]) * p.cache_stride));
-                item = PCGRL_NEXT_ITEM(item);
-                active = item < M;
-                if (active) m.init(s_bb + item * BBW, p, base + s_list[item]);
-            }
-        }
-#else
         while (active) {
             int out[K];
             // PCGRL_EXPAND_R expansions per trip: the transition stream (a few lanes) is then paid once per R
@@ -297,14 +157,11 @@ __global__ void __launch_bounds__(THREADS, NW <= 8 ? PCGRL_MIN_CTAS : 1) k_step_
                 if constexpr (Machine::HAS_CACHE)
                     if (p.cache && p.mode != MODE_STATS)
                         m.store_cache((uint32_t*)(p.cache + (base + s_list[item]) * p.cache_stride));
-                item = PCGRL_NEXT_ITEM(item);
+                item = atomicAdd(&s_next, 1);
                 active = item < M;
                 if (active) m.init(s_bb + item * BBW, p, base + s_list[item]);
             }
         }
-#endif
-#endif
-#endif
     }
     __syncthreads();
 
@@ -320,13 +177,6 @@ static cudaError_t launch(const KParams& p, cudaStream_t s) {
     constexpr int TILE = tile_for(Machine::Prob::P * NW);
     const int64_t ctas = (p.n_envs + TILE - 1) / TILE;
     if (ctas == 0) return cudaSuccess;
-#if PCGRL_CARVEOUT > 0
-    static bool carved = false;   // ask for enough shared memory per SM that PCGRL_MIN_CTAS CTAs fit
-    if (!carved) {
-        cudaFuncSetAttribute(k_step_bitboard<Machine, NW, TWO>, cudaFuncAttributePreferredSharedMemoryCarveout, PCGRL_CARVEOUT);
-        carved = true;
-    }
-#endif
     k_step_bitboard<Machine, NW, TWO><<<(unsigned)ctas, THREADS, 0, s>>>(p);
     return cudaGetLastError();
 }

@@ -101,7 +101,7 @@ struct Holey3DProb {
             uint4* bz = (uint4*)c.best;
             for (int i = lane; i < c.best_bytes / 16; i += 32) bz[i] = make_uint4(0, 0, 0, 0);
             __syncwarp();
-            const int n = Maze3DProb::PCGRL_MAZE_SEARCH<true>(c, entrance, lane, overflow);                  // :81
+            const int n = Maze3DProb::search<true>(c, entrance, lane, overflow);                             // :81
             const uint16_t bx = c.best[exit_c];
             v2 = (bx & 0x8000u) ? (bx & 0x7FFF) : -1;                                            // :84 connected-path-length
             v3 = 0;
@@ -150,7 +150,7 @@ struct Holey3DProb {
             __syncwarp();
             int path = 0, nj = 0, nearest = 0;
             if (n_enemy > 0 || n_chest > 0) {
-                const int n = Maze3DProb::PCGRL_MAZE_SEARCH<false>(c, entrance, lane, overflow);            // :113 / :131
+                const int n = Maze3DProb::search<false>(c, entrance, lane, overflow);                       // :113 / :131
                 if (n_enemy > 0) {                                                               // :114-124
                     // enemy cells are found again in the grid in HBM (the stage was cleared for the search)
                     uint32_t best = 0xFFFFFFFFu;
@@ -179,7 +179,7 @@ struct Holey3DProb {
                 }
                 Maze3DProb::clear_search(c, n, lane);
                 if (chest >= 0) {                                                                // :137-141
-                    const int n2 = Maze3DProb::PCGRL_MAZE_SEARCH<false>(c, chest, lane, overflow);
+                    const int n2 = Maze3DProb::search<false>(c, chest, lane, overflow);
                     const uint16_t b = c.best[exit_c];
                     if (b & 0x8000u) {
                         path += b & 0x7FFF;

@@ -13,9 +13,6 @@
 
 namespace pcgrl {
 
-#ifndef PCGRL_UF_HALVING
-#define PCGRL_UF_HALVING 1
-#endif
 constexpr int SEARCH_WARPS = 8;   // default warps per CTA (a problem may ask for more)
 #ifndef PCGRL_SEARCH_TILE
 #define PCGRL_SEARCH_TILE 64
@@ -49,7 +46,6 @@ __device__ __forceinline__ int run_start(uint32_t a, int b) {
 __device__ inline void uf_union(volatile uint16_t* parent, int a, int b) {
     for (;;) {
         int pa, pb;
-#if PCGRL_UF_HALVING
         // find with path halving: every visited node is re-pointed at its grandparent.  Racing lanes only ever
         // replace a pointer by another ancestor of the same node, so the forest stays valid without locks.
         while ((pa = parent[a]) != a) {
@@ -62,10 +58,6 @@ __device__ inline void uf_union(volatile uint16_t* parent, int a, int b) {
             if (gb != pb) parent[b] = (uint16_t)gb;
             b = gb;
         }
-#else
-        while ((pa = parent[a]) != a) a = pa;
-        while ((pb = parent[b]) != b) b = pb;
-#endif
         if (a == b) return;
         if (a < b) {
             const int t = a;

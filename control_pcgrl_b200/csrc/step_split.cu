@@ -20,8 +20,7 @@
 //               from their warp's slice of the list instead of running in batches.
 //   k_split_out    thread-per-changed-env: fp64 loss(new) - loss(old), stats / reward / packed record; the list is
 //                  handed from step to step through ping-pong counters (see the header layout below).
-//   k_step_inc     all three in ONE launch for mid-size shards; k_split_stats_inc_multi / k_wait_list: the progressive
-//                  host pipeline (measured, off by default).  step_lanegroup.cu holds the small-shard kernel.
+//   k_step_inc     all three in ONE launch for mid-size shards.  step_lanegroup.cu holds the small-shard kernel.
 //
 // Reference path replaced: the same as step_bitboard.cu (envs/pcgrl_env.py:267-342, envs/reps/*_rep.py,
 // envs/probs/binary/binary_prob.py:152-158, envs/probs/zelda/zelda_ctrl_prob.py:90-168, envs/helper.py:200-276,
@@ -47,19 +46,10 @@ namespace pcgrl {
                                      // copies on the compute streams; with separate copy streams 3 / 4 / 5 / 8:
                                      // 2.56 / 2.75 / 2.71 / 2.42e9, profiles/r02_e2e_cps_chunks_split.txt)
 #endif
-#ifndef PCGRL_PROG_CTAS_PER_SM
-#define PCGRL_PROG_CTAS_PER_SM 6
-#endif
 #ifndef PCGRL_INC_MIN_CLAIM
 #define PCGRL_INC_MIN_CLAIM 12       // lanes that must be waiting before a warp hands out new items: the claim / init
                                      // stream then runs with that many lanes (A/B 1 / 4 / 8 at R=3: 0.412 / 0.390 / 0.387; at
                                      // R=12, 8 / 12 / 16 / 24: 0.2978 / 0.2996 / 0.3022 / 0.3263 ms, profiles/r02_ab_inc_claim_window.txt)
-#endif
-#ifndef PCGRL_INC_DYNAMIC
-#define PCGRL_INC_DYNAMIC 0          // > 0: items per fetch from the global list counter (see k_split_stats_inc); 0: static slices.
-                                     // A/B static / 16 / 32 / 64 (400 steps, 1 Mi envs, profiles/r02_ab_inc_dynamic.txt): 0.300-0.304 /
-                                     // 0.304 / 0.295 / 0.313 ms per step; as the default (32) the 800-step bench line did not move
-                                     // (0.2909 against 0.2913 ms) and e2e fell 2.60 -> 2.51e9: the tail is not where the time goes.  Off.
 #endif
 #ifndef PCGRL_INC_EXPAND_R
 #define PCGRL_INC_EXPAND_R 12        // board expansions per trip.  Every trip also issues each transition stream that
@@ -68,18 +58,6 @@ namespace pcgrl {
                                      // lanes idle inside the window: A/B 2 / 3 / 4 / 6 / 8 / 12 -> 0.466 / 0.412 / 0.356 /
                                      // 0.325 / 0.308 / 0.303 ms per step (1 Mi envs, 8 CTAs per SM); 16 / 20 -> 0.3018 / 0.3140
                                      // against 0.2996 for 12 in a later run
-#endif
-#ifndef PCGRL_CONVERGE
-#define PCGRL_CONVERGE 1             // 1: every lane of a warp starts every search trip together (vote at the loop head)
-#endif
-#ifndef PCGRL_THETA
-#define PCGRL_THETA 0                // static search: expand while >= THETA/32 of the running lanes are alive (0: fixed
-                                     // windows).  A/B 8 / 12 / 16 / 20 / 24: 0.59 / 0.50 / 0.45 / 0.43 / 0.42 ms per step
-                                     // against 0.38 with fixed windows of 3 -- waiting lanes cost more than the
-                                     // fuller transition stream saves
-#endif
-#ifndef PCGRL_INC_THETA
-#define PCGRL_INC_THETA 0            // the same for the incremental search (16: 0.334 ms against 0.303 with R=12)
 #endif
 #ifndef PCGRL_EXPAND_R_SPLIT
 #define PCGRL_EXPAND_R_SPLIT 3       // board expansions per trip of the static search (as in the fused kernel)
@@ -94,8 +72,7 @@ constexpr int OUT_THREADS = 256;
 // stats per item.  The headers of all pipeline chunks live together at the front of pcgrl_state.worklist, where no
 // body ever lands, so they stay zero whatever chunking the previous step used.
 // Header (all zero before the first step): [0], [1] item counters used alternately, [3] the step count, whose parity
-// picks the counter, [4] the step's final item count, [5] search warps that reported the list (progressive host
-// pipeline), [6], [7] fetch counters of the dynamic distribution, alternating like [0], [1].  k_split_act adds to counter [par]; the search kernel clears
+// picks the counter, [4] the step's final item count.  k_split_act adds to counter [par]; the search kernel clears
 // counter [par ^ 1] for the next step and publishes the count in [4]; k_split_out reads [4] and bumps [3] -- every
 // word is written by exactly one thread of a kernel none of whose CTAs reads it, so the three launches need no
 // "last CTA out" atomics or fences to hand the list over.
@@ -105,7 +82,6 @@ __device__ __forceinline__ int wl_count_search(const KParams& p) {
     const int count = *(volatile const int*)(p.wl_hdr + par);
     if (blockIdx.x == 0 && threadIdx.x == 0) {
         p.wl_hdr[par ^ 1] = 0;
-        p.wl_hdr[6 + (par ^ 1)] = 0;    // the next step's fetch counter (k_split_stats_inc, dynamic distribution)
         p.wl_hdr[4] = count;
     }
     return count;
@@ -207,39 +183,18 @@ k_split_stats(const KParams p) {
         }
     }
     __syncwarp();
-#if !PCGRL_CONVERGE
-    if (lane >= n_here) return;
-#endif
     const bool mine = lane < n_here;
     const int64_t env = mine ? items[lane].x : 0;
     Machine m;
     if (mine) m.init(wbb + lane * BBW, p, env);
     int out[K];
-#if PCGRL_CONVERGE
     // One trip = PCGRL_EXPAND_R_SPLIT board expansions, then the transition stream for the lanes whose frontier
     // died.  The warp-wide vote at the top makes every lane start every trip together: without it the lanes that
-    // `continue` run ahead of the ones in a transition, the warp falls apart into groups that never re-merge, and
-    // both streams are issued once per group (ncu: transitions at 3.7 lanes, expansions at 19).
+    // loop back early run ahead of the ones in a transition, the warp falls apart into groups that never re-merge, and
+    // both streams are issued once per group (ncu: transitions at 3.7 lanes, expansions at 19; 0.432 against 0.381 ms
+    // per step).  Fixed windows: adaptive rounds (expand while a share of the running lanes is alive) measured
+    // 0.42-0.59 ms against 0.38 -- waiting lanes cost more than the fuller transition stream saves.
     bool running = mine;
-#if PCGRL_THETA > 0
-    // Rounds instead of fixed windows: the warp keeps expanding while at least PCGRL_THETA/32 of its running lanes
-    // still have a live frontier (the others wait), then every waiting lane takes its transition in ONE pass of
-    // the transition stream -- both instruction streams run with many lanes instead of one of them with a few.
-    bool alive = false;   // a fresh machine has an empty frontier: its first act is a transition
-    for (;;) {
-        const unsigned run = __ballot_sync(0xffffffffu, running);
-        if (!run) break;
-        const int need = max(1, (__popc(run) * PCGRL_THETA) >> 5);
-        for (;;) {
-            if (__popc(__ballot_sync(0xffffffffu, running && alive)) < need) break;
-            if (running && alive) alive = m.expand();
-        }
-        if (running && !alive) {
-            if (m.transition(out)) running = false;
-            else alive = true;
-        }
-    }
-#else
     for (;;) {
         if (!__any_sync(0xffffffffu, running)) break;
         bool dead = false;
@@ -253,18 +208,7 @@ k_split_stats(const KParams p) {
         __syncwarp();
         if (dead && m.transition(out)) running = false;
     }
-#endif
     if (!mine) return;
-#else
-    for (;;) {
-        bool alive = m.expand();
-#pragma unroll
-        for (int r = 1; r < PCGRL_EXPAND_R_SPLIT; ++r)
-            if (alive) alive = m.expand();
-        if (alive) continue;
-        if (m.transition(out)) break;
-    }
-#endif
     int32_t* o = wl_stats(p) + (int64_t)(first + lane) * K;
 #pragma unroll
     for (int k = 0; k < K; ++k) o[k] = out[k];
@@ -465,7 +409,10 @@ struct BinaryIncMachine {
 
 // ------------------------------------------------------------------------------------------------
 // k_split_stats, incremental variant: persistent-size grid, every warp owns a contiguous slice of the work list
-// and its lanes claim items from it one by one (ballot-ranked at a convergent point, no atomics).
+// and its lanes claim items from it one by one (ballot-ranked at a convergent point, no atomics).  Static slices:
+// fetching items from a global counter instead did not move the bench line (0.2909 against 0.2913 ms per step) and
+// cut e2e from 2.60 to 2.51e9 (profiles/r02_ab_inc_dynamic.txt).  Fixed windows of PCGRL_INC_EXPAND_R expansions:
+// adaptive rounds measured 0.334 ms against 0.303.
 // ------------------------------------------------------------------------------------------------
 template <int NW, bool TWO>
 __global__ void __launch_bounds__(STAT_THREADS) k_split_stats_inc(const KParams p) {
@@ -473,51 +420,22 @@ __global__ void __launch_bounds__(STAT_THREADS) k_split_stats_inc(const KParams 
     __shared__ uint32_t s_work[STAT_THREADS * M::SMEM_WORDS];
     const int tid = threadIdx.x, lane = tid & 31;
     const int count = wl_count_search(p);
-#if PCGRL_INC_DYNAMIC > 0
-    // Dynamic distribution: a warp fetches the next PCGRL_INC_DYNAMIC items of the list from a global counter (header
-    // words 6 / 7, alternating with the step parity like the item counters; block 0 clears the one the NEXT step uses)
-    // whenever its lanes need items.  With static slices of ~110 items whose cost varies 0..135 expansions each, the
-    // slowest of the 4 736 warps carries ~25 % more work than the average one and the kernel ends with a thin tail.
-    int* ctr = p.wl_hdr + 6 + wl_parity(p);     // (wl_count_search cleared it one step ago, whichever split kernel ran)
-    int lo = 0, hi = 0;
-    bool drained = count == 0, last_batch = false;
-#else
     const int n_warps = gridDim.x * (STAT_THREADS / 32);
     const int gw = blockIdx.x * (STAT_THREADS / 32) + (tid >> 5);
     const int per = (count + n_warps - 1) / n_warps;
     int lo = min(count, gw * per);
     const int hi = min(count, lo + per);
     if (lo >= hi) return;
-#endif
     const int2* items = wl_items(p);
     int32_t* stats_out = wl_stats(p);
     const int W = p.d1;
     M m;
-    bool active = false, alive = false;
+    bool active = false;
     int item = 0;
     int64_t env = 0;
     for (;;) {
-        unsigned need = __ballot_sync(0xffffffffu, !active);
-#if PCGRL_INC_DYNAMIC > 0
-        // up to two rounds per trip: lanes left over when a batch runs out take theirs from the next one at once
-        for (int round = 0; round < 2 && need; ++round) {
-            if (!(round || __popc(need) >= PCGRL_INC_MIN_CLAIM || need == 0xffffffffu || (last_batch && lo < hi))) break;
-            if (lo >= hi) {
-                if (drained) break;
-                int b = 0;
-                if (lane == 0) b = atomicAdd(ctr, PCGRL_INC_DYNAMIC);
-                b = __shfl_sync(0xffffffffu, b, 0);
-                lo = min(count, b);
-                hi = min(count, b + PCGRL_INC_DYNAMIC);
-                last_batch = b + PCGRL_INC_DYNAMIC >= count;      // the counter is past the end: nothing after this batch
-                if (lo >= hi) {
-                    drained = true;
-                    break;
-                }
-            }
-#else
+        const unsigned need = __ballot_sync(0xffffffffu, !active);
         if (need && lo < hi && (__popc(need) >= PCGRL_INC_MIN_CLAIM || need == 0xffffffffu || hi - lo < PCGRL_INC_MIN_CLAIM)) {
-#endif
             const int mine = lo + __popc(need & ((1u << lane) - 1u));
             if (!active && mine < hi) {
                 item = mine;
@@ -528,40 +446,11 @@ __global__ void __launch_bounds__(STAT_THREADS) k_split_stats_inc(const KParams 
                 const int32_t* st = p.stats + env * 2;
                 m.init(s_work + tid * M::SMEM_WORDS, (const uint32_t*)(p.cache + env * p.cache_stride), bitpos, st[0], st[1]);
                 active = true;
-                alive = true;
             }
             lo = min(hi, lo + __popc(need));
-#if PCGRL_INC_DYNAMIC > 0
-            if (lo < hi) break;                                    // the batch served every idle lane
-            need = __ballot_sync(0xffffffffu, !active);
-#endif
         }
         const unsigned act = __ballot_sync(0xffffffffu, active);
-#if PCGRL_INC_DYNAMIC > 0
-        if (!act) {
-            if (drained) break;
-            continue;          // every lane is idle: the next trip fetches a batch
-        }
-#else
         if (!act) break;
-#endif
-#if PCGRL_INC_THETA > 0
-        const int want = max(1, (__popc(act) * PCGRL_INC_THETA) >> 5);
-        for (;;) {
-            if (__popc(__ballot_sync(0xffffffffu, active && alive)) < want) break;
-            if (active && alive) alive = m.expand();
-        }
-        if (active && !alive) {
-            if (m.transition()) {
-                int out[2];
-                m.finish(out, (uint32_t*)(p.cache + env * p.cache_stride));
-                *(int2*)(stats_out + (int64_t)item * 2) = make_int2(out[0], out[1]);
-                active = false;
-            } else {
-                alive = true;
-            }
-        }
-#else
         if (active) {
             bool alive = m.expand();
 #pragma unroll
@@ -574,126 +463,7 @@ __global__ void __launch_bounds__(STAT_THREADS) k_split_stats_inc(const KParams 
                 active = false;
             }
         }
-#endif
     }
-}
-
-// ------------------------------------------------------------------------------------------------
-// k_split_stats_inc_multi: ONE incremental search over the work lists of every chunk of the host pipeline.
-//
-// The chunked pipeline used to run one search launch per chunk on rotating streams; every launch has a tail in which
-// its lanes run dry, and concurrent launches share the SMs so that the first chunk's result was ready only after 2/3
-// of the whole step (profiles/r02_host_trace.txt: kernels done at 190 / 270 / 274 / 361 us).  Here every warp walks
-// the lists in chunk order -- its slice of list 0, then of list 1, ... -- and its lanes keep claiming across the list
-// boundaries, so the SIMT fill is that of the whole-shard search while chunk c is finished after about (c + 1) / n of
-// the kernel.  A warp reports a list (atomicAdd on header word 5, after a fence) once it has claimed its whole
-// slice of it and none of its lanes still works on one of its items; when all warps have reported, the chunk's
-// k_wait_list lets the output kernel and the download go (k_wait_list runs on another stream while this kernel is
-// still busy with the later lists).
-// ------------------------------------------------------------------------------------------------
-template <int NW, bool TWO>
-__global__ void __launch_bounds__(STAT_THREADS, NW >= 8 ? PCGRL_PROG_CTAS_PER_SM : 1) k_split_stats_inc_multi(const KParams p) {
-    using M = BinaryIncMachine<NW, TWO>;
-    __shared__ uint32_t s_work[STAT_THREADS * M::SMEM_WORDS];
-    const int tid = threadIdx.x, lane = tid & 31;
-    const unsigned lt = (1u << lane) - 1u;
-    const int n_lists = p.ml_lists;
-    const int n_warps = gridDim.x * (STAT_THREADS / 32);
-    const int gw = blockIdx.x * (STAT_THREADS / 32) + (tid >> 5);
-    if (blockIdx.x == 0 && tid < n_lists) {   // publish every list's count, clear the other counter (as wl_count_search)
-        int32_t* hdr = p.wl_hdr + 16 * tid;
-        const int par = *(volatile const int*)(hdr + 3) & 1;
-        hdr[4] = *(volatile const int*)(hdr + par);
-        hdr[par ^ 1] = 0;
-        hdr[6 + (par ^ 1)] = 0;
-    }
-    const int W = p.d1;
-    int cl = -1, lo = 0, hi = 0, sig = 0;                  // warp-uniform: list being claimed from, slice, next list to report
-    M m;
-    bool active = false;
-    int my_list = 0, my_item = 0;                          // per lane; pointers are rebuilt from them (registers)
-    for (;;) {
-        unsigned need = __ballot_sync(0xffffffffu, !active);
-        if (need && (__popc(need) >= PCGRL_INC_MIN_CLAIM || need == 0xffffffffu || (cl == n_lists - 1 && hi - lo < PCGRL_INC_MIN_CLAIM))) {
-            for (;;) {
-                while (lo >= hi && cl + 1 < n_lists) {     // next list: this warp's slice of it
-                    ++cl;
-                    const int32_t* hdr = p.wl_hdr + 16 * cl;
-                    const int par = *(volatile const int*)(hdr + 3) & 1;
-                    const int count = *(volatile const int*)(hdr + par);
-                    const int per_w = (count + n_warps - 1) / n_warps;
-                    lo = min(count, gw * per_w);
-                    hi = min(count, lo + per_w);
-                }
-                if (lo >= hi) break;                       // every list is claimed
-                const int mine = lo + __popc(need & lt);
-                if (!active && mine < hi) {
-                    const int64_t first = (int64_t)cl * p.ml_per;
-                    const int2 it = ((const int2*)(p.worklist + 4 * first))[mine];
-                    const int y = it.y / W, x = it.y - y * W;
-                    const int bitpos = TWO ? y * 16 + x : y * 32 + x;
-                    const int32_t* st = p.stats + 2 * (first + it.x);
-                    m.init(s_work + tid * M::SMEM_WORDS, (const uint32_t*)(p.cache + (first + it.x) * p.cache_stride), bitpos, st[0], st[1]);
-                    my_item = mine;
-                    my_list = cl;
-                    active = true;
-                }
-                lo = min(hi, lo + __popc(need));
-                need = __ballot_sync(0xffffffffu, !active);
-                if (!need || lo < hi) break;               // lanes left over at the end of a slice go on to the next list
-            }
-        }
-        const unsigned act = __ballot_sync(0xffffffffu, active);
-        // lists below the oldest one that is still in flight or not claimed to the end are finished for this warp
-        const int oldest = __reduce_min_sync(0xffffffffu, active ? my_list : (lo < hi ? cl : cl + 1));
-        while (sig < oldest) {
-            __threadfence();                               // every lane's stats / cache rows of that list
-            __syncwarp();
-            if (lane == 0) {
-                __threadfence();
-                atomicAdd(p.wl_hdr + 16 * sig + 5, 1);
-            }
-            ++sig;
-        }
-        if (!act) {
-            if (lo >= hi && cl + 1 >= n_lists) break;
-            continue;
-        }
-        if (active) {
-            bool alive = m.expand();
-#pragma unroll
-            for (int r = 1; r < PCGRL_INC_EXPAND_R; ++r)
-                if (alive) alive = m.expand();
-            if (!alive && m.transition()) {
-                int out[2];
-                m.finish(out, const_cast<uint32_t*>(m.cache));
-                const int64_t first = (int64_t)my_list * p.ml_per;
-                const int64_t cap = min(p.ml_per, p.n_envs - first);
-                *(int2*)(p.worklist + 4 * first + 2 * cap + 2 * (int64_t)my_item) = make_int2(out[0], out[1]);
-                active = false;
-            }
-        }
-    }
-}
-
-// One thread waits until every search warp has reported the chunk's list, then re-arms the counter for the next
-// step.  Launched AFTER the search kernel (so it can never sit in front of it in a hardware queue) on the stream
-// that carries the chunk's output kernel and download.  A wait of more than two seconds sets status bit 5.
-__global__ void k_wait_list(int32_t* hdr, int target, int32_t* status) {
-    if (threadIdx.x != 0) return;
-    volatile int* f = hdr + 5;
-    unsigned long long t0, t1;
-    asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t0));
-    while (*f < target) {
-        __nanosleep(400);
-        asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t1));
-        if (t1 - t0 > 2000000000ull) {
-            if (status) atomicOr(status, 32);
-            break;
-        }
-    }
-    __threadfence();
-    *f = 0;
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -857,30 +627,6 @@ static cudaError_t sm_count(int& n) {
     return cudaSuccess;
 }
 
-// CTAs of the progressive pipeline's search: one short of filling the SMs' register files (8 CTAs of 64 registers x
-// 128 threads), so that the chunks' wait / output kernels become resident beside it.  PCGRL_PROG_CPS overrides (A/B).
-static int64_t prog_search_ctas(int64_t n, int n_sm) {
-    static int env_v = -1;
-    if (env_v < 0) {
-        const char* e = getenv("PCGRL_PROG_CPS");
-        env_v = e ? atoi(e) : 0;
-    }
-    const int64_t want = (n + STAT_THREADS - 1) / STAT_THREADS;
-    const int64_t cap = (int64_t)n_sm * (env_v > 0 ? env_v : PCGRL_PROG_CTAS_PER_SM);
-    return want < cap ? want : cap;
-}
-// search warps of that launch (= reports every chunk's k_wait_list waits for); < 0 on error
-int split_prog_search_warps(int64_t n) {
-    int n_sm = 0;
-    if (sm_count(n_sm) != cudaSuccess) return -1;
-    return (int)prog_search_ctas(n, n_sm) * (STAT_THREADS / 32);
-}
-// can this config run the progressive host pipeline (binary, one-cell edits, maps <= 16x16, cache + work list)?
-bool split_prog_supported(const KParams& p, int problem) {
-    return problem == PCGRL_PROB_BINARY && p.ndim == 2 && p.d0 <= 16 && p.d1 <= 16 && p.cache && p.worklist &&
-           p.rep != PCGRL_REP_CELLULAR && p.action_kind != PCGRL_ACT_PATCH;
-}
-
 template <class Machine, int NW, bool TWO>
 static cudaError_t launch_split(const KParams& p, cudaStream_t s, int incremental) {
     constexpr int K = Machine::Prob::K;
@@ -911,23 +657,8 @@ static cudaError_t launch_split(const KParams& p, cudaStream_t s, int incrementa
             return cudaGetLastError();
         }
     }
-    if constexpr (Machine::HAS_CACHE && TWO) {
-        if (p.split_phase == 2) {   // progressive host pipeline: one search over every chunk's list
-            int n_sm = 0;
-            if ((e = sm_count(n_sm)) != cudaSuccess) return e;
-            k_split_stats_inc_multi<NW, TWO><<<(unsigned)prog_search_ctas(n, n_sm), STAT_THREADS, 0, s>>>(p);
-            return cudaGetLastError();
-        }
-    }
-    if (p.split_phase == 3) {       // ... and per chunk: wait for its list, then the output kernel
-        k_wait_list<<<1, 32, 0, s>>>(p.wl_hdr, p.ml_target, p.status);
-        if ((e = cudaGetLastError()) != cudaSuccess) return e;
-        k_split_out<K><<<(unsigned)((n + OUT_THREADS - 1) / OUT_THREADS), OUT_THREADS, 0, s>>>(p);
-        return cudaGetLastError();
-    }
     k_split_act<<<(unsigned)((n + ACT_THREADS - 1) / ACT_THREADS), ACT_THREADS, 0, s>>>(p);
     if ((e = cudaGetLastError()) != cudaSuccess) return e;
-    if (p.split_phase == 1) return cudaSuccess;
     bool ran_inc = false;
     if constexpr (Machine::HAS_CACHE && TWO) {
         if (incremental == 1) {
@@ -975,9 +706,8 @@ static cudaError_t dispatch_split(const KParams& p, cudaStream_t s, int incremen
 cudaError_t launch_bitboard_split(const KParams& p, int problem, cudaStream_t s, int incremental, bool& supported,
                                   int& n_launches) {
     supported = false;
-    n_launches = p.split_phase == 0 ? 3 : p.split_phase == 3 ? 2 : 1;
+    n_launches = 3;
     if (p.mode != MODE_STEP || !p.worklist || p.rep == PCGRL_REP_CELLULAR) return cudaSuccess;
-    if (p.split_phase != 0 && (!split_prog_supported(p, problem) || incremental != 1)) return cudaSuccess;
     if (problem == PCGRL_PROB_BINARY) {
         const int inc = p.cache != nullptr && p.d0 <= 16 && p.d1 <= 16 ? incremental : 0;
         if (inc == 2) n_launches = 1;

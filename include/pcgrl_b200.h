@@ -143,9 +143,7 @@ typedef struct pcgrl_state {
                               bit1 (2) minecraft_3D_maze: the reference would raise IndexError on this map
                               (helper_3D.py:531, a recorded x or y >= depth); bit2 (4) a search workspace
                               overflowed; bit3 (8) sokoban: more crates than a packed solver state holds (15);
-                              bit4 (16) a stat did not fit cfg.record_stat_bytes in the packed record;
-                              bit5 (32) pcgrl_step_host: a chunk's results waited more than two seconds for the
-                              search kernel (progressive host pipeline) -- the outputs of that step are invalid */
+                              bit4 (16) a stat did not fit cfg.record_stat_bytes in the packed record */
     void*    scratch;      /* pcgrl_scratch_bytes() bytes, may be NULL when that returns 0.  Must be zero-filled
                               once before its first use (it holds hash-table generation counters, solver job
                               lists and, for smb, 4 bytes per env of playthrough-length history, which is why

@@ -3,7 +3,7 @@
 # against the one-launch / three-launch thread-per-grid paths.
 set -u
 mkdir -p gpurun_out
-timeout 900 python -m pytest tests/test_gpu_split.py -m gpu -x -q -k progressive 2>&1 | tail -8
+timeout 900 python -m pytest tests/test_gpu_split.py -m gpu -x -q -k chunked_host_pipeline 2>&1 | tail -8
 sweep() {
   n=$1; path=$2; shift 2
   env PCGRL_STEP_PATH=$path "$@" timeout 200 python bench.py --envs $n --steps 300 --warmup 10 --no-e2e --no-cpu-baseline --no-configs > gpurun_out/lg_tmp.json 2> gpurun_out/lg_tmp.err

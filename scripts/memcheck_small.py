@@ -40,16 +40,10 @@ def roll(problem, rep, shape, n, steps, path=None, **kw):
     print("ok", problem, rep, shape, path or "", flush=True)
 
 
-# the kernels added last (lane groups; the progressive host pipeline's multi-list search and wait kernel).
-# MEMCHECK_ONLY=new stops after them.
+# the kernels added last (lane groups).  MEMCHECK_ONLY=new stops after them.
 for shape, rep in (((16, 16), "narrow"), ((7, 5), "turtle"), ((3, 4), "narrow"), ((2, 16), "narrow")):
     roll("binary", rep, shape, 3000, 40, "lg")
 roll("binary", "narrow", (16, 16), 50000, 12, "lg")            # 16 envs per warp
-os.environ["PCGRL_HOST_PROG"], os.environ["PCGRL_HOST_PROG_MIN"], os.environ["PCGRL_HOST_CHUNKS"] = "1", "1024", "5"
-roll("binary", "narrow", (16, 16), 70000, 6, compact=True)
-roll("binary", "turtle", (7, 5), 20000, 6, compact=True)
-for k in ("PCGRL_HOST_PROG", "PCGRL_HOST_PROG_MIN", "PCGRL_HOST_CHUNKS"):
-    os.environ.pop(k)
 if os.environ.get("MEMCHECK_ONLY") == "new":
     sys.exit(0)
 for path in ("fused", "split", "inc", "incfused"):

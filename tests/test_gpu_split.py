@@ -186,12 +186,11 @@ def test_incremental_hand_built_maps():
                                                         ("turtle", (7, 5), None, True),
                                                         ("narrow", (3, 4), None, False),
                                                         ("narrow", (2, 16), None, True)])
-def test_progressive_host_pipeline_equals_device_step(rep, shape, controls, compact, monkeypatch):
-    """pcgrl_step_host's progressive pipeline (per-chunk update kernels, ONE search over every chunk's work list in
-    chunk order, per-chunk wait + output + download) must give exactly what a whole-shard pcgrl_step gives, for every
-    chunk count (ragged last chunk, chunks smaller than a warp's slice, more chunks than the search has lists to
-    fill), across auto-resets, and interleaved with the chunk-per-stream pipeline and plain device steps on the same
-    work-list headers."""
+def test_chunked_host_pipeline_equals_device_step(rep, shape, controls, compact, monkeypatch):
+    """pcgrl_step_host's chunked pipeline (per chunk: upload, the three kernels of the incremental split path on one
+    of the rotating compute streams, download) must give exactly what a whole-shard pcgrl_step gives, for every chunk
+    count (ragged last chunk, chunks smaller than a warp's slice, up to the 64 work-list headers), across
+    auto-resets, and interleaved with plain device steps on the same work-list headers."""
     import control_pcgrl_b200 as P
     n = 70_001
     kw = dict(obs_window=shape) if rep == "wide" else {}
@@ -207,24 +206,21 @@ def test_progressive_host_pipeline_equals_device_step(rep, shape, controls, comp
     b.reset()
     n_act = _n_act(a, rep, shape)
     rng = np.random.default_rng(0)
-    monkeypatch.setenv("PCGRL_HOST_PROG_MIN", "1024")
     launches = a.lib.pcgrl_launch_count
-    for t, (chunks, prog) in enumerate([("2", 1), ("8", 1), ("5", 1), ("64", 1), ("3", 0), ("", 1), ("7", 1), ("1", 1),
-                                        ("4", 0), ("16", 1)] * 3):
+    for t, chunks in enumerate(["2", "8", "5", "64", "3", "", "7", "1", "4", "16"] * 3):
         if chunks:
             monkeypatch.setenv("PCGRL_HOST_CHUNKS", chunks)
         else:
             monkeypatch.delenv("PCGRL_HOST_CHUNKS", raising=False)
-        monkeypatch.setenv("PCGRL_HOST_PROG", str(prog))
         act = rng.integers(0, n_act, size=n).astype(a.action_shape_dtype()[1])
         l0 = launches()
         r, d, s = a.step_host(act)
         launched = launches() - l0
-        if prog and chunks not in ("1", ""):      # (the default is one chunk below 128 Ki envs: plain upload / step / download)
+        if chunks not in ("1", ""):      # (the default is one chunk below 128 Ki envs: plain upload / step / download)
             n_ck = int(chunks)
             n_ck = -(-n // ((-(-n // n_ck) + 255) // 256 * 256))      # ragged: chunks of whole 256-env tiles
-            # n_ck update kernels + 1 search + n_ck (wait + output) [+ the auto-reset launch]
-            assert launched in (3 * n_ck + 1, 3 * n_ck + 2), (chunks, launched)
+            # 3 kernels per chunk [+ the auto-reset launch]
+            assert launched in (3 * n_ck, 3 * n_ck + 1), (chunks, launched)
         if t % 4 == 3:     # a plain device step in between (header 0 is shared by all paths)
             act2 = rng.integers(0, n_act, size=n).astype(np.int32)
             a.step(torch.from_numpy(act2.astype(a.action_shape_dtype()[1])).to(a.device))
@@ -243,10 +239,10 @@ def test_progressive_host_pipeline_equals_device_step(rep, shape, controls, comp
 
 
 def test_one_shard_may_alternate_between_all_step_paths(monkeypatch):
-    """The split paths hand their work list from step to step through alternating header words (item counters, the
-    dynamic search's fetch counters); a shard that switches path from step to step -- three-launch incremental,
-    three-launch from scratch, one-launch, lane groups, fused -- must keep giving the fused kernel's results, and the
-    incremental cache must survive the steps that do not use it."""
+    """The split paths hand their work list from step to step through alternating header words (the item counters);
+    a shard that switches path from step to step -- three-launch incremental, three-launch from scratch, one-launch,
+    lane groups, fused -- must keep giving the fused kernel's results, and the incremental cache must survive the
+    steps that do not use it."""
     n = 40_000
     a, b = _envs("binary", "narrow", (16, 16), n, ["inc", "fused"], max_board_scans=0.05)
     a.reset()
