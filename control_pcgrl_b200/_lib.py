@@ -20,7 +20,7 @@ ACT_INT32, ACT_WIDE_COORDS, ACT_WIDE_FLAT, ACT_CA_TILES, ACT_CA_LOGITS, ACT_PATC
 REWARD_CONTROL, REWARD_RANGE = 0, 1
 
 LIB_NAME = "libpcgrl_sm100.so"
-# PCGRL_B200_LIB lets kernel experiments load an alternative build of the same ABI (scripts/ab_variants.sh)
+# PCGRL_B200_LIB loads another build of the same ABI instead of the in-tree one (e.g. to time two builds side by side)
 LIB_PATH = os.environ.get("PCGRL_B200_LIB") or os.path.join(os.path.dirname(os.path.abspath(__file__)), LIB_NAME)
 
 

@@ -138,10 +138,11 @@ static int step_path(int64_t n_envs, int problem, bool has_cache) {
     return path_of(getenv("PCGRL_STEP_PATH"), dflt);
 }
 // Chunks of the host pipeline run on different streams.  With the search kernel of the three-launch incremental
-// path limited to 3 CTAs per SM (PCGRL_INC_CTAS_PER_SM_HOST) the memory-bound update / output kernels of the
+// path limited to 3 CTAs per SM (INC_CTAS_PER_SM_HOST, step_split.cu) the memory-bound update / output kernels of the
 // neighbouring chunks run NEXT TO it: e2e 2.60e9 env-steps/s at 4 chunks, against 2.24e9 with the fused kernel and
-// 2.11e9 when the search holds every SM for itself (8 CTAs per SM); shards without a search cache keep the fused kernel
-static int host_chunk_path(bool has_cache) { return has_cache ? path_of(getenv("PCGRL_HOST_PATH"), 2) : 0; }
+// 2.11e9 when the search holds every SM for itself (8 CTAs per SM).  The one-launch incremental kernel lost too: e2e
+// 2.74e9 against at most 2.38e9 (profiles/r02_e2e_hostpath.txt).  Shards without a search cache keep the fused kernel.
+static int host_chunk_path(bool has_cache) { return has_cache ? 2 : 0; }
 static int action_elem(const pcgrl_config* c) { return c->action_elem_bytes ? c->action_elem_bytes : 4; }
 static int record_stride(const pcgrl_config* c) {
     return c->record_stat_bytes ? (4 + c->n_stats * c->record_stat_bytes + 2 + 3) / 4 * 4 : 0;
@@ -279,12 +280,10 @@ static int run(const KParams& p, int cfg_problem, void* stream, int force_path =
 // download stream (events in between), so uploads, kernels and downloads of different chunks overlap (two copy
 // engines + the SMs) and a chunk never waits for another chunk's download.
 // Only for kernels that keep no cross-launch device state (scratch == 0, i.e. not the persistent solvers).
-constexpr int PIPE_COMPUTE_MAX = 6;             // streams the chunks' kernels rotate over: n_compute of them (PCGRL_HOST_STREAMS)
-constexpr int PIPE_STREAMS = PIPE_COMPUTE_MAX + 2;  // + one upload stream and one download stream (the last two)
-static int pipe_compute() {
-    static const int v = getenv("PCGRL_HOST_STREAMS") ? std::min(std::max(atoi(getenv("PCGRL_HOST_STREAMS")), 1), PIPE_COMPUTE_MAX) : 3;
-    return v;
-}
+// Streams the chunks' kernels rotate over: 3 beat 4 and 6 (e2e at 4 / 6 chunks: 2.73 / 2.76e9 with 3 streams, 2.48 /
+// 2.72e9 with 4, 2.37 / 2.43e9 with 6, profiles/r02_e2e_streams.txt)
+constexpr int PIPE_COMPUTE = 3;
+constexpr int PIPE_STREAMS = PIPE_COMPUTE + 2;  // + one upload stream and one download stream (the last two)
 struct HostGraphKey {            // everything the queued operations depend on (compared bytewise)
     pcgrl_config cfg;
     pcgrl_state st;
@@ -292,7 +291,7 @@ struct HostGraphKey {            // everything the queued operations depend on (
     int64_t action_bytes;
     int64_t has_host_actions;
     void *reward_host, *done_host, *stats_host, *records_host;
-    int32_t chunks, chunk_path;
+    int32_t chunks;
 };
 struct HostGraph {
     struct Upload {
@@ -613,8 +612,7 @@ static int32_t step_host_impl(const pcgrl_config* cfg, const pcgrl_state* st, co
             }
             q.a_dev = (char*)actions_dev + off * a_stride;
         }
-        const int PIPE_COMPUTE = pipe_compute();
-        cudaStream_t up = hp.s[PIPE_COMPUTE_MAX], down = hp.s[PIPE_COMPUTE_MAX + 1];
+        cudaStream_t up = hp.s[PIPE_COMPUTE], down = hp.s[PIPE_COMPUTE + 1];
         // every upload first: 1 B per env, on its own stream, long before the chunk's turn comes
         for (int c = 0; c < n_ck && actions_host; ++c) {
             if ((e = cudaMemcpyAsync(ck[c].a_dev, (const char*)actions_host + ck[c].off * a_env, (size_t)(ck[c].m * a_env),
@@ -657,9 +655,9 @@ static int32_t step_host_impl(const pcgrl_config* cfg, const pcgrl_state* st, co
     // cannot return before the last event is.  The operations only depend on the pointers, so they are captured ONCE
     // (stream capture on helper stream 0, the others forked / joined by events inside the capture) and replayed
     // with one cudaGraphLaunch; only the source addresses of the uploads change from step to step
-    // (cudaGraphExecMemcpyNodeSetParams1D).  PCGRL_HOST_GRAPH=0 queues the operations directly, as before.
-    static const bool use_graph = !(getenv("PCGRL_HOST_GRAPH") && atoi(getenv("PCGRL_HOST_GRAPH")) == 0);
-    if (use_graph && !hp.graph_broken && !trace) {
+    // (cudaGraphExecMemcpyNodeSetParams1D).  Tracing, and a driver that cannot capture the pipeline, queue the
+    // operations directly (below).
+    if (!hp.graph_broken && !trace) {
         HostGraphKey key;
         std::memset(&key, 0, sizeof(key));
         key.cfg = *cfg;
@@ -672,7 +670,6 @@ static int32_t step_host_impl(const pcgrl_config* cfg, const pcgrl_state* st, co
         key.stats_host = stats_host;
         key.records_host = records_host;
         key.chunks = chunks;
-        key.chunk_path = chunk_path;
         HostGraph* hg = nullptr;
         for (auto& g : hp.graphs)
             if (g.exec && !std::memcmp(&g.key, &key, sizeof(key))) hg = &g;
@@ -780,7 +777,7 @@ static int32_t step_host_impl(const pcgrl_config* cfg, const pcgrl_state* st, co
         for (int c = 0; c < chunks; ++c) {
             float t[3] = {0, 0, 0};
             for (int k = 0; k < 3; ++k) cudaEventElapsedTime(&t[k], trace[3 * WL_CHUNKS], trace[3 * c + k]);
-            fprintf(stderr, "[pcgrl host trace]   chunk %d (stream %d): %8.1f | %8.1f | %8.1f\n", c, c % pipe_compute(),
+            fprintf(stderr, "[pcgrl host trace]   chunk %d (stream %d): %8.1f | %8.1f | %8.1f\n", c, c % PIPE_COMPUTE,
                     t[0] * 1e3f, t[1] * 1e3f, t[2] * 1e3f);
         }
     }

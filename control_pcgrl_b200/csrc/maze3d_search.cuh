@@ -6,13 +6,9 @@
 namespace pcgrl {
 
 constexpr int MAZE_QCAP = 256;    // FIFO ring capacity (entries); measured maximum with push filtering: 50
-#ifndef PCGRL_UF_RUNS32
-#define PCGRL_UF_RUNS32 1   // A/B on B200 (14^3): u16 per-cell parents / u32 run parents -> 2.12 / 2.26e7 env-steps/s
-#endif
-#ifndef PCGRL_MAZE_WARPS
-#define PCGRL_MAZE_WARPS 6   // A/B on B200 (14^3, 65 536 envs): 4 / 6 / 8 / 16 warps per CTA -> 1.81 / 2.13 / 2.05 / 1.41e7 env-steps/s
-#endif
-constexpr int MAZE_WARPS = PCGRL_MAZE_WARPS;     // small CTAs, several per SM: finer-grained tile barriers
+// small CTAs, several per SM: finer-grained tile barriers.  A/B on B200 (14^3, 65 536 envs): 4 / 6 / 8 / 16 warps per
+// CTA -> 1.81 / 2.13 / 2.05 / 1.41e7 env-steps/s
+constexpr int MAZE_WARPS = 6;
 constexpr int MAZE_CTAS_PER_SM = 32 / MAZE_WARPS;
 constexpr int MAZE_MAX_CTAS = 160 * MAZE_CTAS_PER_SM;   // sizes the global scratch (>= 148 SMs x 8 CTAs)
 constexpr int MAZE_NJ_SLICE = 16 * 16 * 16 * 2;         // bytes of nj per warp (maps up to 16^3)
@@ -28,9 +24,7 @@ __host__ __device__ inline MazeLayout maze_layout(int Z, int Y, int X, int row_s
     const int cells = Z * Y * X;
     int bb = 2 * cells;
     if (bb < row_stride) bb = row_stride;      // the raw grid is staged here first
-#if PCGRL_UF_RUNS32
     if (bb < Z * Y * 32) bb = Z * Y * 32;      // ... and the region count's 32-bit run parents live here last
-#endif
     bb = (bb + 15) / 16 * 16;
     L.best_bytes = bb;
     L.order_cap = (Z / 2 + 1) * Y * X;
@@ -275,11 +269,8 @@ struct Maze3DProb {
         }
 
         // ---- calc_num_regions (helper_3D.py:396-406): 6-neighbour AIR components by union-find over runs ---
-#if PCGRL_UF_RUNS32
+        // (u32 run parents; u16 per-cell parents, count_regions_rows, ran at 2.12 against 2.26e7 env-steps/s on B200, 14^3)
         const int regions = count_regions_runs32(c.row, Z, Y, X, (uint32_t*)c.best, lane);
-#else
-        const int regions = count_regions_rows(c.row, Z, Y, X, c.best, lane);
-#endif
 
         if (lane == 0) {
             // jumps[far] of the last processed component: nj[] still holds that search's recordings (lane 0

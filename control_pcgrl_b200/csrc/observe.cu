@@ -9,7 +9,6 @@
 // One thread per output pixel writes all of its channels (channels-last => contiguous per thread, and
 // consecutive threads write consecutive pixels => coalesced stores).  The int8 grid rows are re-read
 // through L1/L2; nothing else is loaded.
-#include <cstdlib>
 #include "pcgrl_device.cuh"
 
 namespace pcgrl {
@@ -161,7 +160,7 @@ __device__ __forceinline__ uint32_t fdiv(uint32_t n, uint32_t d, uint32_t magic,
 constexpr int OBS_MAX_CTA_ENVS = 64;   // GB * G
 constexpr int OBS_THREADS = 256;
 
-template <typename T, bool CROP, bool STATIC, bool D3, int ROWN /* 0, or 4 / 8 / 32: pixels per thread, all in one image row */>
+template <typename T, bool CROP, bool STATIC, bool D3, int ROWN /* 0, or 4 / 7 / 8 / 11 / 32: pixels per thread, all in one image row */>
 __global__ void __launch_bounds__(OBS_THREADS) k_observe_staged(const ObsParams p, const ObsVec v) {
     extern __shared__ __align__(16) uint8_t obs_smem[];
     T* stage = (T*)obs_smem;                                         // [envs of the trip][pix][n_ch]
@@ -518,8 +517,7 @@ static cudaError_t launch_vec(const ObsParams& p, cudaStream_t s, bool& done) {
     int dyn = v.stage_bytes + v.planes_bytes + v.GB * v.G * (p.row_stride * (p.static_mask ? 2 : 1) + 12);
     // two-tile crops of maps up to 16 wide in windows up to 32 wide (u8 one-hot or codes, no extra planes): row-mask path
     v.bits = sizeof(T) == 1 && p.crop && p.ndim == 2 && p.n_tiles == 2 && p.d1 <= 16 && p.o1 <= 32 && p.o1 % 8 == 0 &&
-             !p.static_mask && !p.holes && p.n_ctrl == 0 && (p.raw ? n_ch == 1 : n_ch == 3) &&
-             !getenv("PCGRL_OBSERVE_NO_BITS");
+             !p.static_mask && !p.holes && p.n_ctrl == 0 && (p.raw ? n_ch == 1 : n_ch == 3);
     v.lut_off = (dyn + 15) / 16 * 16;
     if (v.bits) dyn = v.lut_off + 256 * 16 + 256 * 4 + (v.GB * v.G * p.d0 * 2 + 15) / 16 * 16;
     const bool d3 = p.ndim == 3, st = p.static_mask != nullptr, cr = p.crop != 0;
@@ -534,29 +532,17 @@ static cudaError_t launch_vec(const ObsParams& p, cudaStream_t s, bool& done) {
         : (d3 ? k_observe_staged<T, false, false, true, RN> : k_observe_staged<T, false, false, false, RN>))
     void (*kern)(const ObsParams, const ObsVec) = rown == 8 ? OBS_PICK(8) : (rown == 4 ? OBS_PICK(4) : OBS_PICK(0));
 #undef OBS_PICK
-    // u8 windows 22 wide (zelda 7x11 behind its 22x22 crop: neither a multiple of 8 nor of 4, so it ran the 4-pixel path
-    // with carries): half a window row (11 pixels) or a whole one per thread.  PCGRL_OBSERVE_ROW22 = 0 / 11 / 22 (A/B).
     if constexpr (sizeof(T) == 1) {
-        if (rown == 0 && p.o1 == 22 && !d3 && !st && cr && !p.holes) {
-            const char* e22 = getenv("PCGRL_OBSERVE_ROW22");
-            const int r22 = e22 ? atoi(e22) : 11;
-            if (r22 == 11) kern = k_observe_staged<T, true, false, false, 11>;
-            if (r22 == 22) kern = k_observe_staged<T, true, false, false, 22>;
-        }
-    }
-    // ... and for the 3D maze's 14-wide last axis (14^3 window of a 14^3 level): PCGRL_OBSERVE_ROW14 = 0 / 7 / 14 (A/B)
-    if constexpr (sizeof(T) == 1) {
-        if (rown == 0 && d3 && p.o2 == 14 && !st && cr && !p.holes) {
-            const char* e14 = getenv("PCGRL_OBSERVE_ROW14");
-            const int r14 = e14 ? atoi(e14) : 7;
-            if (r14 == 7) kern = k_observe_staged<T, true, false, true, 7>;
-            if (r14 == 14) kern = k_observe_staged<T, true, false, true, 14>;
-        }
-    }
-    // row-mask crops whose window is exactly 32 wide (binary 16x16 behind its 32x32 crop): a whole window row per thread
-    if constexpr (sizeof(T) == 1) {
-        if (v.bits && rown == 8 && p.o1 == 32 && !d3 && !st && cr && !getenv("PCGRL_OBSERVE_NO_ROW32"))
-            kern = k_observe_staged<T, true, false, false, 32>;
+        // u8 windows 22 wide (zelda 7x11 behind its 22x22 crop: neither a multiple of 8 nor of 4, so it ran the 4-pixel
+        // path with carries): half a window row (11 pixels) per thread, 0.2339 ms against 0.3465 ms with 4 and 0.2607 ms
+        // with a whole row (profiles/r02_observe_row22.txt)
+        if (rown == 0 && p.o1 == 22 && !d3 && !st && cr && !p.holes) kern = k_observe_staged<T, true, false, false, 11>;
+        // ... and the 3D maze's 14-wide last axis (14^3 window of a 14^3 level): 7 pixels per thread, 0.776 ms against
+        // 1.6133 ms with 4 and 0.8206 ms with 14 (profiles/r02_observe_row14.txt)
+        if (rown == 0 && d3 && p.o2 == 14 && !st && cr && !p.holes) kern = k_observe_staged<T, true, false, true, 7>;
+        // row-mask crops whose window is exactly 32 wide (binary 16x16 behind its 32x32 crop): a whole window row per
+        // thread, 0.1649 ms against 0.1852 ms with 8 pixels per thread (profiles/r02_observe_row32.jsonl)
+        if (v.bits && rown == 8 && p.o1 == 32 && !d3 && !st && cr) kern = k_observe_staged<T, true, false, false, 32>;
     }
     cudaError_t e;
     if (dyn > 48 * 1024 &&
@@ -624,7 +610,7 @@ cudaError_t launch_observe(const pcgrl_config& cfg, const pcgrl_state& st, const
     const int64_t total = st.n_envs * (int64_t)p.o0 * p.o1 * p.o2;
     if (total == 0) return cudaSuccess;
     // the staged writer knows the 2D border frame only; the bordered 3D map goes through the pixel-per-thread kernel
-    if (!holey3d && !getenv("PCGRL_OBSERVE_SCALAR")) {   // (the env var keeps that kernel reachable for A/B runs)
+    if (!holey3d) {
         bool done = false;
         cudaError_t e = (a.out_kind == 0 || a.out_kind == 3) ? launch_vec<uint8_t>(p, s, done)
                       : a.out_kind == 1 ? launch_vec<float>(p, s, done)

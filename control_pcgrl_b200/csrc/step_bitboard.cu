@@ -22,27 +22,18 @@
 
 namespace pcgrl {
 
-#ifndef PCGRL_THREADS
-#define PCGRL_THREADS 128
-#endif
-#ifndef PCGRL_MIN_CTAS
-#define PCGRL_MIN_CTAS 10  // boards of <= 8 words: 48 registers, 10 CTAs (40 warps) per SM; A/B 1 / 10 -> 2.88 / 2.95e9
-#endif
-#ifndef PCGRL_EXPAND_R
-#define PCGRL_EXPAND_R 3
-#endif
-#ifndef PCGRL_TILE8
-#define PCGRL_TILE8 256   // envs per CTA when a board is <= 8 words (binary 16x16); A/B: 2 envs per thread is best
-#endif
-constexpr int THREADS = PCGRL_THREADS;
+constexpr int THREADS = 128;
+constexpr int MIN_CTAS = 10;   // boards of <= 8 words: 48 registers, 10 CTAs (40 warps) per SM; A/B 1 / 10 -> 2.88 / 2.95e9
+constexpr int EXPAND_R = 3;
+constexpr int TILE8 = 256;     // envs per CTA when a board is <= 8 words (binary 16x16); A/B: 2 envs per thread is best
 // envs per CTA, bounded so the shared-memory bit-boards stay under the 48 KB static limit
-__host__ __device__ constexpr int tile_for(int bbw) { return bbw == 8 ? PCGRL_TILE8 : bbw < 8 ? 256 : (bbw <= 32 ? 256 : (bbw <= 80 ? 128 : 64)); }
+__host__ __device__ constexpr int tile_for(int bbw) { return bbw == 8 ? TILE8 : bbw < 8 ? 256 : (bbw <= 32 ? 256 : (bbw <= 80 ? 128 : 64)); }
 
 // ------------------------------------------------------------------------------------------------
 // the kernel
 // ------------------------------------------------------------------------------------------------
 template <class Machine, int NW, bool TWO>
-__global__ void __launch_bounds__(THREADS, NW <= 8 ? PCGRL_MIN_CTAS : 1) k_step_bitboard(const KParams p) {
+__global__ void __launch_bounds__(THREADS, NW <= 8 ? MIN_CTAS : 1) k_step_bitboard(const KParams p) {
     using Prob = typename Machine::Prob;
     constexpr int P = Prob::P;
     constexpr int K = Prob::K;
@@ -133,7 +124,7 @@ __global__ void __launch_bounds__(THREADS, NW <= 8 ? PCGRL_MIN_CTAS : 1) k_step_
     // Each thread pulls the next changed env from the shared-memory queue as soon as it finishes one, so
     // lanes with short searches do not idle behind long ones; the search itself is a flat loop (one board
     // expansion per trip) so lanes in different phases of different grids execute the same instructions.
-    // Fixed windows of PCGRL_EXPAND_R expansions: adaptive rounds (expand while a share of the warp's lanes is
+    // Fixed windows of EXPAND_R expansions: adaptive rounds (expand while a share of the warp's lanes is
     // alive) measured 0.45-0.60 ms per step against 0.385, and a warp-wide vote that starts every trip together
     // 0.393 against 0.385 (it pays in the split kernel, step_split.cu).
     {
@@ -143,12 +134,12 @@ __global__ void __launch_bounds__(THREADS, NW <= 8 ? PCGRL_MIN_CTAS : 1) k_step_
         if (active) m.init(s_bb + item * BBW, p, base + s_list[item]);
         while (active) {
             int out[K];
-            // PCGRL_EXPAND_R expansions per trip: the transition stream (a few lanes) is then paid once per R
+            // EXPAND_R expansions per trip: the transition stream (a few lanes) is then paid once per R
             // expansions of the warp instead of once per expansion; a lane whose frontier dies early idles for
             // the rest of the trip
             bool alive = m.expand();
 #pragma unroll
-            for (int r = 1; r < PCGRL_EXPAND_R; ++r)
+            for (int r = 1; r < EXPAND_R; ++r)
                 if (alive) alive = m.expand();
             if (alive) continue;
             if (m.transition(out)) {

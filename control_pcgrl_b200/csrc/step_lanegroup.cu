@@ -24,17 +24,14 @@
 //
 // Reference path replaced: the same as step_split.cu (envs/pcgrl_env.py:267-342, envs/reps/*_rep.py,
 // envs/probs/binary/binary_prob.py:152-158, envs/helper.py:200-276, control_wrappers.py:216-244, 318-345).
-#include <cstdlib>
 #include "pcgrl_device.cuh"
 #include "step_common.cuh"
 
 namespace pcgrl {
 
-#ifndef PCGRL_LG_EXPAND_R
-#define PCGRL_LG_EXPAND_R 12      // BFS levels per trip (computed blind, see expand_window).  A/B 4 / 6 / 8 / 12 (kernel time, CUDA
+constexpr int LG_EXPAND_R = 12;   // BFS levels per trip (computed blind, see expand_window).  A/B 4 / 6 / 8 / 12 (kernel time, CUDA
                                   // events): 2 Ki envs 28.8 / 26.4 / 25.7 / 25.0 us, 16 Ki envs 34.9 / 32.4 / 31.8 / 31.5 us -- a small
                                   // shard has issue slots to spare, so few long trips beat many short ones
-#endif
 constexpr int LG_THREADS = 128;
 
 // Every collective below (shuffle, ballot) is issued by ALL 32 lanes with the full mask at warp-uniform points of the
@@ -115,15 +112,15 @@ struct LaneGroupInc {
             hit = false;
         }
     }
-    // PCGRL_LG_EXPAND_R BFS levels of the groups with `run`; returns whether the group's frontier is still alive
+    // LG_EXPAND_R BFS levels of the groups with `run`; returns whether the group's frontier is still alive
     // afterwards (false for !run).  The levels are computed blind, one straight dependent chain of shuffles and
     // logic ops -- a dead frontier stays dead and leaves avail alone, so running past the end is harmless -- and only
     // then the ballots (independent of each other, off the chain) say how many levels were real: front must end up
     // as the LAST NON-EMPTY level (its lowest cell is the far tile) and level counts only those.
     __device__ __forceinline__ bool expand_window(bool run) {
-        uint32_t f = front, av = avail, hist[PCGRL_LG_EXPAND_R];
+        uint32_t f = front, av = avail, hist[LG_EXPAND_R];
 #pragma unroll
-        for (int r = 0; r < PCGRL_LG_EXPAND_R; ++r) {
+        for (int r = 0; r < LG_EXPAND_R; ++r) {
             const uint32_t n = nbr(f) & av;
             av &= ~n;
             f = n;
@@ -132,7 +129,7 @@ struct LaneGroupInc {
         int adv = 0;
         uint32_t last = front;
 #pragma unroll
-        for (int r = 0; r < PCGRL_LG_EXPAND_R; ++r) {
+        for (int r = 0; r < LG_EXPAND_R; ++r) {
             const bool some = gany(run && hist[r] != 0u);   // monotone: once a level is empty the later ones are too
             adv += some ? 1 : 0;
             last = some ? hist[r] : last;
@@ -142,7 +139,7 @@ struct LaneGroupInc {
             front = last;
             level += adv;
         }
-        return run && adv == PCGRL_LG_EXPAND_R;
+        return run && adv == LG_EXPAND_R;
     }
     // The groups with `dead` (busy, frontier died) take their transition; returns true for the groups whose search is
     // over.  Each phase is one block entered by the whole warp if any group needs it.
@@ -267,7 +264,7 @@ __global__ void __launch_bounds__(LG_THREADS) k_step_lanegroup(const __grid_cons
         s_cell[warp][lane] = cell;
         __syncwarp();
         // ---- search.  One flat loop, warp-uniform control flow: idle groups take the next changed env, every busy
-        // group runs PCGRL_LG_EXPAND_R levels, the groups whose frontier died take their transition.
+        // group runs LG_EXPAND_R levels, the groups whose frontier died take their transition.
         bool active = false;
         int slot = 0;
         uint32_t* row = nullptr;
@@ -324,16 +321,11 @@ static cudaError_t launch_lg(const KParams& p, cudaStream_t s) {
         if ((e = cudaDeviceGetAttribute(&g_lg_sm, cudaDevAttrMultiProcessorCount, dev)) != cudaSuccess) return e;
     }
     // tile size: the smallest of 8 / 16 / 32 envs per warp whose grid still fits the GPU in one wave (every warp then
-    // runs as few searches one after the other as possible); PCGRL_LG_TILE overrides (A/B)
-    static int env_t = -1;
-    if (env_t < 0) {
-        const char* e = getenv("PCGRL_LG_TILE");
-        env_t = e ? atoi(e) : 0;
-    }
+    // runs as few searches one after the other as possible).  At 64 Ki envs, where this picks 16, 8 / 16 / 32 envs per
+    // warp gave 0.0810 / 0.0749 / 0.0847 ms per step (profiles/r02_lanegroup_by_size.txt).
     const int64_t resident_warps = (int64_t)g_lg_sm * 32;      // 8 CTAs of 4 warps per SM (64 registers per thread)
     int T = 32;
-    if (env_t == 8 || env_t == 16 || env_t == 32) T = env_t;
-    else if ((p.n_envs + 7) / 8 <= resident_warps) T = 8;
+    if ((p.n_envs + 7) / 8 <= resident_warps) T = 8;
     else if ((p.n_envs + 15) / 16 <= resident_warps) T = 16;
     const int64_t warps = (p.n_envs + T - 1) / T;
     const int64_t want = (warps + LG_THREADS / 32 - 1) / (LG_THREADS / 32);

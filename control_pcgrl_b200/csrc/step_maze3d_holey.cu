@@ -195,11 +195,7 @@ struct Holey3DProb {
             v3 = nj;
         }
         // ---- calc_num_regions over AIR of the bordered map (helper_3D.py:396-406) ----------------------------------
-#if PCGRL_UF_RUNS32
         const int regions = count_regions_runs32(c.row, Z, Y, X, (uint32_t*)c.best, lane);
-#else
-        const int regions = count_regions_rows(c.row, Z, Y, X, c.best, lane);
-#endif
         if (lane == 0) {
             out[0] = regions;
             if (!DUNGEON) {

@@ -14,10 +14,7 @@
 namespace pcgrl {
 
 constexpr int SEARCH_WARPS = 8;   // default warps per CTA (a problem may ask for more)
-#ifndef PCGRL_SEARCH_TILE
-#define PCGRL_SEARCH_TILE 64
-#endif
-constexpr int SEARCH_TILE = PCGRL_SEARCH_TILE;   // envs per CTA iteration (a CTA-wide barrier closes each one).  A/B on the 3D
+constexpr int SEARCH_TILE = 64;                  // envs per CTA iteration (a CTA-wide barrier closes each one).  A/B on the 3D
                                                  // maze (65 536 envs): 32 / 64 / 128 / 256 -> 2.19 / 2.25 / 2.18 / 1.41e7 env-steps/s
 constexpr int SEARCH_SLOTS = 64;  // concurrent launches that can share the tile counters below
 // Dynamic tile scheduling: CTAs pull tile indices from g_tile_ctr[slot]; the last CTA to leave resets the

@@ -40,14 +40,8 @@ namespace pcgrl {
 
 constexpr int SMB_POWER = 10000;                 // smb_prob.py:21 _solver_power
 constexpr int SMB_NODES = 4 * SMB_POWER + 8;
-#ifndef PCGRL_SMB_WARPS
-#define PCGRL_SMB_WARPS 8
-#endif
-constexpr int SMB_WARPS = PCGRL_SMB_WARPS;   // warps per CTA
-#ifndef PCGRL_SMB_CTAS_PER_SM
-#define PCGRL_SMB_CTAS_PER_SM 4   // A/B on B200 (116x16, 65 536 envs): 2 / 3 / 4 CTAs per SM -> 7.0 / 8.5 / 9.7e6 env-steps/s
-#endif
-constexpr int SMB_MAX_CTAS_PER_SM = PCGRL_SMB_CTAS_PER_SM;
+constexpr int SMB_WARPS = 8;             // warps per CTA
+constexpr int SMB_MAX_CTAS_PER_SM = 4;   // A/B on B200 (116x16, 65 536 envs): 2 / 3 / 4 CTAs per SM -> 7.0 / 8.5 / 9.7e6 env-steps/s
 constexpr int SMB_MAX_CTAS = 160 * SMB_MAX_CTAS_PER_SM;   // sizes the global scratch (>= 148 SMs x CTAs per SM)
 constexpr int SMB_YOFF = 8;                      // y >= -5 (four rows per jump, re-jump possible from y = -1)
 
@@ -58,16 +52,14 @@ struct SmbScratch {
 };
 
 // ---- jobs, per-group slices, fallback slices (in this order in the global scratch) --------------------------
-#ifndef PCGRL_SMB_SOLVE_CTAS_PER_SM
-#define PCGRL_SMB_SOLVE_CTAS_PER_SM 2   // 64 lane groups x SMB_G_SMEM_WORDS words of shared memory per CTA = 112 KB
-#endif
+constexpr int SMB_SOLVE_CTAS_PER_SM = 2;   // 64 lane groups x SMB_G_SMEM_WORDS words of shared memory per CTA = 112 KB
 constexpr int SMB_G_CAP = 4096;                  // heap entries == node slots of one lane group
 constexpr int SMB_G_SMEM_WORDS = 447;            // shared-memory words per lane group (heap top + bit map): 64 groups
                                                  // per CTA, two CTAs per SM
 constexpr int SMB_G_SOLID = 128;                 // words of a group's shared-memory bit map: H * ceil((W + 6) / 32)
 constexpr int SMB_G_VISITED = 5120;              // bytes of its visited-key map: (H + 8) * (W + 6)
 constexpr int SMB_SOLVE_WARPS = 8;
-constexpr int SMB_SOLVE_CTAS = 160 * PCGRL_SMB_SOLVE_CTAS_PER_SM;
+constexpr int SMB_SOLVE_CTAS = 160 * SMB_SOLVE_CTAS_PER_SM;
 constexpr int SMB_FALLBACK_CTAS = 160;
 struct SmbJobs {
     static constexpr int CAP = 1 << 18;          // jobs per launch; launch_smb walks larger shards in ranges of CAP envs
@@ -778,7 +770,7 @@ cudaError_t launch_smb(const KParams& p, cudaStream_t s, bool& supported, int& n
             auto k2 = hybrid ? k_smb_solve<SMB_SOLVE_WARPS, true> : k_smb_solve<SMB_SOLVE_WARPS, false>;
             const int dyn = SMB_SOLVE_WARPS * 8 * SMB_G_SMEM_WORDS * 4;
             if ((e = cudaFuncSetAttribute(k2, cudaFuncAttributeMaxDynamicSharedMemorySize, dyn)) != cudaSuccess) return e;
-            const int ctas = std::min(n_sm * PCGRL_SMB_SOLVE_CTAS_PER_SM, SMB_SOLVE_CTAS);
+            const int ctas = std::min(n_sm * SMB_SOLVE_CTAS_PER_SM, SMB_SOLVE_CTAS);
             k2<<<ctas, SMB_SOLVE_WARPS * 32, dyn, s>>>(p, g_cap);
             if ((e = cudaGetLastError()) != cudaSuccess) return e;
             ++n_launches;

@@ -29,10 +29,7 @@ constexpr int SOK_POWER = 10000;                 // sokoban_prob.py:40 _solver_p
 constexpr int SOK_NODES = 4 * SOK_POWER + 8;     // root + <= 4 children per iteration
 constexpr int SOK_TABLE = 32768;                 // visited hash slots (<= 10 000 insertions per search)
 constexpr int SOK_MAX_CRATES = 15;
-#ifndef PCGRL_SOK_CTAS_PER_SM
-#define PCGRL_SOK_CTAS_PER_SM 2   // A/B on B200: 2 / 3 / 4 CTAs per SM change nothing (bounded by the longest solve)
-#endif
-constexpr int SOK_MAX_CTAS_PER_SM = PCGRL_SOK_CTAS_PER_SM;
+constexpr int SOK_MAX_CTAS_PER_SM = 2;   // A/B on B200: 2 / 3 / 4 CTAs per SM change nothing (bounded by the longest solve)
 constexpr int SOK_MAX_CTAS = 160 * SOK_MAX_CTAS_PER_SM;   // sizes the global scratch (>= 148 SMs x CTAs per SM)
 
 struct SokScratch {

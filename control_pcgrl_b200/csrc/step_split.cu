@@ -25,43 +25,30 @@
 // Reference path replaced: the same as step_bitboard.cu (envs/pcgrl_env.py:267-342, envs/reps/*_rep.py,
 // envs/probs/binary/binary_prob.py:152-158, envs/probs/zelda/zelda_ctrl_prob.py:90-168, envs/helper.py:200-276,
 // control_wrappers.py:216-244, 318-345).
-#include <cstdlib>
 #include "pcgrl_device.cuh"
 #include "step_common.cuh"
 #include "bitboard_machines.cuh"
 
 namespace pcgrl {
 
-#ifndef PCGRL_SPLIT_MIN_CTAS
-#define PCGRL_SPLIT_MIN_CTAS 10
-#endif
-#ifndef PCGRL_INC_CTAS_PER_SM
-#define PCGRL_INC_CTAS_PER_SM 8      // 128-thread CTAs of the incremental search resident per SM (A/B 4 / 6 / 8 / 12 at
-                                     // R=3: 0.412 / 0.393 / 0.384 / 0.378 ms per step)
-#endif
-#ifndef PCGRL_INC_CTAS_PER_SM_HOST
-#define PCGRL_INC_CTAS_PER_SM_HOST 4 // the same inside the host pipeline: most of the SM's registers stay free, so the
-                                     // update / output kernels of the neighbouring chunks run next to the search
-                                     // (e2e at 4 chunks, 2 / 3 / 4 / 5 / 8 CTAs per SM: 2.48 / 2.60 / 2.51 / 2.36 / 2.11e9 with the
-                                     // copies on the compute streams; with separate copy streams 3 / 4 / 5 / 8:
-                                     // 2.56 / 2.75 / 2.71 / 2.42e9, profiles/r02_e2e_cps_chunks_split.txt)
-#endif
-#ifndef PCGRL_INC_MIN_CLAIM
-#define PCGRL_INC_MIN_CLAIM 12       // lanes that must be waiting before a warp hands out new items: the claim / init
-                                     // stream then runs with that many lanes (A/B 1 / 4 / 8 at R=3: 0.412 / 0.390 / 0.387; at
-                                     // R=12, 8 / 12 / 16 / 24: 0.2978 / 0.2996 / 0.3022 / 0.3263 ms, profiles/r02_ab_inc_claim_window.txt)
-#endif
-#ifndef PCGRL_INC_EXPAND_R
-#define PCGRL_INC_EXPAND_R 12        // board expansions per trip.  Every trip also issues each transition stream that
-                                     // some lane needs (flood done / next component / second sweep / re-sweep / finish,
-                                     // ~580 instructions at 2-3 lanes), so few long trips beat many short ones although
-                                     // lanes idle inside the window: A/B 2 / 3 / 4 / 6 / 8 / 12 -> 0.466 / 0.412 / 0.356 /
-                                     // 0.325 / 0.308 / 0.303 ms per step (1 Mi envs, 8 CTAs per SM); 16 / 20 -> 0.3018 / 0.3140
-                                     // against 0.2996 for 12 in a later run
-#endif
-#ifndef PCGRL_EXPAND_R_SPLIT
-#define PCGRL_EXPAND_R_SPLIT 3       // board expansions per trip of the static search (as in the fused kernel)
-#endif
+constexpr int SPLIT_MIN_CTAS = 10;
+constexpr int INC_CTAS_PER_SM = 8;       // 128-thread CTAs of the incremental search resident per SM (A/B 4 / 6 / 8 / 12 at
+                                         // R=3: 0.412 / 0.393 / 0.384 / 0.378 ms per step)
+constexpr int INC_CTAS_PER_SM_HOST = 4;  // the same inside the host pipeline: most of the SM's registers stay free, so the
+                                         // update / output kernels of the neighbouring chunks run next to the search
+                                         // (e2e at 4 chunks, 2 / 3 / 4 / 5 / 8 CTAs per SM: 2.48 / 2.60 / 2.51 / 2.36 / 2.11e9 with the
+                                         // copies on the compute streams; with separate copy streams 3 / 4 / 5 / 8:
+                                         // 2.56 / 2.75 / 2.71 / 2.42e9, profiles/r02_e2e_cps_chunks_split.txt)
+constexpr int INC_MIN_CLAIM = 12;        // lanes that must be waiting before a warp hands out new items: the claim / init
+                                         // stream then runs with that many lanes (A/B 1 / 4 / 8 at R=3: 0.412 / 0.390 / 0.387; at
+                                         // R=12, 8 / 12 / 16 / 24: 0.2978 / 0.2996 / 0.3022 / 0.3263 ms, profiles/r02_ab_inc_claim_window.txt)
+constexpr int INC_EXPAND_R = 12;         // board expansions per trip.  Every trip also issues each transition stream that
+                                         // some lane needs (flood done / next component / second sweep / re-sweep / finish,
+                                         // ~580 instructions at 2-3 lanes), so few long trips beat many short ones although
+                                         // lanes idle inside the window: A/B 2 / 3 / 4 / 6 / 8 / 12 -> 0.466 / 0.412 / 0.356 /
+                                         // 0.325 / 0.308 / 0.303 ms per step (1 Mi envs, 8 CTAs per SM); 16 / 20 -> 0.3018 / 0.3140
+                                         // against 0.2996 for 12 in a later run
+constexpr int EXPAND_R_SPLIT = 3;        // board expansions per trip of the static search (as in the fused kernel)
 
 constexpr int ACT_THREADS = 256;
 constexpr int STAT_THREADS = 128;
@@ -121,7 +108,7 @@ __global__ void __launch_bounds__(ACT_THREADS) k_split_act(const KParams p) {
 // k_split_stats, static variant: one from-scratch search per lane, 32 consecutive list items per warp
 // ------------------------------------------------------------------------------------------------
 template <class Machine, int NW, bool TWO>
-__global__ void __launch_bounds__(stat_threads(Machine::Prob::P * NW), NW <= 8 ? PCGRL_SPLIT_MIN_CTAS : 1)
+__global__ void __launch_bounds__(stat_threads(Machine::Prob::P * NW), NW <= 8 ? SPLIT_MIN_CTAS : 1)
 k_split_stats(const KParams p) {
     using Prob = typename Machine::Prob;
     constexpr int P = Prob::P;
@@ -188,7 +175,7 @@ k_split_stats(const KParams p) {
     Machine m;
     if (mine) m.init(wbb + lane * BBW, p, env);
     int out[K];
-    // One trip = PCGRL_EXPAND_R_SPLIT board expansions, then the transition stream for the lanes whose frontier
+    // One trip = EXPAND_R_SPLIT board expansions, then the transition stream for the lanes whose frontier
     // died.  The warp-wide vote at the top makes every lane start every trip together: without it the lanes that
     // loop back early run ahead of the ones in a transition, the warp falls apart into groups that never re-merge, and
     // both streams are issued once per group (ncu: transitions at 3.7 lanes, expansions at 19; 0.432 against 0.381 ms
@@ -201,7 +188,7 @@ k_split_stats(const KParams p) {
         if (running) {
             bool alive = m.expand();
 #pragma unroll
-            for (int r = 1; r < PCGRL_EXPAND_R_SPLIT; ++r)
+            for (int r = 1; r < EXPAND_R_SPLIT; ++r)
                 if (alive) alive = m.expand();
             dead = !alive;
         }
@@ -411,7 +398,7 @@ struct BinaryIncMachine {
 // k_split_stats, incremental variant: persistent-size grid, every warp owns a contiguous slice of the work list
 // and its lanes claim items from it one by one (ballot-ranked at a convergent point, no atomics).  Static slices:
 // fetching items from a global counter instead did not move the bench line (0.2909 against 0.2913 ms per step) and
-// cut e2e from 2.60 to 2.51e9 (profiles/r02_ab_inc_dynamic.txt).  Fixed windows of PCGRL_INC_EXPAND_R expansions:
+// cut e2e from 2.60 to 2.51e9 (profiles/r02_ab_inc_dynamic.txt).  Fixed windows of INC_EXPAND_R expansions:
 // adaptive rounds measured 0.334 ms against 0.303.
 // ------------------------------------------------------------------------------------------------
 template <int NW, bool TWO>
@@ -435,7 +422,7 @@ __global__ void __launch_bounds__(STAT_THREADS) k_split_stats_inc(const KParams 
     int64_t env = 0;
     for (;;) {
         const unsigned need = __ballot_sync(0xffffffffu, !active);
-        if (need && lo < hi && (__popc(need) >= PCGRL_INC_MIN_CLAIM || need == 0xffffffffu || hi - lo < PCGRL_INC_MIN_CLAIM)) {
+        if (need && lo < hi && (__popc(need) >= INC_MIN_CLAIM || need == 0xffffffffu || hi - lo < INC_MIN_CLAIM)) {
             const int mine = lo + __popc(need & ((1u << lane) - 1u));
             if (!active && mine < hi) {
                 item = mine;
@@ -454,7 +441,7 @@ __global__ void __launch_bounds__(STAT_THREADS) k_split_stats_inc(const KParams 
         if (active) {
             bool alive = m.expand();
 #pragma unroll
-            for (int r = 1; r < PCGRL_INC_EXPAND_R; ++r)
+            for (int r = 1; r < INC_EXPAND_R; ++r)
                 if (alive) alive = m.expand();
             if (!alive && m.transition()) {
                 int out[2];
@@ -472,7 +459,7 @@ __global__ void __launch_bounds__(STAT_THREADS) k_split_stats_inc(const KParams 
 // (nearly) all 32 lanes:
 //   update  the next 32 envs of the slice: representation update, counters, done, zero reward for unchanged
 //           maps (thread-per-env, as k_split_act); the changed ones go into the warp's item ring in shared memory;
-//   search  lanes pick items from the ring as they become free (at least PCGRL_INC_MIN_CLAIM at a time) and run
+//   search  lanes pick items from the ring as they become free (at least INC_MIN_CLAIM at a time) and run
 //           BinaryIncMachine trips; a finished lane writes its env's cache row and parks (env, regions,
 //           path-length) in the warp's result ring;
 //   output  once 32 results wait (or nothing else is left): one lane per result does the fp64 reward and writes
@@ -488,14 +475,10 @@ __device__ __noinline__ void inc_output_env(const KParams& p, int64_t env, int r
     finish_env<2>(p, env, nw);
 }
 
-#ifndef PCGRL_STEP_INC_MIN_CTAS
-#define PCGRL_STEP_INC_MIN_CTAS 6
-#endif
-#ifndef PCGRL_STEP_INC_ROUNDS
-#define PCGRL_STEP_INC_ROUNDS 1      // update rounds (of 32 envs) per warp the grid is sized for, see launch_split
-#endif
+constexpr int STEP_INC_MIN_CTAS = 6;
+constexpr int STEP_INC_ROUNDS = 1;   // update rounds (of 32 envs) per warp the grid is sized for below 48 Ki envs, see launch_split
 template <int NW, bool TWO>
-__global__ void __launch_bounds__(STAT_THREADS, PCGRL_STEP_INC_MIN_CTAS) k_step_inc(const __grid_constant__ KParams p) {
+__global__ void __launch_bounds__(STAT_THREADS, STEP_INC_MIN_CTAS) k_step_inc(const __grid_constant__ KParams p) {
     using M = BinaryIncMachine<NW, TWO>;
     constexpr int WARPS = STAT_THREADS / 32;
     constexpr int RING = 64;
@@ -532,7 +515,7 @@ __global__ void __launch_bounds__(STAT_THREADS, PCGRL_STEP_INC_MIN_CTAS) k_step_
         const bool drained = e_next >= e_hi;
         // ---- hand items to free lanes
         const unsigned idle = __ballot_sync(0xffffffffu, !active);
-        if (idle && it_cnt > 0 && (__popc(idle) >= PCGRL_INC_MIN_CLAIM || idle == 0xffffffffu || drained)) {
+        if (idle && it_cnt > 0 && (__popc(idle) >= INC_MIN_CLAIM || idle == 0xffffffffu || drained)) {
             const int rank = __popc(idle & lt);
             if (!active && rank < it_cnt) {
                 const int2 it = items[(it_head + rank) & (RING - 1)];
@@ -569,7 +552,7 @@ __global__ void __launch_bounds__(STAT_THREADS, PCGRL_STEP_INC_MIN_CTAS) k_step_
         if (active) {
             bool alive = m.expand();
 #pragma unroll
-            for (int r = 1; r < PCGRL_INC_EXPAND_R; ++r)
+            for (int r = 1; r < INC_EXPAND_R; ++r)
                 if (alive) alive = m.expand();
             if (!alive && m.transition()) {
                 m.finish(out, (uint32_t*)(p.cache + env * p.cache_stride));
@@ -605,16 +588,8 @@ __global__ void __launch_bounds__(OUT_THREADS) k_split_out(const KParams p) {
 // ------------------------------------------------------------------------------------------------
 // host-side dispatch
 // ------------------------------------------------------------------------------------------------
-// resident CTAs per SM of the persistent incremental kernels; PCGRL_INC_CPS overrides the compiled default (A/B)
-static int inc_ctas_per_sm(bool host_chunk) {
-    static int env_v = -1;
-    if (env_v < 0) {
-        const char* e = getenv("PCGRL_INC_CPS");
-        env_v = e ? atoi(e) : 0;
-    }
-    if (env_v > 0) return env_v;
-    return host_chunk ? PCGRL_INC_CTAS_PER_SM_HOST : PCGRL_INC_CTAS_PER_SM;
-}
+// resident CTAs per SM of the persistent incremental kernels
+static int inc_ctas_per_sm(bool host_chunk) { return host_chunk ? INC_CTAS_PER_SM_HOST : INC_CTAS_PER_SM; }
 static int g_n_sm = 0;
 static cudaError_t sm_count(int& n) {
     if (!g_n_sm) {
@@ -642,14 +617,9 @@ static cudaError_t launch_split(const KParams& p, cudaStream_t s, int incrementa
             // sized so that EVERY CTA gets work: with the plain cap (6 CTAs per SM) a 128 Ki-env shard ran 64 envs per warp
             // on 512 of its 888 CTAs while the others exited at once.  A/B of m (profiles/r02_step_inc_rounds.txt, kernel
             // ms, m = 1 / 2 / 3 / 4): 32 Ki envs 0.042 / 0.048 / 0.062 / 0.075, 64 Ki 0.060 / 0.056 / 0.070 / 0.077,
-            // 128 Ki 0.095 / 0.075 / 0.083 / 0.089.  PCGRL_STEP_INC_ROUNDS overrides.
-            static int rounds = -1;
-            if (rounds < 0) {
-                const char* ev = getenv("PCGRL_STEP_INC_ROUNDS");
-                rounds = ev ? atoi(ev) : 0;
-            }
+            // 128 Ki 0.095 / 0.075 / 0.083 / 0.089.
             const int64_t cap = (int64_t)n_sm * inc_ctas_per_sm(p.host_chunk != 0);
-            int64_t m = rounds > 0 ? rounds : (n >= (48 << 10) ? 2 : PCGRL_STEP_INC_ROUNDS);
+            int64_t m = n >= (48 << 10) ? 2 : STEP_INC_ROUNDS;
             const int64_t need_m = (n + STAT_THREADS * cap - 1) / (STAT_THREADS * cap);
             if (m < need_m) m = need_m;
             const int64_t want = (n + STAT_THREADS * m - 1) / (STAT_THREADS * m);

@@ -12,5 +12,4 @@ for path in fused split inc; do
   echo -n "65k path=$path: "
   PCGRL_STEP_PATH=$path timeout 200 python bench.py --steps 800 --warmup 10 --no-cpu-baseline --no-configs --envs 65536 2>>gpurun_out/r02b.err | python -c "import json,sys; d=json.loads(sys.stdin.read()); print('value %.4g e2e %.4g kernel_ms %.4f' % (d['value'], d['e2e']['value'], d['roofline']['kernel_ms_per_launch']))"
 done | tee -a gpurun_out/r02b_paths.txt
-bash scripts/ab_variants.sh run --steps 800 --warmup 10 2>&1 | tail -30
 tail -5 gpurun_out/r02b.err

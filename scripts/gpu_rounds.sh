@@ -14,7 +14,6 @@ run 98304 incfused
 run 163840 incfused
 run 163840 inc
 run 262144 incfused
-run 262144 incfused PCGRL_STEP_INC_ROUNDS=3
 run 262144 inc
 run 393216 incfused
 run 393216 inc

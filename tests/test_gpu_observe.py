@@ -18,23 +18,18 @@ from oracle import obs_oracle
 
 pytestmark = pytest.mark.gpu
 
-A_B_VARS = ("PCGRL_OBSERVE_SCALAR", "PCGRL_OBSERVE_NO_BITS", "PCGRL_OBSERVE_NO_ROW32", "PCGRL_OBSERVE_ROW22",
-            "PCGRL_OBSERVE_ROW14")
 KINDS = {"u8": (torch.uint8, True), "f32": (torch.float32, True), "f64": (torch.float64, True),
          "codes": (torch.uint8, False)}
 ELEM = {"u8": 1, "codes": 1, "f32": 4, "f64": 8}
 
 
-def writer_variant(kind, crop, shape, window, n_tiles, n_ctrl=0, static=False, env=(), aligned=True):
+def writer_variant(kind, crop, shape, window, n_tiles, n_ctrl=0, static=False, aligned=True):
     """(variant, G, GB) the observation writer takes for one observe() call.
 
-    This mirrors launch_observe / launch_vec in csrc/observe.cu (the dispatch at lines 495-560, the scalar-kernel
-    switch at line 627, and the pack3 / pack1 / bits flags at the top of k_observe_staged) and must change with them.
+    This mirrors launch_observe / launch_vec in csrc/observe.cu (the dispatch at lines 494-546, the scalar-kernel
+    switch at line 613, and the pack3 / pack1 / bits flags at the top of k_observe_staged) and must change with them.
     Nothing checks it against that code automatically: review it line by line when the dispatch changes.
     (The occupancy query's per_sm < 1 fallback is not mirrored; no case here comes near it.)"""
-    env = dict(env)
-    if "PCGRL_OBSERVE_SCALAR" in env:
-        return "scalar_env", 0, 0
     if not aligned:
         return "scalar_unaligned", 0, 0
     size, raw, d3 = ELEM[kind], kind == "codes", len(shape) == 3
@@ -53,16 +48,14 @@ def writer_variant(kind, crop, shape, window, n_tiles, n_ctrl=0, static=False, e
     while GB * G * 2 <= 64 and GB * 2 * group_bytes <= 24 * 1024:
         GB *= 2
     bits = (size == 1 and crop and not d3 and n_tiles == 2 and shape[1] <= 16 and o[1] <= 32 and o[1] % 8 == 0 and
-            not static and n_ctrl == 0 and n_ch == (1 if raw else 3) and "PCGRL_OBSERVE_NO_BITS" not in env)
+            not static and n_ctrl == 0 and n_ch == (1 if raw else 3))
     last = o[-1]
     rown = 8 if size == 1 and last % 8 == 0 else (4 if last % 4 == 0 else 0)
     if size == 1 and rown == 0 and o[1] == 22 and not d3 and not static and crop:
-        r22 = int(env.get("PCGRL_OBSERVE_ROW22", 11))
-        rown = r22 if r22 in (11, 22) else rown
+        rown = 11
     if size == 1 and rown == 0 and d3 and o[2] == 14 and not static and crop:
-        r14 = int(env.get("PCGRL_OBSERVE_ROW14", 7))
-        rown = r14 if r14 in (7, 14) else rown
-    if bits and rown == 8 and o[1] == 32 and not d3 and not static and crop and "PCGRL_OBSERVE_NO_ROW32" not in env:
+        rown = 7
+    if bits and rown == 8 and o[1] == 32 and not d3 and not static and crop:
         rown = 32
     r8 = rown in (8, 32)
     pack3 = size == 1 and r8 and not static and n_ch == 3 and not raw and n_ctrl == 0
@@ -73,12 +66,11 @@ def writer_variant(kind, crop, shape, window, n_tiles, n_ctrl=0, static=False, e
         v = "row8_bits" if bits and (pack3 or pack1) else \
             "row8_pack3" if pack3 else "row8_pack1" if pack1 else "row8_generic"
     else:
-        v = {0: "row0", 4: "row4", 11: "row22_11", 22: "row22_22", 7: "row14_7", 14: "row14_14"}[rown]
+        v = {0: "row0", 4: "row4", 11: "row22_11", 7: "row14_7"}[rown]
     return v, G, GB
 
 
-Case = namedtuple("Case", "id problem rep shape window kinds env controls static big",
-                  defaults=((), None, False, None))
+Case = namedtuple("Case", "id problem rep shape window kinds controls static big", defaults=(None, False, None))
 U8C = ("u8", "codes")
 ALL4 = ("u8", "f32", "f64", "codes")
 CASES = [
@@ -87,30 +79,24 @@ CASES = [
     Case("row32_binary40x16", "binary", "narrow", (40, 16), (32, 32), U8C),
     Case("row32_binary16x5", "binary", "narrow", (16, 5), (32, 32), U8C),
     Case("row32_binary9x13_odd_height", "binary", "turtle", (9, 13), (15, 32), U8C),
-    # staged, 8 pixels per thread from row bit masks: windows smaller than the map, 24 wide, 32 wide without ROW32
+    # staged, 8 pixels per thread from row bit masks: windows smaller than the map, 24 wide
     Case("bits_binary16_w8", "binary", "narrow", (16, 16), (8, 8), U8C),
     Case("bits_binary16_w24", "binary", "narrow", (16, 16), (24, 24), U8C),
     Case("bits_binary9x13_w16x24", "binary", "turtle", (9, 13), (16, 24), U8C),
-    Case("bits_binary16_no_row32", "binary", "narrow", (16, 16), (32, 32), U8C, env={"PCGRL_OBSERVE_NO_ROW32": "1"}),
     # staged, 8 packed records per thread without bit masks (whole groups outside the map: constant records)
     Case("pack_binary20x24_w48", "binary", "narrow", (20, 24), (48, 48), U8C),
-    Case("pack_binary16_no_bits", "binary", "narrow", (16, 16), (32, 32), U8C, env={"PCGRL_OBSERVE_NO_BITS": "1"}),
     Case("pack_binary64_default_window", "binary", "narrow", (64, 64), (32, 32), U8C),
     # staged, 8 pixels per thread, one store per pixel
     Case("generic8_zelda_w24", "zelda", "narrow", (7, 11), (24, 24), ("u8", "f32", "codes")),
     Case("generic8_smb", "smb", "narrow", (116, 16), (32, 32), U8C),
     Case("nocrop_binary_wide", "binary", "wide", (16, 16), None, ALL4),
-    # 22-wide u8 windows: 11 (default) or 22 pixels per thread
-    Case("row22_zelda", "zelda", "narrow", (7, 11), (22, 22), U8C, big="u8"),
-    Case("row22_zelda_whole_row", "zelda", "turtle", (7, 11), (22, 22), U8C, env={"PCGRL_OBSERVE_ROW22": "22"}),
-    Case("row22_off_zelda", "zelda", "narrow", (7, 11), (22, 22), U8C, env={"PCGRL_OBSERVE_ROW22": "0"}),
+    # 22-wide u8 windows: 11 pixels per thread (f32 / f64 take the general path)
+    Case("row22_zelda", "zelda", "narrow", (7, 11), (22, 22), ALL4, big="u8"),
     Case("row22_binary16", "binary", "narrow", (16, 16), (22, 22), U8C),
     Case("row22_sokoban5", "sokoban", "narrow", (5, 5), (22, 22), U8C),
     Case("row22_zelda30_map_wider", "zelda", "narrow", (30, 30), (22, 22), U8C),
-    # 3D crops whose last window axis is 14: 7 (default) or 14 pixels per thread
-    Case("row14_maze14", "minecraft_3D_maze", "narrow", (14, 14, 14), (14, 14, 14), U8C, big="u8"),
-    Case("row14_maze14_whole_row", "minecraft_3D_maze", "turtle", (14, 14, 14), (14, 14, 14), U8C,
-         env={"PCGRL_OBSERVE_ROW14": "14"}),
+    # 3D crops whose last window axis is 14: 7 u8 pixels per thread (f32 / f64 take the general path)
+    Case("row14_maze14", "minecraft_3D_maze", "narrow", (14, 14, 14), (14, 14, 14), ALL4, big="u8"),
     Case("row14_maze7", "minecraft_3D_maze", "narrow", (7, 7, 7), (14, 14, 14), U8C),
     Case("row14_maze5x9x7", "minecraft_3D_maze", "narrow", (5, 9, 7), (10, 18, 14), U8C),
     # 3D, 8 pixels per thread (packed one-hot / codes), 4 per thread in f32 / f64
@@ -124,7 +110,7 @@ CASES = [
     Case("odd_binary16_w21", "binary", "narrow", (16, 16), (21, 21), U8C),
     Case("odd_zelda_w21", "zelda", "narrow", (7, 11), (21, 21), ("u8", "f64", "codes")),
     Case("odd_maze6_w9", "minecraft_3D_maze", "narrow", (6, 6, 6), (9, 9, 9), ALL4),
-    Case("general_binary_turtle", "binary", "turtle", (9, 13), (18, 26), ("u8", "f32", "codes")),
+    Case("general_binary_turtle", "binary", "turtle", (9, 13), (18, 26), ALL4),
     # frozen-tile plane
     Case("static_binary16", "binary", "narrow", (16, 16), (32, 32), ("u8", "f32", "f64"), static=True, big="u8"),
     Case("static_zelda", "zelda", "narrow", (7, 11), (22, 22), ("u8", "f32", "f64"), static=True),
@@ -139,20 +125,18 @@ CASES = [
     Case("ctrl_binary_narrow", "binary", "narrow", (16, 16), (32, 32), ("f32", "f64"), controls=("path-length",)),
     Case("ctrl_zelda_static", "zelda", "narrow", (7, 11), (22, 22), ("f32", "f64"),
          controls=("nearest-enemy", "path-length"), static=True),
-    # the one-thread-per-pixel kernel: forced, and for groups too large for the stage (3D maze's default 30^3 window)
-    Case("scalar_binary16", "binary", "narrow", (16, 16), (32, 32), ALL4, env={"PCGRL_OBSERVE_SCALAR": "1"}),
-    Case("scalar_maze_odd", "minecraft_3D_maze", "narrow", (6, 7, 8), (9, 9, 9), ("u8", "f32", "codes"),
-         env={"PCGRL_OBSERVE_SCALAR": "1"}),
+    # the one-thread-per-pixel kernel for groups too large for the stage (3D maze's default 30^3 window); every case
+    # also runs it through an unaligned output buffer
     Case("oversize_maze15", "minecraft_3D_maze", "narrow", (15, 15, 15), (30, 30, 30), ("u8", "f32", "f64")),
 ]
 # every dispatch target of launch_vec, the 3D / frozen-tile / whole-map / control-plane forms of the staged paths,
-# and the three ways into the scalar kernel
+# and the two ways into the scalar kernel
 REQUIRED_LABELS = {
-    "row32", "row8_bits", "row8_pack3", "row8_pack1", "row8_generic", "row22_11", "row22_22", "row14_7", "row14_14",
+    "row32", "row8_bits", "row8_pack3", "row8_pack1", "row8_generic", "row22_11", "row14_7",
     "row4", "row0", "row8_pack3/3d", "row8_pack1/3d", "row8_generic/3d", "row4/3d", "row0/3d",
     "row8_generic/static", "row4/static", "row0/static", "row8_generic/3d/static", "row4/3d/static",
     "row8_generic/nocrop", "row8_generic/3d/nocrop", "row0/3d/nocrop", "row4/ctrl", "row4/ctrl/nocrop",
-    "row0/ctrl/static", "scalar_env", "scalar_unaligned", "scalar_oversize",
+    "row0/ctrl/static", "scalar_unaligned", "scalar_oversize",
 }
 N_TILES = {"binary": 2, "zelda": 8, "sokoban": 5, "smb": 7, "minecraft_2D_maze": 2, "minecraft_3D_maze": 2}
 
@@ -160,7 +144,7 @@ N_TILES = {"binary": 2, "zelda": 8, "sokoban": 5, "smb": 7, "minecraft_2D_maze":
 def _variant(case, kind, aligned=True):
     crop = case.rep in ("narrow", "turtle")
     return writer_variant(kind, crop, case.shape, case.window, N_TILES[case.problem], len(case.controls or ()),
-                          case.static, case.env, aligned)
+                          case.static, aligned)
 
 
 def case_labels(case):
@@ -273,11 +257,7 @@ def _observe_into_buffer(env, kind, want, aligned, what):
 
 
 @pytest.mark.parametrize("case", CASES, ids=[c.id for c in CASES])
-def test_observe_matches_reference(case, monkeypatch):
-    for v in A_B_VARS:
-        monkeypatch.delenv(v, raising=False)
-    for k, v in dict(case.env).items():
-        monkeypatch.setenv(k, v)
+def test_observe_matches_reference(case):
     sizes, big = _sizes(case, torch.cuda.get_device_properties(0).multi_processor_count)
     for n in sizes + ([big] if big else []):
         env = _make_env(case, n, seed=n)

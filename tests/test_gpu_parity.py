@@ -531,51 +531,11 @@ def test_action_patch_rollout_vs_oracle(problem, shape, aw):
     env.check_status()
 
 
-@pytest.mark.parametrize("problem,rep,shape,obs,kw", [
-    ("binary", "narrow", (16, 16), (32, 32), {}),
-    ("binary", "turtle", (9, 13), (18, 26), {}),
-    ("binary", "wide", (16, 16), (16, 16), {"controls": ["regions", "path-length"]}),
-    ("binary", "narrow", (16, 16), (32, 32), {"controls": ["path-length"]}),
-    ("zelda", "turtle", (7, 11), (22, 22), {}),
-    ("zelda", "narrow", (7, 11), (22, 22), {"static_tile_wrapper": True, "static_prob": 0.5, "n_static_walls": 2}),
-    ("sokoban", "cellular", (5, 5), (5, 5), {}),
-    ("minecraft_3D_maze", "narrow", (14, 14, 14), (14, 14, 14), {}),
-    ("minecraft_3D_maze", "turtle", (6, 7, 8), (12, 14, 16), {}),
-])
-def test_staged_observation_writer_equals_pixel_writer(problem, rep, shape, obs, kw, monkeypatch):
-    """The shared-memory staged writer (128-bit stores) against the one-thread-per-pixel writer it replaced (which
-    the trace replays pinned on the reference's wrapped observations): every dtype, odd env counts (partly filled
-    groups / vector tails), controls, frozen-tile plane, 2D and 3D crops."""
-    for n in (1, 3, 67, 130):
-        env = _mk(problem, rep, shape, n, obs_window=obs, seed=n, **kw)
-        if kw.get("controls"):
-            env.sample_uniform_targets()
-        env.reset()
-        if rep in ("narrow", "turtle"):
-            for i, d in enumerate(shape):
-                env.pos[:, i] = torch.randint(0, d, (n,), device=env.device, dtype=torch.int32)
-        for dt in (torch.uint8, torch.float32, torch.float64):
-            if dt == torch.uint8 and kw.get("controls"):
-                continue
-            monkeypatch.delenv("PCGRL_OBSERVE_SCALAR", raising=False)
-            a = env.observe(dtype=dt).clone()
-            monkeypatch.setenv("PCGRL_OBSERVE_SCALAR", "1")
-            b = env.observe(dtype=dt)
-            monkeypatch.delenv("PCGRL_OBSERVE_SCALAR", raising=False)
-            assert torch.equal(a, b), (problem, rep, n, dt)
-            assert float(a.sum()) > 0
-            # an unaligned output pointer falls back to the pixel writer and still agrees
-            if dt == torch.uint8:
-                buf = torch.empty(a.numel() + 16, dtype=dt, device=env.device)
-                view = buf[1:1 + a.numel()].view(a.shape)
-                assert torch.equal(env.observe(out=view), a)
-
-
 @pytest.mark.parametrize("problem,rep,shape,obs", [("binary", "narrow", (16, 16), (32, 32)),
                                                    ("zelda", "turtle", (7, 11), (22, 22)),
                                                    ("minecraft_3D_maze", "narrow", (6, 7, 8), (12, 14, 16)),
                                                    ("binary", "wide", (16, 16), (16, 16))])
-def test_tile_code_observation_is_the_argmax_of_the_onehot(problem, rep, shape, obs, monkeypatch):
+def test_tile_code_observation_is_the_argmax_of_the_onehot(problem, rep, shape, obs):
     """observe(onehot=False) = Cropped's own output: the channel index of the one-hot record of every pixel."""
     for n in (5, 64):
         env = _mk(problem, rep, shape, n, obs_window=obs, seed=n, action_kind="wide_flat" if rep == "wide" else None)
@@ -588,17 +548,13 @@ def test_tile_code_observation_is_the_argmax_of_the_onehot(problem, rep, shape, 
         assert raw.shape == (*onehot.shape[:-1], 1) and raw.dtype == torch.uint8
         assert torch.equal(raw[..., 0].long(), onehot.argmax(dim=-1))
         assert int(onehot.sum()) == raw[..., 0].numel()
-        monkeypatch.setenv("PCGRL_OBSERVE_SCALAR", "1")
-        assert torch.equal(env.observe(onehot=False), raw)
-        monkeypatch.delenv("PCGRL_OBSERVE_SCALAR", raising=False)
 
 
 @pytest.mark.parametrize("shape,obs", [((16, 16), (32, 32)), ((10, 16), (20, 32)), ((5, 12), (10, 32)), ((16, 9), (32, 32))])
-def test_row_per_thread_observation_writer(shape, obs, monkeypatch):
+def test_row_per_thread_observation_writer(shape, obs):
     """Two-tile crops whose window is exactly 32 wide take the 32-pixels-per-thread path of the staged writer (a whole
     window row from two funnel shifts and eight table lookups): uint8 one-hot and tile codes must equal the float
-    writer's output (which shares none of that code) and the 8-pixel path, for positions all over the map, ragged last
-    trips included."""
+    writer's output (which shares none of that code), for positions all over the map, ragged last trips included."""
     for n in (5, 333, 4099):
         env = _mk("binary", "narrow", shape, n, obs_window=obs, seed=n)
         env.reset()
@@ -611,41 +567,28 @@ def test_row_per_thread_observation_writer(shape, obs, monkeypatch):
         codes = env.observe(onehot=False)
         assert torch.equal(u8.float(), want)
         assert torch.equal(codes[..., 0].long(), want.argmax(dim=-1))
-        monkeypatch.setenv("PCGRL_OBSERVE_NO_ROW32", "1")
-        assert torch.equal(env.observe(dtype=torch.uint8), u8) and torch.equal(env.observe(onehot=False), codes)
-        monkeypatch.delenv("PCGRL_OBSERVE_NO_ROW32", raising=False)
 
 
-def test_zelda_u8_observation_rows_per_thread(monkeypatch):
+def test_zelda_u8_observation_rows_per_thread():
     """zelda's 22-wide window takes 11 pixels (half a window row) per thread in the staged u8 writer; it must equal the
-    float writer and the 4-pixel path, with control planes absent / present and positions all over the map."""
+    float writer, with positions all over the map."""
     for n in (3, 1000):
         env = _mk("zelda", "turtle", (7, 11), n, obs_window=(22, 22), seed=n)
         env.reset()
         for i, d in enumerate((7, 11)):
             env.pos[:, i] = torch.randint(0, d, (n,), device=env.device, dtype=torch.int32)
         want = env.observe(dtype=torch.float32)
-        got = {}
-        for mode in ("11", "22", "0"):
-            monkeypatch.setenv("PCGRL_OBSERVE_ROW22", mode)
-            got[mode] = env.observe(dtype=torch.uint8)
-            assert torch.equal(got[mode].float(), want), mode
-            codes = env.observe(onehot=False)
-            assert torch.equal(codes[..., 0].long(), want.argmax(dim=-1)), mode
-        monkeypatch.delenv("PCGRL_OBSERVE_ROW22", raising=False)
+        assert torch.equal(env.observe(dtype=torch.uint8).float(), want)
+        assert torch.equal(env.observe(onehot=False)[..., 0].long(), want.argmax(dim=-1))
 
 
-def test_maze3d_u8_observation_rows_per_thread(monkeypatch):
-    """The 3D maze's 14-wide last window axis: 14 (or 7) pixels per thread in the staged u8 writer against the float
-    writer and the 4-pixel path."""
+def test_maze3d_u8_observation_rows_per_thread():
+    """The 3D maze's 14-wide last window axis: 7 pixels per thread in the staged u8 writer against the float writer."""
     for n in (3, 700):
         env = _mk("minecraft_3D_maze", "narrow", (14, 14, 14), n, obs_window=(14, 14, 14), seed=n)
         env.reset()
         for i in range(3):
             env.pos[:, i] = torch.randint(0, 14, (n,), device=env.device, dtype=torch.int32)
         want = env.observe(dtype=torch.float32)
-        for mode in ("14", "7", "0"):
-            monkeypatch.setenv("PCGRL_OBSERVE_ROW14", mode)
-            assert torch.equal(env.observe(dtype=torch.uint8).float(), want), mode
-            assert torch.equal(env.observe(onehot=False)[..., 0].long(), want.argmax(dim=-1)), mode
-        monkeypatch.delenv("PCGRL_OBSERVE_ROW14", raising=False)
+        assert torch.equal(env.observe(dtype=torch.uint8).float(), want)
+        assert torch.equal(env.observe(onehot=False)[..., 0].long(), want.argmax(dim=-1))

@@ -151,7 +151,7 @@ def test_random_and_fixed_holes_on_reset():
 @pytest.mark.gpu
 @pytest.mark.parametrize("rep,shape,window", [("narrow", (16, 16), (32, 32)), ("turtle", (9, 12), (18, 24)),
                                               ("wide", (10, 10), (10, 10))])
-def test_holey_observation_matches_oracle(rep, shape, window, monkeypatch):
+def test_holey_observation_matches_oracle(rep, shape, window):
     """HoleyRepresentation.get_observation (envs/reps/wrappers.py:153-174): the bordered map with the two holes,
     positions + 1, through the usual Cropped / OneHot stack whose window is then two cells larger."""
     import torch
@@ -172,13 +172,13 @@ def test_holey_observation_matches_oracle(rep, shape, window, monkeypatch):
         env.pos[:, :2] = torch.from_numpy(pos).to(env.device, torch.int32)
     obs = env.observe(dtype=torch.float64).cpu().numpy()
     codes = env.observe(onehot=False).cpu().numpy()[..., 0]
-    # the staged writer (default) and the pixel-per-thread writer agree, every dtype
+    # the staged writer (default) and the pixel-per-thread writer agree, every dtype: an output view one element past
+    # a 16-byte boundary takes the pixel writer
     for dt in (torch.uint8, torch.float32, torch.float64):
-        a = env.observe(dtype=dt).clone()
-        monkeypatch.setenv("PCGRL_OBSERVE_SCALAR", "1")
-        b2 = env.observe(dtype=dt)
-        monkeypatch.delenv("PCGRL_OBSERVE_SCALAR", raising=False)
-        assert torch.equal(a, b2), (rep, dt)
+        a = env.observe(dtype=dt)
+        view = torch.empty(a.numel() + 1, dtype=dt, device=env.device)[1:].view(a.shape)
+        assert view.data_ptr() % 16 != 0
+        assert torch.equal(env.observe(out=view), a), (rep, dt)
     ow = tuple(d + 2 for d in (window if rep != "wide" else shape))
     assert obs.shape == (n, *ow, 3 if rep != "wide" else 2)
     for e in range(n):
