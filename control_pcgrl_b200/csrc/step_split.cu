@@ -12,9 +12,9 @@
 //       incremental (binary): the one changed cell only touches the components next to it.  From the per-env
 //               cache (passable board, one far tile per non-isolated component, a cell of the component that
 //               attains path-length) the machine floods the affected region U, redoes calc_longest_path's two
-//               sweeps inside U only, and re-sweeps the untouched components only when the one that held the
-//               maximum was touched: 34 instead of 93 board expansions and 2.3 instead of 13.7 component
-//               transitions per changed grid on random 16x16 maps, bit-identical results (helper.py:255-276 is a
+//               sweeps inside U only, and sweeps the untouched components too (in the same final sweep) only when
+//               the one that held the maximum was touched: 32 instead of 93 board expansions per changed grid on
+//               16x16 narrow rollouts (scripts/inc_work_counts.py), bit-identical results (helper.py:255-276 is a
 //               per-component computation; components the edit does not touch keep their first tile, far tile
 //               and eccentricity).  Work per item is uneven (0..135 expansions), so lanes claim items one by one
 //               from their warp's slice of the list instead of running in batches.
@@ -33,7 +33,8 @@ namespace pcgrl {
 
 constexpr int SPLIT_MIN_CTAS = 10;
 constexpr int INC_CTAS_PER_SM = 8;       // 128-thread CTAs of the incremental search resident per SM (A/B 4 / 6 / 8 / 12 at
-                                         // R=3: 0.412 / 0.393 / 0.384 / 0.378 ms per step)
+                                         // R=3: 0.412 / 0.393 / 0.384 / 0.378 ms per step; with the joint final sweep, 6 / 8 / 9:
+                                         // 0.2686 / 0.2697 / 0.2712, profiles/r03_inc_joint_sweep.txt)
 constexpr int INC_CTAS_PER_SM_HOST = 4;  // the same inside the host pipeline: most of the SM's registers stay free, so the
                                          // update / output kernels of the neighbouring chunks run next to the search
                                          // (e2e at 4 chunks, 2 / 3 / 4 / 5 / 8 CTAs per SM: 2.48 / 2.60 / 2.51 / 2.36 / 2.11e9 with the
@@ -41,13 +42,16 @@ constexpr int INC_CTAS_PER_SM_HOST = 4;  // the same inside the host pipeline: m
                                          // 2.56 / 2.75 / 2.71 / 2.42e9, profiles/r02_e2e_cps_chunks_split.txt)
 constexpr int INC_MIN_CLAIM = 12;        // lanes that must be waiting before a warp hands out new items: the claim / init
                                          // stream then runs with that many lanes (A/B 1 / 4 / 8 at R=3: 0.412 / 0.390 / 0.387; at
-                                         // R=12, 8 / 12 / 16 / 24: 0.2978 / 0.2996 / 0.3022 / 0.3263 ms, profiles/r02_ab_inc_claim_window.txt)
+                                         // R=12, 8 / 12 / 16 / 24: 0.2978 / 0.2996 / 0.3022 / 0.3263 ms, profiles/r02_ab_inc_claim_window.txt;
+                                         // with the joint final sweep 8 / 12: 0.2675 / 0.2697 in the split path, k_step_inc not
+                                         // measured at 8, profiles/r03_inc_joint_sweep.txt)
 constexpr int INC_EXPAND_R = 12;         // board expansions per trip.  Every trip also issues each transition stream that
-                                         // some lane needs (flood done / next component / second sweep / re-sweep / finish,
-                                         // ~580 instructions at 2-3 lanes), so few long trips beat many short ones although
+                                         // some lane needs (flood done / next component / final sweep / finish, several
+                                         // hundred instructions at 2-3 lanes), so few long trips beat many short ones although
                                          // lanes idle inside the window: A/B 2 / 3 / 4 / 6 / 8 / 12 -> 0.466 / 0.412 / 0.356 /
                                          // 0.325 / 0.308 / 0.303 ms per step (1 Mi envs, 8 CTAs per SM); 16 / 20 -> 0.3018 / 0.3140
-                                         // against 0.2996 for 12 in a later run
+                                         // against 0.2996 for 12 in a later run; with the joint final sweep 8 / 12 / 16 -> 0.2729 /
+                                         // 0.2697 / 0.2733 (profiles/r03_inc_joint_sweep.txt)
 constexpr int EXPAND_R_SPLIT = 3;        // board expansions per trip of the static search (as in the fused kernel)
 
 constexpr int ACT_THREADS = 256;
@@ -209,26 +213,34 @@ k_split_stats(const KParams p) {
 // calc_num_regions (helper.py:200-210) counts components; calc_longest_path (:255-276) takes, per component in
 // row-major order of its first tile, BFS(first tile) -> far tile (np.argmax: row-major-first maximum) -> BFS(far)
 // and keeps the largest second-sweep maximum.  Both are sums / maxima of per-component terms, and a component the
-// edit does not touch keeps its first tile, far tile and eccentricity.  With D+ the cells that became passable, D-
-// the cells that became solid, P' the new passable board:
+// edit does not touch keeps its first tile, far tile and eccentricity.  With c the edited cell, D+ / D- the cells
+// that became passable / solid (c or nothing), P' the new passable board:
 //   U  = flood fill in P' from D+ and from the passable neighbours of D-   (every new component that is affected)
 //   A  = U | D-                                          (covers every OLD component that is affected, entirely)
 //   regions' = regions - #old components in A + #components of U
 //              (#old in A = far tiles in A + old isolated cells in A: each non-isolated component owns one far tile)
 //   path'    = max(two-sweep maximum inside U, maximum over the untouched components), where the latter is the
-//              old path-length if the cached cell of a maximal component lies outside A, else the joint second
-//              sweep from the remaining far tiles.
-// Validated bit-for-bit against the from-scratch restatement on random rollouts before it was written for the GPU
-// (and on the GPU by tests/test_gpu_split.py: every step of every env equals pcgrl_stats recomputed from scratch).
+//              old path-length if the cached cell of a maximal component lies outside A.  Otherwise ONE sweep from
+//              the far tiles of U and of the untouched components together gives both maxima at once: they are
+//              different components, so a multi-source BFS takes max(lu, lold) levels instead of lu + lold.
+// Isolated cells are counted next to c only: with Q = P' \ {c} and iso(Q) its cells without a neighbour in Q,
+//   c became solid:     old isolated in A = {c} if c has no neighbour in Q,  new isolated in U = N(c) & iso(Q)
+//   c became passable:  old isolated in A = N(c) & iso(Q),  new isolated in U = {c} if c has no neighbour in Q
+// (U is connected from c or from c's neighbours, so a cell of U without a neighbour in P_old or in P' can only have
+// touched the rest of U through c).
+// A Python restatement of this update is pinned by the CPU tests, edit by edit, on the from-scratch computation and on
+// the two sweeps it replaced (same cache rows bit for bit, so the step paths can still share them), and
+// tests/test_gpu_split.py checks every step of every env against pcgrl_stats recomputed from scratch.
 // ------------------------------------------------------------------------------------------------
 template <int NW, bool TWO>
 struct BinaryIncMachine {
+    static_assert(TWO, "the isolated-cell test reads 16-bit rows");
     using B = Board<NW, TWO>;
     static constexpr int SMEM_WORDS = 3 * NW;   // per thread: P' | U (non-isolated part) | far tiles of the rest
     uint32_t avail[NW], front[NW], fars[NW];
     uint32_t* sm;
     const uint32_t* cache;   // this env's cache row (still the OLD state until finish())
-    int phase, level, regions, lu, mcu, mold, lold;
+    int phase, level, regions, path, mcell, cell;   // path / mcell: the cache's path-length and m, old until the end
     bool hit;
 
     static __device__ __forceinline__ int lowest_pos(const uint32_t (&x)[NW]) {
@@ -246,7 +258,8 @@ struct BinaryIncMachine {
         sm = smem;
         cache = c;
         regions = regions_old;
-        lold = path_old;
+        path = path_old;
+        cell = bitpos;
         const uint4* c4 = (const uint4*)c;
         uint32_t pn[NW], d[NW], seed[NW];
         static_assert(NW % 4 == 0 || NW < 4, "cache rows are read as 128-bit vectors");
@@ -260,7 +273,7 @@ struct BinaryIncMachine {
 #pragma unroll
             for (int i = 0; i < NW; ++i) pn[i] = c[i];
         }
-        mold = (int)c[2 * NW];
+        mcell = (int)c[2 * NW];
         const int w = bitpos >> 5;
         const uint32_t bit = 1u << (bitpos & 31);
         uint32_t now_pass = 0;
@@ -281,8 +294,6 @@ struct BinaryIncMachine {
         }
         phase = 0;
         level = 0;
-        lu = 0;
-        mcu = -1;
         hit = false;
     }
     __device__ __forceinline__ bool expand() {
@@ -300,35 +311,58 @@ struct BinaryIncMachine {
     __device__ __forceinline__ bool transition() {
         if (phase == 0) {
             // flood done: U = P' \\ avail.  Account for the old components it swallowed, set up the sweeps inside U.
-            uint32_t pn[NW], po[NW], ones[NW], nb[NW], nbo[NW];
+            int k_old = 0;
 #pragma unroll
             for (int i = 0; i < NW; ++i) {
-                pn[i] = sm[i];
-                po[i] = cache[i];
-                ones[i] = 0xFFFFFFFFu;
-            }
-            B::expand_and(pn, ones, nb);
-            B::expand_and(po, ones, nbo);
-            int k_old = 0, k_iso = 0;
-            uint32_t hitm = 0;
-            const int mw = mold >> 5;
-            const uint32_t mb = mold >= 0 ? 1u << (mold & 31) : 0u;
-#pragma unroll
-            for (int i = 0; i < NW; ++i) {
-                const uint32_t u = pn[i] & ~avail[i];
-                const uint32_t a = u | (po[i] & ~pn[i]);           // U | D-
                 const uint32_t fo = cache[NW + i];
-                k_old += __popc(fo & a) + __popc(po[i] & ~nbo[i] & a);
-                sm[2 * NW + i] = fo & ~a;                          // far tiles of the untouched components
-                if (i == mw) hitm |= a & mb;
-                const uint32_t iso = u & ~nb[i];
-                k_iso += __popc(iso);
-                avail[i] = u & ~iso;
-                sm[NW + i] = avail[i];
+                const uint32_t u = sm[i] & ~avail[i];
+                const uint32_t rest = fo & avail[i];               // avail = P' \ U: far tiles of the untouched components
+                k_old += __popc(fo ^ rest);                        // far tiles in A (fo lies in P_old, P_old \ A = P' \ U)
+                sm[NW + i] = u;
+                sm[2 * NW + i] = rest;
+                avail[i] = u;
                 front[i] = 0;
             }
-            hit = hitm != 0;
-            regions += k_iso - k_old;
+            hit = mcell >= 0 && (mcell == cell || (sm[NW + (mcell >> 5)] >> (mcell & 31)) & 1u);   // m in U | D-
+            // isolated cells next to c.  Rows y-2 .. y+2 of Q = P' \ {c} (c = (y, x) at word w, bit b; a word holds
+            // rows 2w and 2w+1, so row y sits at bit 16 * (y & 1) = b & 16 of word w).
+            const int w = cell >> 5, b = cell & 31, s = b & 16;
+            const uint32_t bit = 1u << b, mx = 1u << (b & 15);
+            const uint32_t pw = sm[w], q = pw & ~bit;
+            const bool grew = pw & bit;
+            const uint32_t qlo = w > 0 ? sm[w - 1] : 0u, qhi = w + 1 < NW ? sm[w + 1] : 0u;
+            const uint32_t r01 = __funnelshift_r(qlo, q, s);       // rows y-2 | y-1 << 16
+            const uint32_t r23 = __funnelshift_r(q, qhi, s);       // rows y   | y+1 << 16
+            const uint32_t r2 = r23 & 0xFFFFu;
+            const uint32_t x13 = (r01 >> 16) | (r23 & 0xFFFF0000u);   // rows y-1 | y+1 << 16
+            const uint32_t v13 = (r01 & 0xFFFFu) | r2 * 0x10001u | ((qhi >> s) << 16);   // their vertical neighbours
+            const uint32_t iso13 = x13 & ~(v13 | ((x13 + x13) & 0xFFFEFFFEu) | ((x13 >> 1) & 0x7FFF7FFFu));
+            const uint32_t iso2 = r2 & ~((x13 | x13 >> 16) | (r2 << 1) | (r2 >> 1));
+            const uint32_t nb13 = mx * 0x10001u, nb2 = (mx << 1) | (mx >> 1);   // c's neighbours in those rows
+            const uint32_t up = iso13 & nb13 & 0xFFFFu, dn = (iso13 & nb13) >> 16, lr = iso2 & nb2;
+            const int n_iso = (up != 0) + (dn != 0) + __popc(lr);
+            const bool alone = !((x13 & nb13) | (r2 & nb2));
+            // the new isolated cells of U leave it: c, or the isolated neighbours of c (rows y-1 | y | y+1 back at
+            // their words w-1, w, w+1)
+            uint32_t cl_lo = 0, cl_mid, cl_hi = 0;
+            if (grew) {
+                cl_mid = alone ? bit : 0u;
+                regions += alone - n_iso;
+            } else {
+                const uint32_t rows = up | (lr << 16);
+                cl_lo = s ? 0u : rows << 16;
+                cl_mid = s ? rows : __funnelshift_l(rows, dn, 16);
+                cl_hi = s ? dn : 0u;
+                regions += n_iso - alone;
+            }
+            regions -= k_old;
+            if (cl_lo | cl_mid | cl_hi) {
+                if (cl_lo) sm[NW + w - 1] &= ~cl_lo;
+                sm[NW + w] &= ~cl_mid;
+                if (cl_hi) sm[NW + w + 1] &= ~cl_hi;
+#pragma unroll
+                for (int i = 0; i < NW; ++i) avail[i] = sm[NW + i];
+            }
             phase = 1;
         }
         if (phase == 1) {   // first sweeps inside U, one component at a time (BinaryMachine phase 0)
@@ -345,52 +379,43 @@ struct BinaryIncMachine {
                 ++regions;
                 return false;
             }
-            phase = 2;      // joint second sweep inside U
+            // final sweep: from the far tiles of U, and when the component that held the maximum was touched, from
+            // those of the untouched components too (isolated cells may stay in avail: the sweep never reaches them)
+            phase = 2;
             uint32_t any = 0;
 #pragma unroll
             for (int i = 0; i < NW; ++i) {
-                front[i] = fars[i];
-                avail[i] = sm[NW + i] & ~fars[i];
-                any |= fars[i];
+                front[i] = fars[i] | (hit ? sm[2 * NW + i] : 0u);
+                avail[i] = sm[i] & ~front[i];
+                any |= front[i];
             }
             level = 0;
             if (any) return false;
         }
-        if (phase == 2) {
-            lu = level;
-            mcu = lowest_pos(front);
-            if (hit) {      // the component that held the maximum was touched: re-sweep the untouched ones
-                uint32_t any = 0;
+        // the final sweep died (or had no sources)
+        if (hit) {      // the maximum over all components; on a tie the untouched ones keep m, as before the edit
+            uint32_t rest[NW];
 #pragma unroll
-                for (int i = 0; i < NW; ++i) {
-                    front[i] = sm[2 * NW + i];
-                    avail[i] = sm[i] & ~sm[NW + i] & ~front[i];   // isolated cells may stay: never reached
-                    any |= front[i];
-                }
-                phase = 3;
-                level = 0;
-                lold = 0;
-                mold = -1;
-                if (any) return false;
-                return true;
-            }
-            return true;
+            for (int i = 0; i < NW; ++i) rest[i] = front[i] & ~sm[NW + i];
+            const int mr = lowest_pos(rest);
+            mcell = mr >= 0 ? mr : lowest_pos(front);
+            path = level;
+        } else if (level > path) {
+            mcell = lowest_pos(front);
+            path = level;
         }
-        // phase 3 died
-        lold = level;
-        mold = lowest_pos(front);
         return true;
     }
     // results + the new cache row
     __device__ __forceinline__ void finish(int* out, uint32_t* c) const {
         out[0] = regions;
-        out[1] = max(lu, lold);
+        out[1] = path;
 #pragma unroll
         for (int i = 0; i < NW; ++i) {
             c[i] = sm[i];
             c[NW + i] = sm[2 * NW + i] | fars[i];
         }
-        c[2 * NW] = (uint32_t)(lu > lold ? mcu : mold);
+        c[2 * NW] = (uint32_t)mcell;
     }
 };
 
