@@ -72,6 +72,8 @@ SYMBOLS = {
     "pcgrl_stats_holey": (C.c_int32, [C.POINTER(Config), C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p,
                                       C.c_void_p]),
     "pcgrl_observe": (C.c_int32, [C.POINTER(Config), C.POINTER(State), C.POINTER(ObsArgs), C.c_void_p]),
+    "pcgrl_observe_envs": (C.c_int32, [C.POINTER(Config), C.POINTER(State), C.POINTER(ObsArgs), C.c_void_p,
+                                       C.c_int64, C.c_void_p]),
     "pcgrl_step_host": (C.c_int32, [C.POINTER(Config), C.POINTER(State), C.c_void_p, C.c_void_p, C.c_int64,
                                     C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
     "pcgrl_step_host_packed": (C.c_int32, [C.POINTER(Config), C.POINTER(State), C.c_void_p, C.c_void_p, C.c_int64,

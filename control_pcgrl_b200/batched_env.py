@@ -670,34 +670,69 @@ class BatchedPcgrlEnv:
         ch += 1 if self.show_agents else 0                  # 'agent_occupancy' plane
         return (*dims, ch)
 
-    def _agent_occupancy(self, agent, dims, dtype):
-        """[N, *dims]: 1 where any agent stands, in agent `agent`'s window (Cropped pads this key with 0)."""
+    def _agent_occupancy(self, agent, dims, dtype, rows=None):
+        """[N, *dims] (rows: [M] env indices -> [M, *dims]): 1 where any agent stands, in agent `agent`'s window
+        (Cropped pads this key with 0)."""
         nd, dev = self.ndim, self.device
-        occ = torch.zeros((self.n_envs, *dims), dtype=dtype, device=dev)
-        center = self.agent_pos[agent, :, :nd].long()
+        sel = slice(None) if rows is None else rows.long()
+        pos = self.agent_pos[:, sel, :nd].long()
+        occ = torch.zeros((pos.shape[1], *dims), dtype=dtype, device=dev)
+        center = pos[agent]
         half = torch.tensor([d // 2 for d in dims], device=dev)
         lim = torch.tensor(list(dims), device=dev)
-        env_idx = torch.arange(self.n_envs, device=dev)
+        env_idx = torch.arange(pos.shape[1], device=dev)
         for b in range(self.n_agents):
-            rel = self.agent_pos[b, :, :nd].long() - center + half
+            rel = pos[b] - center + half
             ok = ((rel >= 0) & (rel < lim)).all(dim=1)
             occ[(env_idx[ok],) + tuple(rel[ok, i] for i in range(nd))] = 1
         return occ
 
-    def observe(self, out: torch.Tensor | None = None, dtype=torch.float32, onehot: bool = True, agent: int = 0):
+    def observe(self, out: torch.Tensor | None = None, dtype=torch.float32, onehot: bool = True, agent: int = 0,
+                env_ids=None):
         """The wrapped observation of every env: [N, *obs_dims, channels] (channels last), exactly what
         CroppedImagePCGRLWrapper / ActionMapImagePCGRLWrapper + ControlWrapper return per env.
         onehot=False (uint8 only, no controls): the tile codes of the crop instead of their one-hot records --
         Cropped's own output (wrappers.py:407-437: 0 = out of bounds, tile t -> t + 1), one channel, for policies
         that embed the tile themselves (SURVEY 8f rank 3).
-        agent: with n_agents > 1, whose crop (every agent sees the shared map around its own position)."""
+        agent: with n_agents > 1, whose crop (every agent sees the shared map around its own position).
+        env_ids: a 1-D integer array / tensor of M env indices (any order, duplicates allowed): returns [M, ...],
+        row j being row env_ids[j] of the full observation (pcgrl_observe_envs); `out` must then be [M, ...].  An index
+        outside [0, N) raises IndexError before anything is launched (a device tensor costs one reduction and one
+        sync for that check)."""
+        rows = None if env_ids is None else self._check_env_ids(env_ids)
+        return self._observe(out, dtype, onehot, agent, rows)
+
+    def _check_env_ids(self, env_ids):
+        """-> int32 device tensor of validated env indices."""
+        if torch.is_tensor(env_ids):
+            t = env_ids
+            if t.dim() != 1 or (t.numel() and (t.dtype.is_floating_point or t.dtype.is_complex or t.dtype == torch.bool)):
+                raise IndexError(f"env_ids must be a 1-D integer index, got {tuple(t.shape)} {t.dtype}")
+            if t.numel():
+                lo, hi = torch.stack(torch.aminmax(t)).tolist()      # host tensors: no device work
+                if lo < 0 or hi >= self.n_envs:
+                    raise IndexError(f"env_ids in [{lo}, {hi}] outside [0, {self.n_envs})")
+            return t.to(device=self.device, dtype=torch.int32).contiguous()
+        a = np.asarray(env_ids)
+        if a.ndim != 1 or (a.size and a.dtype.kind not in "iu"):
+            raise IndexError(f"env_ids must be a 1-D integer index, got shape {a.shape} {a.dtype}")
+        if a.size and (int(a.min()) < 0 or int(a.max()) >= self.n_envs):
+            raise IndexError(f"env_ids in [{int(a.min())}, {int(a.max())}] outside [0, {self.n_envs})")
+        return torch.from_numpy(a.astype(np.int32)).to(self.device)
+
+    def _observe_envs(self, rows, out=None, dtype=torch.float32, onehot: bool = True, agent: int = 0):
+        """observe(env_ids=rows) without the range check, for indices this library produced itself (a nonzero of the
+        done flags, an env the caller just reset)."""
+        return self._observe(out, dtype, onehot, agent, rows.to(device=self.device, dtype=torch.int32).contiguous())
+
+    def _observe(self, out, dtype, onehot, agent, rows):
         if self.ctrl_metrics:
             self._check_fresh("observe with control planes")
         if not onehot:
             if self.ctrl_metrics or (out is not None and out.dtype != torch.uint8):
                 raise ValueError("onehot=False is a uint8 observation without control planes")
             dtype = torch.uint8
-        shape = (self.n_envs, *self.obs_shape(onehot))
+        shape = (self.n_envs if rows is None else rows.numel(), *self.obs_shape(onehot))
         final = None
         if self.show_agents:
             # the kernel writes the map (+ target / static) channels; the occupancy plane is appended here (a handful
@@ -729,10 +764,16 @@ class BatchedPcgrlEnv:
         oa.out_kind = {torch.uint8: 0, torch.float32: 1, torch.float64: 2}[out.dtype] if onehot else 3
         oa.out = out.data_ptr()
         oa.static_channel = 1 if self.static_mask is not None else 0
-        with self._on_device():
-            _lib.check(self.lib.pcgrl_observe(self._cc, self._agent_state(agent), oa, self._stream()), "pcgrl_observe")
+        st = self._agent_state(agent)
+        if rows is None:
+            with self._on_device():
+                _lib.check(self.lib.pcgrl_observe(self._cc, st, oa, self._stream()), "pcgrl_observe")
+        elif rows.numel():
+            with self._on_device():
+                _lib.check(self.lib.pcgrl_observe_envs(self._cc, st, oa, rows.data_ptr(), rows.numel(), self._stream()),
+                           "pcgrl_observe_envs")
         if self.show_agents:
-            occ = self._agent_occupancy(agent, shape[1:-1], out.dtype)
+            occ = self._agent_occupancy(agent, shape[1:-1], out.dtype, rows)
             if final is None:
                 return torch.cat([out, occ[..., None]], dim=-1)
             final[..., :-1] = out
@@ -749,6 +790,7 @@ class BatchedPcgrlEnv:
         (8, RuntimeError, "sokoban: a level with more than 15 crates met the solver preconditions; a packed solver "
                           "state holds 15, so its dist-win / sol-length were not computed"),
         (16, OverflowError, "a stat did not fit the packed result record (record_stat_bytes too small)"),
+        (64, IndexError, "observe: env index out of range (pcgrl_observe_envs loaded nothing through it)"),
     )
 
     def check_status(self):

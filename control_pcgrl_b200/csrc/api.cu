@@ -25,7 +25,8 @@ cudaError_t launch_smb(const KParams& p, cudaStream_t s, bool& supported, int& n
 int64_t sokoban_scratch_bytes();
 int64_t smb_scratch_bytes(int64_t n_envs);
 int64_t maze3d_scratch_bytes();
-cudaError_t launch_observe(const pcgrl_config& cfg, const pcgrl_state& st, const pcgrl_obs_args& o, cudaStream_t s);
+cudaError_t launch_observe(const pcgrl_config& cfg, const pcgrl_state& st, const pcgrl_obs_args& o, cudaStream_t s,
+                           const int32_t* env_idx, int64_t n_idx);
 cudaError_t launch_update(const KParams& p, cudaStream_t s);
 
 // split step path: up to WL_CHUNKS host-pipeline chunks, one 16-int work-list header each at the front of
@@ -485,16 +486,33 @@ int32_t pcgrl_stats_holey(const pcgrl_config* cfg, const int8_t* grids, const in
     return run(p, cfg->problem, stream);
 }
 
-int32_t pcgrl_observe(const pcgrl_config* cfg, const pcgrl_state* st, const pcgrl_obs_args* obs, void* stream) {
+// Shared body of pcgrl_observe / pcgrl_observe_envs (env_idx NULL: every env of the shard).
+static int32_t observe_impl(const pcgrl_config* cfg, const pcgrl_state* st, const pcgrl_obs_args* obs,
+                            const int32_t* env_idx, int64_t n_idx, void* stream) {
     int r = check(cfg);
     if (r) return r;
     if (!st || !st->grids || !st->pos || !obs || !obs->out) return fail(PCGRL_E_ARG, "bad observe arguments");
     if (obs->n_ctrl < 0 || obs->n_ctrl > PCGRL_MAX_STATS) return fail(PCGRL_E_ARG, "n_ctrl out of range");
     if (obs->n_ctrl > 0 && (!st->stats || !st->targets)) return fail(PCGRL_E_ARG, "control channels need stats/targets");
-    cudaError_t e = launch_observe(*cfg, *st, *obs, (cudaStream_t)stream);
+    cudaError_t e = launch_observe(*cfg, *st, *obs, (cudaStream_t)stream, env_idx, n_idx);
     if (e != cudaSuccess) return cuda_fail(e, "observe launch");
     g_launches.fetch_add(1, std::memory_order_relaxed);
     return 0;
+}
+
+int32_t pcgrl_observe(const pcgrl_config* cfg, const pcgrl_state* st, const pcgrl_obs_args* obs, void* stream) {
+    return observe_impl(cfg, st, obs, nullptr, 0, stream);
+}
+
+int32_t pcgrl_observe_envs(const pcgrl_config* cfg, const pcgrl_state* st, const pcgrl_obs_args* obs,
+                           const int32_t* env_idx, int64_t n_idx, void* stream) {
+    if (n_idx < 0) return fail(PCGRL_E_ARG, "n_idx < 0");
+    if (n_idx > 0 && !env_idx) return fail(PCGRL_E_ARG, "env_idx is NULL");
+    int r = check(cfg);
+    if (r) return r;
+    if (!st || !obs) return fail(PCGRL_E_ARG, "bad observe arguments");
+    if (n_idx == 0) return 0;   // nothing to write, nothing launched
+    return observe_impl(cfg, st, obs, env_idx, n_idx, stream);
 }
 
 // Shared body of pcgrl_step_host / pcgrl_step_host_packed: with records_host the only download is the packed

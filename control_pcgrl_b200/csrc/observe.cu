@@ -33,15 +33,43 @@ struct ObsParams {
     void* out;
 };
 
-template <typename T>
-__global__ void __launch_bounds__(256) k_observe(const ObsParams p) {
+// Observation of a list of envs (pcgrl_observe_envs): output row r shows env idx[r] of the shard.  A separate kernel
+// argument after ObsParams / ObsVec, so that the identity instantiations (IDX == false, pcgrl_observe) keep their
+// parameter offsets and code.  With IDX the writers' ObsParams::n_envs is the number of output rows.
+struct ObsIdx {
+    const int32_t* idx;   // [rows] env index of each output row
+    int64_t n_envs;       // envs of the shard: nothing is loaded through an index outside [0, n_envs)
+    int32_t* status;      // pcgrl_state.status or NULL: bit 64 for such an index
+};
+// the env that output row `row` shows, or -1 for an index outside the shard
+template <bool IDX>
+__device__ __forceinline__ int64_t obs_src(const ObsIdx& ix, int64_t row) {
+    if constexpr (!IDX) {
+        return row;
+    } else {
+        const int64_t e = ix.idx[row];
+        return (uint64_t)e < (uint64_t)ix.n_envs ? e : -1;
+    }
+}
+__device__ __forceinline__ void obs_flag_bad_index(const ObsIdx& ix) {
+    if (ix.status) atomicOr(ix.status, 64);
+}
+
+template <typename T, bool IDX>
+__global__ void __launch_bounds__(256) k_observe(const ObsParams p, const ObsIdx ix) {
     const int64_t pix_per_env = (int64_t)p.o0 * p.o1 * p.o2;
     const int64_t total = p.n_envs * pix_per_env;
     const int n_map_ch = p.raw ? 1 : (p.crop ? p.n_tiles + 1 : p.n_tiles);
     const int n_ch = 2 * p.n_ctrl + n_map_ch + (p.static_mask ? 1 : 0);
     for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (int64_t)gridDim.x * blockDim.x) {
-        const int64_t env = i / pix_per_env;
-        int r = (int)(i - env * pix_per_env);
+        const int64_t row = i / pix_per_env;
+        int r = (int)(i - row * pix_per_env);
+        const int64_t env = obs_src<IDX>(ix, row);
+        if (IDX && env < 0) {   // bad index: a zero record, nothing loaded
+            if (r == 0) obs_flag_bad_index(ix);
+            for (int c = 0; c < n_ch; ++c) ((T*)p.out)[i * n_ch + c] = (T)0;
+            continue;
+        }
         const int q2 = r % p.o2;
         r /= p.o2;
         const int q1 = r % p.o1;
@@ -160,8 +188,11 @@ __device__ __forceinline__ uint32_t fdiv(uint32_t n, uint32_t d, uint32_t magic,
 constexpr int OBS_MAX_CTA_ENVS = 64;   // GB * G
 constexpr int OBS_THREADS = 256;
 
-template <typename T, bool CROP, bool STATIC, bool D3, int ROWN /* 0, or 4 / 7 / 8 / 11 / 32: pixels per thread, all in one image row */>
-__global__ void __launch_bounds__(OBS_THREADS) k_observe_staged(const ObsParams p, const ObsVec v) {
+// IDX: rows come from ObsIdx (see there); only the staging loads below differ, the records and the copy-out are the
+// same code over the trip's output rows
+template <typename T, bool CROP, bool STATIC, bool D3, int ROWN /* 0, or 4 / 7 / 8 / 11 / 32: pixels per thread, all in one image row */,
+          bool IDX>
+__global__ void __launch_bounds__(OBS_THREADS) k_observe_staged(const ObsParams p, const ObsVec v, const ObsIdx ix) {
     extern __shared__ __align__(16) uint8_t obs_smem[];
     T* stage = (T*)obs_smem;                                         // [envs of the trip][pix][n_ch]
     T* s_planes = (T*)(obs_smem + v.stage_bytes);                    // [envs of the trip][2 * n_ctrl]
@@ -215,11 +246,21 @@ __global__ void __launch_bounds__(OBS_THREADS) k_observe_staged(const ObsParams 
             for (int i = tid; i < nz; i += OBS_THREADS) ((uint4*)stage)[i] = z;
             const int nv = n_here * (p.row_stride / 16);
             const uint4* g = (const uint4*)(p.grids + env0 * p.row_stride);
+            if constexpr (IDX) {
+                if (ix.status)
+                    for (int i = tid; i < n_here; i += OBS_THREADS)
+                        if (obs_src<IDX>(ix, env0 + i) < 0) obs_flag_bad_index(ix);
+            }
             if (bits) {
                 // one thread per map row: its tiles' low bits as a mask over x
                 for (int i = tid; i < n_here * p.d0; i += OBS_THREADS) {
                     const int el = i / p.d0, y = i - el * p.d0;
-                    const int8_t* row = p.grids + (env0 + el) * p.row_stride + y * p.d1;
+                    const int64_t src = obs_src<IDX>(ix, env0 + el);
+                    if (IDX && src < 0) {   // bad index: an empty map, nothing loaded
+                        s_rowbits[i] = 0;
+                        continue;
+                    }
+                    const int8_t* row = p.grids + src * p.row_stride + y * p.d1;
                     uint32_t m = 0;
                     if (p.d1 == 16) {
                         // one 128-bit load; the low bits of four tiles are gathered into a nibble by one multiply
@@ -234,19 +275,50 @@ __global__ void __launch_bounds__(OBS_THREADS) k_observe_staged(const ObsParams 
                     }
                     s_rowbits[i] = (uint16_t)m;
                 }
+            } else if constexpr (IDX) {
+                // one 128-bit copy per vector of each listed env's row (a bad index stages an empty map)
+                const int vpr = p.row_stride / 16;
+                for (int i = tid; i < nv; i += OBS_THREADS) {
+                    const int el = i / vpr;
+                    const int64_t src = obs_src<IDX>(ix, env0 + el);
+                    ((uint4*)s_grid)[i] = src < 0 ? make_uint4(0, 0, 0, 0)
+                                                  : ((const uint4*)p.grids)[src * vpr + (i - el * vpr)];
+                }
             } else
             for (int i = tid; i < nv; i += OBS_THREADS) ((uint4*)s_grid)[i] = g[i];
             if (p.static_mask) {
+                if constexpr (IDX) {
+                    const int vpr = p.row_stride / 16;
+                    for (int i = tid; i < nv; i += OBS_THREADS) {
+                        const int el = i / vpr;
+                        const int64_t src = obs_src<IDX>(ix, env0 + el);
+                        ((uint4*)s_mask)[i] = src < 0 ? make_uint4(0, 0, 0, 0)
+                                                      : ((const uint4*)p.static_mask)[src * vpr + (i - el * vpr)];
+                    }
+                } else {
                 const uint4* m = (const uint4*)(p.static_mask + env0 * p.row_stride);
                 for (int i = tid; i < nv; i += OBS_THREADS) ((uint4*)s_mask)[i] = m[i];
+                }
             }
-            if (p.crop)
+            if (p.crop) {
+                if constexpr (IDX) {
+                    for (int i = tid; i < n_here * 3; i += OBS_THREADS) {
+                        const int el = i / 3;
+                        const int64_t src = obs_src<IDX>(ix, env0 + el);
+                        ((int32_t*)s_pos)[i] = src < 0 ? 0 : p.pos[src * 3 + (i - el * 3)];
+                    }
+                } else
                 for (int i = tid; i < n_here * 3; i += OBS_THREADS) ((int32_t*)s_pos)[i] = p.pos[env0 * 3 + i];
+            }
         }
         if (p.n_ctrl > 0) {
             for (int i = tid; i < n_here * p.n_ctrl; i += OBS_THREADS) {
                 const int el = i / p.n_ctrl, c = i - el * p.n_ctrl;
-                const int64_t env = env0 + el;
+                const int64_t env = obs_src<IDX>(ix, env0 + el);
+                if (IDX && env < 0) {   // bad index: zero planes
+                    s_planes[el * n_pl + 2 * c] = s_planes[el * n_pl + 2 * c + 1] = (T)0;
+                    continue;
+                }
                 const int k = p.ctrl_idx[c];
                 const double* trg = p.targets + ((p.targets_per_env ? env * p.n_stats : 0) + k) * 2;
                 double t = trg[0];
@@ -415,13 +487,15 @@ __global__ void __launch_bounds__(OBS_THREADS) k_observe_staged(const ObsParams 
                     if (p.holes) {
                         // holey (2D): (s0, s1) address the BORDERED map -- level inside, border tile around it, the
                         // two holes empty (see k_observe)
-                        const int32_t* h = p.holes + (env0 + el) * 4;
+                        const int64_t src = obs_src<IDX>(ix, env0 + el);
+                        const int32_t* h = p.holes + src * 4;
                         int val = -1;
                         if ((unsigned)s0 < (unsigned)(p.d0 + 2) && (unsigned)s1 < (unsigned)(p.d1 + 2)) {
                             if (s0 >= 1 && s0 <= p.d0 && s1 >= 1 && s1 <= p.d1)
                                 val = grid[(s0 - 1) * p.d1 + (s1 - 1)];
-                            else
-                                val = ((s0 == h[0] && s1 == h[1]) || (s0 == h[2] && s1 == h[3])) ? 0 : p.border_tile;
+                            else   // (a bad index: no holes)
+                                val = ((!IDX || src >= 0) &&
+                                       ((s0 == h[0] && s1 == h[1]) || (s0 == h[2] && s1 == h[3]))) ? 0 : p.border_tile;
                         }
                         hot = CROP ? val + 1 : val;
                     } else {
@@ -490,8 +564,8 @@ __global__ void __launch_bounds__(OBS_THREADS) k_observe_staged(const ObsParams 
     if (tid == 0) asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory");   // the stage must outlive its last reader
 }
 
-template <typename T>
-static cudaError_t launch_vec(const ObsParams& p, cudaStream_t s, bool& done) {
+template <typename T, bool IDX>
+static cudaError_t launch_vec(const ObsParams& p, const ObsIdx& ix, cudaStream_t s, bool& done) {
     done = false;
     if ((uintptr_t)p.out % 16) return cudaSuccess;
     const int64_t pix = (int64_t)p.o0 * p.o1 * p.o2;
@@ -527,22 +601,22 @@ static cudaError_t launch_vec(const ObsParams& p, cudaStream_t s, bool& done) {
     const int rown = p.holes ? 0   // the border frame is only handled by the general path
                    : (sizeof(T) == 1 && last_axis % 8 == 0) ? 8 : (last_axis % 4 == 0 ? 4 : 0);
 #define OBS_PICK(RN)                                                                                                     \
-    (cr ? (st ? (d3 ? k_observe_staged<T, true, true, true, RN> : k_observe_staged<T, true, true, false, RN>)            \
-              : (d3 ? k_observe_staged<T, true, false, true, RN> : k_observe_staged<T, true, false, false, RN>))         \
-        : (d3 ? k_observe_staged<T, false, false, true, RN> : k_observe_staged<T, false, false, false, RN>))
-    void (*kern)(const ObsParams, const ObsVec) = rown == 8 ? OBS_PICK(8) : (rown == 4 ? OBS_PICK(4) : OBS_PICK(0));
+    (cr ? (st ? (d3 ? k_observe_staged<T, true, true, true, RN, IDX> : k_observe_staged<T, true, true, false, RN, IDX>)  \
+              : (d3 ? k_observe_staged<T, true, false, true, RN, IDX> : k_observe_staged<T, true, false, false, RN, IDX>)) \
+        : (d3 ? k_observe_staged<T, false, false, true, RN, IDX> : k_observe_staged<T, false, false, false, RN, IDX>))
+    void (*kern)(const ObsParams, const ObsVec, const ObsIdx) = rown == 8 ? OBS_PICK(8) : (rown == 4 ? OBS_PICK(4) : OBS_PICK(0));
 #undef OBS_PICK
     if constexpr (sizeof(T) == 1) {
         // u8 windows 22 wide (zelda 7x11 behind its 22x22 crop: neither a multiple of 8 nor of 4, so it ran the 4-pixel
         // path with carries): half a window row (11 pixels) per thread, 0.2339 ms against 0.3465 ms with 4 and 0.2607 ms
         // with a whole row (profiles/r02_observe_row22.txt)
-        if (rown == 0 && p.o1 == 22 && !d3 && !st && cr && !p.holes) kern = k_observe_staged<T, true, false, false, 11>;
+        if (rown == 0 && p.o1 == 22 && !d3 && !st && cr && !p.holes) kern = k_observe_staged<T, true, false, false, 11, IDX>;
         // ... and the 3D maze's 14-wide last axis (14^3 window of a 14^3 level): 7 pixels per thread, 0.776 ms against
         // 1.6133 ms with 4 and 0.8206 ms with 14 (profiles/r02_observe_row14.txt)
-        if (rown == 0 && d3 && p.o2 == 14 && !st && cr && !p.holes) kern = k_observe_staged<T, true, false, true, 7>;
+        if (rown == 0 && d3 && p.o2 == 14 && !st && cr && !p.holes) kern = k_observe_staged<T, true, false, true, 7, IDX>;
         // row-mask crops whose window is exactly 32 wide (binary 16x16 behind its 32x32 crop): a whole window row per
         // thread, 0.1649 ms against 0.1852 ms with 8 pixels per thread (profiles/r02_observe_row32.jsonl)
-        if (v.bits && rown == 8 && p.o1 == 32 && !d3 && !st && cr) kern = k_observe_staged<T, true, false, false, 32>;
+        if (v.bits && rown == 8 && p.o1 == 32 && !d3 && !st && cr) kern = k_observe_staged<T, true, false, false, 32, IDX>;
     }
     cudaError_t e;
     if (dyn > 48 * 1024 &&
@@ -556,12 +630,38 @@ static cudaError_t launch_vec(const ObsParams& p, cudaStream_t s, bool& done) {
     const int64_t trips = (p.n_envs + v.GB * v.G - 1) / (v.GB * v.G);
     const int64_t cap = (int64_t)n_sm * per_sm;
     const unsigned blocks = (unsigned)(trips < cap ? trips : cap);
-    kern<<<blocks, OBS_THREADS, dyn, s>>>(p, v);
+    kern<<<blocks, OBS_THREADS, dyn, s>>>(p, v, ix);
     done = true;
     return cudaGetLastError();
 }
 
-cudaError_t launch_observe(const pcgrl_config& cfg, const pcgrl_state& st, const pcgrl_obs_args& a, cudaStream_t s) {
+template <bool IDX>
+static cudaError_t launch_writers(const ObsParams& p, const ObsIdx& ix, int out_kind, bool holey3d, int64_t total,
+                                  cudaStream_t s) {
+    // the staged writer knows the 2D border frame only; the bordered 3D map goes through the pixel-per-thread kernel
+    if (!holey3d) {
+        bool done = false;
+        cudaError_t e = (out_kind == 0 || out_kind == 3) ? launch_vec<uint8_t, IDX>(p, ix, s, done)
+                      : out_kind == 1 ? launch_vec<float, IDX>(p, ix, s, done)
+                      : out_kind == 2 ? launch_vec<double, IDX>(p, ix, s, done) : cudaErrorInvalidValue;
+        if (e != cudaSuccess || done) return e;
+    }
+    const int64_t want = (total + 255) / 256;
+    const unsigned blocks = (unsigned)(want < 148 * 32 ? want : 148 * 32);
+    if (out_kind == 0 || out_kind == 3)
+        k_observe<uint8_t, IDX><<<blocks, 256, 0, s>>>(p, ix);
+    else if (out_kind == 1)
+        k_observe<float, IDX><<<blocks, 256, 0, s>>>(p, ix);
+    else if (out_kind == 2)
+        k_observe<double, IDX><<<blocks, 256, 0, s>>>(p, ix);
+    else
+        return cudaErrorInvalidValue;
+    return cudaGetLastError();
+}
+
+// env_idx: NULL observes every env of the shard into row env; else n_idx rows, row j showing env env_idx[j]
+cudaError_t launch_observe(const pcgrl_config& cfg, const pcgrl_state& st, const pcgrl_obs_args& a, cudaStream_t s,
+                           const int32_t* env_idx, int64_t n_idx) {
     ObsParams p;
     p.ndim = cfg.ndim;
     p.d0 = cfg.dims[0];
@@ -581,7 +681,7 @@ cudaError_t launch_observe(const pcgrl_config& cfg, const pcgrl_state& st, const
         p.ctrl_range[i] = a.ctrl_range[i];
     }
     p.targets_per_env = cfg.targets_per_env;
-    p.n_envs = st.n_envs;
+    p.n_envs = env_idx ? n_idx : st.n_envs;   // output rows
     p.grids = st.grids;
     p.pos = st.pos;
     p.stats = st.stats;
@@ -607,27 +707,10 @@ cudaError_t launch_observe(const pcgrl_config& cfg, const pcgrl_state& st, const
     const int grow = holey ? 2 : 0;   // without a crop the whole (bordered) map is observed
     if (!a.crop && (p.o0 != p.d0 + grow || p.o1 != p.d1 + grow || p.o2 != p.d2 + (holey3d ? grow : 0))) return cudaErrorInvalidValue;
     if ((a.out_kind == 0 || a.out_kind == 3) && a.n_ctrl > 0) return cudaErrorInvalidValue;  // target planes are fractional
-    const int64_t total = st.n_envs * (int64_t)p.o0 * p.o1 * p.o2;
+    const int64_t total = p.n_envs * (int64_t)p.o0 * p.o1 * p.o2;
     if (total == 0) return cudaSuccess;
-    // the staged writer knows the 2D border frame only; the bordered 3D map goes through the pixel-per-thread kernel
-    if (!holey3d) {
-        bool done = false;
-        cudaError_t e = (a.out_kind == 0 || a.out_kind == 3) ? launch_vec<uint8_t>(p, s, done)
-                      : a.out_kind == 1 ? launch_vec<float>(p, s, done)
-                      : a.out_kind == 2 ? launch_vec<double>(p, s, done) : cudaErrorInvalidValue;
-        if (e != cudaSuccess || done) return e;
-    }
-    const int64_t want = (total + 255) / 256;
-    const unsigned blocks = (unsigned)(want < 148 * 32 ? want : 148 * 32);
-    if (a.out_kind == 0 || a.out_kind == 3)
-        k_observe<uint8_t><<<blocks, 256, 0, s>>>(p);
-    else if (a.out_kind == 1)
-        k_observe<float><<<blocks, 256, 0, s>>>(p);
-    else if (a.out_kind == 2)
-        k_observe<double><<<blocks, 256, 0, s>>>(p);
-    else
-        return cudaErrorInvalidValue;
-    return cudaGetLastError();
+    return env_idx ? launch_writers<true>(p, ObsIdx{env_idx, st.n_envs, st.status}, a.out_kind, holey3d, total, s)
+                   : launch_writers<false>(p, ObsIdx{nullptr, st.n_envs, nullptr}, a.out_kind, holey3d, total, s);
 }
 
 }  // namespace pcgrl

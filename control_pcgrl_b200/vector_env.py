@@ -96,11 +96,24 @@ class PcgrlVectorEnv:
         # lock-step episodes (no change budget, every env reset together): the episode end is known on the host
         # without a device-to-host sync, and STAYS known afterwards because the reset below is a full one
         lock_step = b.max_changes is None and b._synced_steps is not None
-        any_done = (b._synced_steps > b.max_iterations) if lock_step else bool(done.any())
+        if lock_step:
+            any_done = b._synced_steps > b.max_iterations
+        else:
+            ended = done.nonzero().squeeze(1)        # the step's one host sync
+            any_done = ended.numel() > 0
         if any_done:
             d = done.bool()
+            # the terminal observations, before the targets are redrawn and the envs reset: their target / value
+            # planes show the targets and stats the episodes ended with
+            if lock_step:
+                final_obs = b.observe(dtype=self.obs_dtype, onehot=self.onehot)
+                final_idx = torch.arange(lo, hi, dtype=torch.int64, device=b.device)
+            else:
+                final_obs = b._observe_envs(ended, dtype=self.obs_dtype, onehot=self.onehot)
+                final_idx = ended + lo
             infos.append((lo, {"final_stats": b.stats.clone(), "final_return": ret.clone(),
-                               "final_length": length.clone(), "_final": d}))
+                               "final_length": length.clone(), "_final": d,
+                               "final_obs": final_obs, "final_idx": final_idx}))
             if lock_step:
                 if self.uniform_targets:
                     b.sample_uniform_targets()
@@ -122,8 +135,11 @@ class PcgrlVectorEnv:
         """-> obs, reward, terminated(False), truncated(done), info; finished envs are reset in place and
         their `obs` row is the first observation of the new episode (gymnasium autoreset semantics);
         info carries the final stats of finished episodes (rows where info["_final"] is set; with shards > 1 the
-        rows of ranges that saw no episode end are zero).  reward / done are the env's own output tensors: a
-        reset leaves them alone (include/pcgrl_b200.h, pcgrl_reset), so they need no copies."""
+        rows of ranges that saw no episode end are zero), and their terminal observations as compact rows:
+        info["final_obs"] [M, *obs_shape] is the observation of env info["final_idx"][j] ([M] int64, ascending) after
+        its last step, before its reset -- what a value bootstrap of the truncated episode needs.  reward / done are
+        the env's own output tensors: a reset leaves them alone (include/pcgrl_b200.h, pcgrl_reset), so they need no
+        copies."""
         infos = []
         if len(self.shards) == 1:
             reward, done = self._step_shard(self.env, actions, 0, self.num_envs, infos)
@@ -143,7 +159,11 @@ class PcgrlVectorEnv:
                     "_final": torch.zeros(self.num_envs, dtype=torch.bool, device=self.env.device)}
             for lo, part in infos:
                 for k, v in part.items():
-                    info[k][lo:lo + v.shape[0]] = v
+                    if k not in ("final_obs", "final_idx"):
+                        info[k][lo:lo + v.shape[0]] = v
+            # the ranges' compact rows in range order: final_idx stays ascending
+            info["final_obs"] = torch.cat([part["final_obs"] for _, part in infos])
+            info["final_idx"] = torch.cat([part["final_idx"] for _, part in infos])
         return self._obs, self._reward, torch.zeros_like(self._done), self._done, info
 
 
@@ -236,7 +256,9 @@ def make_rllib_vector_env(cfg, num_envs: int, device="cuda:0", obs_dtype=np.floa
             self.num_envs = num_envs
             self._obs_dev = torch.empty((num_envs, *shp), dtype=tdt, device=b.device)
             self._obs_host = torch.empty((num_envs, *shp), dtype=tdt, pin_memory=True)      # current observations
-            self._new_host = torch.empty((num_envs, *shp), dtype=tdt, pin_memory=True)      # first obs after auto-reset
+            # first observations after the auto-reset of vector_step, compact: row _new_row[i] for env i
+            self._new_host = torch.empty((num_envs, *shp), dtype=tdt, pin_memory=True)
+            self._new_row = np.zeros(num_envs, dtype=np.int64)
             self._fresh = np.zeros(num_envs, dtype=bool)    # envs reset inside the last vector_step, not yet handed out
             self._views = [_SubEnvView(self, i) for i in range(num_envs)]
 
@@ -245,6 +267,14 @@ def make_rllib_vector_env(cfg, num_envs: int, device="cuda:0", obs_dtype=np.floa
             host.copy_(self._obs_dev, non_blocking=True)
             torch.cuda.current_stream(self.env.device).synchronize()
             return host.numpy()
+
+        def _observe_rows_into(self, ids, host):
+            """Observe the envs `ids` only (numpy int array) into host[:len(ids)]: M rows written, M rows copied."""
+            m = len(ids)
+            rows = torch.from_numpy(np.ascontiguousarray(ids, dtype=np.int32)).to(self.env.device)
+            self.env._observe_envs(rows, out=self._obs_dev[:m])
+            host[:m].copy_(self._obs_dev[:m], non_blocking=True)
+            torch.cuda.current_stream(self.env.device).synchronize()
 
         def vector_reset(self, *, seeds=None, options=None):
             b = self.env
@@ -261,12 +291,13 @@ def make_rllib_vector_env(cfg, num_envs: int, device="cuda:0", obs_dtype=np.floa
             i = 0 if index is None else int(index)
             if self._fresh[i]:                     # already reset (with every other finished env) by vector_step
                 self._fresh[i] = False
-                self._obs_host[i].copy_(self._new_host[i])
+                self._obs_host[i].copy_(self._new_host[self._new_row[i]])
                 return self._obs_host.numpy()[i], {}
             mask = torch.zeros(self.num_envs, dtype=torch.uint8, device=self.env.device)
             mask[i] = 1
             self.env.reset(mask=mask)
-            return self._observe_into(self._obs_host)[i], {}
+            self._observe_rows_into(np.array([i]), self._obs_host[i:i + 1])
+            return self._obs_host.numpy()[i], {}
 
         def restart_at(self, index=None):
             self.reset_at(index)
@@ -285,8 +316,10 @@ def make_rllib_vector_env(cfg, num_envs: int, device="cuda:0", obs_dtype=np.floa
                 # RLlib calls reset_at(i) for every finished env next: reset them all in ONE launch now and keep
                 # their first observations ready (the terminal observations above are already on the host)
                 self._fresh[:] = d.astype(bool)
+                ids = np.flatnonzero(self._fresh)
+                self._new_row[ids] = np.arange(len(ids))
                 b.reset(mask=b.done)
-                self._observe_into(self._new_host)
+                self._observe_rows_into(ids, self._new_host)
             return [obs[i] for i in range(self.num_envs)], rewards, [False] * self.num_envs, dones, infos
 
         def get_sub_environments(self):

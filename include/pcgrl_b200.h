@@ -143,7 +143,8 @@ typedef struct pcgrl_state {
                               bit1 (2) minecraft_3D_maze: the reference would raise IndexError on this map
                               (helper_3D.py:531, a recorded x or y >= depth); bit2 (4) a search workspace
                               overflowed; bit3 (8) sokoban: more crates than a packed solver state holds (15);
-                              bit4 (16) a stat did not fit cfg.record_stat_bytes in the packed record */
+                              bit4 (16) a stat did not fit cfg.record_stat_bytes in the packed record; bit5 (32)
+                              is retired; bit6 (64) pcgrl_observe_envs: an env index outside [0, n_envs) */
     void*    scratch;      /* pcgrl_scratch_bytes() bytes, may be NULL when that returns 0.  Must be zero-filled
                               once before its first use (it holds hash-table generation counters, solver job
                               lists and, for smb, 4 bytes per env of playthrough-length history, which is why
@@ -264,6 +265,15 @@ typedef struct pcgrl_obs_args {
                                  the map dims + 2 (no crop), :162-174 */
 } pcgrl_obs_args;
 int32_t pcgrl_observe(const pcgrl_config* cfg, const pcgrl_state* st, const pcgrl_obs_args* obs, void* stream);
+
+/* The observation of a list of envs of the shard, as compact rows: env_idx is a DEVICE array of n_idx int32 env
+ * indices, and row j of obs->out ([n_idx, *obs_dims, channels]) is byte for byte what pcgrl_observe writes into row
+ * env_idx[j].  Any order, duplicates allowed; n_idx == 0 launches nothing.  Every option of pcgrl_observe applies
+ * (targets / stats / holes / static mask / pos of env env_idx[j]).  Nothing is loaded through an index outside
+ * [0, st->n_envs): such a row's contents are unspecified and status bit 64 is set (when st->status is set).
+ * For a trainer's terminal observations of finished episodes, or the fresh rows after a masked reset. */
+int32_t pcgrl_observe_envs(const pcgrl_config* cfg, const pcgrl_state* st, const pcgrl_obs_args* obs,
+                           const int32_t* env_idx, int64_t n_idx, void* stream);
 
 /* -- host-buffer convenience (the end-to-end path timed as `e2e` in bench.py) ------------------ */
 /* Copies `actions` (host, pinned or pageable) to `actions_dev`, runs pcgrl_step, copies reward/done/stats
