@@ -82,6 +82,9 @@ SYMBOLS = {
     "pcgrl_worklist_ints": (C.c_int64, [C.POINTER(Config), C.c_int64]),
     "pcgrl_cache_stride": (C.c_int32, [C.POINTER(Config)]),
     "pcgrl_launch_count": (C.c_int64, []),
+    "pcgrl_lookahead_work_bytes": (C.c_int64, [C.POINTER(Config), C.c_int64]),
+    "pcgrl_lookahead": (C.c_int32, [C.POINTER(Config), C.POINTER(State), C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p,
+                                    C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
 }
 
 _lib = None

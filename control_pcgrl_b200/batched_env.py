@@ -473,6 +473,79 @@ class BatchedPcgrlEnv:
         self._stats_stale = True
         return self.changed
 
+    # ------------------------------------------------------------------ lookahead
+    def lookahead(self, actions: torch.Tensor, env_ids=None, agent: int = 0):
+        """What step() would return for a list of (env, action) candidates, without stepping.  Candidate j pairs env
+        env_ids[j] (j when env_ids is None) with row j of `actions` (the step layout with M rows, M = len(env_ids) or
+        n_envs).  Returns fresh device tensors (reward[M] f32, done[M] u8, stats[M, K] i32, changed[M] u8): the
+        reward (bit for bit), done, stats row and changed flag that env would get from step() if it took that action
+        next.  Indices may come in any order and repeat.  agent: with n_agents > 1, whose turtle would act.
+        Nothing of the env changes, except that check_status() then reports what such a step would (an invalid
+        action: ValueError); no auto-reset.  A bad env index raises IndexError before anything is launched (a device
+        tensor costs one reduction and one sync for that check)."""
+        self._check_fresh("lookahead")
+        rows = None if env_ids is None else self._check_env_ids(env_ids)
+        m = self.n_envs if rows is None else rows.numel()
+        a = self._check_actions(actions, m)
+        K = self.K
+        out = (torch.empty(m, dtype=torch.float32, device=self.device), torch.empty(m, dtype=torch.uint8, device=self.device),
+               torch.empty((m, K), dtype=torch.int32, device=self.device), torch.empty(m, dtype=torch.uint8, device=self.device))
+        self._lookahead(a, rows, m, agent, *out)
+        return out
+
+    def _lookahead(self, a, rows, m, agent, reward, done, stats, changed):
+        if m == 0:
+            return
+        need = int(self.lib.pcgrl_lookahead_work_bytes(self._cc, m))
+        if self._la_work is None or self._la_work.numel() < need:
+            # zero-filled when allocated: the solver kernels keep generation counters in it
+            self._la_work = None
+            self._la_work = torch.zeros(need, dtype=torch.uint8, device=self.device)
+        with self._on_device():
+            _lib.check(self.lib.pcgrl_lookahead(self._cc, self._agent_state(agent), a.data_ptr(), _ptr(rows), m,
+                                                reward.data_ptr(), done.data_ptr(), changed.data_ptr(), stats.data_ptr(),
+                                                self._la_work.data_ptr(), self._stream()), "pcgrl_lookahead")
+
+    _la_work = None
+    LOOKAHEAD_CHUNK = 1 << 22     # candidates per launch of lookahead_all: bounds the work buffer
+
+    def n_discrete_actions(self):
+        """Size of the Discrete action space (narrow C, turtle 4 + C, flat wide act_h * act_w * C)."""
+        if self.action_kind not in ("int32", "wide_flat"):
+            raise ValueError(f"action_kind {self.action_kind!r} is not a Discrete action space")
+        return {"narrow": self.n_tiles, "turtle": 4 + self.n_tiles}.get(
+            self.representation, self._cc.act_h * self._cc.act_w * self.n_tiles)
+
+    def lookahead_all(self, env_ids=None, agent: int = 0):
+        """lookahead() of every action of the Discrete action space for each env of env_ids (default all): returns
+        reward [M, A] f32, done [M, A] u8, stats [M, A, K] i32 and changed [M, A] u8, column a being action a.
+        Runs in chunks of at most LOOKAHEAD_CHUNK candidates, env-major, without a host sync (env_ids=None).
+        Raises ValueError for cellular, patch and wide-coordinate actions, and for flat wide actions whose ActionMap
+        (act_h, act_w) reaches past the map: part of that space is actions the reference rejects."""
+        self._check_fresh("lookahead_all")
+        A = self.n_discrete_actions()
+        if self.action_kind == "wide_flat":
+            # action (y, x, v): the write goes to _map[x, y], so x must be a row and y a column (wrappers.py:304-323)
+            if self._cc.act_w > self.map_shape[0] or self._cc.act_h > self.map_shape[1]:
+                raise ValueError(f"ActionMap ({self._cc.act_h}, {self._cc.act_w}) reaches past the map {self.map_shape}")
+        rows = None if env_ids is None else self._check_env_ids(env_ids)
+        M = self.n_envs if rows is None else rows.numel()
+        dev, K = self.device, self.K
+        reward = torch.empty((M, A), dtype=torch.float32, device=dev)
+        done = torch.empty((M, A), dtype=torch.uint8, device=dev)
+        stats = torch.empty((M, A, K), dtype=torch.int32, device=dev)
+        changed = torch.empty((M, A), dtype=torch.uint8, device=dev)
+        _, _, tdt = self._action_layout()
+        per = max(1, self.LOOKAHEAD_CHUNK // A)
+        for lo in range(0, M, per):
+            hi = min(M, lo + per)
+            c = torch.arange((hi - lo) * A, dtype=torch.int32, device=dev)
+            env = c // A + lo if rows is None else rows[lo:hi].repeat_interleave(A, output_size=(hi - lo) * A)
+            acts = (c % A).to(tdt)
+            self._lookahead(acts, env.to(torch.int32).contiguous(), (hi - lo) * A, agent, reward[lo:hi], done[lo:hi],
+                            stats[lo:hi], changed[lo:hi])
+        return reward, done, stats, changed
+
     def _check_fresh(self, what):
         if self._stats_stale:
             raise RuntimeError(f"{what}: update() edited the maps without recomputing stats, so stats (and the step's "
@@ -520,9 +593,9 @@ class BatchedPcgrlEnv:
         else:
             self.reset(mask=self.done)
 
-    def _action_layout(self):
-        """(shape, numpy dtype, torch dtype) of one action batch for this env's action_kind."""
-        N = self.n_envs
+    def _action_layout(self, n=None):
+        """(shape, numpy dtype, torch dtype) of one action batch (n rows, default n_envs) for this env's action_kind."""
+        N = self.n_envs if n is None else n
         scalar = {4: (np.int32, torch.int32), 1: (np.uint8, torch.uint8), 2: (np.uint16, torch.uint16)}[self._act_elem]
         return {"int32": ((N,), *scalar), "wide_flat": ((N,), *scalar),
                 "wide_coords": ((N, self.ndim + 1), np.int32, torch.int32),
@@ -530,10 +603,10 @@ class BatchedPcgrlEnv:
                 "ca_logits": ((N, self.n_tiles * self.cells), np.float32, torch.float32),
                 "patch": ((N, int(np.prod(self.act_window or (1,)))), np.int32, torch.int32)}[self.action_kind]
 
-    def _check_actions(self, actions):
+    def _check_actions(self, actions, n=None):
         if not torch.is_tensor(actions) or actions.device != self.device:
             raise TypeError("actions must be a tensor on the env's device (use step_host for host arrays)")
-        shape, _, tdt = self._action_layout()
+        shape, _, tdt = self._action_layout(n)
         if actions.dtype != tdt:
             raise TypeError(f"actions dtype {actions.dtype} != {tdt} for action_kind {self.action_kind}")
         if actions.numel() != int(np.prod(shape)):
@@ -791,6 +864,7 @@ class BatchedPcgrlEnv:
                           "state holds 15, so its dist-win / sol-length were not computed"),
         (16, OverflowError, "a stat did not fit the packed result record (record_stat_bytes too small)"),
         (64, IndexError, "observe: env index out of range (pcgrl_observe_envs loaded nothing through it)"),
+        (128, IndexError, "lookahead: env index out of range (pcgrl_lookahead loaded nothing through it)"),
     )
 
     def check_status(self):

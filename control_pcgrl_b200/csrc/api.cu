@@ -28,6 +28,9 @@ int64_t maze3d_scratch_bytes();
 cudaError_t launch_observe(const pcgrl_config& cfg, const pcgrl_state& st, const pcgrl_obs_args& o, cudaStream_t s,
                            const int32_t* env_idx, int64_t n_idx);
 cudaError_t launch_update(const KParams& p, cudaStream_t s);
+cudaError_t launch_lookahead_inc(const KParams& p, const LaOut& o, cudaStream_t s);
+cudaError_t launch_lookahead_gather(const pcgrl_state& src, const pcgrl_state& dst, const int32_t* env_idx,
+                                    int row_stride, int K, int hole_ints, bool targets_per_env, cudaStream_t s);
 
 // split step path: up to WL_CHUNKS host-pipeline chunks, one 16-int work-list header each at the front of
 // pcgrl_state.worklist
@@ -335,6 +338,36 @@ static int host_chunks(const pcgrl_config* cfg, int64_t n, bool packed) {
     if (n < (1 << 19)) return 2;
     return 4;
 }
+// Layout of the lookahead's work buffer for n candidates.  The first 256 bytes hold the work-list header of the
+// incremental path (only that path touches them).  Behind them, either the incremental path's work-list body or the
+// generic path's solver scratch (at a fixed offset: it keeps generation counters from call to call) and the sub-shard.
+struct LaLayout {
+    int64_t inc_body, scratch, grids, mask, pos, n_step, iteration, changes, targets, holes, total;
+};
+static int64_t la_align(int64_t x) { return (x + 255) / 256 * 256; }
+static LaLayout la_layout(const pcgrl_config* c, int64_t n) {
+    LaLayout l;
+    const int64_t K = c->n_stats;
+    l.inc_body = 256;
+    const int64_t inc_end = cache_stride(c) > 0 ? l.inc_body + la_align((2 + K + 1) * 4 * n) : 0;
+    l.scratch = 256;
+    int64_t off = l.scratch + la_align(pcgrl_scratch_bytes(c, n));
+    auto take = [&](int64_t bytes) {
+        const int64_t at = off;
+        off += la_align(bytes);
+        return at;
+    };
+    l.grids = take(n * c->row_stride);
+    l.mask = take(n * c->row_stride);
+    l.pos = take(n * 12);
+    l.n_step = take(n * 4);
+    l.iteration = take(n * 4);
+    l.changes = take(n * 4);
+    l.targets = take(c->targets_per_env ? n * K * 16 : 0);
+    l.holes = take(is_holey(c) ? n * hole_ints(c) * 4 : 0);
+    l.total = std::max(off, inc_end);
+    return l;
+}
 }  // namespace pcgrl
 
 using namespace pcgrl;
@@ -513,6 +546,67 @@ int32_t pcgrl_observe_envs(const pcgrl_config* cfg, const pcgrl_state* st, const
     if (!st || !obs) return fail(PCGRL_E_ARG, "bad observe arguments");
     if (n_idx == 0) return 0;   // nothing to write, nothing launched
     return observe_impl(cfg, st, obs, env_idx, n_idx, stream);
+}
+
+int64_t pcgrl_lookahead_work_bytes(const pcgrl_config* cfg, int64_t n) {
+    if (check(cfg) || n < 0) return -1;
+    return la_layout(cfg, n).total;
+}
+
+int32_t pcgrl_lookahead(const pcgrl_config* cfg, const pcgrl_state* st, const void* actions, const int32_t* env_idx,
+                        int64_t n, float* reward, uint8_t* done, uint8_t* changed, int32_t* stats, void* work,
+                        void* stream) {
+    int r = check(cfg);
+    if (r) return r;
+    if ((r = check_state(st))) return r;
+    if (n < 0 || n > INT32_MAX) return fail(PCGRL_E_ARG, "n must be in [0, 2^31)");
+    if (!env_idx && n > st->n_envs) return fail(PCGRL_E_ARG, "without env_idx candidate j is env j: n > n_envs");
+    if (n > 0 && (!actions || !reward || !done || !changed || !stats || !work))
+        return fail(PCGRL_E_ARG, "actions, reward, done, changed, stats and work must not be NULL");
+    if (is_holey(cfg) && !st->holes) return fail(PCGRL_E_ARG, "a holey problem needs pcgrl_state.holes");
+    if (n == 0) return 0;   // nothing to write, nothing launched
+    KParams p;
+    fill(p, cfg, st);
+    uint8_t* w = (uint8_t*)work;
+    const cudaStream_t s = (cudaStream_t)stream;
+    cudaError_t e;
+    if (p.cache) {   // the shard keeps a search cache: incremental searches from it
+        LaOut o{env_idx, st->n_envs, reward, done, changed, stats};
+        p.mode = MODE_STEP;
+        p.actions = actions;
+        p.n_envs = n;
+        p.records = nullptr;
+        p.wl_hdr = (int32_t*)w;
+        p.worklist = (int32_t*)(w + la_layout(cfg, 0).inc_body);
+        if ((e = launch_lookahead_inc(p, o, s)) != cudaSuccess) return cuda_fail(e, "lookahead launch");
+        g_launches.fetch_add(3, std::memory_order_relaxed);
+        return 0;
+    }
+    // every other config: the candidates' rows as a sub-shard of n envs, then the ordinary step on it
+    const LaLayout l = la_layout(cfg, n);
+    pcgrl_state sub;
+    std::memset(&sub, 0, sizeof(sub));
+    sub.n_envs = n;
+    sub.env_offset = st->env_offset;
+    sub.grids = (int8_t*)(w + l.grids);
+    sub.static_mask = st->static_mask ? w + l.mask : nullptr;
+    sub.pos = (int32_t*)(w + l.pos);
+    sub.n_step = (int32_t*)(w + l.n_step);
+    sub.iteration = (int32_t*)(w + l.iteration);
+    sub.changes = (int32_t*)(w + l.changes);
+    sub.stats = stats;
+    sub.targets = cfg->targets_per_env ? (const double*)(w + l.targets) : st->targets;
+    sub.holes = st->holes && is_holey(cfg) ? (int32_t*)(w + l.holes) : nullptr;
+    sub.reward = reward;
+    sub.done = done;
+    sub.changed = changed;
+    sub.status = st->status;
+    sub.scratch = pcgrl_scratch_bytes(cfg, n) > 0 ? w + l.scratch : nullptr;
+    if ((e = launch_lookahead_gather(*st, sub, env_idx, cfg->row_stride, cfg->n_stats, hole_ints(cfg),
+                                     cfg->targets_per_env != 0, s)) != cudaSuccess)
+        return cuda_fail(e, "lookahead gather launch");
+    g_launches.fetch_add(1, std::memory_order_relaxed);
+    return step_launch(cfg, &sub, actions, stream, nullptr, 0, 0);
 }
 
 // Shared body of pcgrl_step_host / pcgrl_step_host_packed: with records_host the only download is the packed

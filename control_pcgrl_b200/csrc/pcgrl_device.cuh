@@ -59,6 +59,16 @@ struct KParams {
     int32_t host_chunk;           // 1: this launch is one chunk of the host pipeline (other chunks run beside it)
 };
 
+// Outputs of one incremental lookahead (lookahead.cu); the KParams beside it have n_envs = the candidate count.
+struct LaOut {
+    const int32_t* env_idx;   // NULL: candidate j is env j
+    int64_t n_src;            // envs of the shard
+    float* reward;
+    uint8_t* done;
+    uint8_t* changed;
+    int32_t* stats;
+};
+
 // one scalar action (narrow / turtle / flat wide) in the width the caller chose (cfg.action_elem_bytes)
 __device__ __forceinline__ int load_action(const KParams& p, int64_t gid) {
     if (p.act_bytes == 1) return ((const uint8_t*)p.actions)[gid];

@@ -12,6 +12,96 @@ __device__ __forceinline__ int cell_index(const KParams& p, int a0, int a1, int 
     return (a0 * p.d1 + a1) * p.d2 + a2;
 }
 
+// One action that addresses a single cell (narrow / turtle / wide: not patch, not cellular), element `ai` of
+// p.actions, on env `gid`.  APPLY: the representation update -- grid, pos and n_step in HBM.  !APPLY (the lookahead,
+// lookahead.cu): the same decode against the env's grid, position and frozen mask, writing nothing (but status).
+// Returns bit0 = change, bit1 = the grid is (or would be) modified, as apply_action; *cell_out as there.
+template <bool APPLY>
+__device__ __forceinline__ int one_cell_action(const KParams& p, int64_t ai, int64_t gid, int* cell_out) {
+    int8_t* grid = p.grids + gid * p.row_stride;
+    int32_t* pos = p.pos + gid * 3;
+    const uint8_t* frozen = p.static_mask ? p.static_mask + gid * p.row_stride : nullptr;
+    int change = 0, wrote = 0;
+    if (p.rep == PCGRL_REP_NARROW) {
+        // reps/narrow_rep.py:89-102: write at _pos, then _pos = coords[n_step % N], then n_step += 1
+        const int a = load_action(p, ai);
+        const int c = cell_index(p, pos[0], pos[1], pos[2]);
+        if (cell_out) *cell_out = c;
+        if ((unsigned)a >= (unsigned)p.n_tiles) {
+            if (p.status) atomicOr(p.status, 1);
+        } else {
+            const int old = grid[c];
+            change = old != a;
+            wrote = change && !(frozen && frozen[c]);
+            if (APPLY && wrote) grid[c] = (int8_t)a;
+        }
+        if constexpr (APPLY) {
+            const int ns = p.n_step[gid];
+            const int k = ns % p.cells;
+            pos[2] = k % p.d2;
+            pos[1] = (k / p.d2) % p.d1;
+            pos[0] = k / (p.d2 * p.d1);
+            p.n_step[gid] = ns + 1;
+        }
+    } else if (p.rep == PCGRL_REP_TURTLE) {
+        // reps/turtle_rep.py:87-107: 0..3 move along axis 0 / axis 1 (clamped), >= 4 writes tile a-4
+        const int a = load_action(p, ai);
+        if (a >= 0 && a < 4) {
+            if constexpr (APPLY) {
+                const int axis = a >> 1;
+                const int lim = (axis == 0 ? p.d0 : p.d1) - 1;
+                int v = pos[axis] + ((a & 1) ? 1 : -1);
+                pos[axis] = v < 0 ? 0 : (v > lim ? lim : v);
+            }
+        } else if (a >= 4 && a - 4 < p.n_tiles) {
+            const int c = cell_index(p, pos[0], pos[1], pos[2]);
+            if (cell_out) *cell_out = c;
+            const int t = a - 4;
+            const int old = grid[c];
+            change = old != t;
+            wrote = change && !(frozen && frozen[c]);
+            if (APPLY && wrote) grid[c] = (int8_t)t;
+        } else if (p.status) {
+            atomicOr(p.status, 1);
+        }
+    } else {  // PCGRL_REP_WIDE
+        int q0, q1, q2 = 0, v;
+        if (p.action_kind == PCGRL_ACT_WIDE_FLAT) {
+            // wrappers.py:304-323: (y, x, v) = unravel(a, (h, w, C)); env.step([x, y, v]) -> _map[x, y] = v
+            const int a = load_action(p, ai);
+            v = a % p.n_tiles;
+            const int x = (a / p.n_tiles) % p.act_w;
+            const int y = a / (p.n_tiles * p.act_w);
+            q0 = x;
+            q1 = y;
+            if (a < 0 || y >= p.act_h) q0 = -1;
+        } else {
+            const int32_t* a = (const int32_t*)p.actions + ai * (p.ndim + 1);
+            q0 = a[0];
+            q1 = a[1];
+            if (p.ndim == 3) q2 = a[2];
+            v = a[p.ndim];
+        }
+        if ((unsigned)q0 >= (unsigned)p.d0 || (unsigned)q1 >= (unsigned)p.d1 || (unsigned)q2 >= (unsigned)p.d2 ||
+            (unsigned)v >= (unsigned)p.n_tiles) {
+            if (p.status) atomicOr(p.status, 1);
+        } else {
+            const int c = cell_index(p, q0, q1, q2);
+            if (cell_out) *cell_out = c;
+            const int old = grid[c];
+            change = old != v;
+            wrote = change;   // the reference's wide / cellular reps do not run under StaticTileRepresentation
+            if constexpr (APPLY) {
+                if (change) grid[c] = (int8_t)v;
+                pos[0] = q0;
+                pos[1] = q1;
+                pos[2] = q2;
+            }
+        }
+    }
+    return change | (wrote << 1);
+}
+
 // Apply one non-cellular action to env `gid`; updates pos / n_step in HBM.
 // Returns bit0 = change (what PcgrlEnv counts in _changes), bit1 = the grid was actually modified.  The two
 // differ only under StaticTileRepresentation (envs/reps/wrappers.py:358-376): an edit of a frozen cell is
@@ -19,12 +109,12 @@ __device__ __forceinline__ int cell_index(const KParams& p, int a0, int a1, int 
 // against the pre-undo array, so it still counts as a change (and the reference recomputes identical stats).
 // *cell_out (optional): linear index of the one cell the action addressed, -1 for multi-cell actions (patch).
 __device__ __forceinline__ int apply_action(const KParams& p, int64_t gid, int* cell_out = nullptr) {
-    int8_t* grid = p.grids + gid * p.row_stride;
-    int32_t* pos = p.pos + gid * 3;
-    const uint8_t* frozen = p.static_mask ? p.static_mask + gid * p.row_stride : nullptr;
-    int change = 0, wrote = 0;
     if (cell_out) *cell_out = -1;
     if (p.rep == PCGRL_REP_NARROW && p.action_kind == PCGRL_ACT_PATCH) {
+        int8_t* grid = p.grids + gid * p.row_stride;
+        int32_t* pos = p.pos + gid * 3;
+        const uint8_t* frozen = p.static_mask ? p.static_mask + gid * p.row_stride : nullptr;
+        int change = 0, wrote = 0;
         // MultiActionRepresentation.update (envs/reps/wrappers.py:466-528): the patch action.reshape(act_window)
         // replaces map[pos - l_pad : pos + r_pad + 1], l_pad = floor((a-1)/2), r_pad = ceil((a-1)/2) (:404-411);
         // change = any cell differs; then pos = act_coords[n_step % len], n_step += 1 (:517-518)
@@ -63,78 +153,9 @@ __device__ __forceinline__ int apply_action(const KParams& p, int64_t gid, int* 
         pos[0] = l0 + (k / n1) % n0;
         pos[2] = l2 + k / (n1 * n0);
         p.n_step[gid] = ns + 1;
-    } else if (p.rep == PCGRL_REP_NARROW) {
-        // reps/narrow_rep.py:89-102: write at _pos, then _pos = coords[n_step % N], then n_step += 1
-        const int a = load_action(p, gid);
-        const int c = cell_index(p, pos[0], pos[1], pos[2]);
-        if (cell_out) *cell_out = c;
-        if ((unsigned)a >= (unsigned)p.n_tiles) {
-            if (p.status) atomicOr(p.status, 1);
-        } else {
-            const int old = grid[c];
-            change = old != a;
-            wrote = change && !(frozen && frozen[c]);
-            if (wrote) grid[c] = (int8_t)a;
-        }
-        const int ns = p.n_step[gid];
-        const int k = ns % p.cells;
-        pos[2] = k % p.d2;
-        pos[1] = (k / p.d2) % p.d1;
-        pos[0] = k / (p.d2 * p.d1);
-        p.n_step[gid] = ns + 1;
-    } else if (p.rep == PCGRL_REP_TURTLE) {
-        // reps/turtle_rep.py:87-107: 0..3 move along axis 0 / axis 1 (clamped), >= 4 writes tile a-4
-        const int a = load_action(p, gid);
-        if (a >= 0 && a < 4) {
-            const int axis = a >> 1;
-            const int lim = (axis == 0 ? p.d0 : p.d1) - 1;
-            int v = pos[axis] + ((a & 1) ? 1 : -1);
-            pos[axis] = v < 0 ? 0 : (v > lim ? lim : v);
-        } else if (a >= 4 && a - 4 < p.n_tiles) {
-            const int c = cell_index(p, pos[0], pos[1], pos[2]);
-            if (cell_out) *cell_out = c;
-            const int t = a - 4;
-            const int old = grid[c];
-            change = old != t;
-            wrote = change && !(frozen && frozen[c]);
-            if (wrote) grid[c] = (int8_t)t;
-        } else if (p.status) {
-            atomicOr(p.status, 1);
-        }
-    } else {  // PCGRL_REP_WIDE
-        int q0, q1, q2 = 0, v;
-        if (p.action_kind == PCGRL_ACT_WIDE_FLAT) {
-            // wrappers.py:304-323: (y, x, v) = unravel(a, (h, w, C)); env.step([x, y, v]) -> _map[x, y] = v
-            const int a = load_action(p, gid);
-            v = a % p.n_tiles;
-            const int x = (a / p.n_tiles) % p.act_w;
-            const int y = a / (p.n_tiles * p.act_w);
-            q0 = x;
-            q1 = y;
-            if (a < 0 || y >= p.act_h) q0 = -1;
-        } else {
-            const int32_t* a = (const int32_t*)p.actions + gid * (p.ndim + 1);
-            q0 = a[0];
-            q1 = a[1];
-            if (p.ndim == 3) q2 = a[2];
-            v = a[p.ndim];
-        }
-        if ((unsigned)q0 >= (unsigned)p.d0 || (unsigned)q1 >= (unsigned)p.d1 || (unsigned)q2 >= (unsigned)p.d2 ||
-            (unsigned)v >= (unsigned)p.n_tiles) {
-            if (p.status) atomicOr(p.status, 1);
-        } else {
-            const int c = cell_index(p, q0, q1, q2);
-            if (cell_out) *cell_out = c;
-            const int old = grid[c];
-            change = old != v;
-            wrote = change;   // the reference's wide / cellular reps do not run under StaticTileRepresentation
-            if (change) grid[c] = (int8_t)v;
-            pos[0] = q0;
-            pos[1] = q1;
-            pos[2] = q2;
-        }
+        return change | (wrote << 1);
     }
-    return change | (wrote << 1);
+    return one_cell_action<true>(p, gid, gid, cell_out);
 }
 
 // HoleyProblem.gen_holes (envs/probs/holey_prob.py:32-60) for a 2D map.  Border cells are numbered in the
@@ -378,6 +399,13 @@ __device__ static void reset_env(const KParams& p, int64_t gid) {
 }
 
 
+// PcgrlEnv.step's done == truncated after the step that brought the counters to `it` / `ch` (pcgrl_env.py:307-310)
+__device__ __forceinline__ bool episode_done(const KParams& p, int it, int ch) {
+    bool done = it > p.max_iterations;     // :307
+    if (p.max_changes >= 0) done = done || ch > p.max_changes;  // :308-309
+    return done;
+}
+
 // PcgrlEnv.step's bookkeeping for env `gid` after its representation update returned `cw` (bit0 change, bit1 the
 // grid was modified): iteration / changes counters, done, change flag, zero reward for an unchanged map.
 // Returns true when the stats must be recomputed (pcgrl_env.py:314).
@@ -387,8 +415,7 @@ __device__ __forceinline__ bool step_counters(const KParams& p, int64_t gid, int
     const int ch = p.changes[gid] + change;
     p.iteration[gid] = it;
     if (change) p.changes[gid] = ch;
-    bool done = it > p.max_iterations;     // :307
-    if (p.max_changes >= 0) done = done || ch > p.max_changes;  // :308-309
+    const bool done = episode_done(p, it, ch);
     p.done[gid] = done;
     if (p.changed) p.changed[gid] = change != 0;
     record_flags(p, gid, done, change);
@@ -399,6 +426,16 @@ __device__ __forceinline__ bool step_counters(const KParams& p, int64_t gid, int
         record_reward(p, gid, 0.f);
     }
     return need;
+}
+
+// reward = loss(nw) - loss(od) in fp64 under the targets `trg` (or the range-reward sum)
+template <int K>
+__device__ __forceinline__ float step_reward(const KParams& p, const double* trg, const int32_t (&nw)[K],
+                                             const int32_t (&od)[K]) {
+    const double r = p.reward_mode == PCGRL_REWARD_RANGE
+                         ? range_reward_sum(nw, od, trg, p.weights, K)
+                         : control_loss(nw, trg, p.weights, K) - control_loss(od, trg, p.weights, K);
+    return (float)r;
 }
 
 // Phase D for one env: reward = loss(new stats) - loss(old stats) in fp64 (or the range-reward sum), then the new
@@ -413,12 +450,9 @@ __device__ __forceinline__ void finish_env(const KParams& p, int64_t gid, const 
         int32_t od[K];
 #pragma unroll
         for (int k = 0; k < K; ++k) od[k] = old ? old[k] : st[k];
-        const double* trg = p.targets + (p.targets_per_env ? gid * K * 2 : 0);
-        const double r = p.reward_mode == PCGRL_REWARD_RANGE
-                             ? range_reward_sum(nw, od, trg, p.weights, K)
-                             : control_loss(nw, trg, p.weights, K) - control_loss(od, trg, p.weights, K);
-        p.reward[gid] = (float)r;
-        record_reward(p, gid, (float)r);
+        const float r = step_reward<K>(p, p.targets + (p.targets_per_env ? gid * K * 2 : 0), nw, od);
+        p.reward[gid] = r;
+        record_reward(p, gid, r);
     }
     record_stats<K>(p, gid, nw);
 #pragma unroll

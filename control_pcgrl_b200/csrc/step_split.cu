@@ -28,6 +28,7 @@
 #include "pcgrl_device.cuh"
 #include "step_common.cuh"
 #include "bitboard_machines.cuh"
+#include "worklist.cuh"
 
 namespace pcgrl {
 
@@ -59,53 +60,16 @@ constexpr int STAT_THREADS = 128;
 // threads per CTA of the static search: as many warps as keep the staged bit-boards under 48 KB of shared memory
 __host__ __device__ constexpr int stat_threads(int bbw) { return bbw <= 96 ? 128 : 64; }
 constexpr int OUT_THREADS = 256;
-// Work list of one launch: p.wl_hdr = 16 header ints, p.worklist = the body: (env, cell) pairs for up to n_envs items, then n_stats new
-// stats per item.  The headers of all pipeline chunks live together at the front of pcgrl_state.worklist, where no
-// body ever lands, so they stay zero whatever chunking the previous step used.
-// Header (all zero before the first step): [0], [1] item counters used alternately, [3] the step count, whose parity
-// picks the counter, [4] the step's final item count.  k_split_act adds to counter [par]; the search kernel clears
-// counter [par ^ 1] for the next step and publishes the count in [4]; k_split_out reads [4] and bumps [3] -- every
-// word is written by exactly one thread of a kernel none of whose CTAs reads it, so the three launches need no
-// "last CTA out" atomics or fences to hand the list over.
-__device__ __forceinline__ int wl_parity(const KParams& p) { return *(volatile const int*)(p.wl_hdr + 3) & 1; }
-__device__ __forceinline__ int wl_count_search(const KParams& p) {
-    const int par = wl_parity(p);
-    const int count = *(volatile const int*)(p.wl_hdr + par);
-    if (blockIdx.x == 0 && threadIdx.x == 0) {
-        p.wl_hdr[par ^ 1] = 0;
-        p.wl_hdr[4] = count;
-    }
-    return count;
-}
-__device__ __forceinline__ int2* wl_items(const KParams& p) { return (int2*)p.worklist; }
-__device__ __forceinline__ int32_t* wl_stats(const KParams& p) { return p.worklist + 2 * p.n_envs; }
-
 // ------------------------------------------------------------------------------------------------
 // k_split_act
 // ------------------------------------------------------------------------------------------------
 __global__ void __launch_bounds__(ACT_THREADS) k_split_act(const KParams p) {
-    __shared__ int s_warp[ACT_THREADS / 32];
-    __shared__ int s_base;
-    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-    const int64_t gid = (int64_t)blockIdx.x * ACT_THREADS + tid;
+    const int64_t gid = (int64_t)blockIdx.x * ACT_THREADS + threadIdx.x;
     bool need = false;
     int cell = -1;
     if (gid < p.n_envs) need = step_counters(p, gid, apply_action(p, gid, &cell));
-    const unsigned bal = __ballot_sync(0xffffffffu, need);
-    if (lane == 0) s_warp[warp] = __popc(bal);
-    __syncthreads();
-    if (tid == 0) {
-        int tot = 0;
-#pragma unroll
-        for (int w = 0; w < ACT_THREADS / 32; ++w) {
-            const int c = s_warp[w];
-            s_warp[w] = tot;
-            tot += c;
-        }
-        s_base = tot ? atomicAdd(p.wl_hdr + wl_parity(p), tot) : 0;
-    }
-    __syncthreads();
-    if (need) wl_items(p)[s_base + s_warp[warp] + __popc(bal & ((1u << lane) - 1u))] = make_int2((int)gid, cell);
+    const int slot = wl_append_slot<ACT_THREADS>(p, need);
+    if (need) wl_items(p)[slot] = make_int2((int)gid, cell);
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -408,8 +372,14 @@ struct BinaryIncMachine {
     }
     // results + the new cache row
     __device__ __forceinline__ void finish(int* out, uint32_t* c) const {
+        results(out);
+        store_cache(c);
+    }
+    __device__ __forceinline__ void results(int* out) const {
         out[0] = regions;
         out[1] = path;
+    }
+    __device__ __forceinline__ void store_cache(uint32_t* c) const {
 #pragma unroll
         for (int i = 0; i < NW; ++i) {
             c[i] = sm[i];
@@ -425,8 +395,9 @@ struct BinaryIncMachine {
 // fetching items from a global counter instead did not move the bench line (0.2909 against 0.2913 ms per step) and
 // cut e2e from 2.60 to 2.51e9 (profiles/r02_ab_inc_dynamic.txt).  Fixed windows of INC_EXPAND_R expansions:
 // adaptive rounds measured 0.334 ms against 0.303.
+// LOOKAHEAD (lookahead.cu): the items are candidate edits of unchanged envs; the cache rows are read, never written.
 // ------------------------------------------------------------------------------------------------
-template <int NW, bool TWO>
+template <int NW, bool TWO, bool LOOKAHEAD = false>
 __global__ void __launch_bounds__(STAT_THREADS) k_split_stats_inc(const KParams p) {
     using M = BinaryIncMachine<NW, TWO>;
     __shared__ uint32_t s_work[STAT_THREADS * M::SMEM_WORDS];
@@ -470,7 +441,8 @@ __global__ void __launch_bounds__(STAT_THREADS) k_split_stats_inc(const KParams 
                 if (alive) alive = m.expand();
             if (!alive && m.transition()) {
                 int out[2];
-                m.finish(out, (uint32_t*)(p.cache + env * p.cache_stride));
+                if constexpr (LOOKAHEAD) m.results(out);
+                else m.finish(out, (uint32_t*)(p.cache + env * p.cache_stride));
                 *(int2*)(stats_out + (int64_t)item * 2) = make_int2(out[0], out[1]);
                 active = false;
             }
@@ -716,6 +688,23 @@ cudaError_t launch_bitboard_split(const KParams& p, int problem, cudaStream_t s,
         return launch_split<BinaryHoleyMachine<32, false>, 32, false>(p, s, 0);
     }
     return cudaSuccess;
+}
+
+// The search kernel of the incremental lookahead (lookahead.cu): the work list of p holds (env, cell) candidate
+// edits, p.stats / p.cache are the shard's.  Sized as the split path's search.
+cudaError_t launch_lookahead_search(const KParams& p, cudaStream_t s) {
+    int n_sm = 0;
+    cudaError_t e = sm_count(n_sm);
+    if (e != cudaSuccess) return e;
+    const int64_t want = (p.n_envs + STAT_THREADS - 1) / STAT_THREADS;
+    const int64_t cap = (int64_t)n_sm * INC_CTAS_PER_SM;
+    const unsigned grid = (unsigned)(want < cap ? want : cap);
+    const int nw = (p.d0 + 1) / 2;
+    if (nw <= 1) k_split_stats_inc<1, true, true><<<grid, STAT_THREADS, 0, s>>>(p);
+    else if (nw <= 2) k_split_stats_inc<2, true, true><<<grid, STAT_THREADS, 0, s>>>(p);
+    else if (nw <= 4) k_split_stats_inc<4, true, true><<<grid, STAT_THREADS, 0, s>>>(p);
+    else k_split_stats_inc<8, true, true><<<grid, STAT_THREADS, 0, s>>>(p);
+    return cudaGetLastError();
 }
 
 // bytes per env of the incremental search cache (0: this config has none)

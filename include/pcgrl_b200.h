@@ -144,7 +144,8 @@ typedef struct pcgrl_state {
                               (helper_3D.py:531, a recorded x or y >= depth); bit2 (4) a search workspace
                               overflowed; bit3 (8) sokoban: more crates than a packed solver state holds (15);
                               bit4 (16) a stat did not fit cfg.record_stat_bytes in the packed record; bit5 (32)
-                              is retired; bit6 (64) pcgrl_observe_envs: an env index outside [0, n_envs) */
+                              is retired; bit6 (64) pcgrl_observe_envs: an env index outside [0, n_envs); bit7 (128)
+                              pcgrl_lookahead: an env index outside [0, n_envs) */
     void*    scratch;      /* pcgrl_scratch_bytes() bytes, may be NULL when that returns 0.  Must be zero-filled
                               once before its first use (it holds hash-table generation counters, solver job
                               lists and, for smb, 4 bytes per env of playthrough-length history, which is why
@@ -274,6 +275,24 @@ int32_t pcgrl_observe(const pcgrl_config* cfg, const pcgrl_state* st, const pcgr
  * For a trainer's terminal observations of finished episodes, or the fresh rows after a masked reset. */
 int32_t pcgrl_observe_envs(const pcgrl_config* cfg, const pcgrl_state* st, const pcgrl_obs_args* obs,
                            const int32_t* env_idx, int64_t n_idx, void* stream);
+
+/* One-step lookahead: what pcgrl_step would return for a list of (env, action) candidates, with the shard left as it
+ * is.  Candidate j pairs env e = env_idx[j] (a DEVICE array of n int32; NULL: e = j, n <= n_envs) with action j of
+ * `actions` (the pcgrl_step layout, n rows).  Supposing env e took that action as its next one:
+ *   reward[j]  f32, bit for bit the step's      done[j], changed[j]  u8, the step's
+ *   stats[j]   [n, K] int32, env e's stats row after that step
+ * Any order, duplicates allowed; n == 0 launches nothing.  Nothing of the shard changes except st->status, which gets
+ * the bits the step would set (bit 0 for an invalid action, the solvers' bits) and bit 128 for an env index outside
+ * [0, st->n_envs), through which nothing is loaded (that candidate's outputs are unspecified).  No auto-reset.
+ *   work  pcgrl_lookahead_work_bytes(cfg, n) bytes (or more), zero-filled once before its first use (the solver
+ *         kernels keep generation counters in it); not shared by launches that can run concurrently, as scratch.
+ * A shard with a search cache (st->worklist and st->cache set, pcgrl_cache_stride(cfg) > 0) runs the step's
+ * incremental search from the cache row of every changed candidate (three launches, no grid copied); every other
+ * shard copies the candidates' env rows into a sub-shard inside `work` and runs the ordinary step on it. */
+int64_t pcgrl_lookahead_work_bytes(const pcgrl_config* cfg, int64_t n);
+int32_t pcgrl_lookahead(const pcgrl_config* cfg, const pcgrl_state* st, const void* actions, const int32_t* env_idx,
+                        int64_t n, float* reward, uint8_t* done, uint8_t* changed, int32_t* stats, void* work,
+                        void* stream);
 
 /* -- host-buffer convenience (the end-to-end path timed as `e2e` in bench.py) ------------------ */
 /* Copies `actions` (host, pinned or pageable) to `actions_dev`, runs pcgrl_step, copies reward/done/stats
