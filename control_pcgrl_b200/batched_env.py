@@ -438,11 +438,18 @@ class BatchedPcgrlEnv:
             raise IndexError(f"agent {agent} of {max(self.n_agents, 1)}")
         return self._st_agents[int(agent)]
 
-    def step(self, actions: torch.Tensor, agent: int = 0):
+    def step(self, actions: torch.Tensor, agent: int = 0, env_ids=None):
         """One env-step for all N envs.  `actions` is a device tensor laid out per `action_kind`.
         Returns (reward[N] f32, done[N] u8) device tensors (overwritten by the next step).
         agent: with n_agents > 1, whose turtle acts (MultiAgentWrapper.step, wrappers.py:724-731, steps the env once
-        per agent)."""
+        per agent).
+        env_ids: a 1-D integer array / tensor of M DISTINCT env indices (any order): only those envs step, env_ids[j]
+        taking row j of `actions` (the step layout with M rows), and every other env keeps its state and its last
+        outputs bit for bit (pcgrl_step_envs).  Returns fresh compact (reward[M] f32, done[M] u8).  With auto_reset,
+        the listed envs that finished restart.  A bad or repeated index raises IndexError / ValueError before
+        anything is launched (a device tensor costs one sort and one sync for that check)."""
+        if env_ids is not None:
+            return self._step_envs(actions, agent, env_ids)
         self._check_fresh("step")
         a = self._check_actions(actions)
         with self._on_device():
@@ -456,6 +463,28 @@ class BatchedPcgrlEnv:
         return self.reward, self.done
 
     _in_agent_round = False
+
+    def _step_envs(self, actions, agent, env_ids):
+        self._check_fresh("step")
+        rows = self._check_env_ids(env_ids, distinct=True)
+        m = rows.numel()
+        a = self._check_actions(actions, m)
+        st = self._agent_state(agent)
+        if m == 0:
+            return (torch.empty(0, dtype=torch.float32, device=self.device),
+                    torch.empty(0, dtype=torch.uint8, device=self.device))
+        work = self._work(int(self.lib.pcgrl_step_envs_work_bytes(self._cc, m)))
+        with self._on_device():
+            _lib.check(self.lib.pcgrl_step_envs(self._cc, st, a.data_ptr(), rows.data_ptr(), m, work.data_ptr(),
+                                                self._stream()), "pcgrl_step_envs")
+        idx = rows.long()
+        reward, done = self.reward[idx], self.done[idx]
+        self._synced_steps = None
+        if self.auto_reset:     # the listed envs that finished: unlisted rows of self.done are older steps' flags
+            mask = torch.zeros(self.n_envs, dtype=torch.uint8, device=self.device)
+            mask[idx] = done
+            self.reset(mask=mask)
+        return reward, done
 
     def update(self, actions: torch.Tensor, agent: int = 0) -> torch.Tensor:
         """Representation.update for all N envs (envs/reps/*.py), the call evolution's generator loop makes at every
@@ -496,15 +525,20 @@ class BatchedPcgrlEnv:
     def _lookahead(self, a, rows, m, agent, reward, done, stats, changed):
         if m == 0:
             return
-        need = int(self.lib.pcgrl_lookahead_work_bytes(self._cc, m))
+        work = self._work(int(self.lib.pcgrl_lookahead_work_bytes(self._cc, m)))
+        with self._on_device():
+            _lib.check(self.lib.pcgrl_lookahead(self._cc, self._agent_state(agent), a.data_ptr(), _ptr(rows), m,
+                                                reward.data_ptr(), done.data_ptr(), changed.data_ptr(), stats.data_ptr(),
+                                                work.data_ptr(), self._stream()), "pcgrl_lookahead")
+
+    def _work(self, need):
+        """The work buffer of lookahead and of step(env_ids=...), at least `need` bytes (both keep the solver scratch at
+        the same offset, so one buffer serves both)."""
         if self._la_work is None or self._la_work.numel() < need:
             # zero-filled when allocated: the solver kernels keep generation counters in it
             self._la_work = None
             self._la_work = torch.zeros(need, dtype=torch.uint8, device=self.device)
-        with self._on_device():
-            _lib.check(self.lib.pcgrl_lookahead(self._cc, self._agent_state(agent), a.data_ptr(), _ptr(rows), m,
-                                                reward.data_ptr(), done.data_ptr(), changed.data_ptr(), stats.data_ptr(),
-                                                self._la_work.data_ptr(), self._stream()), "pcgrl_lookahead")
+        return self._la_work
 
     _la_work = None
     LOOKAHEAD_CHUNK = 1 << 22     # candidates per launch of lookahead_all: bounds the work buffer
@@ -775,22 +809,31 @@ class BatchedPcgrlEnv:
         rows = None if env_ids is None else self._check_env_ids(env_ids)
         return self._observe(out, dtype, onehot, agent, rows)
 
-    def _check_env_ids(self, env_ids):
-        """-> int32 device tensor of validated env indices."""
+    def _check_env_ids(self, env_ids, distinct=False):
+        """-> int32 device tensor of validated env indices (distinct: a repeated index raises ValueError)."""
         if torch.is_tensor(env_ids):
             t = env_ids
             if t.dim() != 1 or (t.numel() and (t.dtype.is_floating_point or t.dtype.is_complex or t.dtype == torch.bool)):
                 raise IndexError(f"env_ids must be a 1-D integer index, got {tuple(t.shape)} {t.dtype}")
             if t.numel():
-                lo, hi = torch.stack(torch.aminmax(t)).tolist()      # host tensors: no device work
+                if distinct:    # one sort gives the range and the repeats, read back in one sync
+                    srt = t.to(torch.int64).sort().values
+                    lo, hi, rep = torch.stack([srt[0], srt[-1], (srt[1:] == srt[:-1]).any().to(torch.int64)]).tolist()
+                else:
+                    lo, hi = torch.stack(torch.aminmax(t)).tolist()      # host tensors: no device work
+                    rep = 0
                 if lo < 0 or hi >= self.n_envs:
                     raise IndexError(f"env_ids in [{lo}, {hi}] outside [0, {self.n_envs})")
+                if rep:
+                    raise ValueError("env_ids repeat an env index")
             return t.to(device=self.device, dtype=torch.int32).contiguous()
         a = np.asarray(env_ids)
         if a.ndim != 1 or (a.size and a.dtype.kind not in "iu"):
             raise IndexError(f"env_ids must be a 1-D integer index, got shape {a.shape} {a.dtype}")
         if a.size and (int(a.min()) < 0 or int(a.max()) >= self.n_envs):
             raise IndexError(f"env_ids in [{int(a.min())}, {int(a.max())}] outside [0, {self.n_envs})")
+        if distinct and np.unique(a).size != a.size:
+            raise ValueError("env_ids repeat an env index")
         return torch.from_numpy(a.astype(np.int32)).to(self.device)
 
     def _observe_envs(self, rows, out=None, dtype=torch.float32, onehot: bool = True, agent: int = 0):
@@ -865,6 +908,7 @@ class BatchedPcgrlEnv:
         (16, OverflowError, "a stat did not fit the packed result record (record_stat_bytes too small)"),
         (64, IndexError, "observe: env index out of range (pcgrl_observe_envs loaded nothing through it)"),
         (128, IndexError, "lookahead: env index out of range (pcgrl_lookahead loaded nothing through it)"),
+        (256, IndexError, "step: env index out of range (pcgrl_step_envs loaded and wrote nothing through it)"),
     )
 
     def check_status(self):

@@ -15,7 +15,7 @@ namespace pcgrl {
 cudaError_t launch_bitboard(const KParams& p, int problem, cudaStream_t s, bool& supported);
 cudaError_t launch_bigboard(const KParams& p, int problem, cudaStream_t s, bool& supported);
 cudaError_t launch_bitboard_split(const KParams& p, int problem, cudaStream_t s, int incremental, bool& supported,
-                                  int& n_launches);
+                                  int& n_launches, const int32_t* env_idx = nullptr, int64_t n_src = 0);
 cudaError_t launch_bitboard_lanegroup(const KParams& p, int problem, cudaStream_t s, bool& supported);
 int bitboard_cache_stride(int problem, int ndim, int d0, int d1, int rep, int action_kind);
 cudaError_t launch_maze3d(const KParams& p, cudaStream_t s, bool& supported);
@@ -29,8 +29,11 @@ cudaError_t launch_observe(const pcgrl_config& cfg, const pcgrl_state& st, const
                            const int32_t* env_idx, int64_t n_idx);
 cudaError_t launch_update(const KParams& p, cudaStream_t s);
 cudaError_t launch_lookahead_inc(const KParams& p, const LaOut& o, cudaStream_t s);
-cudaError_t launch_lookahead_gather(const pcgrl_state& src, const pcgrl_state& dst, const int32_t* env_idx,
-                                    int row_stride, int K, int hole_ints, bool targets_per_env, cudaStream_t s);
+cudaError_t launch_lookahead_gather(const pcgrl_state& shard, const pcgrl_state& sub, const int32_t* env_idx,
+                                    int row_stride, int K, int hole_ints, bool targets_per_env, int rec_stride,
+                                    int status_bit, cudaStream_t s);
+cudaError_t launch_step_envs_scatter(const pcgrl_state& shard, const pcgrl_state& sub, const int32_t* env_idx,
+                                     int row_stride, int K, int rec_stride, cudaStream_t s);
 
 // split step path: up to WL_CHUNKS host-pipeline chunks, one 16-int work-list header each at the front of
 // pcgrl_state.worklist
@@ -338,14 +341,17 @@ static int host_chunks(const pcgrl_config* cfg, int64_t n, bool packed) {
     if (n < (1 << 19)) return 2;
     return 4;
 }
-// Layout of the lookahead's work buffer for n candidates.  The first 256 bytes hold the work-list header of the
-// incremental path (only that path touches them).  Behind them, either the incremental path's work-list body or the
-// generic path's solver scratch (at a fixed offset: it keeps generation counters from call to call) and the sub-shard.
+// Layout of the work buffer of the lookahead (n candidates) and of pcgrl_step_envs (n envs, `step`).  The first 256
+// bytes hold the work-list header of the incremental lookahead (only that path touches them).  Behind them, either the
+// incremental lookahead's work-list body or the generic path's solver scratch (at a fixed offset: it keeps generation
+// counters from call to call, so one zero-filled buffer serves both calls) and the sub-shard.  The step's sub-shard
+// also holds the outputs it writes back: stats, reward, done, changed and the packed records.
 struct LaLayout {
-    int64_t inc_body, scratch, grids, mask, pos, n_step, iteration, changes, targets, holes, total;
+    int64_t inc_body, scratch, grids, mask, pos, n_step, iteration, changes, targets, holes;
+    int64_t stats, reward, done, changed, records, total;
 };
 static int64_t la_align(int64_t x) { return (x + 255) / 256 * 256; }
-static LaLayout la_layout(const pcgrl_config* c, int64_t n) {
+static LaLayout la_layout(const pcgrl_config* c, int64_t n, bool step = false) {
     LaLayout l;
     const int64_t K = c->n_stats;
     l.inc_body = 256;
@@ -365,7 +371,12 @@ static LaLayout la_layout(const pcgrl_config* c, int64_t n) {
     l.changes = take(n * 4);
     l.targets = take(c->targets_per_env ? n * K * 16 : 0);
     l.holes = take(is_holey(c) ? n * hole_ints(c) * 4 : 0);
-    l.total = std::max(off, inc_end);
+    l.stats = take(step ? n * K * 4 : 0);
+    l.reward = take(step ? n * 4 : 0);
+    l.done = take(step ? n : 0);
+    l.changed = take(step ? n : 0);
+    l.records = take(step ? n * record_stride(c) : 0);
+    l.total = step ? off : std::max(off, inc_end);
     return l;
 }
 }  // namespace pcgrl
@@ -548,6 +559,26 @@ int32_t pcgrl_observe_envs(const pcgrl_config* cfg, const pcgrl_state* st, const
     return observe_impl(cfg, st, obs, env_idx, n_idx, stream);
 }
 
+// The generic path's sub-shard of n envs inside `work` (layout l): grids, frozen mask, pos, counters, per-env targets,
+// holes and solver scratch.  The caller points stats / reward / done / changed / records.
+static pcgrl_state sub_shard(const pcgrl_config* cfg, const pcgrl_state* st, int64_t n, uint8_t* w, const LaLayout& l) {
+    pcgrl_state sub;
+    std::memset(&sub, 0, sizeof(sub));
+    sub.n_envs = n;
+    sub.env_offset = st->env_offset;
+    sub.grids = (int8_t*)(w + l.grids);
+    sub.static_mask = st->static_mask ? w + l.mask : nullptr;
+    sub.pos = (int32_t*)(w + l.pos);
+    sub.n_step = (int32_t*)(w + l.n_step);
+    sub.iteration = (int32_t*)(w + l.iteration);
+    sub.changes = (int32_t*)(w + l.changes);
+    sub.targets = cfg->targets_per_env ? (const double*)(w + l.targets) : st->targets;
+    sub.holes = st->holes && is_holey(cfg) ? (int32_t*)(w + l.holes) : nullptr;
+    sub.status = st->status;
+    sub.scratch = pcgrl_scratch_bytes(cfg, n) > 0 ? w + l.scratch : nullptr;
+    return sub;
+}
+
 int64_t pcgrl_lookahead_work_bytes(const pcgrl_config* cfg, int64_t n) {
     if (check(cfg) || n < 0) return -1;
     return la_layout(cfg, n).total;
@@ -583,30 +614,69 @@ int32_t pcgrl_lookahead(const pcgrl_config* cfg, const pcgrl_state* st, const vo
         return 0;
     }
     // every other config: the candidates' rows as a sub-shard of n envs, then the ordinary step on it
-    const LaLayout l = la_layout(cfg, n);
-    pcgrl_state sub;
-    std::memset(&sub, 0, sizeof(sub));
-    sub.n_envs = n;
-    sub.env_offset = st->env_offset;
-    sub.grids = (int8_t*)(w + l.grids);
-    sub.static_mask = st->static_mask ? w + l.mask : nullptr;
-    sub.pos = (int32_t*)(w + l.pos);
-    sub.n_step = (int32_t*)(w + l.n_step);
-    sub.iteration = (int32_t*)(w + l.iteration);
-    sub.changes = (int32_t*)(w + l.changes);
+    pcgrl_state sub = sub_shard(cfg, st, n, w, la_layout(cfg, n));
     sub.stats = stats;
-    sub.targets = cfg->targets_per_env ? (const double*)(w + l.targets) : st->targets;
-    sub.holes = st->holes && is_holey(cfg) ? (int32_t*)(w + l.holes) : nullptr;
     sub.reward = reward;
     sub.done = done;
     sub.changed = changed;
-    sub.status = st->status;
-    sub.scratch = pcgrl_scratch_bytes(cfg, n) > 0 ? w + l.scratch : nullptr;
     if ((e = launch_lookahead_gather(*st, sub, env_idx, cfg->row_stride, cfg->n_stats, hole_ints(cfg),
-                                     cfg->targets_per_env != 0, s)) != cudaSuccess)
+                                     cfg->targets_per_env != 0, 0, 128, s)) != cudaSuccess)
         return cuda_fail(e, "lookahead gather launch");
     g_launches.fetch_add(1, std::memory_order_relaxed);
     return step_launch(cfg, &sub, actions, stream, nullptr, 0, 0);
+}
+
+int64_t pcgrl_step_envs_work_bytes(const pcgrl_config* cfg, int64_t n) {
+    if (check(cfg) || n < 0) return -1;
+    return la_layout(cfg, n, true).total;
+}
+
+int32_t pcgrl_step_envs(const pcgrl_config* cfg, const pcgrl_state* st, const void* actions, const int32_t* env_idx,
+                        int64_t n, void* work, void* stream) {
+    int r = check(cfg);
+    if (r) return r;
+    if ((r = check_state(st))) return r;
+    if (n < 0 || n > INT32_MAX) return fail(PCGRL_E_ARG, "n must be in [0, 2^31)");
+    if (n > st->n_envs) return fail(PCGRL_E_ARG, "n distinct env indices: n > n_envs");
+    if (n > 0 && (!actions || !env_idx || !work)) return fail(PCGRL_E_ARG, "actions, env_idx and work must not be NULL");
+    if (is_holey(cfg) && !st->holes) return fail(PCGRL_E_ARG, "a holey problem needs pcgrl_state.holes");
+    if (n == 0) return 0;   // nothing to write, nothing launched
+    KParams p;
+    fill(p, cfg, st);
+    p.mode = MODE_STEP;
+    p.actions = actions;
+    p.n_envs = n;
+    const cudaStream_t s = (cudaStream_t)stream;
+    cudaError_t e;
+    if (p.worklist) {   // the split path's three launches through the shard's own work list (chunk 0's header)
+        bool supported = false;
+        int n_launches = 0;
+        e = launch_bitboard_split(p, kernel_problem(cfg->problem), s, 1, supported, n_launches, env_idx, st->n_envs);
+        if (supported) {
+            if (e != cudaSuccess) return cuda_fail(e, "step_envs launch");
+            g_launches.fetch_add(n_launches, std::memory_order_relaxed);
+            return 0;
+        }
+    }
+    // every other config: the listed rows as a sub-shard of n envs, the ordinary step on it, and the rows back
+    uint8_t* w = (uint8_t*)work;
+    const LaLayout l = la_layout(cfg, n, true);
+    pcgrl_state sub = sub_shard(cfg, st, n, w, l);
+    sub.stats = (int32_t*)(w + l.stats);
+    sub.reward = (float*)(w + l.reward);
+    sub.done = w + l.done;
+    sub.changed = w + l.changed;
+    sub.records = p.records ? w + l.records : nullptr;
+    const int rs = p.records ? record_stride(cfg) : 0;
+    if ((e = launch_lookahead_gather(*st, sub, env_idx, cfg->row_stride, cfg->n_stats, hole_ints(cfg),
+                                     cfg->targets_per_env != 0, rs, 256, s)) != cudaSuccess)
+        return cuda_fail(e, "step_envs gather launch");
+    g_launches.fetch_add(1, std::memory_order_relaxed);
+    if ((r = step_launch(cfg, &sub, actions, stream, nullptr, 0, 0))) return r;
+    if ((e = launch_step_envs_scatter(*st, sub, env_idx, cfg->row_stride, cfg->n_stats, rs, s)) != cudaSuccess)
+        return cuda_fail(e, "step_envs scatter launch");
+    g_launches.fetch_add(1, std::memory_order_relaxed);
+    return 0;
 }
 
 // Shared body of pcgrl_step_host / pcgrl_step_host_packed: with records_host the only download is the packed

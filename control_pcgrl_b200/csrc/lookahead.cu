@@ -13,7 +13,8 @@
 // over without a sync and the next lookahead finds its counter cleared.
 //
 // Generic path, for every other config: k_la_gather copies each candidate's env rows into a sub-shard carved from
-// `work`, and api.cu runs the ordinary MODE_STEP on it.
+// `work`, and api.cu runs the ordinary MODE_STEP on it.  pcgrl_step_envs takes the same path for shards without a work
+// list, and k_step_envs_scatter writes the stepped rows back to their envs.
 #include "pcgrl_device.cuh"
 #include "step_common.cuh"
 #include "worklist.cuh"
@@ -96,53 +97,101 @@ cudaError_t launch_lookahead_inc(const KParams& p, const LaOut& o, cudaStream_t 
 }
 
 // ------------------------------------------------------------------------------------------------
-// Generic path: candidate j's rows of the shard `src` -> row j of the sub-shard `dst`.  One thread per 16-byte
-// vector of the grid (and of the frozen mask); the thread of vector 0 also copies the small rows.  The old stats
-// go straight into dst.stats, the caller's output, where the step reads and replaces them.
+// Generic path (also pcgrl_step_envs' path for shards without a work list): row j of the sub-shard `sub` is env
+// e = env_idx[j] (or j) of the shard `shard`.  One thread per 16-byte vector of the grid (and of the frozen mask); the
+// thread of vector 0 also copies the small rows.
+// k_la_gather: shard -> sub.  The old stats go to sub.stats (the lookahead's output, or step_envs' sub-shard), where
+// the step reads and replaces them.  An index outside the shard loads nothing (its row is zeros) and sets status_bit.
+// k_step_envs_scatter: sub -> shard, what the step wrote (grid, pos, counters, stats, reward, done, changed, record);
+// an index outside the shard writes nothing.
 // ------------------------------------------------------------------------------------------------
-struct LaGather {
-    pcgrl_state src, dst;
+struct SubShard {
+    pcgrl_state shard, sub;
     const int32_t* env_idx;
-    int32_t chunks, K, hole_ints, targets_per_env;
+    int32_t chunks, K, hole_ints, targets_per_env, rec_ints, status_bit;
 };
-__global__ void __launch_bounds__(LA_THREADS) k_la_gather(const LaGather g) {
+__global__ void __launch_bounds__(LA_THREADS) k_la_gather(const SubShard g) {
     const int64_t i = (int64_t)blockIdx.x * LA_THREADS + threadIdx.x;
     const int64_t j = i / g.chunks;
     const int c = (int)(i - j * g.chunks);
-    if (j >= g.dst.n_envs) return;
+    if (j >= g.sub.n_envs) return;
     const int64_t e = g.env_idx ? (int64_t)g.env_idx[j] : j;
-    const bool ok = (uint64_t)e < (uint64_t)g.src.n_envs;   // a bad index loads nothing: its row is zeros
+    const bool ok = (uint64_t)e < (uint64_t)g.shard.n_envs;   // a bad index loads nothing: its row is zeros
     const int64_t rs = (int64_t)g.chunks * 16;
     const uint4 z = make_uint4(0, 0, 0, 0);
-    ((uint4*)(g.dst.grids + j * rs))[c] = ok ? ((const uint4*)(g.src.grids + e * rs))[c] : z;
-    if (g.dst.static_mask)
-        ((uint4*)(g.dst.static_mask + j * rs))[c] = ok ? ((const uint4*)(g.src.static_mask + e * rs))[c] : z;
+    ((uint4*)(g.sub.grids + j * rs))[c] = ok ? ((const uint4*)(g.shard.grids + e * rs))[c] : z;
+    if (g.sub.static_mask)
+        ((uint4*)(g.sub.static_mask + j * rs))[c] = ok ? ((const uint4*)(g.shard.static_mask + e * rs))[c] : z;
     if (c) return;
-    if (!ok && g.src.status) atomicOr(g.src.status, 128);
-    for (int k = 0; k < 3; ++k) g.dst.pos[j * 3 + k] = ok ? g.src.pos[e * 3 + k] : 0;
-    g.dst.n_step[j] = ok ? g.src.n_step[e] : 0;
-    g.dst.iteration[j] = ok ? g.src.iteration[e] : 0;
-    g.dst.changes[j] = ok ? g.src.changes[e] : 0;
-    for (int k = 0; k < g.K; ++k) g.dst.stats[j * g.K + k] = ok ? g.src.stats[e * g.K + k] : 0;
+    if (!ok && g.shard.status) atomicOr(g.shard.status, g.status_bit);
+    for (int k = 0; k < 3; ++k) g.sub.pos[j * 3 + k] = ok ? g.shard.pos[e * 3 + k] : 0;
+    g.sub.n_step[j] = ok ? g.shard.n_step[e] : 0;
+    g.sub.iteration[j] = ok ? g.shard.iteration[e] : 0;
+    g.sub.changes[j] = ok ? g.shard.changes[e] : 0;
+    for (int k = 0; k < g.K; ++k) g.sub.stats[j * g.K + k] = ok ? g.shard.stats[e * g.K + k] : 0;
     if (g.targets_per_env)
         for (int k = 0; k < 2 * g.K; ++k)
-            ((double*)g.dst.targets)[j * 2 * g.K + k] = ok ? g.src.targets[e * 2 * g.K + k] : 0.0;
-    if (g.dst.holes)
-        for (int k = 0; k < g.hole_ints; ++k) g.dst.holes[j * g.hole_ints + k] = ok ? g.src.holes[e * g.hole_ints + k] : 0;
+            ((double*)g.sub.targets)[j * 2 * g.K + k] = ok ? g.shard.targets[e * 2 * g.K + k] : 0.0;
+    if (g.sub.holes)
+        for (int k = 0; k < g.hole_ints; ++k) g.sub.holes[j * g.hole_ints + k] = ok ? g.shard.holes[e * g.hole_ints + k] : 0;
+    if (g.sub.records)   // the step leaves parts of the record as they were (the stats of an unchanged map)
+        for (int k = 0; k < g.rec_ints; ++k)
+            ((int32_t*)g.sub.records)[j * g.rec_ints + k] = ok ? ((const int32_t*)g.shard.records)[e * g.rec_ints + k] : 0;
 }
 
-cudaError_t launch_lookahead_gather(const pcgrl_state& src, const pcgrl_state& dst, const int32_t* env_idx,
-                                    int row_stride, int K, int hole_ints, bool targets_per_env, cudaStream_t s) {
-    LaGather g;
-    g.src = src;
-    g.dst = dst;
+__global__ void __launch_bounds__(LA_THREADS) k_step_envs_scatter(const SubShard g) {
+    const int64_t i = (int64_t)blockIdx.x * LA_THREADS + threadIdx.x;
+    const int64_t j = i / g.chunks;
+    const int c = (int)(i - j * g.chunks);
+    if (j >= g.sub.n_envs) return;
+    const int64_t e = g.env_idx[j];
+    if ((uint64_t)e >= (uint64_t)g.shard.n_envs) return;   // the gather set the status bit
+    const int64_t rs = (int64_t)g.chunks * 16;
+    ((uint4*)(g.shard.grids + e * rs))[c] = ((const uint4*)(g.sub.grids + j * rs))[c];
+    if (c) return;
+    for (int k = 0; k < 3; ++k) g.shard.pos[e * 3 + k] = g.sub.pos[j * 3 + k];
+    g.shard.n_step[e] = g.sub.n_step[j];
+    g.shard.iteration[e] = g.sub.iteration[j];
+    g.shard.changes[e] = g.sub.changes[j];
+    for (int k = 0; k < g.K; ++k) g.shard.stats[e * g.K + k] = g.sub.stats[j * g.K + k];
+    g.shard.reward[e] = g.sub.reward[j];
+    g.shard.done[e] = g.sub.done[j];
+    if (g.shard.changed) g.shard.changed[e] = g.sub.changed[j];
+    if (g.sub.records)
+        for (int k = 0; k < g.rec_ints; ++k)
+            ((int32_t*)g.shard.records)[e * g.rec_ints + k] = ((const int32_t*)g.sub.records)[j * g.rec_ints + k];
+}
+
+static SubShard sub_shard(const pcgrl_state& shard, const pcgrl_state& sub, const int32_t* env_idx, int row_stride,
+                          int K, int hole_ints, bool targets_per_env, int rec_stride, int status_bit) {
+    SubShard g;
+    g.shard = shard;
+    g.sub = sub;
     g.env_idx = env_idx;
     g.chunks = row_stride / 16;
     g.K = K;
     g.hole_ints = hole_ints;
     g.targets_per_env = targets_per_env;
-    const int64_t threads = dst.n_envs * g.chunks;
-    k_la_gather<<<(unsigned)((threads + LA_THREADS - 1) / LA_THREADS), LA_THREADS, 0, s>>>(g);
+    g.rec_ints = rec_stride / 4;
+    g.status_bit = status_bit;
+    return g;
+}
+static unsigned sub_blocks(const SubShard& g) {
+    return (unsigned)((g.sub.n_envs * g.chunks + LA_THREADS - 1) / LA_THREADS);
+}
+
+cudaError_t launch_lookahead_gather(const pcgrl_state& shard, const pcgrl_state& sub, const int32_t* env_idx,
+                                    int row_stride, int K, int hole_ints, bool targets_per_env, int rec_stride,
+                                    int status_bit, cudaStream_t s) {
+    const SubShard g = sub_shard(shard, sub, env_idx, row_stride, K, hole_ints, targets_per_env, rec_stride, status_bit);
+    k_la_gather<<<sub_blocks(g), LA_THREADS, 0, s>>>(g);
+    return cudaGetLastError();
+}
+
+cudaError_t launch_step_envs_scatter(const pcgrl_state& shard, const pcgrl_state& sub, const int32_t* env_idx,
+                                     int row_stride, int K, int rec_stride, cudaStream_t s) {
+    const SubShard g = sub_shard(shard, sub, env_idx, row_stride, K, 0, false, rec_stride, 0);
+    k_step_envs_scatter<<<sub_blocks(g), LA_THREADS, 0, s>>>(g);
     return cudaGetLastError();
 }
 

@@ -108,7 +108,8 @@ __device__ __forceinline__ int one_cell_action(const KParams& p, int64_t ai, int
 // undone (`np.where(static_tiles < 1, new, old)`), but `change = np.any(old_state != new_state)` compares
 // against the pre-undo array, so it still counts as a change (and the reference recomputes identical stats).
 // *cell_out (optional): linear index of the one cell the action addressed, -1 for multi-cell actions (patch).
-__device__ __forceinline__ int apply_action(const KParams& p, int64_t gid, int* cell_out = nullptr) {
+// The action is row `ai` of p.actions (pcgrl_step_envs: the list position of env `gid`; ai == gid otherwise).
+__device__ __forceinline__ int apply_action(const KParams& p, int64_t ai, int64_t gid, int* cell_out) {
     if (cell_out) *cell_out = -1;
     if (p.rep == PCGRL_REP_NARROW && p.action_kind == PCGRL_ACT_PATCH) {
         int8_t* grid = p.grids + gid * p.row_stride;
@@ -119,7 +120,7 @@ __device__ __forceinline__ int apply_action(const KParams& p, int64_t gid, int* 
         // replaces map[pos - l_pad : pos + r_pad + 1], l_pad = floor((a-1)/2), r_pad = ceil((a-1)/2) (:404-411);
         // change = any cell differs; then pos = act_coords[n_step % len], n_step += 1 (:517-518)
         const int np_ = p.aw0 * p.aw1 * p.aw2;
-        const int32_t* a = (const int32_t*)p.actions + gid * np_;
+        const int32_t* a = (const int32_t*)p.actions + ai * np_;
         const int l0 = (p.aw0 - 1) / 2, l1 = (p.aw1 - 1) / 2, l2 = (p.aw2 - 1) / 2;
         const int t0 = pos[0] - l0, t1 = pos[1] - l1, t2 = pos[2] - l2;
         if (t0 < 0 || t1 < 0 || t2 < 0 || t0 + p.aw0 > p.d0 || t1 + p.aw1 > p.d1 || t2 + p.aw2 > p.d2) {
@@ -155,7 +156,10 @@ __device__ __forceinline__ int apply_action(const KParams& p, int64_t gid, int* 
         p.n_step[gid] = ns + 1;
         return change | (wrote << 1);
     }
-    return one_cell_action<true>(p, gid, gid, cell_out);
+    return one_cell_action<true>(p, ai, gid, cell_out);
+}
+__device__ __forceinline__ int apply_action(const KParams& p, int64_t gid, int* cell_out = nullptr) {
+    return apply_action(p, gid, gid, cell_out);
 }
 
 // HoleyProblem.gen_holes (envs/probs/holey_prob.py:32-60) for a 2D map.  Border cells are numbered in the

@@ -62,12 +62,24 @@ __host__ __device__ constexpr int stat_threads(int bbw) { return bbw <= 96 ? 128
 constexpr int OUT_THREADS = 256;
 // ------------------------------------------------------------------------------------------------
 // k_split_act
+// IDX (pcgrl_step_envs): p.n_envs is the list length; thread j applies action row j to env env_idx[j] of the shard's
+// n_src envs.  An index outside the shard loads and writes nothing and sets status bit 256.
 // ------------------------------------------------------------------------------------------------
-__global__ void __launch_bounds__(ACT_THREADS) k_split_act(const KParams p) {
-    const int64_t gid = (int64_t)blockIdx.x * ACT_THREADS + threadIdx.x;
+template <bool IDX>
+__global__ void __launch_bounds__(ACT_THREADS) k_split_act(const KParams p, const int32_t* env_idx, int64_t n_src) {
+    const int64_t j = (int64_t)blockIdx.x * ACT_THREADS + threadIdx.x;
+    int64_t gid = j;
     bool need = false;
     int cell = -1;
-    if (gid < p.n_envs) need = step_counters(p, gid, apply_action(p, gid, &cell));
+    if (j < p.n_envs) {
+        if constexpr (IDX) {
+            gid = env_idx[j];
+            if ((uint64_t)gid < (uint64_t)n_src) need = step_counters(p, gid, apply_action(p, j, gid, &cell));
+            else if (p.status) atomicOr(p.status, 256);
+        } else {
+            need = step_counters(p, gid, apply_action(p, gid, &cell));
+        }
+    }
     const int slot = wl_append_slot<ACT_THREADS>(p, need);
     if (need) wl_items(p)[slot] = make_int2((int)gid, cell);
 }
@@ -599,8 +611,10 @@ static cudaError_t sm_count(int& n) {
     return cudaSuccess;
 }
 
+// env_idx (pcgrl_step_envs): the list of p.n_envs env indices into a shard of n_src envs (incremental <= 1).
 template <class Machine, int NW, bool TWO>
-static cudaError_t launch_split(const KParams& p, cudaStream_t s, int incremental) {
+static cudaError_t launch_split(const KParams& p, cudaStream_t s, int incremental, const int32_t* env_idx,
+                                int64_t n_src) {
     constexpr int K = Machine::Prob::K;
     const int64_t n = p.n_envs;
     if (n == 0) return cudaSuccess;
@@ -624,7 +638,9 @@ static cudaError_t launch_split(const KParams& p, cudaStream_t s, int incrementa
             return cudaGetLastError();
         }
     }
-    k_split_act<<<(unsigned)((n + ACT_THREADS - 1) / ACT_THREADS), ACT_THREADS, 0, s>>>(p);
+    const unsigned act_blocks = (unsigned)((n + ACT_THREADS - 1) / ACT_THREADS);
+    if (env_idx) k_split_act<true><<<act_blocks, ACT_THREADS, 0, s>>>(p, env_idx, n_src);
+    else k_split_act<false><<<act_blocks, ACT_THREADS, 0, s>>>(p, nullptr, 0);
     if ((e = cudaGetLastError()) != cudaSuccess) return e;
     bool ran_inc = false;
     if constexpr (Machine::HAS_CACHE && TWO) {
@@ -647,20 +663,21 @@ static cudaError_t launch_split(const KParams& p, cudaStream_t s, int incrementa
 }
 
 template <template <int, bool> class Machine>
-static cudaError_t dispatch_split(const KParams& p, cudaStream_t s, int incremental, bool& supported) {
+static cudaError_t dispatch_split(const KParams& p, cudaStream_t s, int incremental, bool& supported,
+                                  const int32_t* env_idx, int64_t n_src) {
     const int H = p.d0, W = p.d1;
     supported = p.ndim == 2;
     if (!supported) return cudaSuccess;
     if (W <= 16 && H <= 16) {
         const int nw = (H + 1) / 2;
-        if (nw <= 1) return launch_split<Machine<1, true>, 1, true>(p, s, incremental);
-        if (nw <= 2) return launch_split<Machine<2, true>, 2, true>(p, s, incremental);
-        if (nw <= 4) return launch_split<Machine<4, true>, 4, true>(p, s, incremental);
-        return launch_split<Machine<8, true>, 8, true>(p, s, incremental);
+        if (nw <= 1) return launch_split<Machine<1, true>, 1, true>(p, s, incremental, env_idx, n_src);
+        if (nw <= 2) return launch_split<Machine<2, true>, 2, true>(p, s, incremental, env_idx, n_src);
+        if (nw <= 4) return launch_split<Machine<4, true>, 4, true>(p, s, incremental, env_idx, n_src);
+        return launch_split<Machine<8, true>, 8, true>(p, s, incremental, env_idx, n_src);
     }
     if (W <= 32 && H <= 32) {
-        if (H <= 16) return launch_split<Machine<16, false>, 16, false>(p, s, 0);
-        return launch_split<Machine<32, false>, 32, false>(p, s, 0);
+        if (H <= 16) return launch_split<Machine<16, false>, 16, false>(p, s, 0, env_idx, n_src);
+        return launch_split<Machine<32, false>, 32, false>(p, s, 0, env_idx, n_src);
     }
     supported = false;
     return cudaSuccess;
@@ -670,22 +687,24 @@ static cudaError_t dispatch_split(const KParams& p, cudaStream_t s, int incremen
 // (binary only; needs p.cache).  Three kernels are launched: *launches is incremented by the caller accordingly.
 // incremental: 0 = from-scratch searches, 1 = incremental search as the middle kernel of the split path, 2 = the
 // fused incremental step (k_step_inc, one launch).  *n_launches = kernels launched.
+// env_idx (pcgrl_step_envs, incremental <= 1): step only the p.n_envs listed envs of a shard of n_src envs, through
+// the shard's own work list; the search and output kernels address envs through the list items as for a full step.
 cudaError_t launch_bitboard_split(const KParams& p, int problem, cudaStream_t s, int incremental, bool& supported,
-                                  int& n_launches) {
+                                  int& n_launches, const int32_t* env_idx, int64_t n_src) {
     supported = false;
     n_launches = 3;
     if (p.mode != MODE_STEP || !p.worklist || p.rep == PCGRL_REP_CELLULAR) return cudaSuccess;
     if (problem == PCGRL_PROB_BINARY) {
         const int inc = p.cache != nullptr && p.d0 <= 16 && p.d1 <= 16 ? incremental : 0;
         if (inc == 2) n_launches = 1;
-        return dispatch_split<BinaryMachine>(p, s, inc, supported);
+        return dispatch_split<BinaryMachine>(p, s, inc, supported, env_idx, n_src);
     }
-    if (problem == PCGRL_PROB_ZELDA) return dispatch_split<ZeldaMachine>(p, s, 0, supported);
+    if (problem == PCGRL_PROB_ZELDA) return dispatch_split<ZeldaMachine>(p, s, 0, supported, env_idx, n_src);
     if (problem == PCGRL_PROB_BINARY_HOLEY) {
         supported = p.ndim == 2 && p.d1 + 2 <= 32 && p.d0 + 2 <= 32;
         if (!supported) return cudaSuccess;
-        if (p.d0 + 2 <= 18) return launch_split<BinaryHoleyMachine<18, false>, 18, false>(p, s, 0);
-        return launch_split<BinaryHoleyMachine<32, false>, 32, false>(p, s, 0);
+        if (p.d0 + 2 <= 18) return launch_split<BinaryHoleyMachine<18, false>, 18, false>(p, s, 0, env_idx, n_src);
+        return launch_split<BinaryHoleyMachine<32, false>, 32, false>(p, s, 0, env_idx, n_src);
     }
     return cudaSuccess;
 }

@@ -145,7 +145,8 @@ typedef struct pcgrl_state {
                               overflowed; bit3 (8) sokoban: more crates than a packed solver state holds (15);
                               bit4 (16) a stat did not fit cfg.record_stat_bytes in the packed record; bit5 (32)
                               is retired; bit6 (64) pcgrl_observe_envs: an env index outside [0, n_envs); bit7 (128)
-                              pcgrl_lookahead: an env index outside [0, n_envs) */
+                              pcgrl_lookahead: an env index outside [0, n_envs); bit8 (256) pcgrl_step_envs: an
+                              env index outside [0, n_envs) */
     void*    scratch;      /* pcgrl_scratch_bytes() bytes, may be NULL when that returns 0.  Must be zero-filled
                               once before its first use (it holds hash-table generation counters, solver job
                               lists and, for smb, 4 bytes per env of playthrough-length history, which is why
@@ -293,6 +294,26 @@ int64_t pcgrl_lookahead_work_bytes(const pcgrl_config* cfg, int64_t n);
 int32_t pcgrl_lookahead(const pcgrl_config* cfg, const pcgrl_state* st, const void* actions, const int32_t* env_idx,
                         int64_t n, float* reward, uint8_t* done, uint8_t* changed, int32_t* stats, void* work,
                         void* stream);
+
+/* Step a list of envs of the shard in place, leaving every other env untouched.  env_idx is a DEVICE array of n
+ * DISTINCT int32 env indices (a precondition the library does not check; n <= st->n_envs), in any order, and env
+ * e = env_idx[j] takes action row j of `actions` (the pcgrl_step layout, n rows).  Env e gets exactly what pcgrl_step
+ * would give it for that action: grid, pos, n_step, iteration, changes, stats, reward, done, changed, its packed
+ * record and its search-cache row, all in its own rows of `st`.  Every env that is not listed keeps every row bit for
+ * bit.  n == 0 launches nothing.  No auto-reset.  An index outside [0, st->n_envs) loads and writes nothing and sets
+ * status bit 256.
+ *   work  pcgrl_step_envs_work_bytes(cfg, n) bytes (or more), zero-filled once before its first use, not shared by
+ *         launches that can run concurrently; a buffer of max(this, pcgrl_lookahead_work_bytes(cfg, n)) bytes serves
+ *         both calls (the solver scratch sits at the same offset).
+ * A shard with a split-path work list (st->worklist set; binary / minecraft_2D_maze / zelda / binary_holey maps up to
+ * 32x32, not cellular) runs the split step's three launches on the listed envs through its own work list: the
+ * update kernel addresses env_idx[j], the search and output kernels run unchanged.  Every other shard copies the
+ * listed rows into a sub-shard inside `work`, runs the ordinary step on it and copies the stepped rows back.  smb's
+ * per-env playthrough-length history then lives in that sub-shard's scratch, so the env's own history row does not
+ * advance; the history only picks a job class, never a result. */
+int64_t pcgrl_step_envs_work_bytes(const pcgrl_config* cfg, int64_t n);
+int32_t pcgrl_step_envs(const pcgrl_config* cfg, const pcgrl_state* st, const void* actions, const int32_t* env_idx,
+                        int64_t n, void* work, void* stream);
 
 /* -- host-buffer convenience (the end-to-end path timed as `e2e` in bench.py) ------------------ */
 /* Copies `actions` (host, pinned or pageable) to `actions_dev`, runs pcgrl_step, copies reward/done/stats
