@@ -57,6 +57,15 @@ class ObsArgs(C.Structure):
     ]
 
 
+class RowLayout(C.Structure):
+    """pcgrl_row_layout: size, signature and byte offsets (-1 = absent) of one packed env row."""
+    _fields_ = [
+        ("row_bytes", C.c_int32), ("signature", C.c_uint32), ("n_pos", C.c_int32),
+        *((name, C.c_int32) for name in ("grid", "static_mask", "cache", "records", "targets", "stats", "holes", "pos",
+                                         "n_step", "iteration", "changes", "reward", "done", "changed")),
+    ]
+
+
 # name -> (restype, argtypes); every symbol include/pcgrl_b200.h declares
 SYMBOLS = {
     "pcgrl_abi_version": (C.c_int32, []),
@@ -87,6 +96,11 @@ SYMBOLS = {
                                     C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
     "pcgrl_step_envs_work_bytes": (C.c_int64, [C.POINTER(Config), C.c_int64]),
     "pcgrl_step_envs": (C.c_int32, [C.POINTER(Config), C.POINTER(State), C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p,
+                                    C.c_void_p]),
+    "pcgrl_env_row_layout": (C.c_int32, [C.POINTER(Config), C.POINTER(State), C.c_int32, C.POINTER(RowLayout)]),
+    "pcgrl_save_envs": (C.c_int32, [C.POINTER(Config), C.POINTER(State), C.c_int32, C.c_void_p, C.c_int64, C.c_void_p,
+                                    C.c_void_p]),
+    "pcgrl_load_envs": (C.c_int32, [C.POINTER(Config), C.POINTER(State), C.c_int32, C.c_void_p, C.c_void_p, C.c_int64,
                                     C.c_void_p]),
 }
 

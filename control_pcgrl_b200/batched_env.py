@@ -585,6 +585,133 @@ class BatchedPcgrlEnv:
             raise RuntimeError(f"{what}: update() edited the maps without recomputing stats, so stats (and the step's "
                                "search cache) are stale; call reset() (all envs) before stepping again")
 
+    # ------------------------------------------------------------------ packed env rows
+    _row_layout_cache = None
+    _fork_buf = None
+    # row_fields name -> (pcgrl_row_layout field, dtype)
+    _ROW_FIELDS = (("grids", "grid", torch.int8), ("static_mask", "static_mask", torch.uint8),
+                   ("cache", "cache", torch.uint8), ("records", "records", torch.uint8),
+                   ("targets", "targets", torch.float64), ("stats", "stats", torch.int32),
+                   ("holes", "holes", torch.int32), ("agent_pos", "pos", torch.int32),
+                   ("n_step", "n_step", torch.int32), ("iteration", "iteration", torch.int32),
+                   ("changes", "changes", torch.int32), ("reward", "reward", torch.float32),
+                   ("done", "done", torch.uint8), ("changed", "changed", torch.uint8))
+
+    def _row_layout(self):
+        """pcgrl_row_layout of this env's rows, with every agent's position array (agent_pos) in them."""
+        if self._row_layout_cache is None:
+            lay = _lib.RowLayout()
+            _lib.check(self.lib.pcgrl_env_row_layout(self._cc, self._st, self.agent_pos.shape[0], lay),
+                       "pcgrl_env_row_layout")
+            self._row_layout_cache = lay
+        return self._row_layout_cache
+
+    @property
+    def env_row_bytes(self) -> int:
+        """Bytes of one packed env row (save_envs / load_envs / fork_envs), a multiple of 16."""
+        return int(self._row_layout().row_bytes)
+
+    def row_fields(self, rows):
+        """Typed views into a [M, env_row_bytes] uint8 tensor of packed rows, one per section this env's rows have:
+        grids i8 [M, row_stride], static_mask u8 [M, row_stride], cache u8 [M, cache_stride], records u8
+        [M, record_stride], targets f64 [M, K, 2], stats i32 [M, K], holes i32 [M, hole_ints], agent_pos i32
+        [M, n_agents, 3], n_step / iteration / changes i32 [M], reward f32 [M], done / changed u8 [M].  Offsets come
+        from the library (pcgrl_env_row_layout), so an archive can read or filter saved states, by stats say, without
+        loading them."""
+        lay = self._row_layout()
+        if not torch.is_tensor(rows) or rows.dtype != torch.uint8 or rows.dim() != 2 or rows.shape[1] != lay.row_bytes \
+                or rows.stride(1) != 1:
+            raise ValueError(f"rows must be a uint8 [M, {lay.row_bytes}] tensor with contiguous rows")
+        inner = {"grids": (self.row_stride,), "static_mask": (self.row_stride,), "cache": (self.cache_stride,),
+                 "records": (self.record_stride,), "targets": (self.K, 2), "stats": (self.K,),
+                 "holes": (self.hole_ints,), "agent_pos": (lay.n_pos, 3)}
+        m, out = rows.shape[0], {}
+        for name, field, dt in self._ROW_FIELDS:
+            off = getattr(lay, field)
+            if off < 0:
+                continue
+            shape = inner.get(name, ())
+            nbytes = int(np.prod(shape, dtype=np.int64)) * dt.itemsize
+            v = rows[:, off:off + nbytes].view(dt)
+            out[name] = v.view(m, *shape) if shape else v[:, 0]
+        return out
+
+    def save_envs(self, env_ids=None) -> torch.Tensor:
+        """The whole state of envs env_ids (default all) as a new device uint8 tensor [M, env_row_bytes], row j = env
+        env_ids[j]: grid, frozen mask, search cache, packed record, per-env targets, stats, holes, every agent's position,
+        n_step / iteration / changes and the last reward / done / changed (pcgrl_save_envs).  Indices may repeat and come
+        in any order; a bad index raises IndexError before anything is launched (a device tensor costs one reduction and
+        one sync).  Not in a row: shared targets, the reset RNG position (seed, epoch) and smb's playthrough-length
+        history, which only picks a job class of its solver, never a result."""
+        self._check_fresh("save_envs")
+        idx = None if env_ids is None else self._check_env_ids(env_ids)
+        m = self.n_envs if idx is None else idx.numel()
+        rows = torch.empty((m, self.env_row_bytes), dtype=torch.uint8, device=self.device)
+        self._save_rows(idx, m, rows)
+        self._synced_steps = None
+        return rows
+
+    def load_envs(self, rows: torch.Tensor, env_ids=None):
+        """Env env_ids[j] (default j) becomes bit for bit the env row j of `rows` was saved from (pcgrl_load_envs); every
+        other env is untouched and nothing is reset, auto_reset or not.  rows: a contiguous uint8 [M, env_row_bytes]
+        tensor on this env's device, saved by any env with the same row layout (another n_envs, env_offset, seed or
+        device after .to(env.device) included).  env_ids: M DISTINCT indices.  A bad or repeated index (IndexError /
+        ValueError) or a row saved under another layout (ValueError) raises before anything is launched; each check of
+        device data costs one reduction and one sync."""
+        self._check_fresh("load_envs")
+        lay = self._row_layout()
+        if not torch.is_tensor(rows) or rows.dtype != torch.uint8 or rows.dim() != 2 or \
+                rows.shape[1] != lay.row_bytes or not rows.is_contiguous() or rows.device != self.device:
+            raise ValueError(f"rows must be a contiguous uint8 [M, {lay.row_bytes}] tensor on {self.device}")
+        m = rows.shape[0]
+        idx = None
+        if env_ids is None:
+            if m > self.n_envs:
+                raise ValueError(f"{m} rows for {self.n_envs} envs")
+        else:
+            idx = self._check_env_ids(env_ids, distinct=True)
+            if idx.numel() != m:
+                raise ValueError(f"{m} rows for {idx.numel()} env_ids")
+        if m:
+            sig = lay.signature - (1 << 32) if lay.signature >= 1 << 31 else lay.signature   # as int32
+            want = torch.tensor([sig, lay.row_bytes], dtype=torch.int32, device=self.device)
+            if bool((rows[:, :8].view(torch.int32) != want).any()):
+                raise ValueError("rows were not saved from an env with this env's row layout (header mismatch)")
+            self._load_rows(rows, idx, m)
+        self._synced_steps = None
+
+    def fork_envs(self, src_ids, dst_ids):
+        """Env dst_ids[j] becomes a copy of env src_ids[j] as it was before the call (save into a reusable buffer, then
+        load: two launches).  dst_ids are distinct, src_ids may repeat, and the two may overlap: a beam step overwrites
+        the whole shard with copies of its best children.  Bad or repeated indices raise IndexError / ValueError before
+        anything is launched.  Nothing is reset."""
+        self._check_fresh("fork_envs")
+        src = self._check_env_ids(src_ids)
+        dst = self._check_env_ids(dst_ids, distinct=True)
+        m = dst.numel()
+        if src.numel() != m:
+            raise ValueError(f"{src.numel()} src_ids for {m} dst_ids")
+        if m:
+            S = self.env_row_bytes
+            if self._fork_buf is None or self._fork_buf.numel() < m * S:
+                self._fork_buf = None
+                self._fork_buf = torch.empty(m * S, dtype=torch.uint8, device=self.device)
+            buf = self._fork_buf[:m * S].view(m, S)
+            self._save_rows(src, m, buf)
+            self._load_rows(buf, dst, m)     # the library's own rows: no header check
+        self._synced_steps = None
+
+    def _save_rows(self, idx, m, rows):
+        if m:
+            with self._on_device():
+                _lib.check(self.lib.pcgrl_save_envs(self._cc, self._st, self.agent_pos.shape[0], _ptr(idx), m,
+                                                    rows.data_ptr(), self._stream()), "pcgrl_save_envs")
+
+    def _load_rows(self, rows, idx, m):
+        with self._on_device():
+            _lib.check(self.lib.pcgrl_load_envs(self._cc, self._st, self.agent_pos.shape[0], rows.data_ptr(), _ptr(idx), m,
+                                                self._stream()), "pcgrl_load_envs")
+
     def step_agents(self, actions: torch.Tensor):
         """One multi-agent step: actions[N, n_agents], agent a acts a-th (MultiAgentWrapper.step,
         wrappers.py:724-731: a full env step per agent, so iteration advances by n_agents).  Returns
@@ -909,6 +1036,9 @@ class BatchedPcgrlEnv:
         (64, IndexError, "observe: env index out of range (pcgrl_observe_envs loaded nothing through it)"),
         (128, IndexError, "lookahead: env index out of range (pcgrl_lookahead loaded nothing through it)"),
         (256, IndexError, "step: env index out of range (pcgrl_step_envs loaded and wrote nothing through it)"),
+        (512, IndexError, "save / load / fork: env index out of range (pcgrl_save_envs wrote a zero row for it, "
+                          "pcgrl_load_envs wrote nothing)"),
+        (1024, ValueError, "load: a row's header does not match this env's row layout (nothing of it was loaded)"),
     )
 
     def check_status(self):

@@ -10,6 +10,7 @@
 #include <vector>
 
 #include "pcgrl_device.cuh"
+#include "env_rows.cuh"
 
 namespace pcgrl {
 cudaError_t launch_bitboard(const KParams& p, int problem, cudaStream_t s, bool& supported);
@@ -379,6 +380,77 @@ static LaLayout la_layout(const pcgrl_config* c, int64_t n, bool step = false) {
     l.total = step ? off : std::max(off, inc_end);
     return l;
 }
+
+// The packed env row of pcgrl_save_envs / pcgrl_load_envs (format in include/pcgrl_b200.h), decided here and nowhere
+// else: the offsets for the caller, and (rc != NULL) the pieces the copy kernels move.  The shard's arguments have been
+// checked.
+static int32_t env_row_layout(const pcgrl_config* c, const pcgrl_state* st, int32_t n_pos, pcgrl_row_layout* l,
+                              RowCopy* rc) {
+    const int64_t K = c->n_stats, rs = c->row_stride;
+    std::memset(l, 0, sizeof(*l));
+    l->n_pos = n_pos;
+    if (rc) std::memset(rc, 0, sizeof(*rc));
+    int64_t off = 16;                  // the header
+    uint32_t h = 2166136261u;          // FNV-1a over the fields that give the row's bytes their meaning
+    auto mix = [&](int64_t v) {
+        for (int b = 0; b < 8; ++b) h = (h ^ (uint32_t)((uint64_t)v >> (8 * b) & 0xff)) * 16777619u;
+    };
+    // a section of `bytes` bytes (0: absent, offset -1) at the next 16-byte boundary
+    auto section = [&](int64_t bytes) -> int32_t {
+        mix(bytes);
+        if (!bytes) return -1;
+        const int64_t at = off;
+        off += (bytes + 15) / 16 * 16;
+        return (int32_t)at;
+    };
+    auto piece = [&](int32_t at, const void* base, int64_t item, int64_t count, int64_t item_stride) {
+        if (!rc || at < 0) return;
+        RowPiece& q = rc->piece[rc->n_pieces++];
+        q.base = const_cast<void*>(base);
+        q.off = at;
+        q.item = (int32_t)item;
+        q.count = (int32_t)count;
+        q.item_stride = item_stride;
+        const uint64_t m = (uint64_t)at | (uint64_t)item | (uintptr_t)base | (count > 1 ? (uint64_t)item_stride : 0) | 16;
+        q.unit = (int32_t)(m & (~m + 1));   // the lowest set bit
+    };
+    for (const int64_t v : {c->problem, c->representation, c->action_kind, c->ndim, c->n_tiles, c->n_stats, c->row_stride})
+        mix(v);
+    for (int i = 0; i < 3; ++i) mix(i < c->ndim ? c->dims[i] : 1);
+    const int64_t cs = st->worklist && st->cache ? cache_stride(c) : 0;   // the condition fill() uses
+    const int64_t rec = c->record_stat_bytes && st->records ? record_stride(c) : 0;
+    const int64_t hi = is_holey(c) ? hole_ints(c) : 0;
+    piece(l->grid = section(rs), st->grids, rs, 1, 0);
+    piece(l->static_mask = section(st->static_mask ? rs : 0), st->static_mask, rs, 1, 0);
+    piece(l->cache = section(cs), st->cache, cs, 1, 0);
+    piece(l->records = section(rec), st->records, rec, 1, 0);
+    piece(l->targets = section(c->targets_per_env ? 16 * K : 0), st->targets, 16 * K, 1, 0);
+    piece(l->stats = section(4 * K), st->stats, 4 * K, 1, 0);
+    piece(l->holes = section(4 * hi), st->holes, 4 * hi, 1, 0);
+    piece(l->pos = section(12 * (int64_t)n_pos), st->pos, 12, n_pos, 12 * st->n_envs);   // agent a's array: pos + a * N * 3
+    l->n_step = section(12);
+    l->iteration = l->n_step + 4;
+    l->changes = l->n_step + 8;
+    piece(l->n_step, st->n_step, 4, 1, 0);
+    piece(l->iteration, st->iteration, 4, 1, 0);
+    piece(l->changes, st->changes, 4, 1, 0);
+    l->reward = section(st->changed ? 6 : 5);
+    l->done = l->reward + 4;
+    l->changed = st->changed ? l->reward + 5 : -1;
+    piece(l->reward, st->reward, 4, 1, 0);
+    piece(l->done, st->done, 1, 1, 0);
+    piece(l->changed, st->changed, 1, 1, 0);
+    if (off > INT32_MAX) return fail(PCGRL_E_ARG, "row too large (n_pos)");
+    l->row_bytes = (int32_t)off;
+    l->signature = h ? h : 1;          // an all-zero header is never valid
+    if (rc) {
+        rc->row_bytes = l->row_bytes;
+        rc->signature = l->signature;
+        rc->n_envs = st->n_envs;
+        rc->status = st->status;
+    }
+    return 0;
+}
 }  // namespace pcgrl
 
 using namespace pcgrl;
@@ -677,6 +749,56 @@ int32_t pcgrl_step_envs(const pcgrl_config* cfg, const pcgrl_state* st, const vo
         return cuda_fail(e, "step_envs scatter launch");
     g_launches.fetch_add(1, std::memory_order_relaxed);
     return 0;
+}
+
+static int32_t check_rows_shard(const pcgrl_config* cfg, const pcgrl_state* st, int32_t n_pos) {
+    int r = check(cfg);
+    if (r) return r;
+    if ((r = check_state(st))) return r;
+    if (n_pos < 1) return fail(PCGRL_E_ARG, "n_pos must be >= 1");
+    if (is_holey(cfg) && !st->holes) return fail(PCGRL_E_ARG, "a holey problem needs pcgrl_state.holes");
+    return 0;
+}
+
+int32_t pcgrl_env_row_layout(const pcgrl_config* cfg, const pcgrl_state* st, int32_t n_pos, pcgrl_row_layout* out) {
+    int r = check_rows_shard(cfg, st, n_pos);
+    if (r) return r;
+    if (!out) return fail(PCGRL_E_ARG, "out is NULL");
+    return env_row_layout(cfg, st, n_pos, out, nullptr);
+}
+
+// Shared body of pcgrl_save_envs / pcgrl_load_envs: every check before any CUDA call, then one launch.
+static int32_t env_rows_impl(const pcgrl_config* cfg, const pcgrl_state* st, int32_t n_pos, const void* rows,
+                             const int32_t* env_idx, int64_t n, void* stream, bool save) {
+    int r = check_rows_shard(cfg, st, n_pos);
+    if (r) return r;
+    if (n < 0 || n > INT32_MAX) return fail(PCGRL_E_ARG, "n must be in [0, 2^31)");
+    if (!env_idx && n > st->n_envs) return fail(PCGRL_E_ARG, "without env_idx row j is env j: n > n_envs");
+    if (!save && n > st->n_envs) return fail(PCGRL_E_ARG, "load: n distinct env indices: n > n_envs");
+    if (n > 0 && !rows) return fail(PCGRL_E_ARG, "rows is NULL");
+    if ((uintptr_t)rows % 16) return fail(PCGRL_E_ARG, "rows must be 16-byte aligned");
+    pcgrl_row_layout l;
+    RowCopy rc;
+    if ((r = env_row_layout(cfg, st, n_pos, &l, &rc))) return r;
+    if (n * (l.row_bytes / 16) / 256 >= INT32_MAX) return fail(PCGRL_E_ARG, "too many rows for one launch");
+    if (n == 0) return 0;   // nothing to write, nothing launched
+    rc.rows = (uint8_t*)const_cast<void*>(rows);
+    rc.env_idx = env_idx;
+    rc.n_rows = n;
+    const cudaError_t e = save ? launch_save_envs(rc, (cudaStream_t)stream) : launch_load_envs(rc, (cudaStream_t)stream);
+    if (e != cudaSuccess) return cuda_fail(e, save ? "save_envs launch" : "load_envs launch");
+    g_launches.fetch_add(1, std::memory_order_relaxed);
+    return 0;
+}
+
+int32_t pcgrl_save_envs(const pcgrl_config* cfg, const pcgrl_state* st, int32_t n_pos, const int32_t* env_idx,
+                        int64_t n, void* rows, void* stream) {
+    return env_rows_impl(cfg, st, n_pos, rows, env_idx, n, stream, true);
+}
+
+int32_t pcgrl_load_envs(const pcgrl_config* cfg, const pcgrl_state* st, int32_t n_pos, const void* rows,
+                        const int32_t* env_idx, int64_t n, void* stream) {
+    return env_rows_impl(cfg, st, n_pos, rows, env_idx, n, stream, false);
 }
 
 // Shared body of pcgrl_step_host / pcgrl_step_host_packed: with records_host the only download is the packed

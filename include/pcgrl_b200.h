@@ -135,7 +135,8 @@ typedef struct pcgrl_state {
     int32_t* stats;        /* [N, K] current _rep_stats; read (old) and written (new) by step */
     const double* targets; /* [N or 1, K, 2] (lo, hi): hi = NaN -> scalar target lo, else the integer range
                               np.arange(lo, hi) (control_wrappers.py:336-343).  With PCGRL_REWARD_RANGE: the
-                              (lo, hi) band of get_range_reward for each stat */
+                              (lo, hi) band of get_range_reward for each stat.  `const`: no step writes it;
+                              pcgrl_load_envs is the one call that writes its rows (cfg.targets_per_env only) */
     float*   reward;       /* [N] out: loss(new stats) - loss(old stats), evaluated in fp64 */
     uint8_t* done;         /* [N] out: done == truncated (pcgrl_env.py:307-310) */
     uint8_t* changed;      /* [N] out, may be NULL: 1 if the map changed (stats were recomputed) */
@@ -146,7 +147,9 @@ typedef struct pcgrl_state {
                               bit4 (16) a stat did not fit cfg.record_stat_bytes in the packed record; bit5 (32)
                               is retired; bit6 (64) pcgrl_observe_envs: an env index outside [0, n_envs); bit7 (128)
                               pcgrl_lookahead: an env index outside [0, n_envs); bit8 (256) pcgrl_step_envs: an
-                              env index outside [0, n_envs) */
+                              env index outside [0, n_envs); bit9 (512) pcgrl_save_envs / pcgrl_load_envs: an env index
+                              outside [0, n_envs); bit10 (1024) pcgrl_load_envs: a row whose header does not match this
+                              shard's row layout */
     void*    scratch;      /* pcgrl_scratch_bytes() bytes, may be NULL when that returns 0.  Must be zero-filled
                               once before its first use (it holds hash-table generation counters, solver job
                               lists and, for smb, 4 bytes per env of playthrough-length history, which is why
@@ -314,6 +317,48 @@ int32_t pcgrl_lookahead(const pcgrl_config* cfg, const pcgrl_state* st, const vo
 int64_t pcgrl_step_envs_work_bytes(const pcgrl_config* cfg, int64_t n);
 int32_t pcgrl_step_envs(const pcgrl_config* cfg, const pcgrl_state* st, const void* actions, const int32_t* env_idx,
                         int64_t n, void* work, void* stream);
+
+/* -- packed env rows: save, load and fork individual envs ------------------------------------------------------------
+ * The whole state of one env as one row of row_bytes bytes (a multiple of 16), for beam search / MCTS over edits
+ * (copy the best children over the rest), Go-Explore archives, elite copies and fixed mid-episode start states.
+ *   header (16 bytes)  uint32 signature, uint32 row_bytes, 8 zero bytes.  The signature is a 32-bit FNV-1a hash of
+ *                      problem, representation, action_kind, ndim, dims, n_tiles, n_stats, row_stride and the size of
+ *                      every section (0 = absent); never 0, so an all-zero row never loads.  Episode and reward
+ *                      parameters (max_iterations, max_changes, weights, reward_mode, init / static probabilities) are
+ *                      not in it: a row loads under another budget.
+ *   sections           each on a 16-byte boundary of the row, present only where the shard has them, in this order:
+ *                      grid (row_stride), frozen-tile mask (st->static_mask), search-cache row (st->worklist and
+ *                      st->cache set and pcgrl_cache_stride(cfg) > 0), packed record (cfg.record_stat_bytes and
+ *                      st->records), per-env targets (cfg.targets_per_env), stats, holes (holey problems), positions
+ *                      (n_pos int32 triples), n_step | iteration | changes, reward | done | changed (st->changed set).
+ * Not in the row: the scratch (smb's per-env playthrough-length history only picks a job class, never a result) and
+ * the work list, shared [1, K, 2] targets, and the reset RNG position (seed and epoch belong to the shard).
+ * n_pos: the number of position arrays, [n_envs, 3] int32 each, laid back to back from st->pos (one per agent of a
+ * multi-agent turtle shard; 1 for a single agent).  n_pos < 1 is PCGRL_E_ARG. */
+typedef struct pcgrl_row_layout {
+    int32_t  row_bytes;
+    uint32_t signature;
+    int32_t  n_pos;
+    /* byte offsets into the row, -1 = section absent */
+    int32_t  grid, static_mask, cache, records, targets, stats, holes, pos, n_step, iteration, changes,
+             reward, done, changed;
+} pcgrl_row_layout;
+/* Host only (no CUDA call): the row layout of this shard. */
+int32_t pcgrl_env_row_layout(const pcgrl_config* cfg, const pcgrl_state* st, int32_t n_pos, pcgrl_row_layout* out);
+/* Row j of `rows` (a DEVICE array of n rows) = env env_idx[j] (a DEVICE array of n int32; NULL: env j, n <= n_envs).
+ * Any order, duplicates allowed; n == 0 launches nothing.  An index outside [0, n_envs) loads nothing: its row is
+ * written as zeros, header included, so it can never be loaded, and status bit 512 is set.  One launch. */
+int32_t pcgrl_save_envs(const pcgrl_config* cfg, const pcgrl_state* st, int32_t n_pos, const int32_t* env_idx,
+                        int64_t n, void* rows, void* stream);
+/* Env env_idx[j] gets row j of `rows` (NULL env_idx: env j, n <= n_envs): afterwards it is bit for bit the env the row
+ * was saved from, in every section the row has; every env that is not listed is untouched.  The indices must be
+ * DISTINCT (a precondition the library does not check).  n == 0 launches nothing.  An index outside [0, n_envs) writes
+ * nothing and sets status bit 512; a row whose signature or row_bytes does not match this shard's layout writes nothing
+ * to that env and sets status bit 1024.  Writes st->targets rows when cfg.targets_per_env is set.  One launch.
+ * A fork (env dst[j] becomes a copy of env src[j]) is pcgrl_save_envs of src into a buffer, then this call with dst:
+ * src and dst may overlap. */
+int32_t pcgrl_load_envs(const pcgrl_config* cfg, const pcgrl_state* st, int32_t n_pos, const void* rows,
+                        const int32_t* env_idx, int64_t n, void* stream);
 
 /* -- host-buffer convenience (the end-to-end path timed as `e2e` in bench.py) ------------------ */
 /* Copies `actions` (host, pinned or pageable) to `actions_dev`, runs pcgrl_step, copies reward/done/stats
