@@ -94,6 +94,10 @@ SYMBOLS = {
     "pcgrl_lookahead_work_bytes": (C.c_int64, [C.POINTER(Config), C.c_int64]),
     "pcgrl_lookahead": (C.c_int32, [C.POINTER(Config), C.POINTER(State), C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p,
                                     C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
+    "pcgrl_lookahead_obs_work_bytes": (C.c_int64, [C.POINTER(Config), C.c_int64]),
+    "pcgrl_lookahead_obs": (C.c_int32, [C.POINTER(Config), C.POINTER(State), C.POINTER(ObsArgs), C.c_void_p, C.c_void_p,
+                                        C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
+                                        C.c_void_p]),
     "pcgrl_step_envs_work_bytes": (C.c_int64, [C.POINTER(Config), C.c_int64]),
     "pcgrl_step_envs": (C.c_int32, [C.POINTER(Config), C.POINTER(State), C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p,
                                     C.c_void_p]),

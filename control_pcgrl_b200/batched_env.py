@@ -503,7 +503,8 @@ class BatchedPcgrlEnv:
         return self.changed
 
     # ------------------------------------------------------------------ lookahead
-    def lookahead(self, actions: torch.Tensor, env_ids=None, agent: int = 0):
+    def lookahead(self, actions: torch.Tensor, env_ids=None, agent: int = 0, obs_dtype=None, onehot: bool = True,
+                  obs_out: torch.Tensor | None = None):
         """What step() would return for a list of (env, action) candidates, without stepping.  Candidate j pairs env
         env_ids[j] (j when env_ids is None) with row j of `actions` (the step layout with M rows, M = len(env_ids) or
         n_envs).  Returns fresh device tensors (reward[M] f32, done[M] u8, stats[M, K] i32, changed[M] u8): the
@@ -511,7 +512,12 @@ class BatchedPcgrlEnv:
         next.  Indices may come in any order and repeat.  agent: with n_agents > 1, whose turtle would act.
         Nothing of the env changes, except that check_status() then reports what such a step would (an invalid
         action: ValueError); no auto-reset.  A bad env index raises IndexError before anything is launched (a device
-        tensor costs one reduction and one sync for that check)."""
+        tensor costs one reduction and one sync for that check).
+        obs_dtype / obs_out: also return the observation [M, *obs_shape] as a fifth tensor, row j byte for byte what
+        observe(dtype=obs_dtype, onehot=onehot, agent=agent) would return for that env right after that step
+        (pcgrl_lookahead_obs): target planes from the candidate's new stats, the terminal observation of a candidate
+        that would end the episode.  obs_out, a contiguous [M, *obs_shape] tensor, receives it; onehot=False is the
+        uint8 tile codes, as for observe()."""
         self._check_fresh("lookahead")
         rows = None if env_ids is None else self._check_env_ids(env_ids)
         m = self.n_envs if rows is None else rows.numel()
@@ -519,17 +525,49 @@ class BatchedPcgrlEnv:
         K = self.K
         out = (torch.empty(m, dtype=torch.float32, device=self.device), torch.empty(m, dtype=torch.uint8, device=self.device),
                torch.empty((m, K), dtype=torch.int32, device=self.device), torch.empty(m, dtype=torch.uint8, device=self.device))
-        self._lookahead(a, rows, m, agent, *out)
-        return out
+        if obs_dtype is None and obs_out is None:
+            self._lookahead(a, rows, m, agent, *out)
+            return out
+        return (*out, self._lookahead_obs(a, rows, m, agent, out, obs_out, obs_dtype or torch.float32, onehot))
 
-    def _lookahead(self, a, rows, m, agent, reward, done, stats, changed):
+    def _lookahead(self, a, rows, m, agent, reward, done, stats, changed, obs=None):
+        """pcgrl_lookahead, or with `obs` (pcgrl_obs_args) pcgrl_lookahead_obs."""
         if m == 0:
             return
-        work = self._work(int(self.lib.pcgrl_lookahead_work_bytes(self._cc, m)))
+        st = self._agent_state(agent)
+        if obs is None:
+            work = self._work(int(self.lib.pcgrl_lookahead_work_bytes(self._cc, m)))
+            with self._on_device():
+                _lib.check(self.lib.pcgrl_lookahead(self._cc, st, a.data_ptr(), _ptr(rows), m, reward.data_ptr(),
+                                                    done.data_ptr(), changed.data_ptr(), stats.data_ptr(),
+                                                    work.data_ptr(), self._stream()), "pcgrl_lookahead")
+            return
+        work = self._work(int(self.lib.pcgrl_lookahead_obs_work_bytes(self._cc, m)))
         with self._on_device():
-            _lib.check(self.lib.pcgrl_lookahead(self._cc, self._agent_state(agent), a.data_ptr(), _ptr(rows), m,
-                                                reward.data_ptr(), done.data_ptr(), changed.data_ptr(), stats.data_ptr(),
-                                                work.data_ptr(), self._stream()), "pcgrl_lookahead")
+            _lib.check(self.lib.pcgrl_lookahead_obs(self._cc, st, obs, a.data_ptr(), _ptr(rows), m, reward.data_ptr(),
+                                                    done.data_ptr(), changed.data_ptr(), stats.data_ptr(),
+                                                    work.data_ptr(), self._stream()), "pcgrl_lookahead_obs")
+
+    def _lookahead_obs(self, a, rows, m, agent, outs, obs_out, dtype, onehot):
+        """_lookahead with the observation: -> obs [m, *obs_shape]."""
+        final, ob, oa = self._obs_buffers(m, obs_out, dtype, onehot)
+        self._lookahead(a, rows, m, agent, *outs, obs=oa)
+        occ = None
+        if self.show_agents:
+            ids = torch.arange(m, device=self.device) if rows is None else rows
+            occ = self._agent_occupancy(agent, ob.shape[1:-1], ob.dtype, ids, self._turtle_after(a, ids, agent))
+        return self._obs_finish(final, ob, occ)
+
+    def _turtle_after(self, a, rows, agent):
+        """[M, 3]: where agent `agent`'s turtle stands after action a[j] in env rows[j] (reps/turtle_rep.py:87-107:
+        0..3 move along axis 0 / 1, clamped to the map; a write or an invalid action stays).  The library returns no
+        positions, and multi-agent envs are turtle-only, so the occupancy plane of a lookahead takes them from here."""
+        pos = self.agent_pos[agent][rows.long()].long()
+        a = a.reshape(-1).to(torch.int64)
+        for axis in (0, 1):
+            step = (a == 2 * axis + 1).long() - (a == 2 * axis).long()
+            pos[:, axis] = (pos[:, axis] + step).clamp(0, self.map_shape[axis] - 1)
+        return pos
 
     def _work(self, need):
         """The work buffer of lookahead and of step(env_ids=...), at least `need` bytes (both keep the solver scratch at
@@ -542,6 +580,7 @@ class BatchedPcgrlEnv:
 
     _la_work = None
     LOOKAHEAD_CHUNK = 1 << 22     # candidates per launch of lookahead_all: bounds the work buffer
+    LOOKAHEAD_OBS_CHUNK_BYTES = 1 << 30   # ... and the observation bytes of one launch (and its temporaries)
 
     def n_discrete_actions(self):
         """Size of the Discrete action space (narrow C, turtle 4 + C, flat wide act_h * act_w * C)."""
@@ -550,12 +589,16 @@ class BatchedPcgrlEnv:
         return {"narrow": self.n_tiles, "turtle": 4 + self.n_tiles}.get(
             self.representation, self._cc.act_h * self._cc.act_w * self.n_tiles)
 
-    def lookahead_all(self, env_ids=None, agent: int = 0):
+    def lookahead_all(self, env_ids=None, agent: int = 0, obs_dtype=None, onehot: bool = True):
         """lookahead() of every action of the Discrete action space for each env of env_ids (default all): returns
         reward [M, A] f32, done [M, A] u8, stats [M, A, K] i32 and changed [M, A] u8, column a being action a.
         Runs in chunks of at most LOOKAHEAD_CHUNK candidates, env-major, without a host sync (env_ids=None).
         Raises ValueError for cellular, patch and wide-coordinate actions, and for flat wide actions whose ActionMap
-        (act_h, act_w) reaches past the map: part of that space is actions the reference rejects."""
+        (act_h, act_w) reaches past the map: part of that space is actions the reference rejects.
+        obs_dtype: also return obs [M, A, *obs_shape], lookahead()'s observation of every candidate; chunks then hold at
+        most LOOKAHEAD_OBS_CHUNK_BYTES of it.  Mind the size: it is M * A observations, so wide actions are expensive
+        (16 Ki binary-wide envs x 512 actions x 6 KB of float32 crop is about 50 GB).  It is meant for narrow and turtle
+        envs; elsewhere call lookahead() on chosen candidates."""
         self._check_fresh("lookahead_all")
         A = self.n_discrete_actions()
         if self.action_kind == "wide_flat":
@@ -570,15 +613,28 @@ class BatchedPcgrlEnv:
         stats = torch.empty((M, A, K), dtype=torch.int32, device=dev)
         changed = torch.empty((M, A), dtype=torch.uint8, device=dev)
         _, _, tdt = self._action_layout()
-        per = max(1, self.LOOKAHEAD_CHUNK // A)
+        per_cand = self.LOOKAHEAD_CHUNK
+        obs = None
+        if obs_dtype is not None:
+            oshape = self.obs_shape(onehot)
+            obs = torch.empty((M, A, *oshape), dtype=obs_dtype if onehot else torch.uint8, device=dev)
+            per_cand = max(1, min(per_cand, self.LOOKAHEAD_OBS_CHUNK_BYTES // (math.prod(oshape) * obs.element_size())))
+        per = max(1, per_cand // A)
         for lo in range(0, M, per):
             hi = min(M, lo + per)
             c = torch.arange((hi - lo) * A, dtype=torch.int32, device=dev)
             env = c // A + lo if rows is None else rows[lo:hi].repeat_interleave(A, output_size=(hi - lo) * A)
             acts = (c % A).to(tdt)
-            self._lookahead(acts, env.to(torch.int32).contiguous(), (hi - lo) * A, agent, reward[lo:hi], done[lo:hi],
-                            stats[lo:hi], changed[lo:hi])
-        return reward, done, stats, changed
+            env = env.to(torch.int32).contiguous()
+            outs = (reward[lo:hi], done[lo:hi], stats[lo:hi], changed[lo:hi])
+            if obs is None:
+                self._lookahead(acts, env, (hi - lo) * A, agent, *outs)
+            else:
+                self._lookahead_obs(acts, env, (hi - lo) * A, agent, outs, obs[lo:hi].view(-1, *oshape), obs.dtype,
+                                    onehot)
+        if obs is None:
+            return reward, done, stats, changed
+        return reward, done, stats, changed, obs
 
     def _check_fresh(self, what):
         if self._stats_stale:
@@ -904,12 +960,15 @@ class BatchedPcgrlEnv:
         ch += 1 if self.show_agents else 0                  # 'agent_occupancy' plane
         return (*dims, ch)
 
-    def _agent_occupancy(self, agent, dims, dtype, rows=None):
+    def _agent_occupancy(self, agent, dims, dtype, rows=None, acting_pos=None):
         """[N, *dims] (rows: [M] env indices -> [M, *dims]): 1 where any agent stands, in agent `agent`'s window
-        (Cropped pads this key with 0)."""
+        (Cropped pads this key with 0).  acting_pos: [M, 3] positions that replace agent `agent`'s own (a lookahead's
+        after-state)."""
         nd, dev = self.ndim, self.device
         sel = slice(None) if rows is None else rows.long()
         pos = self.agent_pos[:, sel, :nd].long()
+        if acting_pos is not None:
+            pos[agent] = acting_pos[:, :nd].long()
         occ = torch.zeros((pos.shape[1], *dims), dtype=dtype, device=dev)
         center = pos[agent]
         half = torch.tensor([d // 2 for d in dims], device=dev)
@@ -969,13 +1028,29 @@ class BatchedPcgrlEnv:
         return self._observe(out, dtype, onehot, agent, rows.to(device=self.device, dtype=torch.int32).contiguous())
 
     def _observe(self, out, dtype, onehot, agent, rows):
+        final, out, oa = self._obs_buffers(self.n_envs if rows is None else rows.numel(), out, dtype, onehot)
+        st = self._agent_state(agent)
+        if rows is None:
+            with self._on_device():
+                _lib.check(self.lib.pcgrl_observe(self._cc, st, oa, self._stream()), "pcgrl_observe")
+        elif rows.numel():
+            with self._on_device():
+                _lib.check(self.lib.pcgrl_observe_envs(self._cc, st, oa, rows.data_ptr(), rows.numel(), self._stream()),
+                           "pcgrl_observe_envs")
+        occ = self._agent_occupancy(agent, out.shape[1:-1], out.dtype, rows) if self.show_agents else None
+        return self._obs_finish(final, out, occ)
+
+    def _obs_buffers(self, m, out, dtype, onehot):
+        """Checks and buffers of an observation of m rows, before anything is launched: -> (final, out, oa).  The
+        kernel writes `out` (every channel but the occupancy plane) as pcgrl_obs_args `oa` describes; `final` is the
+        caller's tensor that _obs_finish completes, or None."""
         if self.ctrl_metrics:
             self._check_fresh("observe with control planes")
         if not onehot:
             if self.ctrl_metrics or (out is not None and out.dtype != torch.uint8):
                 raise ValueError("onehot=False is a uint8 observation without control planes")
             dtype = torch.uint8
-        shape = (self.n_envs if rows is None else rows.numel(), *self.obs_shape(onehot))
+        shape = (m, *self.obs_shape(onehot))
         final = None
         if self.show_agents:
             # the kernel writes the map (+ target / static) channels; the occupancy plane is appended here (a handful
@@ -1007,22 +1082,17 @@ class BatchedPcgrlEnv:
         oa.out_kind = {torch.uint8: 0, torch.float32: 1, torch.float64: 2}[out.dtype] if onehot else 3
         oa.out = out.data_ptr()
         oa.static_channel = 1 if self.static_mask is not None else 0
-        st = self._agent_state(agent)
-        if rows is None:
-            with self._on_device():
-                _lib.check(self.lib.pcgrl_observe(self._cc, st, oa, self._stream()), "pcgrl_observe")
-        elif rows.numel():
-            with self._on_device():
-                _lib.check(self.lib.pcgrl_observe_envs(self._cc, st, oa, rows.data_ptr(), rows.numel(), self._stream()),
-                           "pcgrl_observe_envs")
-        if self.show_agents:
-            occ = self._agent_occupancy(agent, shape[1:-1], out.dtype, rows)
-            if final is None:
-                return torch.cat([out, occ[..., None]], dim=-1)
-            final[..., :-1] = out
-            final[..., -1] = occ
-            return final
-        return out
+        return final, out, oa
+
+    def _obs_finish(self, final, out, occ):
+        """The observation: `out` with the occupancy plane `occ` appended (show_agents), into `final` if given."""
+        if not self.show_agents:
+            return out
+        if final is None:
+            return torch.cat([out, occ[..., None]], dim=-1)
+        final[..., :-1] = out
+        final[..., -1] = occ
+        return final
 
     STATUS_BITS = (
         (1, ValueError, "an action outside the action space reached pcgrl_step (ignored on device)"),

@@ -28,6 +28,7 @@ int64_t smb_scratch_bytes(int64_t n_envs);
 int64_t maze3d_scratch_bytes();
 cudaError_t launch_observe(const pcgrl_config& cfg, const pcgrl_state& st, const pcgrl_obs_args& o, cudaStream_t s,
                            const int32_t* env_idx, int64_t n_idx);
+const char* obs_args_error(const pcgrl_config& cfg, const pcgrl_state& st, const pcgrl_obs_args& a);
 cudaError_t launch_update(const KParams& p, cudaStream_t s);
 cudaError_t launch_lookahead_inc(const KParams& p, const LaOut& o, cudaStream_t s);
 cudaError_t launch_lookahead_gather(const pcgrl_state& shard, const pcgrl_state& sub, const int32_t* env_idx,
@@ -35,6 +36,7 @@ cudaError_t launch_lookahead_gather(const pcgrl_state& shard, const pcgrl_state&
                                     int status_bit, cudaStream_t s);
 cudaError_t launch_step_envs_scatter(const pcgrl_state& shard, const pcgrl_state& sub, const int32_t* env_idx,
                                      int row_stride, int K, int rec_stride, cudaStream_t s);
+cudaError_t launch_lookahead_apply(const KParams& p, const int32_t* env_idx, int64_t n_src, cudaStream_t s);
 
 // split step path: up to WL_CHUNKS host-pipeline chunks, one 16-int work-list header each at the front of
 // pcgrl_state.worklist
@@ -342,21 +344,24 @@ static int host_chunks(const pcgrl_config* cfg, int64_t n, bool packed) {
     if (n < (1 << 19)) return 2;
     return 4;
 }
-// Layout of the work buffer of the lookahead (n candidates) and of pcgrl_step_envs (n envs, `step`).  The first 256
-// bytes hold the work-list header of the incremental lookahead (only that path touches them).  Behind them, either the
-// incremental lookahead's work-list body or the generic path's solver scratch (at a fixed offset: it keeps generation
-// counters from call to call, so one zero-filled buffer serves both calls) and the sub-shard.  The step's sub-shard
-// also holds the outputs it writes back: stats, reward, done, changed and the packed records.
+// Layout of the work buffer of the lookahead (n candidates), of pcgrl_step_envs (n envs, `step`) and of
+// pcgrl_lookahead_obs (n candidates, `obs`).  The first 256 bytes hold the work-list header of the incremental lookahead
+// (only that path touches them).  Behind them, either the incremental lookahead's work-list body or the generic path's
+// solver scratch (at a fixed offset: it keeps generation counters from call to call, so one zero-filled buffer serves
+// every call) and the sub-shard.  The step's sub-shard also holds the outputs it writes back: stats, reward, done,
+// changed and the packed records.  The observation needs the sub-shard beside the incremental path's body, so there the
+// body goes behind the sub-shard.
 struct LaLayout {
     int64_t inc_body, scratch, grids, mask, pos, n_step, iteration, changes, targets, holes;
     int64_t stats, reward, done, changed, records, total;
 };
 static int64_t la_align(int64_t x) { return (x + 255) / 256 * 256; }
-static LaLayout la_layout(const pcgrl_config* c, int64_t n, bool step = false) {
+static LaLayout la_layout(const pcgrl_config* c, int64_t n, bool step = false, bool obs = false) {
     LaLayout l;
     const int64_t K = c->n_stats;
+    const int64_t inc_bytes = cache_stride(c) > 0 ? (2 + K + 1) * 4 * n : 0;
     l.inc_body = 256;
-    const int64_t inc_end = cache_stride(c) > 0 ? l.inc_body + la_align((2 + K + 1) * 4 * n) : 0;
+    const int64_t inc_end = inc_bytes ? l.inc_body + la_align(inc_bytes) : 0;
     l.scratch = 256;
     int64_t off = l.scratch + la_align(pcgrl_scratch_bytes(c, n));
     auto take = [&](int64_t bytes) {
@@ -377,7 +382,8 @@ static LaLayout la_layout(const pcgrl_config* c, int64_t n, bool step = false) {
     l.done = take(step ? n : 0);
     l.changed = take(step ? n : 0);
     l.records = take(step ? n * record_stride(c) : 0);
-    l.total = step ? off : std::max(off, inc_end);
+    if (obs) l.inc_body = take(inc_bytes);
+    l.total = step || obs ? off : std::max(off, inc_end);
     return l;
 }
 
@@ -656,9 +662,15 @@ int64_t pcgrl_lookahead_work_bytes(const pcgrl_config* cfg, int64_t n) {
     return la_layout(cfg, n).total;
 }
 
-int32_t pcgrl_lookahead(const pcgrl_config* cfg, const pcgrl_state* st, const void* actions, const int32_t* env_idx,
-                        int64_t n, float* reward, uint8_t* done, uint8_t* changed, int32_t* stats, void* work,
-                        void* stream) {
+int64_t pcgrl_lookahead_obs_work_bytes(const pcgrl_config* cfg, int64_t n) {
+    if (check(cfg) || n < 0) return -1;
+    return la_layout(cfg, n, false, true).total;
+}
+
+// Shared body of pcgrl_lookahead (obs NULL) and pcgrl_lookahead_obs: every check before any CUDA call.
+static int32_t lookahead_impl(const pcgrl_config* cfg, const pcgrl_state* st, const pcgrl_obs_args* obs,
+                              const void* actions, const int32_t* env_idx, int64_t n, float* reward, uint8_t* done,
+                              uint8_t* changed, int32_t* stats, void* work, void* stream) {
     int r = check(cfg);
     if (r) return r;
     if ((r = check_state(st))) return r;
@@ -667,35 +679,75 @@ int32_t pcgrl_lookahead(const pcgrl_config* cfg, const pcgrl_state* st, const vo
     if (n > 0 && (!actions || !reward || !done || !changed || !stats || !work))
         return fail(PCGRL_E_ARG, "actions, reward, done, changed, stats and work must not be NULL");
     if (is_holey(cfg) && !st->holes) return fail(PCGRL_E_ARG, "a holey problem needs pcgrl_state.holes");
+    if (obs) {
+        if (n > 0 && !obs->out) return fail(PCGRL_E_ARG, "obs->out is NULL");
+        if (obs->n_ctrl < 0 || obs->n_ctrl > PCGRL_MAX_STATS) return fail(PCGRL_E_ARG, "n_ctrl out of range");
+        if (obs->out_kind < 0 || obs->out_kind > 3) return fail(PCGRL_E_ARG, "out_kind out of range");
+        if (const char* m = obs_args_error(*cfg, *st, *obs)) return fail(PCGRL_E_ARG, m);
+    }
     if (n == 0) return 0;   // nothing to write, nothing launched
     KParams p;
     fill(p, cfg, st);
     uint8_t* w = (uint8_t*)work;
     const cudaStream_t s = (cudaStream_t)stream;
+    const LaLayout l = la_layout(cfg, n, false, obs != nullptr);
+    // the candidates' rows as a sub-shard of n envs; the lookahead's outputs are its stats / reward / done / changed
+    pcgrl_state sub = sub_shard(cfg, st, n, w, l);
+    sub.stats = stats;
+    sub.reward = reward;
+    sub.done = done;
+    sub.changed = changed;
+    auto gather = [&]() {
+        const cudaError_t e = launch_lookahead_gather(*st, sub, env_idx, cfg->row_stride, cfg->n_stats, hole_ints(cfg),
+                                                      cfg->targets_per_env != 0, 0, 128, s);
+        if (e != cudaSuccess) return cuda_fail(e, "lookahead gather launch");
+        g_launches.fetch_add(1, std::memory_order_relaxed);
+        return 0;
+    };
     cudaError_t e;
     if (p.cache) {   // the shard keeps a search cache: incremental searches from it
+        // the observation's copy of e's rows first: the gather writes e's old stats, the incremental path the new ones
+        if (obs && (r = gather())) return r;
         LaOut o{env_idx, st->n_envs, reward, done, changed, stats};
         p.mode = MODE_STEP;
         p.actions = actions;
         p.n_envs = n;
         p.records = nullptr;
         p.wl_hdr = (int32_t*)w;
-        p.worklist = (int32_t*)(w + la_layout(cfg, 0).inc_body);
+        p.worklist = (int32_t*)(w + l.inc_body);
         if ((e = launch_lookahead_inc(p, o, s)) != cudaSuccess) return cuda_fail(e, "lookahead launch");
         g_launches.fetch_add(3, std::memory_order_relaxed);
-        return 0;
+        if (!obs) return 0;
+        // the candidate's edit and position advance, on the copy
+        KParams q;
+        fill(q, cfg, &sub);
+        q.mode = MODE_STEP;
+        q.actions = actions;
+        if ((e = launch_lookahead_apply(q, env_idx, st->n_envs, s)) != cudaSuccess)
+            return cuda_fail(e, "lookahead apply launch");
+        g_launches.fetch_add(1, std::memory_order_relaxed);
+    } else {   // every other config: the ordinary step on the sub-shard
+        if ((r = gather())) return r;
+        if ((r = step_launch(cfg, &sub, actions, stream, nullptr, 0, 0))) return r;
+        if (!obs) return 0;
     }
-    // every other config: the candidates' rows as a sub-shard of n envs, then the ordinary step on it
-    pcgrl_state sub = sub_shard(cfg, st, n, w, la_layout(cfg, n));
-    sub.stats = stats;
-    sub.reward = reward;
-    sub.done = done;
-    sub.changed = changed;
-    if ((e = launch_lookahead_gather(*st, sub, env_idx, cfg->row_stride, cfg->n_stats, hole_ints(cfg),
-                                     cfg->targets_per_env != 0, 0, 128, s)) != cudaSuccess)
-        return cuda_fail(e, "lookahead gather launch");
+    // the after-states are rows 0..n-1 of the sub-shard: the unchanged observation writer on it
+    if ((e = launch_observe(*cfg, sub, *obs, s, nullptr, 0)) != cudaSuccess) return cuda_fail(e, "observe launch");
     g_launches.fetch_add(1, std::memory_order_relaxed);
-    return step_launch(cfg, &sub, actions, stream, nullptr, 0, 0);
+    return 0;
+}
+
+int32_t pcgrl_lookahead(const pcgrl_config* cfg, const pcgrl_state* st, const void* actions, const int32_t* env_idx,
+                        int64_t n, float* reward, uint8_t* done, uint8_t* changed, int32_t* stats, void* work,
+                        void* stream) {
+    return lookahead_impl(cfg, st, nullptr, actions, env_idx, n, reward, done, changed, stats, work, stream);
+}
+
+int32_t pcgrl_lookahead_obs(const pcgrl_config* cfg, const pcgrl_state* st, const pcgrl_obs_args* obs,
+                            const void* actions, const int32_t* env_idx, int64_t n, float* reward, uint8_t* done,
+                            uint8_t* changed, int32_t* stats, void* work, void* stream) {
+    if (!obs) return fail(PCGRL_E_ARG, "obs is NULL");
+    return lookahead_impl(cfg, st, obs, actions, env_idx, n, reward, done, changed, stats, work, stream);
 }
 
 int64_t pcgrl_step_envs_work_bytes(const pcgrl_config* cfg, int64_t n) {

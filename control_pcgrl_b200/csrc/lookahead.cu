@@ -15,6 +15,10 @@
 // Generic path, for every other config: k_la_gather copies each candidate's env rows into a sub-shard carved from
 // `work`, and api.cu runs the ordinary MODE_STEP on it.  pcgrl_step_envs takes the same path for shards without a work
 // list, and k_step_envs_scatter writes the stepped rows back to their envs.
+//
+// With the observation (pcgrl_lookahead_obs) every candidate's after-state is a row of the sub-shard, and api.cu runs
+// the unchanged observation writer on it.  The generic path leaves it there already; the incremental path runs
+// k_la_gather before its three launches and k_la_apply (the step's apply_action on the copy) after them.
 #include "pcgrl_device.cuh"
 #include "step_common.cuh"
 #include "worklist.cuh"
@@ -192,6 +196,22 @@ cudaError_t launch_step_envs_scatter(const pcgrl_state& shard, const pcgrl_state
                                      int row_stride, int K, int rec_stride, cudaStream_t s) {
     const SubShard g = sub_shard(shard, sub, env_idx, row_stride, K, 0, false, rec_stride, 0);
     k_step_envs_scatter<<<sub_blocks(g), LA_THREADS, 0, s>>>(g);
+    return cudaGetLastError();
+}
+
+// pcgrl_lookahead_obs on a shard with a search cache: the incremental lookahead gives the outputs but no grid, so
+// k_la_gather copies e's rows into the sub-shard and this kernel, a thread per candidate, applies the candidate's edit
+// and position advance to row j of the copy with the step's own decode (apply_action).  p: the sub-shard (n_envs =
+// the candidate count), actions = the candidates'.  A row gathered through a bad index stays as the gather left it.
+__global__ void __launch_bounds__(LA_THREADS) k_la_apply(const KParams p, const int32_t* env_idx, int64_t n_src) {
+    const int64_t j = (int64_t)blockIdx.x * LA_THREADS + threadIdx.x;
+    if (j >= p.n_envs) return;
+    if (env_idx && (uint64_t)env_idx[j] >= (uint64_t)n_src) return;
+    apply_action(p, j);
+}
+
+cudaError_t launch_lookahead_apply(const KParams& p, const int32_t* env_idx, int64_t n_src, cudaStream_t s) {
+    k_la_apply<<<(unsigned)((p.n_envs + LA_THREADS - 1) / LA_THREADS), LA_THREADS, 0, s>>>(p, env_idx, n_src);
     return cudaGetLastError();
 }
 

@@ -659,9 +659,30 @@ static cudaError_t launch_writers(const ObsParams& p, const ObsIdx& ix, int out_
     return cudaGetLastError();
 }
 
+// What launch_observe refuses (it then returns cudaErrorInvalidValue), as a message; NULL if it launches.  Host only,
+// so that pcgrl_lookahead_obs can check the observation before its first launch.
+const char* obs_args_error(const pcgrl_config& cfg, const pcgrl_state& st, const pcgrl_obs_args& a) {
+    const bool holey3d = cfg.problem == PCGRL_PROB_MINECRAFT_3D_HOLEY_MAZE || cfg.problem == PCGRL_PROB_MINECRAFT_3D_DUNGEON_HOLEY;
+    const bool holey = cfg.problem == PCGRL_PROB_BINARY_HOLEY || holey3d;
+    if (holey) {
+        if (!st.holes || cfg.ndim != (holey3d ? 3 : 2) || a.static_channel)
+            return "a holey problem's observation needs holes and has no static_builds plane";
+        if (a.holey_border_tile < 0 || a.holey_border_tile >= cfg.n_tiles) return "holey_border_tile out of range";
+    }
+    if (a.static_channel && (!a.crop || !st.static_mask)) return "the static_builds plane needs a crop and a static mask";
+    const int grow = holey ? 2 : 0;   // without a crop the whole (bordered) map is observed
+    const int o2 = cfg.ndim == 3 ? a.obs_dims[2] : 1, d2 = cfg.ndim == 3 ? cfg.dims[2] : 1;
+    if (!a.crop && (a.obs_dims[0] != cfg.dims[0] + grow || a.obs_dims[1] != cfg.dims[1] + grow ||
+                    o2 != d2 + (holey3d ? grow : 0)))
+        return "without a crop obs_dims must be the (bordered) map dims";
+    if ((a.out_kind == 0 || a.out_kind == 3) && a.n_ctrl > 0) return "uint8 observations have no target planes";
+    return nullptr;   // an out_kind outside 0..3 fails at the launch (and passes when there is nothing to write)
+}
+
 // env_idx: NULL observes every env of the shard into row env; else n_idx rows, row j showing env env_idx[j]
 cudaError_t launch_observe(const pcgrl_config& cfg, const pcgrl_state& st, const pcgrl_obs_args& a, cudaStream_t s,
                            const int32_t* env_idx, int64_t n_idx) {
+    if (obs_args_error(cfg, st, a)) return cudaErrorInvalidValue;
     ObsParams p;
     p.ndim = cfg.ndim;
     p.d0 = cfg.dims[0];
@@ -692,21 +713,12 @@ cudaError_t launch_observe(const pcgrl_config& cfg, const pcgrl_state& st, const
     const bool holey3d = cfg.problem == PCGRL_PROB_MINECRAFT_3D_HOLEY_MAZE || cfg.problem == PCGRL_PROB_MINECRAFT_3D_DUNGEON_HOLEY;
     const bool holey = cfg.problem == PCGRL_PROB_BINARY_HOLEY || holey3d;
     if (holey) {
-        if (!st.holes || cfg.ndim != (holey3d ? 3 : 2) || a.static_channel) return cudaErrorInvalidValue;
         p.hole_ints = holey3d ? 6 : 4;
-        if (a.holey_border_tile < 0 || a.holey_border_tile >= cfg.n_tiles) return cudaErrorInvalidValue;
         p.holes = st.holes;
         p.border_tile = a.holey_border_tile;
     }
-    p.static_mask = nullptr;
-    if (a.static_channel) {
-        if (!a.crop || !st.static_mask) return cudaErrorInvalidValue;
-        p.static_mask = st.static_mask;
-    }
+    p.static_mask = a.static_channel ? st.static_mask : nullptr;
     p.out = a.out;
-    const int grow = holey ? 2 : 0;   // without a crop the whole (bordered) map is observed
-    if (!a.crop && (p.o0 != p.d0 + grow || p.o1 != p.d1 + grow || p.o2 != p.d2 + (holey3d ? grow : 0))) return cudaErrorInvalidValue;
-    if ((a.out_kind == 0 || a.out_kind == 3) && a.n_ctrl > 0) return cudaErrorInvalidValue;  // target planes are fractional
     const int64_t total = p.n_envs * (int64_t)p.o0 * p.o1 * p.o2;
     if (total == 0) return cudaSuccess;
     return env_idx ? launch_writers<true>(p, ObsIdx{env_idx, st.n_envs, st.status}, a.out_kind, holey3d, total, s)

@@ -298,6 +298,26 @@ int32_t pcgrl_lookahead(const pcgrl_config* cfg, const pcgrl_state* st, const vo
                         int64_t n, float* reward, uint8_t* done, uint8_t* changed, int32_t* stats, void* work,
                         void* stream);
 
+/* One-step lookahead with the observation: pcgrl_lookahead's arguments and outputs (reward, done, changed and stats
+ * exactly as it returns them) plus obs (pcgrl_obs_args as for pcgrl_observe, obs->out [n, *obs_dims, channels]).  Row j
+ * of obs->out is byte for byte what pcgrl_observe would write for env e = env_idx[j] (or j) right after pcgrl_step gave
+ * that env action row j: crop or whole map, one-hot or tile codes, target planes from the candidate's NEW stats and e's
+ * targets, the static_builds plane from e's frozen mask, the holey bordered map with e's holes.  A candidate that would
+ * end the episode shows its terminal observation (no auto-reset).  Nothing of the shard changes except st->status, as
+ * for pcgrl_lookahead; an index outside the shard loads nothing, sets bit 128 and leaves that row unspecified.  The
+ * observation arguments are checked before anything is launched; n == 0 launches nothing.
+ *   work  pcgrl_lookahead_obs_work_bytes(cfg, n) bytes (or more), zero-filled once before its first use, not shared by
+ *         launches that can run concurrently.  One buffer of the largest of pcgrl_lookahead_work_bytes,
+ *         pcgrl_step_envs_work_bytes and this size serves all three calls (the solver scratch sits at the same offset).
+ * Every candidate's after-state becomes a row of a sub-shard inside `work`, and the ordinary observation writer runs on
+ * it.  A shard with a search cache keeps pcgrl_lookahead's three incremental launches for reward / done / changed /
+ * stats, then copies e's rows and applies the edit and position advance on the copy (two launches); every other shard
+ * steps the sub-shard as pcgrl_lookahead does.  Then one observation launch. */
+int64_t pcgrl_lookahead_obs_work_bytes(const pcgrl_config* cfg, int64_t n);
+int32_t pcgrl_lookahead_obs(const pcgrl_config* cfg, const pcgrl_state* st, const pcgrl_obs_args* obs,
+                            const void* actions, const int32_t* env_idx, int64_t n, float* reward, uint8_t* done,
+                            uint8_t* changed, int32_t* stats, void* work, void* stream);
+
 /* Step a list of envs of the shard in place, leaving every other env untouched.  env_idx is a DEVICE array of n
  * DISTINCT int32 env indices (a precondition the library does not check; n <= st->n_envs), in any order, and env
  * e = env_idx[j] takes action row j of `actions` (the pcgrl_step layout, n rows).  Env e gets exactly what pcgrl_step
