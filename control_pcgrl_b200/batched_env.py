@@ -519,6 +519,8 @@ class BatchedPcgrlEnv:
         that would end the episode.  obs_out, a contiguous [M, *obs_shape] tensor, receives it; onehot=False is the
         uint8 tile codes, as for observe()."""
         self._check_fresh("lookahead")
+        if obs_dtype is not None and onehot:
+            self._check_obs_dtype(obs_dtype)
         rows = None if env_ids is None else self._check_env_ids(env_ids)
         m = self.n_envs if rows is None else rows.numel()
         a = self._check_actions(actions, m)
@@ -597,9 +599,11 @@ class BatchedPcgrlEnv:
         (act_h, act_w) reaches past the map: part of that space is actions the reference rejects.
         obs_dtype: also return obs [M, A, *obs_shape], lookahead()'s observation of every candidate; chunks then hold at
         most LOOKAHEAD_OBS_CHUNK_BYTES of it.  Mind the size: it is M * A observations, so wide actions are expensive
-        (16 Ki binary-wide envs x 512 actions x 6 KB of float32 crop is about 50 GB).  It is meant for narrow and turtle
-        envs; elsewhere call lookahead() on chosen candidates."""
+        (16 Ki binary-wide envs x 512 actions x 6 KB of float32 crop is about 50 GB; bfloat16 halves that).  It is meant
+        for narrow and turtle envs; elsewhere call lookahead() on chosen candidates."""
         self._check_fresh("lookahead_all")
+        if obs_dtype is not None and onehot:
+            self._check_obs_dtype(obs_dtype)
         A = self.n_discrete_actions()
         if self.action_kind == "wide_flat":
             # action (y, x, v): the write goes to _map[x, y], so x must be a row and y a column (wrappers.py:304-323)
@@ -984,6 +988,9 @@ class BatchedPcgrlEnv:
                 env_ids=None):
         """The wrapped observation of every env: [N, *obs_dims, channels] (channels last), exactly what
         CroppedImagePCGRLWrapper / ActionMapImagePCGRLWrapper + ControlWrapper return per env.
+        dtype: uint8 (no control planes), float32, float64, or float16 / bfloat16 for a policy that runs in half
+        precision -- byte for byte the float32 observation converted (round to nearest even), written directly at 2
+        bytes per element.  Any other dtype raises TypeError before anything is allocated or launched.
         onehot=False (uint8 only, no controls): the tile codes of the crop instead of their one-hot records --
         Cropped's own output (wrappers.py:407-437: 0 = out of bounds, tile t -> t + 1), one channel, for policies
         that embed the tile themselves (SURVEY 8f rank 3).
@@ -1061,6 +1068,7 @@ class BatchedPcgrlEnv:
             if final is not None:
                 dtype = final.dtype
             shape = (*shape[:-1], shape[-1] - 1)
+        self._check_obs_dtype(dtype if out is None else out.dtype)
         if out is None:
             out = torch.empty(shape, dtype=dtype, device=self.device)
         if tuple(out.shape) != shape or not out.is_contiguous():
@@ -1079,10 +1087,18 @@ class BatchedPcgrlEnv:
         for i, k in enumerate(self.ctrl_metrics):
             oa.ctrl_idx[i] = self.stat_names.index(k)
             oa.ctrl_range[i] = float(self.param_ranges[k])
-        oa.out_kind = {torch.uint8: 0, torch.float32: 1, torch.float64: 2}[out.dtype] if onehot else 3
+        oa.out_kind = self.OBS_KINDS[out.dtype] if onehot else 3
         oa.out = out.data_ptr()
         oa.static_channel = 1 if self.static_mask is not None else 0
         return final, out, oa
+
+    # element type of a one-hot observation -> pcgrl_obs_args.out_kind (tile codes are uint8, kind 3).  float16 and
+    # bfloat16 are the float32 observation rounded to nearest even, for policies that run in half precision.
+    OBS_KINDS = {torch.uint8: 0, torch.float32: 1, torch.float64: 2, torch.float16: 5, torch.bfloat16: 6}
+
+    def _check_obs_dtype(self, dtype):
+        if dtype not in self.OBS_KINDS:
+            raise TypeError(f"observation dtype {dtype} is not one of {', '.join(map(str, self.OBS_KINDS))}")
 
     def _obs_finish(self, final, out, occ):
         """The observation: `out` with the occupancy plane `occ` appended (show_agents), into `final` if given."""

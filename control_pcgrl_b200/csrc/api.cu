@@ -682,7 +682,8 @@ static int32_t lookahead_impl(const pcgrl_config* cfg, const pcgrl_state* st, co
     if (obs) {
         if (n > 0 && !obs->out) return fail(PCGRL_E_ARG, "obs->out is NULL");
         if (obs->n_ctrl < 0 || obs->n_ctrl > PCGRL_MAX_STATS) return fail(PCGRL_E_ARG, "n_ctrl out of range");
-        if (obs->out_kind < 0 || obs->out_kind > 3) return fail(PCGRL_E_ARG, "out_kind out of range");
+        if ((obs->out_kind < 0 || obs->out_kind > 3) && obs->out_kind != 5 && obs->out_kind != 6)
+            return fail(PCGRL_E_ARG, "out_kind out of range");
         if (const char* m = obs_args_error(*cfg, *st, *obs)) return fail(PCGRL_E_ARG, m);
     }
     if (n == 0) return 0;   // nothing to write, nothing launched

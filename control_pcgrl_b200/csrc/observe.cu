@@ -9,9 +9,27 @@
 // One thread per output pixel writes all of its channels (channels-last => contiguous per thread, and
 // consecutive threads write consecutive pixels => coalesced stores).  The int8 grid rows are re-read
 // through L1/L2; nothing else is loaded.
+#include <cuda_bf16.h>
+#include <cuda_fp16.h>
+
+#include <type_traits>
+
 #include "pcgrl_device.cuh"
 
 namespace pcgrl {
+
+// An element of type T from a plane value or a small integer.  The 2-byte types (float16, bfloat16) round the FLOAT32
+// element to nearest even, so a half observation is byte for byte the float32 one converted: x / range is rounded to
+// float first.  (A double converted straight to a half type rounds once and differs on rare ties.)
+template <typename T, typename S>
+__device__ __forceinline__ T obs_elem(S x) {
+    if constexpr (std::is_same_v<T, __half>) return __float2half_rn((float)x);
+    else if constexpr (std::is_same_v<T, __nv_bfloat16>) return __float2bfloat16_rn((float)x);
+    else return (T)x;
+}
+// the 16 bits of 1.0 in a 2-byte element type
+template <typename T>
+__host__ __device__ constexpr uint32_t half_one_bits() { return std::is_same_v<T, __half> ? 0x3C00u : 0x3F80u; }
 
 struct ObsParams {
     int32_t ndim, d0, d1, d2, row_stride, n_tiles, n_stats;
@@ -67,7 +85,7 @@ __global__ void __launch_bounds__(256) k_observe(const ObsParams p, const ObsIdx
         const int64_t env = obs_src<IDX>(ix, row);
         if (IDX && env < 0) {   // bad index: a zero record, nothing loaded
             if (r == 0) obs_flag_bad_index(ix);
-            for (int c = 0; c < n_ch; ++c) ((T*)p.out)[i * n_ch + c] = (T)0;
+            for (int c = 0; c < n_ch; ++c) ((T*)p.out)[i * n_ch + c] = obs_elem<T>(0);
             continue;
         }
         const int q2 = r % p.o2;
@@ -146,16 +164,16 @@ __global__ void __launch_bounds__(256) k_observe(const ObsParams p, const ObsIdx
             const double* trg = p.targets + ((p.targets_per_env ? env * p.n_stats : 0) + k) * 2;
             double t = trg[0];
             if (!isnan(trg[1])) t = (trg[0] + trg[1]) / 2;
-            o[2 * c] = (T)(t / p.ctrl_range[c]);
-            o[2 * c + 1] = (T)((double)p.stats[env * p.n_stats + k] / p.ctrl_range[c]);
+            o[2 * c] = obs_elem<T>(t / p.ctrl_range[c]);
+            o[2 * c + 1] = obs_elem<T>((double)p.stats[env * p.n_stats + k] / p.ctrl_range[c]);
         }
         o += 2 * p.n_ctrl;
         if (p.raw) {
-            o[0] = (T)hot;
+            o[0] = obs_elem<T>(hot);
         } else {
-            for (int c = 0; c < n_map_ch; ++c) o[c] = (T)(c == hot ? 1 : 0);
+            for (int c = 0; c < n_map_ch; ++c) o[c] = obs_elem<T>(c == hot ? 1 : 0);
         }
-        if (p.static_mask) o[n_map_ch] = (T)frozen;
+        if (p.static_mask) o[n_map_ch] = obs_elem<T>(frozen);
     }
 }
 
@@ -212,13 +230,15 @@ __global__ void __launch_bounds__(OBS_THREADS) k_observe_staged(const ObsParams 
     const bool pack3 = sizeof(T) == 1 && R8 && !STATIC && v.n_ch == 3 && !p.raw && n_pl == 0;
     // uint8 tile codes (one byte per pixel): 8 pixels are one 64-bit word
     const bool pack1 = sizeof(T) == 1 && R8 && !STATIC && v.n_ch == 1 && p.raw && n_pl == 0;
+    // 2-byte one-hot records of 3 channels on the row-mask path below: the u8 table's records, each byte widened
+    const bool wide3 = sizeof(T) == 2 && ROWN == 8 && v.bits != 0 && !STATIC && v.n_ch == 3 && !p.raw && n_pl == 0;
     // Two-tile maps behind a crop (binary: the headline observation).  75 % of a 32x32 window on a 16x16 map is
     // padding, and the in-map / padding split of a warp's pixel groups made every warp run both record builders
     // (157 instructions per 24-byte group, issue-bound at 0.63 of the HBM peak).  Instead: the trip's map rows are
     // kept as 16-bit masks, a group's 8 tile bits and 8 inside bits are two clamped funnel shifts of its row, and
     // the records of 4 pixels at a time come from a 256-entry table indexed by (inside nibble, tile nibble) --
     // one instruction stream for padding and map pixels alike.
-    const bool bits = v.bits != 0 && (pack3 || pack1);
+    const bool bits = v.bits != 0 && (pack3 || pack1 || wide3);
     uint16_t* s_rowbits = (uint16_t*)(obs_smem + v.lut_off + 256 * 16 + 256 * 4);   // [envs of the trip][d0]
     uint4* s_lut3 = (uint4*)(obs_smem + v.lut_off);                                  // 4 one-hot records (12 bytes)
     uint32_t* s_lut1 = (uint32_t*)(obs_smem + v.lut_off + 256 * 16);                 // 4 tile codes
@@ -241,7 +261,7 @@ __global__ void __launch_bounds__(OBS_THREADS) k_observe_staged(const ObsParams 
         if (tid == 0) asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory");
         __syncthreads();
         {
-            const int nz = (pack3 || pack1) ? 0 : (int)(((int64_t)n_here * v.E * (int64_t)sizeof(T) + 15) / 16);
+            const int nz = (pack3 || pack1 || wide3) ? 0 : (int)(((int64_t)n_here * v.E * (int64_t)sizeof(T) + 15) / 16);
             const uint4 z = make_uint4(0, 0, 0, 0);
             for (int i = tid; i < nz; i += OBS_THREADS) ((uint4*)stage)[i] = z;
             const int nv = n_here * (p.row_stride / 16);
@@ -316,15 +336,15 @@ __global__ void __launch_bounds__(OBS_THREADS) k_observe_staged(const ObsParams 
                 const int el = i / p.n_ctrl, c = i - el * p.n_ctrl;
                 const int64_t env = obs_src<IDX>(ix, env0 + el);
                 if (IDX && env < 0) {   // bad index: zero planes
-                    s_planes[el * n_pl + 2 * c] = s_planes[el * n_pl + 2 * c + 1] = (T)0;
+                    s_planes[el * n_pl + 2 * c] = s_planes[el * n_pl + 2 * c + 1] = obs_elem<T>(0);
                     continue;
                 }
                 const int k = p.ctrl_idx[c];
                 const double* trg = p.targets + ((p.targets_per_env ? env * p.n_stats : 0) + k) * 2;
                 double t = trg[0];
                 if (!isnan(trg[1])) t = (trg[0] + trg[1]) / 2;
-                s_planes[el * n_pl + 2 * c] = (T)(t / p.ctrl_range[c]);
-                s_planes[el * n_pl + 2 * c + 1] = (T)((double)p.stats[env * p.n_stats + k] / p.ctrl_range[c]);
+                s_planes[el * n_pl + 2 * c] = obs_elem<T>(t / p.ctrl_range[c]);
+                s_planes[el * n_pl + 2 * c + 1] = obs_elem<T>((double)p.stats[env * p.n_stats + k] / p.ctrl_range[c]);
             }
         }
         __syncthreads();
@@ -399,14 +419,29 @@ __global__ void __launch_bounds__(OBS_THREADS) k_observe_staged(const ObsParams 
                         o16[0] = make_uint4(w[0], w[1], w[2], w[3]);
                         o16[1] = make_uint4(w[4], w[5], w[6], w[7]);
                     }
-                } else if (sizeof(T) == 1 && ROWN == 8 && bits) {
+                } else if (ROWN == 8 && bits) {
                     // sl + 16 >= 0 (the window is at most 32 wide): bit k of the shifted row is map column sl + k
                     const uint32_t rb = row_ok ? (uint32_t)s_rowbits[el * p.d0 + c0 + (int)q0] : 0u;
                     const uint32_t inr = row_ok ? ((1u << p.d1) - 1u) : 0u;
                     const uint32_t t8 = __funnelshift_rc(rb << 16, 0u, (uint32_t)(sl + 16)) & 0xFFu;
                     const uint32_t in8 = __funnelshift_rc(inr << 16, 0u, (uint32_t)(sl + 16)) & 0xFFu;
                     const uint32_t ilo = ((in8 & 0xFu) << 4) | (t8 & 0xFu), ihi = (in8 & 0xF0u) | (t8 >> 4);
-                    if (pack3) {
+                    if constexpr (sizeof(T) == 2) {
+                        // byte k of a table record (0 or 1) becomes 16-bit lane k: 0 or the bits of 1.0; 8 records
+                        // are 48 bytes at a multiple of 48, three 128-bit stores
+                        const uint4 a = s_lut3[ilo], b = s_lut3[ihi];
+                        const uint32_t w[6] = {a.x, a.y, a.z, b.x, b.y, b.z};
+                        uint32_t h[12];
+#pragma unroll
+                        for (int j = 0; j < 6; ++j) {
+                            h[2 * j] = __byte_perm(w[j], 0u, 0x4140) * half_one_bits<T>();
+                            h[2 * j + 1] = __byte_perm(w[j], 0u, 0x4342) * half_one_bits<T>();
+                        }
+                        uint4* o16 = (uint4*)o;
+                        o16[0] = make_uint4(h[0], h[1], h[2], h[3]);
+                        o16[1] = make_uint4(h[4], h[5], h[6], h[7]);
+                        o16[2] = make_uint4(h[8], h[9], h[10], h[11]);
+                    } else if (pack3) {
                         const uint4 a = s_lut3[ilo], b = s_lut3[ihi];
                         uint2* o8 = (uint2*)o;
                         o8[0] = make_uint2(a.x, a.y);
@@ -458,7 +493,8 @@ __global__ void __launch_bounds__(OBS_THREADS) k_observe_staged(const ObsParams 
                     const bool inside = row_ok && (!CROP || (unsigned)(sl + k) < (unsigned)dl);
                     const int hot = inside ? rowp[sl + k] + (CROP ? 1 : 0) : 0;
                     for (int c = 0; c < n_pl; ++c) o[k * v.n_ch - n_pl + c] = s_planes[el * n_pl + c];
-                    o[k * v.n_ch + (p.raw ? 0 : hot)] = p.raw ? (T)hot : (T)1;
+                    if constexpr (sizeof(T) == 2) o[k * v.n_ch + hot] = obs_elem<T>(1);   // no 2-byte tile codes
+                    else o[k * v.n_ch + (p.raw ? 0 : hot)] = p.raw ? obs_elem<T>(hot) : obs_elem<T>(1);
                     if (STATIC) {   // see k_observe: the bordered frozen-tile mask through the same crop
                         const int s0 = c0 + (int)q0, s1 = D3 ? c1 + (int)q1 : sl + k, s2 = D3 ? sl + k : 0;
                         const int b0 = s0 - 1, b1 = s1 - 1, b2 = D3 ? s2 - 1 : 0;
@@ -468,7 +504,7 @@ __global__ void __launch_bounds__(OBS_THREADS) k_observe_staged(const ObsParams 
                             const bool inner = (unsigned)b0 < (unsigned)p.d0 && (unsigned)b1 < (unsigned)p.d1 &&
                                                (unsigned)b2 < (unsigned)p.d2;
                             if (!inner || s_mask[el * p.row_stride + (b0 * p.d1 + b1) * p.d2 + b2] != 0)
-                                o[k * v.n_ch + v.n_map_ch] = (T)1;
+                                o[k * v.n_ch + v.n_map_ch] = obs_elem<T>(1);
                         }
                     }
                 }
@@ -502,7 +538,8 @@ __global__ void __launch_bounds__(OBS_THREADS) k_observe_staged(const ObsParams 
                         hot = inside ? grid[cell] + (CROP ? 1 : 0) : 0;
                     }
                     for (int c = 0; c < n_pl; ++c) o[k * v.n_ch - n_pl + c] = s_planes[el * n_pl + c];
-                    o[k * v.n_ch + (p.raw ? 0 : hot)] = p.raw ? (T)hot : (T)1;
+                    if constexpr (sizeof(T) == 2) o[k * v.n_ch + hot] = obs_elem<T>(1);   // no 2-byte tile codes
+                    else o[k * v.n_ch + (p.raw ? 0 : hot)] = p.raw ? obs_elem<T>(hot) : obs_elem<T>(1);
                     if (STATIC) {   // see k_observe: the bordered frozen-tile mask through the same crop
                         const int b0 = s0 - 1, b1 = s1 - 1, b2 = D3 ? s2 - 1 : 0;
                         const bool in_bordered = b0 >= -1 && b0 <= p.d0 && b1 >= -1 && b1 <= p.d1 &&
@@ -511,7 +548,7 @@ __global__ void __launch_bounds__(OBS_THREADS) k_observe_staged(const ObsParams 
                             const bool inner = (unsigned)b0 < (unsigned)p.d0 && (unsigned)b1 < (unsigned)p.d1 &&
                                                (unsigned)b2 < (unsigned)p.d2;
                             if (!inner || s_mask[el * p.row_stride + (b0 * p.d1 + b1) * p.d2 + b2] != 0)
-                                o[k * v.n_ch + v.n_map_ch] = (T)1;
+                                o[k * v.n_ch + v.n_map_ch] = obs_elem<T>(1);
                         }
                     }
                     // next pixel: the last image axis is fastest
@@ -589,8 +626,9 @@ static cudaError_t launch_vec(const ObsParams& p, const ObsIdx& ix, cudaStream_t
     v.m_o12 = floor_magic((uint32_t)(p.o1 * p.o2));   // 2D: o2 == 1, i.e. the magic of o1
     v.planes_bytes = (v.GB * v.G * 2 * p.n_ctrl * (int)sizeof(T) + 15) / 16 * 16;
     int dyn = v.stage_bytes + v.planes_bytes + v.GB * v.G * (p.row_stride * (p.static_mask ? 2 : 1) + 12);
-    // two-tile crops of maps up to 16 wide in windows up to 32 wide (u8 one-hot or codes, no extra planes): row-mask path
-    v.bits = sizeof(T) == 1 && p.crop && p.ndim == 2 && p.n_tiles == 2 && p.d1 <= 16 && p.o1 <= 32 && p.o1 % 8 == 0 &&
+    // two-tile crops of maps up to 16 wide in windows up to 32 wide (u8 / 2-byte one-hot or u8 codes, no extra planes):
+    // row-mask path
+    v.bits = sizeof(T) <= 2 && p.crop && p.ndim == 2 && p.n_tiles == 2 && p.d1 <= 16 && p.o1 <= 32 && p.o1 % 8 == 0 &&
              !p.static_mask && !p.holes && p.n_ctrl == 0 && (p.raw ? n_ch == 1 : n_ch == 3);
     v.lut_off = (dyn + 15) / 16 * 16;
     if (v.bits) dyn = v.lut_off + 256 * 16 + 256 * 4 + (v.GB * v.G * p.d0 * 2 + 15) / 16 * 16;
@@ -604,7 +642,22 @@ static cudaError_t launch_vec(const ObsParams& p, const ObsIdx& ix, cudaStream_t
     (cr ? (st ? (d3 ? k_observe_staged<T, true, true, true, RN, IDX> : k_observe_staged<T, true, true, false, RN, IDX>)  \
               : (d3 ? k_observe_staged<T, true, false, true, RN, IDX> : k_observe_staged<T, true, false, false, RN, IDX>)) \
         : (d3 ? k_observe_staged<T, false, false, true, RN, IDX> : k_observe_staged<T, false, false, false, RN, IDX>))
-    void (*kern)(const ObsParams, const ObsVec, const ObsIdx) = rown == 8 ? OBS_PICK(8) : (rown == 4 ? OBS_PICK(4) : OBS_PICK(0));
+    void (*kern)(const ObsParams, const ObsVec, const ObsIdx);
+    if constexpr (sizeof(T) == 2) {
+        // float16 / bfloat16: only the kernels this choice reaches are instantiated.  B200 at 1000 W, 262 144 envs,
+        // bf16 (profiles/r03_observe_half_ab.txt):
+        // - two-tile crops take the row-mask path, 8 pixels (48 bytes, three 128-bit stores) per thread: binary-narrow
+        //   32x32 0.2764 / 0.2759 ms against 0.3231 / 0.3230 ms on the 4-pixel path;
+        // - 14-wide 3D windows take 7 pixels per thread: minecraft 14^3 1.0209 / 1.0181 ms against 1.8901 / 1.8919 ms;
+        // - 4 pixels per thread otherwise (24 bytes of 3-channel records, the bank pattern of the u8 path's 8):
+        //   binary-wide + 2 controls 0.2696 / 0.2693 ms against 0.4347 / 0.4341 ms with 8;
+        // - 22-wide windows keep the general path: zelda 22x22 0.4704 / 0.4707 ms against 0.4919 / 0.4916 ms with 11.
+        if (v.bits) kern = k_observe_staged<T, true, false, false, 8, IDX>;
+        else if (!p.holes && !st && cr && d3 && p.o2 == 14) kern = k_observe_staged<T, true, false, true, 7, IDX>;
+        else kern = rown == 4 ? OBS_PICK(4) : OBS_PICK(0);
+    } else {
+        kern = rown == 8 ? OBS_PICK(8) : (rown == 4 ? OBS_PICK(4) : OBS_PICK(0));
+    }
 #undef OBS_PICK
     if constexpr (sizeof(T) == 1) {
         // u8 windows 22 wide (zelda 7x11 behind its 22x22 crop: neither a multiple of 8 nor of 4, so it ran the 4-pixel
@@ -643,7 +696,9 @@ static cudaError_t launch_writers(const ObsParams& p, const ObsIdx& ix, int out_
         bool done = false;
         cudaError_t e = (out_kind == 0 || out_kind == 3) ? launch_vec<uint8_t, IDX>(p, ix, s, done)
                       : out_kind == 1 ? launch_vec<float, IDX>(p, ix, s, done)
-                      : out_kind == 2 ? launch_vec<double, IDX>(p, ix, s, done) : cudaErrorInvalidValue;
+                      : out_kind == 2 ? launch_vec<double, IDX>(p, ix, s, done)
+                      : out_kind == 5 ? launch_vec<__half, IDX>(p, ix, s, done)
+                      : out_kind == 6 ? launch_vec<__nv_bfloat16, IDX>(p, ix, s, done) : cudaErrorInvalidValue;
         if (e != cudaSuccess || done) return e;
     }
     const int64_t want = (total + 255) / 256;
@@ -654,6 +709,10 @@ static cudaError_t launch_writers(const ObsParams& p, const ObsIdx& ix, int out_
         k_observe<float, IDX><<<blocks, 256, 0, s>>>(p, ix);
     else if (out_kind == 2)
         k_observe<double, IDX><<<blocks, 256, 0, s>>>(p, ix);
+    else if (out_kind == 5)
+        k_observe<__half, IDX><<<blocks, 256, 0, s>>>(p, ix);
+    else if (out_kind == 6)
+        k_observe<__nv_bfloat16, IDX><<<blocks, 256, 0, s>>>(p, ix);
     else
         return cudaErrorInvalidValue;
     return cudaGetLastError();
@@ -676,7 +735,7 @@ const char* obs_args_error(const pcgrl_config& cfg, const pcgrl_state& st, const
                     o2 != d2 + (holey3d ? grow : 0)))
         return "without a crop obs_dims must be the (bordered) map dims";
     if ((a.out_kind == 0 || a.out_kind == 3) && a.n_ctrl > 0) return "uint8 observations have no target planes";
-    return nullptr;   // an out_kind outside 0..3 fails at the launch (and passes when there is nothing to write)
+    return nullptr;   // an out_kind outside 0..3, 5, 6 fails at the launch (and passes when there is nothing to write)
 }
 
 // env_idx: NULL observes every env of the shard into row env; else n_idx rows, row j showing env env_idx[j]

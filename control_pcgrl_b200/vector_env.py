@@ -228,7 +228,8 @@ def make_rllib_vector_env(cfg, num_envs: int, device="cuda:0", obs_dtype=np.floa
         register_env("pcgrl", lambda env_ctx: make_rllib_vector_env(env_ctx, env_ctx["num_envs_per_worker"]))
 
     Observations are what make_env's wrapper stack returns per env (rl/envs.py:28-66: cropped / full one-hot image
-    with the ControlWrapper target planes), as numpy rows of one pinned host array; rewards / truncation flags /
+    with the ControlWrapper target planes), as numpy rows of one pinned host array of obs_dtype (uint8, float32,
+    float64, or float16: half the bytes of float32 over PCIe; numpy has no bfloat16); rewards / truncation flags /
     info stats come back in one packed record array (compact host I/O)."""
     Base = _rllib_base()
 
@@ -238,7 +239,8 @@ def make_rllib_vector_env(cfg, num_envs: int, device="cuda:0", obs_dtype=np.floa
                                        auto_reset=False, compact_host_io=True)
             b = self.env
             shp = b.obs_shape()
-            tdt = {np.float32: torch.float32, np.float64: torch.float64, np.uint8: torch.uint8}[np.dtype(obs_dtype).type]
+            tdt = {np.float32: torch.float32, np.float64: torch.float64, np.float16: torch.float16,
+                   np.uint8: torch.uint8}[np.dtype(obs_dtype).type]
             self.observation_space = spaces.Box(0, 1, shape=shp, dtype=obs_dtype)
             rep = b.representation
             if b.act_window is not None:

@@ -249,7 +249,11 @@ int32_t pcgrl_stats_holey(const pcgrl_config* cfg, const int8_t* grids, const in
  *   stat index, ctrl_range[i] = |hi - lo| of cond_bounds.
  *   out_kind: 0 = uint8, 1 = float32, 2 = float64 (the reference's np.eye dtype), 3 = uint8 TILE CODES instead of
  *   one-hot records (Cropped's own output, the input of OneHotEncoding: 0 = out of bounds, tile t -> t + 1 behind a
- *   crop; for policies that embed the tile themselves -- a third of the bytes; no target planes).
+ *   crop; for policies that embed the tile themselves -- a third of the bytes; no target planes), 5 = float16,
+ *   6 = bfloat16 one-hot records (for policies that run in half precision; target planes allowed).  A half element is
+ *   the float32 element rounded to nearest even, i.e. byte for byte the float32 observation converted: one-hot and
+ *   static_builds elements are exactly 0 / 1, and a target or value plane is round_half((float)(x / range)), rounded
+ *   through float32 (a double rounded straight to the half type differs on rare ties).  4 is not a kind.
  *   Output layout [N, *obs_dims, channels] (channels last):
  *   [2*n_ctrl target planes | C+1 or C one-hot | static_builds]. */
 typedef struct pcgrl_obs_args {
