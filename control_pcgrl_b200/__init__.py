@@ -7,6 +7,7 @@ Public surface (mirrors the reference's names; see INTEGRATION.md):
     PcgrlVectorEnv(cfg, num_envs)          vector-env seam with auto-reset and device observations
     make_rllib_vector_env(cfg, num_envs)   ray.rllib VectorEnv (vector_reset / reset_at / vector_step) over one shard
     make_config(...)                       dataclass with the reference's cfg field names
+    level_distances / level_knn / level_diversity   Hamming distances between levels, kNN novelty, group diversity
 Importing this package never touches CUDA; constructing an env loads libpcgrl_sm100.so and fails
 loudly if it (or a GPU) is missing.
 """
@@ -16,9 +17,9 @@ from .registry import REGISTRY, make, make_batched  # noqa: F401
 
 
 def __getattr__(name):
-    if name in ("BatchedPcgrlEnv",):
-        from .batched_env import BatchedPcgrlEnv
-        return BatchedPcgrlEnv
+    if name in ("BatchedPcgrlEnv", "level_distances", "level_knn", "level_diversity"):
+        from . import batched_env
+        return getattr(batched_env, name)
     if name in ("PcgrlVectorEnv", "make_rllib_vector_env"):
         from . import vector_env
         return getattr(vector_env, name)

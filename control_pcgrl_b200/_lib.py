@@ -106,6 +106,13 @@ SYMBOLS = {
                                     C.c_void_p]),
     "pcgrl_load_envs": (C.c_int32, [C.POINTER(Config), C.POINTER(State), C.c_int32, C.c_void_p, C.c_void_p, C.c_int64,
                                     C.c_void_p]),
+    "pcgrl_level_work_bytes": (C.c_int64, [C.POINTER(Config), C.c_int64, C.c_int64, C.c_int32]),
+    "pcgrl_level_distances": (C.c_int32, [C.POINTER(Config), C.c_void_p, C.c_int64, C.c_int64, C.c_void_p, C.c_int64,
+                                          C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p]),
+    "pcgrl_level_knn": (C.c_int32, [C.POINTER(Config), C.c_void_p, C.c_int64, C.c_int64, C.c_void_p, C.c_int64,
+                                    C.c_int64, C.c_int32, C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
+    "pcgrl_level_group_diversity": (C.c_int32, [C.POINTER(Config), C.c_void_p, C.c_int64, C.c_int64, C.c_int64,
+                                                C.c_void_p, C.c_void_p, C.c_void_p]),
 }
 
 _lib = None

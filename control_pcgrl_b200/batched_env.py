@@ -772,6 +772,23 @@ class BatchedPcgrlEnv:
             _lib.check(self.lib.pcgrl_load_envs(self._cc, self._st, self.agent_pos.shape[0], rows.data_ptr(), _ptr(idx), m,
                                                 self._stream()), "pcgrl_load_envs")
 
+    # ------------------------------------------------------------------ level distances
+    def novelty(self, archive_rows: torch.Tensor, k: int, env_ids=None) -> torch.Tensor:
+        """Novelty of envs env_ids (default all) against an archive of saved rows (save_envs of an env with this row
+        layout): the mean Hamming distance of each env's grid to its k nearest archive grids (level_knn), float32 [M].
+        With fewer than k archive rows the mean is over those there are (NaN for an empty archive).  A bad index raises
+        IndexError before anything is launched (a device tensor costs one reduction and one sync)."""
+        arch = self.row_fields(archive_rows)["grids"]
+        queries = self.grids if env_ids is None else self.grids[self._check_env_ids(env_ids).long()]
+        dist, _ = level_knn(queries, arch, k=k, cfg=self)
+        valid = dist >= 0
+        return (dist.clamp(min=0).sum(1).double() / valid.sum(1)).float()
+
+    def diversity(self, group_size: int) -> torch.Tensor:
+        """Mean pairwise Hamming distance within each group of group_size consecutive envs (level_diversity of the
+        env's own grids), float64 [n_envs / group_size]."""
+        return level_diversity(self.grids, group_size, cfg=self)
+
     def step_agents(self, actions: torch.Tensor):
         """One multi-agent step: actions[N, n_agents], agent a acts a-th (MultiAgentWrapper.step,
         wrappers.py:724-731: a full env step per agent, so iteration advances by n_agents).  Returns
@@ -1174,3 +1191,106 @@ class BatchedPcgrlEnv:
         self.seed = int(sd.get("seed", self.seed))
         self._synced_steps = sd.get("_synced_steps")     # lock-step episode clock (None: envs are out of step)
         self._stats_stale = bool(sd.get("_stats_stale", False))    # checkpoints from before update() have no flag
+
+
+# ---------------------------------------------------------------------- level distances (pcgrl_level_*)
+def _level_config(cfg):
+    """The pcgrl_config whose dims and n_tiles give the level geometry: an env's own, or one built from a config."""
+    if isinstance(cfg, BatchedPcgrlEnv):
+        return cfg._cc
+    c = normalise(cfg)
+    spec = get_spec(c.problem, c.map_shape)
+    cc = _lib.Config()
+    cc.abi_version = _lib.PCGRL_ABI_VERSION
+    cc.problem = _lib.PROB_IDS[c.problem]
+    cc.representation = _lib.REP_IDS["narrow"]
+    cc.action_kind = _lib.ACT_INT32
+    cc.ndim = len(c.map_shape)
+    for i in range(3):
+        cc.dims[i] = c.map_shape[i] if i < cc.ndim else 1
+    cc.n_tiles, cc.n_stats = spec.n_tiles, len(spec.stat_names)
+    cc.max_iterations, cc.max_changes = 1, -1
+    _lib.check(_lib.load().pcgrl_config_check(cc), "pcgrl_config_check")
+    return cc
+
+
+def _levels(t, cc, env, what):
+    """-> (levels tensor, byte stride) of [M, >= cells] int8 / uint8 grids (env grids, [M, cells] maps, a row_fields
+    'grids' view), or of an env's saved rows [M, env_row_bytes] when cfg is that env."""
+    cells = int(np.prod([cc.dims[i] for i in range(cc.ndim)]))
+    if not torch.is_tensor(t) or t.dtype not in (torch.int8, torch.uint8) or t.dim() != 2:
+        raise ValueError(f"{what} must be a 2-D int8 / uint8 tensor of levels")
+    if env is not None and t.dtype == torch.uint8 and t.shape[1] == env.env_row_bytes:
+        t = env.row_fields(t)["grids"]
+    if not t.is_cuda:
+        raise ValueError(f"{what} must be on a CUDA device")
+    stride = t.stride(0) if t.shape[0] > 1 else cells
+    if t.shape[1] < cells or (t.shape[1] > 1 and t.stride(1) != 1) or stride < cells:
+        raise ValueError(f"{what} must hold one level of {cells} tile codes per row, with contiguous rows")
+    return t, stride
+
+
+def _level_call(a, b, cfg):
+    cc = _level_config(cfg)
+    env = cfg if isinstance(cfg, BatchedPcgrlEnv) else None
+    a, sa = _levels(a, cc, env, "a")
+    b, sb = (a, sa) if b is None else _levels(b, cc, env, "b")
+    if a.device != b.device:
+        raise ValueError(f"a is on {a.device}, b on {b.device}")
+    return cc, a, sa, b, sb
+
+
+def level_distances(a: torch.Tensor, b: torch.Tensor | None = None, *, cfg) -> torch.Tensor:
+    """Hamming distances between levels: int32 [M, N], out[i, j] = the number of cells where level a[i] and level b[j]
+    (default: a) hold different tile codes.  a, b: [M, cells] or [M, row_stride] int8 / uint8 grids (only the first cells
+    bytes of a row count), a row_fields(rows)['grids'] view, or, when cfg is a BatchedPcgrlEnv, saved rows of it.  cfg:
+    a make_config config or an env; it gives the map shape and tile count.  Meant for small problems: the output is
+    M * N * 4 bytes; level_knn never writes it."""
+    cc, a, sa, b, sb = _level_call(a, b, cfg)
+    lib, m, n = _lib.load(), a.shape[0], b.shape[0]
+    out = torch.empty((m, n), dtype=torch.int32, device=a.device)
+    work = torch.empty(max(int(lib.pcgrl_level_work_bytes(cc, m, n, 0)), 16), dtype=torch.uint8, device=a.device)
+    with torch.cuda.device(a.device):
+        _lib.check(lib.pcgrl_level_distances(cc, a.data_ptr(), m, sa, b.data_ptr(), n, sb, out.data_ptr(),
+                                             work.data_ptr(), torch.cuda.current_stream().cuda_stream),
+                   "pcgrl_level_distances")
+    return out
+
+
+def level_knn(a: torch.Tensor, b: torch.Tensor | None = None, *, k: int, cfg, exclude_self: bool = False,
+              self_offset: int = 0):
+    """The k nearest levels of b (default: a) to every level of a, 1 <= k <= 64: (dist, idx) int32 [M, k], each row in
+    ascending distance and, on equal distance, ascending index of b, so the result is deterministic.  exclude_self:
+    query i never picks level i + self_offset of b (novelty within a population: b None, offset 0).  With fewer than k
+    candidates a row ends in -1 / -1.  Inputs as for level_distances; no M x N matrix is formed."""
+    if isinstance(k, bool) or not isinstance(k, (int, np.integer)) or not 1 <= k <= 64:
+        raise ValueError(f"k must be an integer in [1, 64], got {k!r}")
+    if exclude_self and self_offset < 0:
+        raise ValueError("self_offset must be >= 0")
+    cc, a, sa, b, sb = _level_call(a, b, cfg)
+    lib, m, n = _lib.load(), a.shape[0], b.shape[0]
+    dist = torch.empty((m, k), dtype=torch.int32, device=a.device)
+    idx = torch.empty((m, k), dtype=torch.int32, device=a.device)
+    work = torch.empty(max(int(lib.pcgrl_level_work_bytes(cc, m, n, k)), 16), dtype=torch.uint8, device=a.device)
+    with torch.cuda.device(a.device):
+        _lib.check(lib.pcgrl_level_knn(cc, a.data_ptr(), m, sa, b.data_ptr(), n, sb, int(k),
+                                       int(self_offset) if exclude_self else -1, dist.data_ptr(), idx.data_ptr(),
+                                       work.data_ptr(), torch.cuda.current_stream().cuda_stream), "pcgrl_level_knn")
+    return dist, idx
+
+
+def level_diversity(a: torch.Tensor, group_size: int, *, cfg) -> torch.Tensor:
+    """Diversity of consecutive groups of group_size levels (group_size >= 2 divides M): float64 [M / group_size], the
+    mean Hamming distance over the unordered pairs of each group (the int64 pair sum from the device over
+    S (S - 1) / 2).  Inputs as for level_distances."""
+    cc, a, sa, _, _ = _level_call(a, None, cfg)
+    lib, m, s = _lib.load(), a.shape[0], int(group_size)
+    if s < 2 or m % s:
+        raise ValueError(f"group_size {group_size} must be >= 2 and divide {m}")
+    sums = torch.empty(m // s, dtype=torch.int64, device=a.device)
+    work = torch.empty(max(int(lib.pcgrl_level_work_bytes(cc, m, 0, 0)), 16), dtype=torch.uint8, device=a.device)
+    with torch.cuda.device(a.device):
+        _lib.check(lib.pcgrl_level_group_diversity(cc, a.data_ptr(), m, sa, s, sums.data_ptr(), work.data_ptr(),
+                                                   torch.cuda.current_stream().cuda_stream),
+                   "pcgrl_level_group_diversity")
+    return sums.double() / (s * (s - 1) // 2)

@@ -11,6 +11,7 @@
 
 #include "pcgrl_device.cuh"
 #include "env_rows.cuh"
+#include "level_distance.cuh"
 
 namespace pcgrl {
 cudaError_t launch_bitboard(const KParams& p, int problem, cudaStream_t s, bool& supported);
@@ -852,6 +853,81 @@ int32_t pcgrl_save_envs(const pcgrl_config* cfg, const pcgrl_state* st, int32_t 
 int32_t pcgrl_load_envs(const pcgrl_config* cfg, const pcgrl_state* st, int32_t n_pos, const void* rows,
                         const int32_t* env_idx, int64_t n, void* stream) {
     return env_rows_impl(cfg, st, n_pos, rows, env_idx, n, stream, false);
+}
+
+// ---- level distances: every check before any CUDA call ------------------------------------------------------------
+static int32_t check_levels(const LdGeom& g, const void* p, int64_t n, int64_t stride, const char* what) {
+    if (n < 0 || n > INT32_MAX) return fail(PCGRL_E_ARG, std::string(what) + ": count must be in [0, 2^31)");
+    if (stride < g.cells) return fail(PCGRL_E_ARG, std::string(what) + ": stride must be >= cells");
+    if (n > 0 && !p) return fail(PCGRL_E_ARG, std::string(what) + " is NULL");
+    if (n * g.W / 8 >= INT32_MAX) return fail(PCGRL_E_ARG, std::string(what) + ": too many levels for one launch");
+    return 0;
+}
+
+static int32_t check_level_call(const pcgrl_config* cfg, LdGeom& g, const void* work) {
+    const int r = check(cfg);
+    if (r) return r;
+    g = ld_geom(cells_of(cfg), cfg->n_tiles);
+    if (!ld_fits(g)) return fail(PCGRL_E_UNSUPPORTED, "level too large for the distance tile's shared memory");
+    if (!work) return fail(PCGRL_E_ARG, "work is NULL");
+    if ((uintptr_t)work % 16) return fail(PCGRL_E_ARG, "work must be 16-byte aligned");
+    return 0;
+}
+
+int64_t pcgrl_level_work_bytes(const pcgrl_config* cfg, int64_t n_query, int64_t n_archive, int32_t k) {
+    if (check(cfg) || n_query < 0 || n_archive < 0 || k < 0 || k > 64) return -1;
+    return ld_work_bytes(ld_geom(cells_of(cfg), cfg->n_tiles), n_query, n_archive, k);
+}
+
+int32_t pcgrl_level_distances(const pcgrl_config* cfg, const void* a, int64_t n_a, int64_t a_stride, const void* b,
+                              int64_t n_b, int64_t b_stride, int32_t* out, void* work, void* stream) {
+    LdGeom g;
+    int r;
+    if ((r = check_level_call(cfg, g, work)) || (r = check_levels(g, a, n_a, a_stride, "a")) ||
+        (r = check_levels(g, b, n_b, b_stride, "b")))
+        return r;
+    if (n_a > 0 && n_b > 0 && !out) return fail(PCGRL_E_ARG, "out is NULL");
+    if (n_a == 0 || n_b == 0) return 0;
+    int launches = 0;
+    const cudaError_t e = launch_level_distances(g, {(const uint8_t*)a, n_a, a_stride}, {(const uint8_t*)b, n_b, b_stride},
+                                                 out, work, (cudaStream_t)stream, launches);
+    g_launches.fetch_add(launches, std::memory_order_relaxed);
+    return e == cudaSuccess ? 0 : cuda_fail(e, "level_distances launch");
+}
+
+int32_t pcgrl_level_knn(const pcgrl_config* cfg, const void* q, int64_t n_q, int64_t q_stride, const void* b,
+                        int64_t n_b, int64_t b_stride, int32_t k, int64_t self_offset, int32_t* dist, int32_t* idx,
+                        void* work, void* stream) {
+    LdGeom g;
+    int r;
+    if ((r = check_level_call(cfg, g, work)) || (r = check_levels(g, q, n_q, q_stride, "queries")) ||
+        (r = check_levels(g, b, n_b, b_stride, "archive")))
+        return r;
+    if (k < 1 || k > 64) return fail(PCGRL_E_ARG, "k must be in [1, 64]");
+    if (self_offset < -1) return fail(PCGRL_E_ARG, "self_offset must be >= -1 (-1: no self-exclusion)");
+    if (n_q > 0 && (!dist || !idx)) return fail(PCGRL_E_ARG, "dist / idx is NULL");
+    if (n_q == 0) return 0;
+    int launches = 0;
+    const cudaError_t e = launch_level_knn(g, {(const uint8_t*)q, n_q, q_stride}, {(const uint8_t*)b, n_b, b_stride}, k,
+                                           self_offset, dist, idx, work, (cudaStream_t)stream, launches);
+    g_launches.fetch_add(launches, std::memory_order_relaxed);
+    return e == cudaSuccess ? 0 : cuda_fail(e, "level_knn launch");
+}
+
+int32_t pcgrl_level_group_diversity(const pcgrl_config* cfg, const void* a, int64_t n, int64_t stride,
+                                    int64_t group_size, int64_t* sums, void* work, void* stream) {
+    LdGeom g;
+    int r;
+    if ((r = check_level_call(cfg, g, work)) || (r = check_levels(g, a, n, stride, "levels"))) return r;
+    if (group_size < 2) return fail(PCGRL_E_ARG, "group_size must be >= 2");
+    if (n % group_size) return fail(PCGRL_E_ARG, "group_size must divide the level count");
+    if (n > 0 && !sums) return fail(PCGRL_E_ARG, "sums is NULL");
+    if (n == 0) return 0;
+    int launches = 0;
+    const cudaError_t e = launch_level_groups(g, {(const uint8_t*)a, n, stride}, group_size, sums, work,
+                                              (cudaStream_t)stream, launches);
+    g_launches.fetch_add(launches, std::memory_order_relaxed);
+    return e == cudaSuccess ? 0 : cuda_fail(e, "level_group_diversity launch");
 }
 
 // Shared body of pcgrl_step_host / pcgrl_step_host_packed: with records_host the only download is the packed

@@ -384,6 +384,39 @@ int32_t pcgrl_save_envs(const pcgrl_config* cfg, const pcgrl_state* st, int32_t 
 int32_t pcgrl_load_envs(const pcgrl_config* cfg, const pcgrl_state* st, int32_t n_pos, const void* rows,
                         const int32_t* env_idx, int64_t n, void* stream);
 
+/* -- level distances: Hamming kNN novelty and per-group diversity ----------------------------------------------------
+ * d(a, b) = the number of cells whose tile codes differ.  A level is the first cells = prod(dims) bytes at a DEVICE
+ * pointer + i * stride; only those bytes are read, so row padding never counts, whatever it holds.  The stride is any
+ * byte count >= cells (no alignment): levels come straight from pcgrl_state.grids (stride row_stride; a holey problem
+ * compares its interior grid) or from the grid section of saved env rows (pointer + pcgrl_row_layout.grid, stride
+ * row_bytes).  Tile codes must lie in [0, cfg->n_tiles).  cfg supplies dims and n_tiles only (it must pass
+ * pcgrl_config_check).  Counts are < 2^31.
+ *   work  at least pcgrl_level_work_bytes(cfg, n_query, n_archive, k) bytes, 16-byte aligned, not shared by launches
+ *         that can run concurrently; it holds the levels packed as ceil(log2 n_tiles) bit-planes and the partial kNN
+ *         lists, every byte written before it is read (so it need not be initialised).  Sizes per call:
+ *         pcgrl_level_distances (n_a, n_b, 0), pcgrl_level_knn (n_q, n_b, k), pcgrl_level_group_diversity (n, 0, 0).
+ *         -1 for a bad config, a negative count or k outside [0, 64].
+ * Every argument is checked on the host before any launch; a level whose packed form does not fit the distance tile's
+ * shared memory (more than 362 words, ceil(cells / 32) per bit-plane) is PCGRL_E_UNSUPPORTED.  Launches are asynchronous on
+ * `stream`; a call with nothing to compute launches nothing. */
+int64_t pcgrl_level_work_bytes(const pcgrl_config* cfg, int64_t n_query, int64_t n_archive, int32_t k);
+/* out [n_a, n_b] int32: out[i][j] = d(a_i, b_j).  a and b may be the same levels.  Three launches. */
+int32_t pcgrl_level_distances(const pcgrl_config* cfg, const void* a, int64_t n_a, int64_t a_stride, const void* b,
+                              int64_t n_b, int64_t b_stride, int32_t* out, void* work, void* stream);
+/* The k nearest archive levels of every query, 1 <= k <= 64: dist and idx [n_q, k] int32, row i in ascending distance
+ * and, on equal distance, ascending archive index, so the result is deterministic.  self_offset >= 0 leaves archive
+ * level i + self_offset out of query i's candidates (0 with the queries as the archive: novelty within a population);
+ * -1 excludes nothing.  With fewer than k candidates the row ends in (-1, -1) pairs.  The distance matrix is never
+ * written.  Three launches, four when a small query count splits the archive into slices (chosen from n_q and n_b) and a
+ * merge combines the slices' lists. */
+int32_t pcgrl_level_knn(const pcgrl_config* cfg, const void* q, int64_t n_q, int64_t q_stride, const void* b,
+                        int64_t n_b, int64_t b_stride, int32_t k, int64_t self_offset, int32_t* dist, int32_t* idx,
+                        void* work, void* stream);
+/* n levels as n / group_size consecutive groups (group_size >= 2 divides n): sums[g] int64 = the sum of d over the
+ * unordered pairs i < j of group g; the mean pairwise distance is sums[g] / (S (S - 1) / 2).  Two launches. */
+int32_t pcgrl_level_group_diversity(const pcgrl_config* cfg, const void* a, int64_t n, int64_t stride,
+                                    int64_t group_size, int64_t* sums, void* work, void* stream);
+
 /* -- host-buffer convenience (the end-to-end path timed as `e2e` in bench.py) ------------------ */
 /* Copies `actions` (host, pinned or pageable) to `actions_dev`, runs pcgrl_step, copies reward/done/stats
  * back to the host buffers, and synchronises the stream.  Any host pointer may be NULL to skip that copy. */
