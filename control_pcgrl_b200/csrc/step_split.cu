@@ -13,7 +13,8 @@
 //               cache (passable board, one far tile per non-isolated component, a cell of the component that
 //               attains path-length) the machine floods the affected region U, redoes calc_longest_path's two
 //               sweeps inside U only, and sweeps the untouched components too (in the same final sweep) only when
-//               the one that held the maximum was touched: 32 instead of 93 board expansions per changed grid on
+//               the one that held the maximum was touched; otherwise it skips the final sweep when the first sweeps
+//               prove that it cannot beat the old path-length: 29 instead of 93 board expansions per changed grid on
 //               16x16 narrow rollouts (scripts/inc_work_counts.py), bit-identical results (helper.py:255-276 is a
 //               per-component computation; components the edit does not touch keep their first tile, far tile
 //               and eccentricity).  Work per item is uneven (0..135 expansions), so lanes claim items one by one
@@ -33,26 +34,36 @@
 namespace pcgrl {
 
 constexpr int SPLIT_MIN_CTAS = 10;
-constexpr int INC_CTAS_PER_SM = 8;       // 128-thread CTAs of the incremental search resident per SM (A/B 4 / 6 / 8 / 12 at
+constexpr int INC_CTAS_PER_SM = 6;       // 128-thread CTAs of the incremental search resident per SM (A/B 4 / 6 / 8 / 12 at
                                          // R=3: 0.412 / 0.393 / 0.384 / 0.378 ms per step; with the joint final sweep, 6 / 8 / 9:
-                                         // 0.2686 / 0.2697 / 0.2712, profiles/r03_inc_joint_sweep.txt)
+                                         // 0.2686 / 0.2697 / 0.2712, profiles/r03_inc_joint_sweep.txt; with the skipped final
+                                         // sweep, 6 / 8: 0.2576 / 0.2590 with claims of 12 lanes, 0.2549 / 0.2566 with claims of 8,
+                                         // profiles/r04_inc_skip_final_sweep.txt)
+constexpr int INC_CTAS_PER_SM_LOOKAHEAD = 8;   // the same for the search of the incremental lookahead, which keeps 8:
+                                               // scripts/bench_lookahead.py, 8 / 6 CTAs per SM, binary-narrow lookahead_all
+                                               // of 1 Mi envs 0.482-0.486 / 0.489 ms, binary-wide 512 actions of 16 Ki envs
+                                               // 1.794-1.795 / 1.830-1.836 ms (profiles/r04_inc_skip_final_sweep.txt)
 constexpr int INC_CTAS_PER_SM_HOST = 4;  // the same inside the host pipeline: most of the SM's registers stay free, so the
                                          // update / output kernels of the neighbouring chunks run next to the search
                                          // (e2e at 4 chunks, 2 / 3 / 4 / 5 / 8 CTAs per SM: 2.48 / 2.60 / 2.51 / 2.36 / 2.11e9 with the
                                          // copies on the compute streams; with separate copy streams 3 / 4 / 5 / 8:
                                          // 2.56 / 2.75 / 2.71 / 2.42e9, profiles/r02_e2e_cps_chunks_split.txt)
-constexpr int INC_MIN_CLAIM = 12;        // lanes that must be waiting before a warp hands out new items: the claim / init
+constexpr int INC_MIN_CLAIM = 8;         // lanes that must be waiting before a warp hands out new items: the claim / init
                                          // stream then runs with that many lanes (A/B 1 / 4 / 8 at R=3: 0.412 / 0.390 / 0.387; at
                                          // R=12, 8 / 12 / 16 / 24: 0.2978 / 0.2996 / 0.3022 / 0.3263 ms, profiles/r02_ab_inc_claim_window.txt;
-                                         // with the joint final sweep 8 / 12: 0.2675 / 0.2697 in the split path, k_step_inc not
-                                         // measured at 8, profiles/r03_inc_joint_sweep.txt)
+                                         // with the joint final sweep 8 / 12: 0.2675 / 0.2697 in the split path,
+                                         // profiles/r03_inc_joint_sweep.txt; with the skipped final sweep 8 / 12: 0.2566 / 0.2590 at 8
+                                         // CTAs per SM, and k_step_inc (64 Ki envs, binary-wide + controls) 0.0596 / 0.0596 ms,
+                                         // profiles/r04_inc_skip_final_sweep.txt)
 constexpr int INC_EXPAND_R = 12;         // board expansions per trip.  Every trip also issues each transition stream that
                                          // some lane needs (flood done / next component / final sweep / finish, several
                                          // hundred instructions at 2-3 lanes), so few long trips beat many short ones although
                                          // lanes idle inside the window: A/B 2 / 3 / 4 / 6 / 8 / 12 -> 0.466 / 0.412 / 0.356 /
                                          // 0.325 / 0.308 / 0.303 ms per step (1 Mi envs, 8 CTAs per SM); 16 / 20 -> 0.3018 / 0.3140
                                          // against 0.2996 for 12 in a later run; with the joint final sweep 8 / 12 / 16 -> 0.2729 /
-                                         // 0.2697 / 0.2733 (profiles/r03_inc_joint_sweep.txt)
+                                         // 0.2697 / 0.2733 (profiles/r03_inc_joint_sweep.txt); with the final sweep skipped under
+                                         // the min(2 e1, |C| - 1) bound, 8 / 12 / 16 -> 0.2653 / 0.2599 / 0.2629
+                                         // (profiles/r04_inc_skip_final_sweep.txt)
 constexpr int EXPAND_R_SPLIT = 3;        // board expansions per trip of the static search (as in the fused kernel)
 
 constexpr int ACT_THREADS = 256;
@@ -199,6 +210,11 @@ k_split_stats(const KParams p) {
 //              old path-length if the cached cell of a maximal component lies outside A.  Otherwise ONE sweep from
 //              the far tiles of U and of the untouched components together gives both maxima at once: they are
 //              different components, so a multi-source BFS takes max(lu, lold) levels instead of lu + lold.
+//              In the first case the final sweep is skipped when the first sweeps already prove lu <= path: the
+//              first sweep of component C_j of U reaches depth e1_j = ecc(first tile), so its far tile has
+//              ecc <= 2 * e1_j; if max_j 2 * e1_j <= path, path and m stay.  (The tighter min(2 * e1_j, |C_j| - 1)
+//              skips the sweep on 4 % more changed grids, but the popcounts it needs cost more than that: 0.2599
+//              against 0.2591 ms per step, profiles/r04_inc_skip_final_sweep.txt.)
 // Isolated cells are counted next to c only: with Q = P' \ {c} and iso(Q) its cells without a neighbour in Q,
 //   c became solid:     old isolated in A = {c} if c has no neighbour in Q,  new isolated in U = N(c) & iso(Q)
 //   c became passable:  old isolated in A = N(c) & iso(Q),  new isolated in U = {c} if c has no neighbour in Q
@@ -218,6 +234,7 @@ struct BinaryIncMachine {
     const uint32_t* cache;   // this env's cache row (still the OLD state until finish())
     int phase, level, regions, path, mcell, cell;   // path / mcell: the cache's path-length and m, old until the end
     bool hit;
+    bool longer;    // phase 1: some far tile of U may have an eccentricity above path (else the final sweep is skipped)
 
     static __device__ __forceinline__ int lowest_pos(const uint32_t (&x)[NW]) {
         int pos = -1;   // branch-free: this runs in the few-lane transition stream
@@ -271,6 +288,7 @@ struct BinaryIncMachine {
         phase = 0;
         level = 0;
         hit = false;
+        longer = false;
     }
     __device__ __forceinline__ bool expand() {
         uint32_t n[NW];
@@ -340,8 +358,11 @@ struct BinaryIncMachine {
                 for (int i = 0; i < NW; ++i) avail[i] = sm[NW + i];
             }
             phase = 1;
+            level = 0;
         }
         if (phase == 1) {   // first sweeps inside U, one component at a time (BinaryMachine phase 0)
+            // the component whose sweep just died (none on entry from phase 0: level 0) reached depth e1 = level
+            longer |= 2 * level > path;
             uint32_t t[NW];
             B::minus_one(front, t);
 #pragma unroll
@@ -353,11 +374,14 @@ struct BinaryIncMachine {
                     avail[i] &= t[i];
                 }
                 ++regions;
+                level = 0;
                 return false;
             }
             // final sweep: from the far tiles of U, and when the component that held the maximum was touched, from
-            // those of the untouched components too (isolated cells may stay in avail: the sweep never reaches them)
+            // those of the untouched components too (isolated cells may stay in avail: the sweep never reaches them).
+            // Untouched: path' = max(path, lu), and the first sweeps bound lu by path -- nothing to sweep.
             phase = 2;
+            if (!hit && !longer) return true;
             uint32_t any = 0;
 #pragma unroll
             for (int i = 0; i < NW; ++i) {
@@ -710,13 +734,13 @@ cudaError_t launch_bitboard_split(const KParams& p, int problem, cudaStream_t s,
 }
 
 // The search kernel of the incremental lookahead (lookahead.cu): the work list of p holds (env, cell) candidate
-// edits, p.stats / p.cache are the shard's.  Sized as the split path's search.
+// edits, p.stats / p.cache are the shard's.  Sized as the split path's search, with INC_CTAS_PER_SM_LOOKAHEAD.
 cudaError_t launch_lookahead_search(const KParams& p, cudaStream_t s) {
     int n_sm = 0;
     cudaError_t e = sm_count(n_sm);
     if (e != cudaSuccess) return e;
     const int64_t want = (p.n_envs + STAT_THREADS - 1) / STAT_THREADS;
-    const int64_t cap = (int64_t)n_sm * INC_CTAS_PER_SM;
+    const int64_t cap = (int64_t)n_sm * INC_CTAS_PER_SM_LOOKAHEAD;
     const unsigned grid = (unsigned)(want < cap ? want : cap);
     const int nw = (p.d0 + 1) / 2;
     if (nw <= 1) k_split_stats_inc<1, true, true><<<grid, STAT_THREADS, 0, s>>>(p);

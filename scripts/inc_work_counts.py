@@ -1,6 +1,7 @@
-"""Work per changed grid of the incremental binary search, for the two-sweep update (oracle/inc_oracle.py) and the
-joint-sweep update BinaryIncMachine runs (tests/inc_oracle_joint.py), on 16x16 narrow-representation rollouts (the
-flagship workload's edit pattern: the cell cursor walks the map in row-major order, each step sets a random tile).
+"""Work per changed grid of the incremental binary search, for the two-sweep update (oracle/inc_oracle.py), the
+joint-sweep update (tests/inc_oracle_joint.py) and the joint-sweep update with the skipped final sweep that
+BinaryIncMachine runs (tests/inc_oracle_skip.py), on 16x16 narrow-representation rollouts (the flagship workload's
+edit pattern: the cell cursor walks the map in row-major order, each step sets a random tile).
 
     segments      BFS runs from a non-empty start (flood, first sweep per component of U, final sweeps)
     expansions    board expansions of those runs, the last (empty) one included
@@ -16,6 +17,7 @@ sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 
 from oracle.inc_oracle import IncBinary  # noqa: E402
 from tests.inc_oracle_joint import IncBinaryJoint  # noqa: E402
+from tests.inc_oracle_skip import IncBinarySkip  # noqa: E402
 
 
 def counting(cls):
@@ -36,8 +38,8 @@ def main():
     ap.add_argument("--seed", type=int, default=3)
     args = ap.parse_args()
     rng = random.Random(args.seed)
-    machines = {"two-sweep": counting(IncBinary), "joint": counting(IncBinaryJoint)}
-    n, no_seed = 0, 0
+    machines = {"two-sweep": counting(IncBinary), "joint": counting(IncBinaryJoint), "skip": counting(IncBinarySkip)}
+    n, no_seed, skipped = 0, 0, 0
     totals = {k: [0, 0] for k in machines}
     for _ in range(args.maps):
         g = [[rng.randrange(2) for _ in range(16)] for _ in range(16)]
@@ -60,11 +62,13 @@ def main():
         for k, m in ms.items():
             totals[k][0] += m.segments
             totals[k][1] += m.expansions
-    assert (ms["two-sweep"].regions, ms["two-sweep"].path) == (ms["joint"].regions, ms["joint"].path)
+        skipped += ms["skip"].skipped
+        assert len({(m.regions, m.path, m.F, m.m) for m in ms.values()}) == 1
     print(f"{n} changed grids ({args.maps} maps x 256 narrow steps, seed {args.seed})")
     print(f"{'':10s} {'segments':>9s} {'expansions':>11s} {'transitions':>12s}   (per changed grid)")
     for k, (seg, exp) in totals.items():
         print(f"{k:10s} {seg / n:9.2f} {exp / n:11.1f} {(seg + no_seed) / n:12.2f}")
+    print(f"final sweep skipped on {skipped / n:.1%} of the changed grids")
 
 
 if __name__ == "__main__":
