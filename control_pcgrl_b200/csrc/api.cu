@@ -16,7 +16,7 @@
 namespace pcgrl {
 cudaError_t launch_bitboard(const KParams& p, int problem, cudaStream_t s, bool& supported);
 cudaError_t launch_bigboard(const KParams& p, int problem, cudaStream_t s, bool& supported);
-cudaError_t launch_bitboard_split(const KParams& p, int problem, cudaStream_t s, int incremental, bool& supported,
+cudaError_t launch_bitboard_split(const KParams& p, int problem, cudaStream_t s, StepPath path, bool& supported,
                                   int& n_launches, const int32_t* env_idx = nullptr, int64_t n_src = 0);
 cudaError_t launch_bitboard_lanegroup(const KParams& p, int problem, cudaStream_t s, bool& supported);
 int bitboard_cache_stride(int problem, int ndim, int d0, int d1, int rep, int action_kind);
@@ -120,17 +120,13 @@ static int cache_stride(const pcgrl_config* c) {
     return bitboard_cache_stride(kernel_problem(c->problem), c->ndim, c->dims[0], c->dims[1], c->representation,
                                  c->action_kind);
 }
-// PCGRL_STEP_PATH = fused | split | inc | incfused | lg (default by shard size, step_path()): which of the equivalent step paths pcgrl_step
-// takes when the caller supplied the buffers for all of them (A/B runs and the path-equivalence tests)
-static int path_of(const char* e, int dflt) {
-    if (!e) return dflt;
-    return !strcmp(e, "fused") ? 0 : !strcmp(e, "split") ? 1 : !strcmp(e, "inc") ? 2 : !strcmp(e, "incfused") ? 3
-         : !strcmp(e, "lg") ? 4 : dflt;
-}
+// The step path of a bit-board shard (StepPath).
+// PCGRL_STEP_PATH = fused | split | inc | incfused | lg (default by shard size, below): which of the equivalent step paths
+// pcgrl_step takes when the caller supplied the buffers for all of them (A/B runs and the path-equivalence tests).
 // Measured on B200, binary 16x16, ms per step of a shard of 64 Ki / 256 Ki / 512 Ki / 1 Mi envs:
 //   fused 0.066 / 0.131 / 0.220 / 0.385   inc (3 launches) 0.063 / 0.114 / 0.175 / 0.304   incfused 0.058 / 0.122 / 0.203 / 0.367
 // so a plain pcgrl_step takes the one-launch incremental kernel for small shards and the three-launch one above.
-// The lane-group kernel (step_lanegroup.cu, path 4 "lg"; kernel times, profiles/r02_lanegroup_by_size.txt): 1 Ki / 4 Ki / 16 Ki
+// The lane-group kernel (step_lanegroup.cu, "lg"; kernel times, profiles/r02_lanegroup_by_size.txt): 1 Ki / 4 Ki / 16 Ki
 // envs 24.9 / 27.1 / 31.5 us against 30.8 / 32.6 / 33.7 us for incfused, 64 Ki 67.5 / 58.0 -- it takes the shards below 24 Ki envs
 // (RLlib-scale batches).
 // With its grid sized so that every CTA works and warps take two update rounds (step_split.cu, launch_split) the
@@ -142,18 +138,22 @@ static int path_of(const char* e, int dflt) {
 // The problems without a search cache (binary_holey, binary maps of 17..32 rows) run the from-scratch machines either
 // way: fused below 128 Ki envs, the split path (full warps from a global list) above (profiles/r02_zelda_paths.txt:
 // binary 24x24 64 Ki envs 0.207 / 0.227 ms fused / split, 512 Ki 1.019 / 0.943; binary_holey 64 Ki 0.087 / 0.086, 1 Mi 0.820 / 0.580).
-static int step_path(int64_t n_envs, int problem, bool has_cache) {
-    const int dflt = problem == PCGRL_PROB_ZELDA ? 0
-                   : !has_cache ? (n_envs < (128 << 10) ? 0 : 1)
-                   : n_envs < (24 << 10) ? 4 : n_envs < (224 << 10) ? 3 : 2;
-    return path_of(getenv("PCGRL_STEP_PATH"), dflt);
-}
-// Chunks of the host pipeline run on different streams.  With the search kernel of the three-launch incremental
+// Chunks of the host pipeline (host_chunk) run on different streams.  With the search kernel of the three-launch incremental
 // path limited to 3 CTAs per SM (INC_CTAS_PER_SM_HOST, step_split.cu) the memory-bound update / output kernels of the
 // neighbouring chunks run NEXT TO it: e2e 2.60e9 env-steps/s at 4 chunks, against 2.24e9 with the fused kernel and
 // 2.11e9 when the search holds every SM for itself (8 CTAs per SM).  The one-launch incremental kernel lost too: e2e
 // 2.74e9 against at most 2.38e9 (profiles/r02_e2e_hostpath.txt).  Shards without a search cache keep the fused kernel.
-static int host_chunk_path(bool has_cache) { return has_cache ? 2 : 0; }
+// PCGRL_STEP_PATH does not apply to host-pipeline chunks.
+static StepPath step_path(int64_t n_envs, int problem, bool has_cache, bool host_chunk) {
+    if (host_chunk) return has_cache ? INC : FUSED;
+    const StepPath dflt = problem == PCGRL_PROB_ZELDA ? FUSED
+                        : !has_cache ? (n_envs < (128 << 10) ? FUSED : SPLIT)
+                        : n_envs < (24 << 10) ? LANEGROUP : n_envs < (224 << 10) ? INC_FUSED : INC;
+    const char* e = getenv("PCGRL_STEP_PATH");
+    if (!e) return dflt;
+    return !strcmp(e, "fused") ? FUSED : !strcmp(e, "split") ? SPLIT : !strcmp(e, "inc") ? INC
+         : !strcmp(e, "incfused") ? INC_FUSED : !strcmp(e, "lg") ? LANEGROUP : dflt;
+}
 static int action_elem(const pcgrl_config* c) { return c->action_elem_bytes ? c->action_elem_bytes : 4; }
 static int record_stride(const pcgrl_config* c) {
     return c->record_stat_bytes ? (4 + c->n_stats * c->record_stat_bytes + 2 + 3) / 4 * 4 : 0;
@@ -239,7 +239,7 @@ static int check_state(const pcgrl_state* st) {
     return 0;
 }
 
-static int run(const KParams& p, int cfg_problem, void* stream, int force_path = -1) {
+static int run(const KParams& p, int cfg_problem, void* stream) {
     const int problem = kernel_problem(cfg_problem);
     bool supported = false;
     int multi = 0;
@@ -253,8 +253,9 @@ static int run(const KParams& p, int cfg_problem, void* stream, int force_path =
     else if (problem == PCGRL_PROB_SMB)
         e = launch_smb(p, (cudaStream_t)stream, supported, multi);   // map statistics + lane-group playthroughs + fallback
     else {
-        int path = force_path >= 0 ? force_path : step_path(p.n_envs, problem, p.cache != nullptr);
-        if (p.mode == MODE_STEP && path == 4) {   // lane groups (step_lanegroup.cu): small binary shards with a search cache
+        // the fallback chain of StepPath: lane groups, the split path, the fused kernel, warp-per-grid boards
+        StepPath path = step_path(p.n_envs, problem, p.cache != nullptr, p.host_chunk != 0);
+        if (p.mode == MODE_STEP && path == LANEGROUP) {
             if (p.cache) {
                 e = launch_bitboard_lanegroup(p, problem, (cudaStream_t)stream, supported);
                 if (supported) {
@@ -263,11 +264,11 @@ static int run(const KParams& p, int cfg_problem, void* stream, int force_path =
                     return 0;
                 }
             }
-            path = 3;
+            path = INC_FUSED;
         }
-        if (p.mode == MODE_STEP && p.worklist && path > 0) {
+        if (p.mode == MODE_STEP && p.worklist && path != FUSED) {
             int n_launches = 0;
-            e = launch_bitboard_split(p, problem, (cudaStream_t)stream, path - 1, supported, n_launches);
+            e = launch_bitboard_split(p, problem, (cudaStream_t)stream, path, supported, n_launches);
             if (supported) {
                 if (e != cudaSuccess) return cuda_fail(e, "kernel launch");
                 g_launches.fetch_add(n_launches, std::memory_order_relaxed);
@@ -329,8 +330,7 @@ struct HostPipe {
 };
 static thread_local HostPipe g_pipe[16];
 
-static int host_chunks(const pcgrl_config* cfg, int64_t n, bool packed) {
-    (void)packed;
+static int host_chunks(const pcgrl_config* cfg, int64_t n) {
     if (!is_bitboard(cfg) || cfg->dims[0] > 32 || cfg->dims[1] > 32) return 1;
     if (const char* e = getenv("PCGRL_HOST_CHUNKS")) {
         const int v = atoi(e);
@@ -515,9 +515,9 @@ int32_t pcgrl_record_stride(const pcgrl_config* cfg) {
 
 // One step launch over `st`.  wl_chunk / wl_off place this launch's work list inside the PARENT shard's
 // pcgrl_state.worklist (host pipeline: st is a sub-range starting wl_off envs into the shard and `wl_base` is the
-// parent's buffer); a plain pcgrl_step is chunk 0 at offset 0 of its own buffer.
+// parent's buffer, host_chunk = true); a plain pcgrl_step is chunk 0 at offset 0 of its own buffer.
 static int32_t step_launch(const pcgrl_config* cfg, const pcgrl_state* st, const void* actions, void* stream,
-                           int32_t* wl_base, int wl_chunk, int64_t wl_off, int force_path = -1) {
+                           int32_t* wl_base, int wl_chunk, int64_t wl_off, bool host_chunk = false) {
     int r = check(cfg);
     if (r) return r;
     if ((r = check_state(st))) return r;
@@ -531,8 +531,8 @@ static int32_t step_launch(const pcgrl_config* cfg, const pcgrl_state* st, const
     }
     p.mode = MODE_STEP;
     p.actions = actions;
-    p.host_chunk = force_path >= 0;
-    return run(p, cfg->problem, stream, force_path);
+    p.host_chunk = host_chunk;
+    return run(p, cfg->problem, stream);
 }
 
 int32_t pcgrl_step(const pcgrl_config* cfg, const pcgrl_state* st, const void* actions, void* stream) {
@@ -777,7 +777,7 @@ int32_t pcgrl_step_envs(const pcgrl_config* cfg, const pcgrl_state* st, const vo
     if (p.worklist) {   // the split path's three launches through the shard's own work list (chunk 0's header)
         bool supported = false;
         int n_launches = 0;
-        e = launch_bitboard_split(p, kernel_problem(cfg->problem), s, 1, supported, n_launches, env_idx, st->n_envs);
+        e = launch_bitboard_split(p, kernel_problem(cfg->problem), s, INC, supported, n_launches, env_idx, st->n_envs);
         if (supported) {
             if (e != cudaSuccess) return cuda_fail(e, "step_envs launch");
             g_launches.fetch_add(n_launches, std::memory_order_relaxed);
@@ -947,7 +947,7 @@ static int32_t step_host_impl(const pcgrl_config* cfg, const pcgrl_state* st, co
         return fail(PCGRL_E_ARG, "packed host step needs cfg.record_stat_bytes and pcgrl_state.records");
     const int64_t n = st->n_envs;
     const int K = cfg->n_stats;
-    const int chunks = (n > 0 && (!actions_host || action_bytes % n == 0)) ? host_chunks(cfg, n, records_host != nullptr) : 1;
+    const int chunks = (n > 0 && (!actions_host || action_bytes % n == 0)) ? host_chunks(cfg, n) : 1;
     if (chunks <= 1) {
         if (actions_host &&
             (e = cudaMemcpyAsync(actions_dev, actions_host, (size_t)action_bytes, cudaMemcpyHostToDevice, s)) != cudaSuccess)
@@ -981,7 +981,6 @@ static int32_t step_host_impl(const pcgrl_config* cfg, const pcgrl_state* st, co
                 return cuda_fail(e, "event create");
         hp.ready = true;
     }
-    const int chunk_path = host_chunk_path(st->worklist && st->cache && cache_stride(cfg) > 0);
     const int64_t per = ((n + chunks - 1) / chunks + 255) / 256 * 256;   // whole CTA tiles per chunk
     const int64_t a_env = actions_host ? action_bytes / n : 0;
 
@@ -1064,7 +1063,7 @@ static int32_t step_host_impl(const pcgrl_config* cfg, const pcgrl_state* st, co
                 cudaEventRecord(trace[3 * c + 0], cs);
             }
             // every chunk gets its own header and its own body range of the shard's work list
-            int rr = step_launch(cfg, &sub, ck[c].a_dev, cs, st->worklist, c, off, chunk_path);
+            int rr = step_launch(cfg, &sub, ck[c].a_dev, cs, st->worklist, c, off, true);
             if (rr) return rr;
             if (trace) cudaEventRecord(trace[3 * c + 1], cs);
             if ((e = cudaEventRecord(hp.k_ev[c], cs)) != cudaSuccess) return cuda_fail(e, "event record");

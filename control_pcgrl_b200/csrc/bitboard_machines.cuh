@@ -370,4 +370,64 @@ __device__ __forceinline__ void pack16(const uint4 v, uint32_t (&out)[Prob::P]) 
     }
 }
 
+// barrier of the threads that cooperate in stage_boards: a warp (GROUP == 32) or the whole CTA
+template <int GROUP>
+__device__ __forceinline__ void group_sync() {
+    if constexpr (GROUP == 32) __syncwarp();
+    else __syncthreads();
+}
+
+// Coalesced 128-bit loads of n level grids -> per-plane bit-boards in shared memory, P * NW words per slot (plane q of
+// slot i at bb[i * P * NW + q * NW]).  The GROUP threads that cooperate call it together, rank = the thread's index
+// among them; row(i) is the grid of slot i.  On return the boards are complete for the whole group.
+template <class Prob, int NW, bool TWO, int GROUP, class Row>
+__device__ __forceinline__ void stage_boards(const KParams& p, int rank, int n, uint32_t* bb, Row row) {
+    constexpr int P = Prob::P;
+    constexpr int BBW = P * NW;
+    const int chunks = p.row_stride / 16;
+    const int W = p.d1;
+    const bool word_is_32_bytes = TWO ? (W == 16) : (W == 32);
+    if (word_is_32_bytes) {
+        // a board word is exactly 32 consecutive cells: one thread builds one word, no atomics
+        for (int i = rank; i < n * NW; i += GROUP) {
+            const int slot = i / NW, j = i - slot * NW;
+            const int8_t* g = row(slot) + j * 32;
+            uint32_t lo[P], hi[P];
+#pragma unroll
+            for (int q = 0; q < P; ++q) lo[q] = hi[q] = 0;
+            if (2 * j < chunks) pack16<Prob>(*(const uint4*)g, lo);
+            if (2 * j + 1 < chunks) pack16<Prob>(*(const uint4*)(g + 16), hi);
+#pragma unroll
+            for (int q = 0; q < P; ++q) bb[slot * BBW + q * NW + j] = lo[q] | (hi[q] << 16);
+        }
+    } else {
+        for (int i = rank; i < n * BBW; i += GROUP) bb[i] = 0;
+        group_sync<GROUP>();
+        for (int i = rank; i < n * chunks; i += GROUP) {
+            const int slot = i / chunks, c = i - slot * chunks;
+            uint32_t lin[P];
+            pack16<Prob>(*(const uint4*)(row(slot) + c * 16), lin);
+            uint32_t* sb = bb + slot * BBW;
+            int cell = c * 16;
+            const int end = min(cell + 16, p.cells);
+            int y = cell / W, x = cell - y * W;
+            while (cell < end) {   // one row segment at a time (at most ceil(16/W)+1 of them)
+                const int len = min(W - x, end - cell);
+                const int word = TWO ? (y >> 1) : y;
+                const int sh = TWO ? ((y & 1) * 16 + x) : x;
+                const uint32_t m = (1u << len) - 1u;
+#pragma unroll
+                for (int q = 0; q < P; ++q) {
+                    const uint32_t seg = (lin[q] >> (cell - c * 16)) & m;
+                    if (seg) atomicOr(&sb[q * NW + word], seg << sh);
+                }
+                cell += len;
+                x = 0;
+                ++y;
+            }
+        }
+    }
+    group_sync<GROUP>();
+}
+
 }  // namespace pcgrl

@@ -678,8 +678,8 @@ static cudaError_t launch_vec(const ObsParams& p, const ObsIdx& ix, cudaStream_t
     int per_sm = 0;
     if ((e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, OBS_THREADS, dyn)) != cudaSuccess) return e;
     if (per_sm < 1) return cudaSuccess;
-    int dev = 0, n_sm = 148;
-    if (cudaGetDevice(&dev) == cudaSuccess) cudaDeviceGetAttribute(&n_sm, cudaDevAttrMultiProcessorCount, dev);
+    int n_sm = 0;
+    if ((e = sm_count(n_sm)) != cudaSuccess) return e;
     const int64_t trips = (p.n_envs + v.GB * v.G - 1) / (v.GB * v.G);
     const int64_t cap = (int64_t)n_sm * per_sm;
     const unsigned blocks = (unsigned)(trips < cap ? trips : cap);

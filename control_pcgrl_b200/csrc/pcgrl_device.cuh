@@ -2,11 +2,25 @@
 #pragma once
 #include <cuda_runtime.h>
 #include <stdint.h>
+#include <atomic>
 #include "../../include/pcgrl_b200.h"
 
 namespace pcgrl {
 
 enum { MODE_STEP = 0, MODE_RESET = 1, MODE_STATS = 2 };
+
+// The equivalent step paths of the bit-board problems (binary, zelda, binary_holey), in the order of PCGRL_STEP_PATH's
+// names fused | split | inc | incfused | lg:
+//   FUSED      k_step_bitboard, one launch (step_bitboard.cu)
+//   SPLIT      act / static search / output, three launches over a global work list (step_split.cu)
+//   INC        the same with the incremental search from the per-env cache
+//   INC_FUSED  the incremental step in one launch, k_step_inc
+//   LANEGROUP  k_step_lanegroup, one launch (step_lanegroup.cu)
+// A path that does not apply to a shard falls back: lane groups without a search cache run INC_FUSED; INC and INC_FUSED
+// without a cache (zelda, binary_holey, maps beyond 16x16) run the static SPLIT; SPLIT on a cellular shard, without a
+// work list or on maps beyond 32x32 runs FUSED, and maps beyond 32x32 then run the warp-per-grid boards
+// (step_bigboard.cu).
+enum StepPath { FUSED, SPLIT, INC, INC_FUSED, LANEGROUP };
 
 // Everything a kernel needs, passed by value (fits the 4 KB parameter space comfortably).
 struct KParams {
@@ -189,6 +203,10 @@ __device__ __forceinline__ double range_reward_sum(const int32_t* nw, const int3
 // ------------------------------------------------------------------------------------------------
 template <int NW, bool TWO>
 struct Board {
+    static constexpr int WORDS = NW;
+    static constexpr bool TWO_ROWS = TWO;
+    // bit position (word * 32 + bit) of cell (y, x)
+    __host__ __device__ static constexpr int bitpos(int y, int x) { return TWO ? y * 16 + x : y * 32 + x; }
     // n = dilate4(f) & av;  returns OR of all words of n (zero <=> frontier died)
     //
     // TWO layout: the "row above" word of board word i and the "row below" word of board word i-1 are the
@@ -286,5 +304,39 @@ struct Board {
         return r;
     }
 };
+
+// The board of a d0 x d1 map (rows x columns): up to 16x16 two rows per word in 1 / 2 / 4 / 8 words, up to 32x32 one
+// row per word in 16 / 32 words.  Returns f(Board<NW, TWO>{}); a larger map has no board: supported = false and f is
+// not called.
+template <class F>
+auto with_board(int d0, int d1, bool& supported, F&& f) -> decltype(f(Board<1, true>{})) {
+    supported = true;
+    if (d1 <= 16 && d0 <= 16) {
+        const int nw = (d0 + 1) / 2;
+        if (nw <= 1) return f(Board<1, true>{});
+        if (nw <= 2) return f(Board<2, true>{});
+        if (nw <= 4) return f(Board<4, true>{});
+        return f(Board<8, true>{});
+    }
+    if (d1 <= 32 && d0 <= 32) {
+        if (d0 <= 16) return f(Board<16, false>{});
+        return f(Board<32, false>{});
+    }
+    supported = false;
+    return {};
+}
+
+// SM count of the current device, queried once per device (ordinals beyond 16 on every call)
+inline cudaError_t sm_count(int& n) {
+    static std::atomic<int> cached[16];
+    int dev = 0;
+    cudaError_t e = cudaGetDevice(&dev);
+    if (e != cudaSuccess) return e;
+    const bool slot = dev >= 0 && dev < 16;
+    if (slot && (n = cached[dev].load(std::memory_order_relaxed)) > 0) return cudaSuccess;
+    if ((e = cudaDeviceGetAttribute(&n, cudaDevAttrMultiProcessorCount, dev)) != cudaSuccess) return e;
+    if (slot) cached[dev].store(n, std::memory_order_relaxed);
+    return cudaSuccess;
+}
 
 }  // namespace pcgrl

@@ -73,52 +73,8 @@ __global__ void __launch_bounds__(THREADS, NW <= 8 ? MIN_CTAS : 1) k_step_bitboa
     // ---------------- phase B: coalesced 128-bit grid loads -> per-plane bit-boards in smem --------
     // 16 cells (one uint4) are turned into a 16-bit membership mask per plane with SIMD-in-register ops:
     // a PRMT table lookup maps 4 tile codes to 4 0/1 bytes, a multiply gathers them into a nibble.
-    {
-        const int chunks = p.row_stride / 16;
-        const int W = (p.ndim == 2) ? p.d1 : p.d2;
-        const bool word_is_32_bytes = TWO ? (W == 16) : (W == 32);
-        if (word_is_32_bytes) {
-            // a board word is exactly 32 consecutive cells: one thread builds one word, no atomics
-            for (int i = tid; i < M * NW; i += THREADS) {
-                const int slot = i / NW, j = i - slot * NW;
-                const int8_t* g = grids_in + (base + s_list[slot]) * p.row_stride + j * 32;
-                uint32_t lo[P], hi[P];
-#pragma unroll
-                for (int q = 0; q < P; ++q) lo[q] = hi[q] = 0;
-                if (2 * j < chunks) pack16<Prob>(*(const uint4*)g, lo);
-                if (2 * j + 1 < chunks) pack16<Prob>(*(const uint4*)(g + 16), hi);
-#pragma unroll
-                for (int q = 0; q < P; ++q) s_bb[slot * BBW + q * NW + j] = lo[q] | (hi[q] << 16);
-            }
-        } else {
-            for (int i = tid; i < M * BBW; i += THREADS) s_bb[i] = 0;
-            __syncthreads();
-            for (int i = tid; i < M * chunks; i += THREADS) {
-                const int slot = i / chunks, c = i - slot * chunks;
-                uint32_t lin[P];
-                pack16<Prob>(*(const uint4*)(grids_in + (base + s_list[slot]) * p.row_stride + c * 16), lin);
-                uint32_t* bb = s_bb + slot * BBW;
-                int cell = c * 16;
-                const int end = min(cell + 16, p.cells);
-                int y = cell / W, x = cell - y * W;
-                while (cell < end) {   // one row segment at a time (at most ceil(16/W)+1 of them)
-                    const int len = min(W - x, end - cell);
-                    const int word = TWO ? (y >> 1) : y;
-                    const int sh = TWO ? ((y & 1) * 16 + x) : x;
-                    const uint32_t m = (1u << len) - 1u;
-#pragma unroll
-                    for (int q = 0; q < P; ++q) {
-                        const uint32_t seg = (lin[q] >> (cell - c * 16)) & m;
-                        if (seg) atomicOr(&bb[q * NW + word], seg << sh);
-                    }
-                    cell += len;
-                    x = 0;
-                    ++y;
-                }
-            }
-        }
-    }
-    __syncthreads();
+    stage_boards<Prob, NW, TWO, THREADS>(p, tid, M, s_bb,
+                                         [&](int slot) { return grids_in + (base + s_list[slot]) * p.row_stride; });
 
     // ---------------- phase C: thread-per-grid stat searches, dynamic queue --------------------------
     // Each thread pulls the next changed env from the shared-memory queue as soon as it finishes one, so
@@ -174,25 +130,12 @@ static cudaError_t launch(const KParams& p, cudaStream_t s) {
 
 template <template <int, bool> class Machine>
 static cudaError_t dispatch_shape(const KParams& p, cudaStream_t s, bool& supported) {
-    const int H = (p.ndim == 2) ? p.d0 : -1, W = p.d1;
-    supported = true;
-    if (p.ndim != 2) {
-        supported = false;
-        return cudaSuccess;
-    }
-    if (W <= 16 && H <= 16) {
-        const int nw = (H + 1) / 2;
-        if (nw <= 1) return launch<Machine<1, true>, 1, true>(p, s);
-        if (nw <= 2) return launch<Machine<2, true>, 2, true>(p, s);
-        if (nw <= 4) return launch<Machine<4, true>, 4, true>(p, s);
-        return launch<Machine<8, true>, 8, true>(p, s);
-    }
-    if (W <= 32 && H <= 32) {
-        if (H <= 16) return launch<Machine<16, false>, 16, false>(p, s);
-        return launch<Machine<32, false>, 32, false>(p, s);
-    }
     supported = false;
-    return cudaSuccess;
+    if (p.ndim != 2) return cudaSuccess;
+    return with_board(p.d0, p.d1, supported, [&](auto b) {
+        using B = decltype(b);
+        return launch<Machine<B::WORDS, B::TWO_ROWS>, B::WORDS, B::TWO_ROWS>(p, s);
+    });
 }
 
 cudaError_t launch_bitboard(const KParams& p, int problem, cudaStream_t s, bool& supported) {

@@ -463,6 +463,15 @@ __device__ __forceinline__ void finish_env(const KParams& p, int64_t gid, const 
     for (int k = 0; k < K; ++k) st[k] = nw[k];
 }
 
+// Update and output of one env in the one-launch incremental binary steps (k_step_inc, k_step_lanegroup)
+__device__ static __noinline__ bool inc_update_env(const KParams& p, int64_t gid, int* cell) {
+    return step_counters(p, gid, apply_action(p, gid, cell));
+}
+__device__ static __noinline__ void inc_output_env(const KParams& p, int64_t env, int regions, int path) {
+    const int32_t nw[2] = {regions, path};
+    finish_env<2>(p, env, nw);
+}
+
 // ------------------------------------------------------------------------------------------------
 // Cellular representation update (reps/ca_rep.py:31-44) of the tile_n envs starting at `base`, cooperative over
 // the CTA: the whole map is replaced by the action.  s_flag[e] = 1 when env base + e's grid changed; the caller

@@ -228,14 +228,6 @@ struct LaneGroupInc {
     }
 };
 
-__device__ __noinline__ bool lg_update_env(const KParams& p, int64_t gid, int* cell) {
-    return step_counters(p, gid, apply_action(p, gid, cell));
-}
-__device__ __noinline__ void lg_output_env(const KParams& p, int64_t env, int regions, int path) {
-    const int32_t nw[2] = {regions, path};
-    finish_env<2>(p, env, nw);
-}
-
 template <int NW>
 __global__ void __launch_bounds__(LG_THREADS) k_step_lanegroup(const __grid_constant__ KParams p, const int T) {
     using M = LaneGroupInc<NW>;
@@ -259,7 +251,7 @@ __global__ void __launch_bounds__(LG_THREADS) k_step_lanegroup(const __grid_cons
         // ---- update
         const int64_t gid = e0 + lane;
         int cell = -1;
-        const bool need = lane < T && gid < p.n_envs && lg_update_env(p, gid, &cell);
+        const bool need = lane < T && gid < p.n_envs && inc_update_env(p, gid, &cell);
         unsigned todo = __ballot_sync(0xffffffffu, need);     // changed envs of the tile not yet handed to a group
         s_cell[warp][lane] = cell;
         __syncwarp();
@@ -279,7 +271,7 @@ __global__ void __launch_bounds__(LG_THREADS) k_step_lanegroup(const __grid_cons
                     const int64_t env = e0 + slot;
                     const int c = s_cell[warp][slot];
                     const int y = c / W, x = c - y * W;
-                    bitpos = y * 16 + x;
+                    bitpos = Board<NW, true>::bitpos(y, x);
                     row = (uint32_t*)(p.cache + env * p.cache_stride);
                     const int2 st = *(const int2*)(p.stats + env * 2);
                     r_old = st.x;
@@ -304,32 +296,27 @@ __global__ void __launch_bounds__(LG_THREADS) k_step_lanegroup(const __grid_cons
         // ---- output
         if (need) {
             const int2 r = s_res[warp][lane];
-            lg_output_env(p, gid, r.x, r.y);
+            inc_output_env(p, gid, r.x, r.y);
         }
         __syncwarp();
     }
 }
 
-static int g_lg_sm = 0;
-
 template <int NW>
 static cudaError_t launch_lg(const KParams& p, cudaStream_t s) {
-    if (!g_lg_sm) {
-        int dev = 0;
-        cudaError_t e = cudaGetDevice(&dev);
-        if (e != cudaSuccess) return e;
-        if ((e = cudaDeviceGetAttribute(&g_lg_sm, cudaDevAttrMultiProcessorCount, dev)) != cudaSuccess) return e;
-    }
+    int n_sm = 0;
+    const cudaError_t e = sm_count(n_sm);
+    if (e != cudaSuccess) return e;
     // tile size: the smallest of 8 / 16 / 32 envs per warp whose grid still fits the GPU in one wave (every warp then
     // runs as few searches one after the other as possible).  At 64 Ki envs, where this picks 16, 8 / 16 / 32 envs per
     // warp gave 0.0810 / 0.0749 / 0.0847 ms per step (profiles/r02_lanegroup_by_size.txt).
-    const int64_t resident_warps = (int64_t)g_lg_sm * 32;      // 8 CTAs of 4 warps per SM (64 registers per thread)
+    const int64_t resident_warps = (int64_t)n_sm * 32;      // 8 CTAs of 4 warps per SM (64 registers per thread)
     int T = 32;
     if ((p.n_envs + 7) / 8 <= resident_warps) T = 8;
     else if ((p.n_envs + 15) / 16 <= resident_warps) T = 16;
     const int64_t warps = (p.n_envs + T - 1) / T;
     const int64_t want = (warps + LG_THREADS / 32 - 1) / (LG_THREADS / 32);
-    const int64_t cap = (int64_t)g_lg_sm * 8;
+    const int64_t cap = (int64_t)n_sm * 8;
     k_step_lanegroup<NW><<<(unsigned)(want < cap ? want : cap), LG_THREADS, 0, s>>>(p, T);
     return cudaGetLastError();
 }
@@ -339,11 +326,11 @@ cudaError_t launch_bitboard_lanegroup(const KParams& p, int problem, cudaStream_
     supported = problem == PCGRL_PROB_BINARY && p.mode == MODE_STEP && p.ndim == 2 && p.d0 <= 16 && p.d1 <= 16 &&
                 p.cache != nullptr && p.rep != PCGRL_REP_CELLULAR && p.action_kind != PCGRL_ACT_PATCH;
     if (!supported || p.n_envs == 0) return cudaSuccess;
-    const int nw = (p.d0 + 1) / 2;
-    if (nw <= 1) return launch_lg<1>(p, s);
-    if (nw <= 2) return launch_lg<2>(p, s);
-    if (nw <= 4) return launch_lg<4>(p, s);
-    return launch_lg<8>(p, s);
+    return with_board(p.d0, p.d1, supported, [&](auto b) {
+        using B = decltype(b);
+        if constexpr (!B::TWO_ROWS) return cudaErrorInvalidValue;   // not reached: maps of at most 16x16
+        else return launch_lg<B::WORDS>(p, s);
+    });
 }
 
 }  // namespace pcgrl

@@ -238,15 +238,11 @@ __global__ void __launch_bounds__(WARPS * 32) k_step_search(const KParams p, con
 template <class Prob, int WARPS = SEARCH_WARPS>
 static cudaError_t launch_search(const KParams& p, cudaStream_t s, int smem_per_warp, int max_ctas_per_sm = 1 << 20,
                                  int max_ctas = SEARCH_MAX_CTAS, int64_t env_begin = 0, int64_t env_end = -1) {
-    static int n_sm = 0;
     static std::atomic<unsigned> next_slot{0};
     constexpr int SEARCH_THREADS = WARPS * 32;
+    int n_sm = 0;
     cudaError_t e;
-    if (!n_sm) {
-        int dev = 0;
-        if ((e = cudaGetDevice(&dev)) != cudaSuccess) return e;
-        if ((e = cudaDeviceGetAttribute(&n_sm, cudaDevAttrMultiProcessorCount, dev)) != cudaSuccess) return e;
-    }
+    if ((e = sm_count(n_sm)) != cudaSuccess) return e;
     const int dyn = smem_per_warp * WARPS;
     auto kern = k_step_search<Prob, WARPS>;
     if ((e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, dyn)) != cudaSuccess) return e;

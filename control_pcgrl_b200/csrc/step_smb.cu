@@ -748,13 +748,9 @@ cudaError_t launch_smb(const KParams& p, cudaStream_t s, bool& supported, int& n
         supported = false;
         return cudaSuccess;
     }
-    static int n_sm = 0;
+    int n_sm = 0;
     cudaError_t e;
-    if (!n_sm) {
-        int dev = 0;
-        if ((e = cudaGetDevice(&dev)) != cudaSuccess) return e;
-        if ((e = cudaDeviceGetAttribute(&n_sm, cudaDevAttrMultiProcessorCount, dev)) != cudaSuccess) return e;
-    }
+    if ((e = sm_count(n_sm)) != cudaSuccess) return e;
     const char* cap_env = getenv("PCGRL_SMB_GROUP_CAP");         // tests shrink it to drive levels into the fallback
     // narrow levels ([116, 16]: heaps of 30-270 entries) keep the whole heap in shared memory; wide ones ([16, 116]:
     // ~1 900) continue in the group's global slice

@@ -897,12 +897,8 @@ cudaError_t launch_sokoban(const KParams& p, cudaStream_t s, bool& supported) {
     const int ctx_smem = SokobanProb::smem_bytes(p.row_stride);
     cudaError_t e = launch_search<SokobanProb>(p, s, ctx_smem, SOK_MAX_CTAS_PER_SM, SOK_MAX_CTAS);   // pass 1
     if (e != cudaSuccess || p.n_envs == 0) return e;
-    static int n_sm = 0;
-    if (!n_sm) {
-        int dev = 0;
-        if ((e = cudaGetDevice(&dev)) != cudaSuccess) return e;
-        if ((e = cudaDeviceGetAttribute(&n_sm, cudaDevAttrMultiProcessorCount, dev)) != cudaSuccess) return e;
-    }
+    int n_sm = 0;
+    if ((e = sm_count(n_sm)) != cudaSuccess) return e;
     {   // pass 2: as many warps as pass 1 may hold (the per-warp scratch slices are shared by the two passes)
         auto k2 = k_sokoban_solve<SEARCH_WARPS>;
         const int dyn = ctx_smem * SEARCH_WARPS;

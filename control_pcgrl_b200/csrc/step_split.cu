@@ -115,52 +115,9 @@ k_split_stats(const KParams p) {
     const int2* items = wl_items(p) + first;
     uint32_t* wbb = s_bb + warp * 32 * BBW;
 
-    // stage the warp's grids as per-plane bit-boards (same packing as phase B of the fused kernel)
-    {
-        const int chunks = p.row_stride / 16;
-        const int W = p.d1;
-        const bool word_is_32_bytes = TWO ? (W == 16) : (W == 32);
-        if (word_is_32_bytes) {
-            for (int i = lane; i < n_here * NW; i += 32) {
-                const int slot = i / NW, j = i - slot * NW;
-                const int8_t* g = p.grids + (int64_t)items[slot].x * p.row_stride + j * 32;
-                uint32_t lo[P], hi[P];
-#pragma unroll
-                for (int q = 0; q < P; ++q) lo[q] = hi[q] = 0;
-                if (2 * j < chunks) pack16<Prob>(*(const uint4*)g, lo);
-                if (2 * j + 1 < chunks) pack16<Prob>(*(const uint4*)(g + 16), hi);
-#pragma unroll
-                for (int q = 0; q < P; ++q) wbb[slot * BBW + q * NW + j] = lo[q] | (hi[q] << 16);
-            }
-        } else {
-            for (int i = lane; i < n_here * BBW; i += 32) wbb[i] = 0;
-            __syncwarp();
-            for (int i = lane; i < n_here * chunks; i += 32) {
-                const int slot = i / chunks, c = i - slot * chunks;
-                uint32_t lin[P];
-                pack16<Prob>(*(const uint4*)(p.grids + (int64_t)items[slot].x * p.row_stride + c * 16), lin);
-                uint32_t* bb = wbb + slot * BBW;
-                int cell = c * 16;
-                const int end = min(cell + 16, p.cells);
-                int y = cell / W, x = cell - y * W;
-                while (cell < end) {
-                    const int len = min(W - x, end - cell);
-                    const int word = TWO ? (y >> 1) : y;
-                    const int sh = TWO ? ((y & 1) * 16 + x) : x;
-                    const uint32_t m = (1u << len) - 1u;
-#pragma unroll
-                    for (int q = 0; q < P; ++q) {
-                        const uint32_t seg = (lin[q] >> (cell - c * 16)) & m;
-                        if (seg) atomicOr(&bb[q * NW + word], seg << sh);
-                    }
-                    cell += len;
-                    x = 0;
-                    ++y;
-                }
-            }
-        }
-    }
-    __syncwarp();
+    // stage the warp's grids as per-plane bit-boards (as phase B of the fused kernel)
+    stage_boards<Prob, NW, TWO, 32>(p, lane, n_here, wbb,
+                                    [&](int slot) { return p.grids + (int64_t)items[slot].x * p.row_stride; });
     const bool mine = lane < n_here;
     const int64_t env = mine ? items[lane].x : 0;
     Machine m;
@@ -300,6 +257,12 @@ struct BinaryIncMachine {
         }
         ++level;
         return true;
+    }
+    // init for the list item (env, cell) of a map W cells wide: the cell's bit, and the env's cache row and old stats
+    __device__ __forceinline__ void start(uint32_t* smem, const KParams& p, int64_t env, int cell_idx, int W) {
+        const int y = cell_idx / W, x = cell_idx - y * W;
+        const int32_t* st = p.stats + env * 2;
+        init(smem, (const uint32_t*)(p.cache + env * p.cache_stride), B::bitpos(y, x), st[0], st[1]);
     }
     // the frontier died; returns true when the search is over (call finish())
     __device__ __forceinline__ bool transition() {
@@ -460,10 +423,7 @@ __global__ void __launch_bounds__(STAT_THREADS) k_split_stats_inc(const KParams 
                 item = mine;
                 const int2 it = items[item];
                 env = it.x;
-                const int y = it.y / W, x = it.y - y * W;
-                const int bitpos = TWO ? y * 16 + x : y * 32 + x;
-                const int32_t* st = p.stats + env * 2;
-                m.init(s_work + tid * M::SMEM_WORDS, (const uint32_t*)(p.cache + env * p.cache_stride), bitpos, st[0], st[1]);
+                m.start(s_work + tid * M::SMEM_WORDS, p, env, it.y, W);
                 active = true;
             }
             lo = min(hi, lo + __popc(need));
@@ -500,14 +460,6 @@ __global__ void __launch_bounds__(STAT_THREADS) k_split_stats_inc(const KParams 
 // The update and output passes are memory-latency work; in the split path they were two separate kernels (42 +
 // 30 us of the 303 us step at 1 Mi envs) during which the ALU pipes idled, here other warps' searches cover them.
 // ------------------------------------------------------------------------------------------------
-__device__ __noinline__ bool inc_update_env(const KParams& p, int64_t gid, int* cell) {
-    return step_counters(p, gid, apply_action(p, gid, cell));
-}
-__device__ __noinline__ void inc_output_env(const KParams& p, int64_t env, int regions, int path) {
-    const int32_t nw[2] = {regions, path};
-    finish_env<2>(p, env, nw);
-}
-
 constexpr int STEP_INC_MIN_CTAS = 6;
 constexpr int STEP_INC_ROUNDS = 1;   // update rounds (of 32 envs) per warp the grid is sized for below 48 Ki envs, see launch_split
 template <int NW, bool TWO>
@@ -553,10 +505,7 @@ __global__ void __launch_bounds__(STAT_THREADS, STEP_INC_MIN_CTAS) k_step_inc(co
             if (!active && rank < it_cnt) {
                 const int2 it = items[(it_head + rank) & (RING - 1)];
                 env = it.x;
-                const int y = it.y / W, x = it.y - y * W;
-                const int bitpos = TWO ? y * 16 + x : y * 32 + x;
-                const int32_t* st = p.stats + env * 2;
-                m.init(s_work + tid * M::SMEM_WORDS, (const uint32_t*)(p.cache + env * p.cache_stride), bitpos, st[0], st[1]);
+                m.start(s_work + tid * M::SMEM_WORDS, p, env, it.y, W);
                 active = true;
             }
             const int taken = min(__popc(idle), it_cnt);
@@ -623,28 +572,17 @@ __global__ void __launch_bounds__(OUT_THREADS) k_split_out(const KParams p) {
 // ------------------------------------------------------------------------------------------------
 // resident CTAs per SM of the persistent incremental kernels
 static int inc_ctas_per_sm(bool host_chunk) { return host_chunk ? INC_CTAS_PER_SM_HOST : INC_CTAS_PER_SM; }
-static int g_n_sm = 0;
-static cudaError_t sm_count(int& n) {
-    if (!g_n_sm) {
-        int dev = 0;
-        cudaError_t e = cudaGetDevice(&dev);
-        if (e != cudaSuccess) return e;
-        if ((e = cudaDeviceGetAttribute(&g_n_sm, cudaDevAttrMultiProcessorCount, dev)) != cudaSuccess) return e;
-    }
-    n = g_n_sm;
-    return cudaSuccess;
-}
 
-// env_idx (pcgrl_step_envs): the list of p.n_envs env indices into a shard of n_src envs (incremental <= 1).
+// env_idx (pcgrl_step_envs): the list of p.n_envs env indices into a shard of n_src envs (path SPLIT or INC).
 template <class Machine, int NW, bool TWO>
-static cudaError_t launch_split(const KParams& p, cudaStream_t s, int incremental, const int32_t* env_idx,
+static cudaError_t launch_split(const KParams& p, cudaStream_t s, StepPath path, const int32_t* env_idx,
                                 int64_t n_src) {
     constexpr int K = Machine::Prob::K;
     const int64_t n = p.n_envs;
     if (n == 0) return cudaSuccess;
     cudaError_t e;
     if constexpr (Machine::HAS_CACHE && TWO) {
-        if (incremental == 2) {     // the whole step in one launch (k_step_inc)
+        if (path == INC_FUSED) {     // the whole step in one launch (k_step_inc)
             int n_sm = 0;
             if ((e = sm_count(n_sm)) != cudaSuccess) return e;
             // envs per warp = 32 * m.  A warp's first 32 envs yield ~16 changed ones, i.e. half-empty warps for the whole
@@ -668,7 +606,7 @@ static cudaError_t launch_split(const KParams& p, cudaStream_t s, int incrementa
     if ((e = cudaGetLastError()) != cudaSuccess) return e;
     bool ran_inc = false;
     if constexpr (Machine::HAS_CACHE && TWO) {
-        if (incremental == 1) {
+        if (path == INC) {
             int n_sm = 0;
             if ((e = sm_count(n_sm)) != cudaSuccess) return e;
             const int64_t want = (n + STAT_THREADS - 1) / STAT_THREADS;
@@ -687,48 +625,36 @@ static cudaError_t launch_split(const KParams& p, cudaStream_t s, int incrementa
 }
 
 template <template <int, bool> class Machine>
-static cudaError_t dispatch_split(const KParams& p, cudaStream_t s, int incremental, bool& supported,
+static cudaError_t dispatch_split(const KParams& p, cudaStream_t s, StepPath path, bool& supported,
                                   const int32_t* env_idx, int64_t n_src) {
-    const int H = p.d0, W = p.d1;
-    supported = p.ndim == 2;
-    if (!supported) return cudaSuccess;
-    if (W <= 16 && H <= 16) {
-        const int nw = (H + 1) / 2;
-        if (nw <= 1) return launch_split<Machine<1, true>, 1, true>(p, s, incremental, env_idx, n_src);
-        if (nw <= 2) return launch_split<Machine<2, true>, 2, true>(p, s, incremental, env_idx, n_src);
-        if (nw <= 4) return launch_split<Machine<4, true>, 4, true>(p, s, incremental, env_idx, n_src);
-        return launch_split<Machine<8, true>, 8, true>(p, s, incremental, env_idx, n_src);
-    }
-    if (W <= 32 && H <= 32) {
-        if (H <= 16) return launch_split<Machine<16, false>, 16, false>(p, s, 0, env_idx, n_src);
-        return launch_split<Machine<32, false>, 32, false>(p, s, 0, env_idx, n_src);
-    }
     supported = false;
-    return cudaSuccess;
+    if (p.ndim != 2) return cudaSuccess;
+    return with_board(p.d0, p.d1, supported, [&](auto b) {
+        using B = decltype(b);
+        return launch_split<Machine<B::WORDS, B::TWO_ROWS>, B::WORDS, B::TWO_ROWS>(p, s, path, env_idx, n_src);
+    });
 }
 
-// MODE_STEP of a bit-board problem through the split path.  `incremental` asks for the cached incremental search
-// (binary only; needs p.cache).  Three kernels are launched: *launches is incremented by the caller accordingly.
-// incremental: 0 = from-scratch searches, 1 = incremental search as the middle kernel of the split path, 2 = the
-// fused incremental step (k_step_inc, one launch).  *n_launches = kernels launched.
-// env_idx (pcgrl_step_envs, incremental <= 1): step only the p.n_envs listed envs of a shard of n_src envs, through
-// the shard's own work list; the search and output kernels address envs through the list items as for a full step.
-cudaError_t launch_bitboard_split(const KParams& p, int problem, cudaStream_t s, int incremental, bool& supported,
+// MODE_STEP of a bit-board problem through the split path: `path` is SPLIT, INC or INC_FUSED, and a shard without a
+// search cache runs SPLIT (StepPath).  *n_launches = kernels launched.
+// env_idx (pcgrl_step_envs, SPLIT / INC): step only the p.n_envs listed envs of a shard of n_src envs, through the
+// shard's own work list; the search and output kernels address envs through the list items as for a full step.
+cudaError_t launch_bitboard_split(const KParams& p, int problem, cudaStream_t s, StepPath path, bool& supported,
                                   int& n_launches, const int32_t* env_idx, int64_t n_src) {
     supported = false;
     n_launches = 3;
     if (p.mode != MODE_STEP || !p.worklist || p.rep == PCGRL_REP_CELLULAR) return cudaSuccess;
     if (problem == PCGRL_PROB_BINARY) {
-        const int inc = p.cache != nullptr && p.d0 <= 16 && p.d1 <= 16 ? incremental : 0;
-        if (inc == 2) n_launches = 1;
-        return dispatch_split<BinaryMachine>(p, s, inc, supported, env_idx, n_src);
+        if (!p.cache || p.d0 > 16 || p.d1 > 16) path = SPLIT;
+        if (path == INC_FUSED) n_launches = 1;
+        return dispatch_split<BinaryMachine>(p, s, path, supported, env_idx, n_src);
     }
-    if (problem == PCGRL_PROB_ZELDA) return dispatch_split<ZeldaMachine>(p, s, 0, supported, env_idx, n_src);
+    if (problem == PCGRL_PROB_ZELDA) return dispatch_split<ZeldaMachine>(p, s, SPLIT, supported, env_idx, n_src);
     if (problem == PCGRL_PROB_BINARY_HOLEY) {
         supported = p.ndim == 2 && p.d1 + 2 <= 32 && p.d0 + 2 <= 32;
         if (!supported) return cudaSuccess;
-        if (p.d0 + 2 <= 18) return launch_split<BinaryHoleyMachine<18, false>, 18, false>(p, s, 0, env_idx, n_src);
-        return launch_split<BinaryHoleyMachine<32, false>, 32, false>(p, s, 0, env_idx, n_src);
+        if (p.d0 + 2 <= 18) return launch_split<BinaryHoleyMachine<18, false>, 18, false>(p, s, SPLIT, env_idx, n_src);
+        return launch_split<BinaryHoleyMachine<32, false>, 32, false>(p, s, SPLIT, env_idx, n_src);
     }
     return cudaSuccess;
 }
@@ -742,21 +668,25 @@ cudaError_t launch_lookahead_search(const KParams& p, cudaStream_t s) {
     const int64_t want = (p.n_envs + STAT_THREADS - 1) / STAT_THREADS;
     const int64_t cap = (int64_t)n_sm * INC_CTAS_PER_SM_LOOKAHEAD;
     const unsigned grid = (unsigned)(want < cap ? want : cap);
-    const int nw = (p.d0 + 1) / 2;
-    if (nw <= 1) k_split_stats_inc<1, true, true><<<grid, STAT_THREADS, 0, s>>>(p);
-    else if (nw <= 2) k_split_stats_inc<2, true, true><<<grid, STAT_THREADS, 0, s>>>(p);
-    else if (nw <= 4) k_split_stats_inc<4, true, true><<<grid, STAT_THREADS, 0, s>>>(p);
-    else k_split_stats_inc<8, true, true><<<grid, STAT_THREADS, 0, s>>>(p);
-    return cudaGetLastError();
+    bool supported = false;
+    e = with_board(p.d0, p.d1, supported, [&](auto b) {
+        using B = decltype(b);
+        if constexpr (!B::TWO_ROWS) {
+            return cudaErrorInvalidValue;   // a shard with a search cache has maps of at most 16x16
+        } else {
+            k_split_stats_inc<B::WORDS, true, true><<<grid, STAT_THREADS, 0, s>>>(p);
+            return cudaGetLastError();
+        }
+    });
+    return supported ? e : cudaErrorInvalidValue;
 }
 
 // bytes per env of the incremental search cache (0: this config has none)
 int bitboard_cache_stride(int problem, int ndim, int d0, int d1, int rep, int action_kind) {
     if (problem != PCGRL_PROB_BINARY || ndim != 2 || d0 > 16 || d1 > 16) return 0;
     if (rep == PCGRL_REP_CELLULAR || action_kind == PCGRL_ACT_PATCH) return 0;   // whole-map / multi-cell edits
-    const int nw = (d0 + 1) / 2;
-    const int NW = nw <= 1 ? 1 : nw <= 2 ? 2 : nw <= 4 ? 4 : 8;
-    return (2 * NW + 4) * 4;
+    bool supported = false;
+    return with_board(d0, d1, supported, [](auto b) { return (2 * decltype(b)::WORDS + 4) * 4; });
 }
 
 }  // namespace pcgrl

@@ -40,16 +40,14 @@ __global__ void __launch_bounds__(UPD_THREADS) k_update(const KParams p, const i
 
 // Persistent grid: as many CTAs as are resident at once, or fewer when the shard is smaller.
 cudaError_t launch_update(const KParams& p, cudaStream_t s) {
-    static int n_sm = 0, per_sm[2] = {0, 0};
+    static int per_sm[2] = {0, 0};
+    int n_sm = 0;
     cudaError_t e;
-    if (!n_sm) {
-        int dev = 0;
-        if ((e = cudaGetDevice(&dev)) != cudaSuccess) return e;
-        if ((e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm[0], k_update<false>, UPD_THREADS, 0)) != cudaSuccess ||
-            (e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm[1], k_update<true>, UPD_THREADS, 0)) != cudaSuccess ||
-            (e = cudaDeviceGetAttribute(&n_sm, cudaDevAttrMultiProcessorCount, dev)) != cudaSuccess)
-            return e;
-    }
+    if ((e = sm_count(n_sm)) != cudaSuccess) return e;
+    if (!per_sm[0] &&
+        ((e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm[0], k_update<false>, UPD_THREADS, 0)) != cudaSuccess ||
+         (e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm[1], k_update<true>, UPD_THREADS, 0)) != cudaSuccess))
+        return e;
     if (p.n_envs == 0) return cudaSuccess;
     const bool ca = p.rep == PCGRL_REP_CELLULAR;
     const int64_t cap = (int64_t)n_sm * (per_sm[ca] > 0 ? per_sm[ca] : 1);
